@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the byte-level BPE hot path on B200 (contract and definitions: DESIGN.md, "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload train|train-tiny|encode] [--bytes B] [--vocab V]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload train|train-tiny|encode] [--bytes B] [--vocab V] [--dump-outputs DIR]
     torchrun --nproc-per-node N bench.py --gpus N ...       # one rank per GPU, NCCL
     python bench.py --impl reference ...                    # the reference's own CPU path on a bounded sample
 
@@ -71,7 +71,15 @@ def parse_args():
     ap.add_argument("--no-files", action="store_true", help="skip the file-level legs (train_bpe(path), encode_file) at N = 1")
     ap.add_argument("--no-slices", action="store_true", help="skip the same-slice legs")
     ap.add_argument("--no-unsharded-check", action="store_true", help="N > 1: do not re-run the unsharded path on rank 0")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float32 / float64): the trained vocab and merges, and "
+                         "a fixed, seeded sample of the encoded ids (at N > 1 drawn from rank 0's shard, the start of the text)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
+    return args
 
 
 def merges_sha(merges) -> str:
@@ -163,6 +171,47 @@ def ncu_traffic_sum(kernels, config: dict):
         return sum(e["dram_bytes_per_step"] for e in hit), "sum over %s; %s" % (", ".join(names), "; ".join(sorted({e["source"] for e in hit})))
     except Exception:
         return None, None
+
+
+# --dump-outputs: the arrays are a pure function of the bench arguments (seeded corpora, fixed sample seed), so two builds
+# run with the same arguments can be compared file by file.
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SAMPLE_IDS, DUMP_SAMPLE_SEED = 1 << 20, 20240601
+
+
+def train_output_arrays(np, vocab, merges) -> dict:
+    """train_bpe's (vocab, merges) as arrays: the ids of the vocab, the bytes of its entries in id order back to back with the
+    offset of each entry's first byte, and every merge as the vocab ids of its two parts."""
+    ids = sorted(vocab)
+    toks = [vocab[i] for i in ids]
+    offsets = np.zeros(len(toks) + 1, dtype=np.float64)
+    np.cumsum([len(t) for t in toks], out=offsets[1:])
+    inv = {t: i for i, t in vocab.items()}
+    return {"train_vocab_ids": np.array(ids, dtype=np.float64),
+            "train_vocab_bytes": np.frombuffer(b"".join(toks), dtype=np.uint8).astype(np.float32),
+            "train_vocab_offsets": offsets,
+            "train_merges": np.array([[inv[a], inv[b]] for a, b in merges], dtype=np.float64).reshape(-1, 2)}
+
+
+def encode_output_arrays(np, torch, ids, n_ids: int) -> dict:
+    """A fixed, seeded sample of the n_ids token ids in the device tensor ids (uint16): their positions, their values, and n_ids."""
+    if n_ids <= DUMP_SAMPLE_IDS:
+        pos = np.arange(n_ids, dtype=np.int64)
+    else:
+        pos = np.sort(np.random.default_rng(DUMP_SAMPLE_SEED).choice(n_ids, size=DUMP_SAMPLE_IDS, replace=False))
+    vals = ids[:n_ids].view(torch.int16)[torch.from_numpy(pos).to(ids.device)].to(torch.int32) & 0xFFFF
+    return {"encode_ids_sample_positions": pos.astype(np.float64), "encode_ids_sample": vals.cpu().numpy().astype(np.float32),
+            "encode_n_ids": np.array([n_ids], dtype=np.float64)}
+
+
+def write_outputs(np, out_dir: str, arrays: dict) -> None:
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ----------------------------------------------------------------------------------------------
@@ -557,11 +606,14 @@ def run_b200(args):
     vocab_size = args.vocab or vocab_size
     line = {}
     train_res = None
+    dumps = {}
 
     # ======================= training =======================
     if is_train:
         nbytes = int(args.bytes or nbytes) // BLOCK * BLOCK
         m, train_res = measure_train(shape, seed, nbytes, vocab_size, args.steps, args.warmup, not args.no_e2e, not args.no_unsharded_check)
+        if args.dump_outputs:
+            dumps.update(train_output_arrays(np, train_res[0], train_res[1]))
         avg = m.pop("_avg")
         merge_ms, pretok_ms, count_ms = avg["ms_merge"], avg["ms_pretok"], avg["ms_count"]
         local_bytes = m["local_bytes"]
@@ -618,7 +670,7 @@ def run_b200(args):
         # ---- BASELINE.json configs[2]: TinyStories shape, 2 GiB, vocab 10000 ----
         if primary == "train" and not args.no_tiny and not args.bytes:
             t_shape, t_seed, t_bytes, t_vocab, t_desc = WORKLOADS["train-tiny"]
-            tm, _ = measure_train(t_shape, t_seed, int(t_bytes) // BLOCK * BLOCK, t_vocab, max(1, min(args.steps, 5)), max(1, min(args.warmup, 3)),
+            tm, _ = measure_train(t_shape, t_seed, int(t_bytes) // BLOCK * BLOCK, t_vocab, args.steps, max(1, min(args.warmup, 3)),
                                   not args.no_e2e, not args.no_unsharded_check)
             tavg = tm.pop("_avg")
             tm.update({"metric": "bpe_train_MBps", "unit": "MB/s", "config": {"workload": t_desc, "corpus_bytes": int(t_bytes), "vocab_size": t_vocab,
@@ -675,6 +727,8 @@ def run_b200(args):
         eclocks = sampler.stop()
         e_launches = L.bpe_launch_count() - l0
         tokens_local = n_tok[-1]
+        if args.dump_outputs and rank == 0:
+            dumps.update(encode_output_arrays(np, torch, out, tokens_local))
         tok_total, bytes_total, first_index = tokens_local, n_loc, 0
         if world > 1:
             t = torch.tensor([tokens_local, n_loc], dtype=torch.int64, device=dev)
@@ -794,7 +848,7 @@ def run_b200(args):
             t.cpu().numpy().tofile(src)
             del t
             walls = []
-            for _ in range(3):                   # (first run: page cache and buffer pools warm up)
+            for _ in range(1 + args.steps):      # (first run: page cache and buffer pools warm up)
                 t0 = time.time()
                 f_vocab_d, f_merges = train_bpe_path(src, f_vocab, SPECIALS, ctx=ctx)
                 walls.append(time.time() - t0)
@@ -802,7 +856,7 @@ def run_b200(args):
             tok_f = Tokenizer(f_vocab_d, f_merges, SPECIALS, ctx=ctx)
             dst = os.path.join(fdir, "tokens.bin")
             ewalls = []
-            for _ in range(2):
+            for _ in range(args.steps):
                 ctx.check(L.bpe_tok_cache_reset(tok_f._device_tok()))
                 t0 = time.time()
                 n_tok_f = encode_file(tok_f, src, dst, np.uint16)
@@ -842,8 +896,8 @@ def run_b200(args):
                 return train_bpe_on_bytes(host.array, SLICE_VOCAB, SPECIALS, ctx=ctx)
 
             dev_step(); host_step()
-            ms_d, _, o = timed(dev_step, 3)
-            _, ms_h, o2 = timed(host_step, 3)
+            ms_d, _, o = timed(dev_step, args.steps)
+            _, ms_h, o2 = timed(host_step, args.steps)
             assert o[-1][1] == o2[-1][1]
             slice_results[name] = o[-1]
             slices.append({"name": name, "corpus_bytes": n_s, "vocab_size": SLICE_VOCAB, "shape": s_shape, "seed": s_seed,
@@ -861,14 +915,14 @@ def run_b200(args):
             data = osynth.synth_host("owt", 4322, n_s)
             stok.encode_to_numpy(data, np.uint16)
             dt = 1e9
-            for _ in range(3):                                   # best of three warm calls (the first ones may still grow the cache tables)
+            for _ in range(args.steps):                          # best of the warm calls (the first ones may still grow the cache tables)
                 t0 = time.perf_counter()
                 ids = stok.encode_to_numpy(data, np.uint16)
                 dt = min(dt, time.perf_counter() - t0)
             enc_slices.append({"name": name, "text_bytes": n_s, "gpu_e2e_ms": round(dt * 1e3, 3), "gpu_e2e_MBps": round(n_s / 1e6 / dt, 2), "n_ids": int(ids.size),
                                "ids_sha": hashlib.sha256(ids.astype("<i8").tobytes()).hexdigest()[:16],
                                "tokenizer": "vocab %d trained on the first %d MiB of the train corpus" % (SLICE_VOCAB, SLICE_REF_BYTES >> 20),
-                               "cache": "warm pretoken cache (best of three calls after a first one)"})
+                               "cache": "warm pretoken cache (best of %d calls after a first one)" % args.steps})
         line["same_slice_encode"] = enc_slices
 
         # ======================= CPU baseline: the CPU arms on those slices, timed in this run (rank 0, N = 1) =======================
@@ -923,6 +977,8 @@ def run_b200(args):
         dist.all_gather_object(allnuma, numa)
         line["numa_binding"] = {"note": "each rank binds itself to the CPUs of its GPU's NUMA node before allocating page-locked buffers (best effort)",
                                 "ranks": allnuma}
+    if args.dump_outputs and rank == 0:
+        write_outputs(np, args.dump_outputs, dumps)
     if rank == 0:
         print(json.dumps(line))
     if world > 1:

@@ -1,8 +1,14 @@
-"""The oracle against the UNMODIFIED reference, run live (CPU; only where /root/reference is mounted, i.e. in the build container --
-it does not exist on the GPU box and the test is skipped there).  The committed goldens (tests/golden, tools/make_golden.py) pin 20
-training and 5 tokenizer set-ups; this differential adds fresh seeded cases on every run of the CPU suite: random small corpora through
-models/tokenizer/train.py:142-231 and random texts through models/tokenizer/tokenizer.py:111-138, compared with oracle/bpe_oracle.c.
-The reference runs in a subprocess (its package is called `models`, like this repository's shim)."""
+"""The oracle against the UNMODIFIED reference, run live (CPU; only where BPE_REFERENCE_DIR names a checkout of the reference, skipped
+elsewhere).  The committed goldens (tests/golden, tools/make_golden.py) pin 20 training and 5 tokenizer set-ups; this differential adds
+fresh seeded cases: random small corpora through models/tokenizer/train.py:142-231 and random texts through
+models/tokenizer/tokenizer.py:111-138, compared with oracle/bpe_oracle.c.  The reference runs in a subprocess (its package is called
+`models`, like this repository's shim).
+
+The reference's results on seed 0 are stored as digests in tests/golden/live_seed0.json, so the oracle is held to them on every run of the
+CPU suite, with or without a reference checkout (test_oracle_equals_the_recorded_reference_results).  They were recorded from the oracle
+after this differential had found the oracle and the reference identical on these inputs; where a checkout is given, the
+differential at seed 0 also holds the reference's own results to them.  Re-record: python -m tests.test_oracle_vs_reference_live"""
+import hashlib
 import json
 import os
 import pathlib
@@ -12,15 +18,30 @@ import sys
 import pytest
 
 from oracle import oracle
+from tests.common import GOLDEN_PATH
 from tests.helpers import live_shapes
 
-REF = pathlib.Path("/root/reference")
 SEED = int(os.environ.get("BPE_LIVE_SEED", "0"))     # other seeds for longer hunts: BPE_LIVE_SEED=k python -m pytest tests/test_oracle_vs_reference_live.py
-pytestmark = pytest.mark.skipif(not (REF / "models" / "tokenizer" / "train.py").exists(), reason="the reference is not mounted here")
+RECORDED = GOLDEN_PATH / "live_seed0.json"
+
+
+def _reference_dir():
+    """The reference checkout named by BPE_REFERENCE_DIR, or None when it is unset or cannot be read."""
+    d = os.environ.get("BPE_REFERENCE_DIR")
+    if not d:
+        return None
+    try:
+        return pathlib.Path(d) if (pathlib.Path(d) / "models" / "tokenizer" / "train.py").is_file() else None
+    except OSError:
+        return None
+
+
+REF = _reference_dir()
+needs_reference = pytest.mark.skipif(REF is None, reason="no readable reference checkout (set BPE_REFERENCE_DIR)")
 
 WORKER = r'''
 import json, sys, logging
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, sys.argv[3])
 logging.disable(logging.CRITICAL)
 from models.tokenizer import train as T
 T.tqdm = lambda x, *a, **k: x
@@ -65,20 +86,69 @@ json.dump(out, open(sys.argv[2], "w"))
 def _run_reference(tmp_path, jobs):
     (tmp_path / "worker.py").write_text(WORKER)
     (tmp_path / "jobs.json").write_text(json.dumps(jobs))
-    subprocess.check_call([sys.executable, str(tmp_path / "worker.py"), str(tmp_path / "jobs.json"), str(tmp_path / "out.json")],
+    subprocess.check_call([sys.executable, str(tmp_path / "worker.py"), str(tmp_path / "jobs.json"), str(tmp_path / "out.json"), str(REF)],
                           cwd=str(REF), env={"PYTHONDONTWRITEBYTECODE": "1", "PATH": "/usr/bin:/bin", "PYTHONHASHSEED": os.environ.get("PYTHONHASHSEED", "random")}, timeout=600)
     return json.loads((tmp_path / "out.json").read_text())
 
 
-def test_train_bpe_equals_the_reference_on_fresh_corpora(tmp_path):
+def _train_jobs(tmp_path, seed):
     jobs, inputs = [], []
-    for k, (data, vocab_size, specials) in enumerate(live_shapes.train_cases(SEED)):
+    for k, (data, vocab_size, specials) in enumerate(live_shapes.train_cases(seed)):
         p = tmp_path / ("c%d.txt" % k)
         p.write_bytes(data)
         jobs.append({"kind": "train", "path": str(p), "vocab_size": vocab_size, "special_tokens": specials})
         inputs.append(data)
+    return jobs, inputs
+
+
+def _encode_jobs(seed):
+    set_ups, texts = live_shapes.encode_cases(seed)
+    jobs = [{"kind": "encode", "vocab": {str(k): v.hex() for k, v in vocab.items()}, "merges": [[a.hex(), b.hex()] for a, b in merges],
+             "special_tokens": specials, "texts": texts} for vocab, merges, specials in set_ups]
+    return set_ups, texts, jobs
+
+
+def _iterable_job(seed):
+    """~2.3 Mi characters in lines of odd lengths through encode_iterable: two buffers."""
+    import random
+    r = random.Random(77 + seed)
+    set_ups, _ = live_shapes.encode_cases(seed)
+    vocab, merges, specials = set_ups[0]
+    words = ["alpha", "beta", "it's", "naïve", "日本語", "12", "<|endoftext|>", "x"]
+    lines, chars = [], 0
+    while chars < 2_400_000:
+        line = " ".join(r.choice(words) for _ in range(r.randint(1, 40))) + r.choice(["\n", " ", "", "\n\n"])
+        lines.append(line)
+        chars += len(line)
+    return (vocab, merges, specials), {"kind": "iterable", "vocab": {str(k): v.hex() for k, v in vocab.items()},
+                                       "merges": [[a.hex(), b.hex()] for a, b in merges], "special_tokens": specials, "lines": lines}
+
+
+def _iterable_digest(ids):
+    import struct
+    h, n = hashlib.sha256(), 0
+    for i in ids:
+        h.update(struct.pack("<i", i))
+        n += 1
+    return {"n": n, "sha": h.hexdigest()}
+
+
+def _digest(result) -> str:
+    return hashlib.sha256(json.dumps(result, sort_keys=True).encode()).hexdigest()
+
+
+def _recorded() -> dict:
+    return json.loads(RECORDED.read_text())
+
+
+@needs_reference
+def test_train_bpe_equals_the_reference_on_fresh_corpora(tmp_path):
+    jobs, inputs = _train_jobs(tmp_path, SEED)
+    refs = _run_reference(tmp_path, jobs)
+    if SEED == 0:
+        assert [_digest(r) for r in refs] == _recorded()["train"]
     n_err = 0
-    for job, data, ref in zip(jobs, inputs, _run_reference(tmp_path, jobs)):
+    for job, data, ref in zip(jobs, inputs, refs):
         if "error" in ref:
             n_err += 1
             with pytest.raises(UnicodeDecodeError) as e:
@@ -91,12 +161,14 @@ def test_train_bpe_equals_the_reference_on_fresh_corpora(tmp_path):
     assert n_err >= 3 or SEED
 
 
+@needs_reference
 def test_tokenizer_encode_equals_the_reference_on_fresh_texts(tmp_path):
-    set_ups, texts = live_shapes.encode_cases(SEED)
-    jobs = [{"kind": "encode", "vocab": {str(k): v.hex() for k, v in vocab.items()}, "merges": [[a.hex(), b.hex()] for a, b in merges],
-             "special_tokens": specials, "texts": texts} for vocab, merges, specials in set_ups]
+    set_ups, texts, jobs = _encode_jobs(SEED)
+    refs = _run_reference(tmp_path, jobs)
+    if SEED == 0:
+        assert [[_digest(r) for r in res] for res in refs] == _recorded()["encode"]
     n_key = n_dec = 0
-    for (vocab, merges, specials), ref in zip(set_ups, _run_reference(tmp_path, jobs)):
+    for (vocab, merges, specials), ref in zip(set_ups, refs):
         tok = oracle.OracleTokenizer(dict(vocab), list(merges), list(specials))
         for text, want in zip(texts, ref):
             if "error" in want:
@@ -117,26 +189,73 @@ def test_tokenizer_encode_equals_the_reference_on_fresh_texts(tmp_path):
     assert (n_key >= 5 and n_dec >= 1) or SEED
 
 
+@needs_reference
 def test_encode_iterable_chunk_rule_equals_the_reference(tmp_path):
     """tokenizer.py:140-153: items are concatenated until the buffer holds >= 2 Mi characters and every buffer is encoded on its own
-    (a pretoken may be cut where two buffers meet, SURVEY A-13).  ~2.3 Mi characters in lines of odd lengths: two buffers."""
-    import hashlib
-    import random
-    import struct
-    r = random.Random(77 + SEED)
-    set_ups, _ = live_shapes.encode_cases(SEED)
-    vocab, merges, specials = set_ups[0]
-    words = ["alpha", "beta", "it's", "naïve", "日本語", "12", "<|endoftext|>", "x"]
-    lines, chars = [], 0
-    while chars < 2_400_000:
-        line = " ".join(r.choice(words) for _ in range(r.randint(1, 40))) + r.choice(["\n", " ", "", "\n\n"])
-        lines.append(line)
-        chars += len(line)
-    job = {"kind": "iterable", "vocab": {str(k): v.hex() for k, v in vocab.items()}, "merges": [[a.hex(), b.hex()] for a, b in merges],
-           "special_tokens": specials, "lines": lines}
+    (a pretoken may be cut where two buffers meet, SURVEY A-13)."""
+    (vocab, merges, specials), job = _iterable_job(SEED)
     (ref,) = _run_reference(tmp_path, [job])
-    h, n = hashlib.sha256(), 0
-    for i in oracle.OracleTokenizer(dict(vocab), list(merges), list(specials)).encode_iterable(iter(lines)):
-        h.update(struct.pack("<i", i))
-        n += 1
-    assert (n, h.hexdigest()) == (ref["n"], ref["sha"])
+    if SEED == 0:
+        assert ref == _recorded()["iterable"]
+    got = _iterable_digest(oracle.OracleTokenizer(dict(vocab), list(merges), list(specials)).encode_iterable(iter(job["lines"])))
+    assert (got["n"], got["sha"]) == (ref["n"], ref["sha"])
+
+
+# ---- the reference's results on seed 0, stored ----
+def _oracle_results(tmp_path):
+    """The oracle's results on the seed-0 inputs, in the form the reference worker above returns them."""
+    train = []
+    for job, data in zip(*_train_jobs(tmp_path, 0)):
+        try:
+            vocab, merges = oracle.train_bpe_on_bytes(data, job["vocab_size"], job["special_tokens"])
+        except UnicodeDecodeError as e:
+            train.append({"error": "UnicodeDecodeError", "start": e.start})
+            continue
+        train.append({"vocab": {str(k): v.hex() for k, v in vocab.items()}, "merges": [[a.hex(), b.hex()] for a, b in merges]})
+    set_ups, texts, _ = _encode_jobs(0)
+    encode = []
+    for vocab, merges, specials in set_ups:
+        tok = oracle.OracleTokenizer(dict(vocab), list(merges), list(specials))
+        res = []
+        for text in texts:
+            try:
+                ids = tok.encode(text)
+            except KeyError as e:
+                res.append({"error": "KeyError", "arg": e.args[0].hex() if isinstance(e.args[0], bytes) else repr(e.args[0])})
+                continue
+            try:
+                res.append({"ids": ids, "decoded": tok.decode(ids)})
+            except KeyError as e:
+                res.append({"ids": ids, "decode_error": repr(e.args[0])})
+        encode.append(res)
+    (vocab, merges, specials), job = _iterable_job(0)
+    iterable = _iterable_digest(oracle.OracleTokenizer(dict(vocab), list(merges), list(specials)).encode_iterable(iter(job["lines"])))
+    return train, encode, iterable
+
+
+def _as_recorded(train, encode, iterable) -> dict:
+    return {"train": [_digest(r) for r in train], "encode": [[_digest(r) for r in res] for res in encode], "iterable": iterable,
+            "n_train_errors": sum("error" in r for r in train), "n_key_errors": sum("error" in r for res in encode for r in res),
+            "n_decode_errors": sum("decode_error" in r for res in encode for r in res)}
+
+
+def test_oracle_equals_the_recorded_reference_results(tmp_path):
+    want = _recorded()
+    got = _as_recorded(*_oracle_results(tmp_path))
+    for k, (g, w) in enumerate(zip(got["train"], want["train"])):
+        assert g == w, ("train case", k, live_shapes.train_cases(0)[k][1:])
+    for s, (gs, ws) in enumerate(zip(got["encode"], want["encode"])):
+        for k, (g, w) in enumerate(zip(gs, ws)):
+            assert g == w, ("encode set-up", s, "text", k)
+    assert got == {k: want[k] for k in got}
+    assert got["n_train_errors"] >= 3 and got["n_key_errors"] >= 5 and got["n_decode_errors"] >= 1
+
+
+if __name__ == "__main__":
+    import tempfile
+    with tempfile.TemporaryDirectory() as td:
+        rec = _as_recorded(*_oracle_results(pathlib.Path(td)))
+    rec = {"source": "oracle/bpe_oracle.c on the seed-0 inputs of tests/helpers/live_shapes.py, identical to the reference's results there "
+                     "(tests/test_oracle_vs_reference_live.py); sha256 of each result as JSON with sorted keys", **rec}
+    RECORDED.write_text(json.dumps(rec, indent=0) + "\n")
+    print("wrote", RECORDED)
