@@ -194,7 +194,19 @@ typedef struct bpe_encode_stats {
  * returns BPE_ERR_ARG (the reference's np.uint16 cast at models/tokenizer/encode.py:37 would wrap). */
 int bpe_encode(bpe_tok *tok, const uint8_t *text_host, uint64_t n, int out_dtype,
                void *out, uint64_t cap, uint64_t *n_out, bpe_encode_stats *stats);
-/* 1 if the text of the last bpe_encode / bpe_encode_dev call on this tokenizer's context held a carriage return (the flags kernel
+/* Replaces [Tokenizer.encode(d) for d in docs]: models/tokenizer/tokenizer.py:111-138 once per document.
+ * text_host holds n_docs UTF-8 documents back to back, document j = text[doc_offs[j] .. doc_offs[j+1])
+ * (doc_offs[0] = 0, doc_offs[n_docs] = n, non-decreasing).  Writes the ids of all documents back to back and
+ * id_offs_out[j] (n_docs + 1 entries) = index of document j's first id.  Same size-query idiom, dtypes and errors as
+ * bpe_encode; BPE_ERR_UTF8 / BPE_ERR_KEY detail = byte offset in text_host.  Every document is encoded on its own: no
+ * pretoken or special-token occurrence spans two documents, and UTF-8 validity is per document.  The error reported is the
+ * first one the device meets: an invalid UTF-8 sequence anywhere in a pipeline chunk (256 MB of documents) comes before a
+ * KeyError in it, so a caller that needs the first failing document in list order re-encodes the documents before the
+ * invalid one (Tokenizer.encode_batch does).  BPE_ERR_UNSUPPORTED when every ASCII byte but '\r' occurs in some special
+ * token (the boundary byte between documents must occur in none).  bpe_tok_saw_cr afterwards: a '\r' in any document. */
+int bpe_encode_batch(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
+                     int out_dtype, void *out, uint64_t cap, uint64_t *n_out, uint64_t *id_offs_out, bpe_encode_stats *stats);
+/* 1 if the text of the last bpe_encode / bpe_encode_dev / bpe_encode_batch call on this tokenizer's context held a carriage return (the flags kernel
  * sees every byte anyway).  Tokenizer.encode takes a str and keeps '\r' as it is; a caller that reads a FILE in text mode, like the
  * reference's bulk driver (models/tokenizer/encode.py:31-34, universal newlines), uses this instead of scanning the text on the host:
  * it translates and encodes the piece again in the rare case. */

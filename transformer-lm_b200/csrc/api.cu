@@ -108,7 +108,7 @@ BPE_API void bpe_ctx_destroy(bpe_ctx *ctx) {
     count_state_free(ctx);
     if (ctx->s_in) { cudaStreamSynchronize(ctx->s_in); cudaStreamSynchronize(ctx->s_out); }
     for (DevBuf *b : {&ctx->text, &ctx->flags, &ctx->spmask, &ctx->spstart, &ctx->scratch, &ctx->tmp0, &ctx->tmp1, &ctx->tmp2, &ctx->sp_dev,
-                      &ctx->text_alt, &ctx->out_a, &ctx->out_b})
+                      &ctx->text_alt, &ctx->out_a, &ctx->out_b, &ctx->doc_bmask, &ctx->doc_offs, &ctx->doc_stage})
         bpe_buf_free(ctx, *b);
     if (ctx->s_in) {
         cudaStreamDestroy(ctx->s_in); cudaStreamDestroy(ctx->s_out);
@@ -207,9 +207,11 @@ int ctx_upload_specials(bpe_ctx *ctx, const uint8_t *blob, const u32 *offs, int 
 //   translate_newlines: apply universal-newline translation when a '\r' is present (training path);
 //                       *n is updated to the translated length.
 //   specials: when n_sp > 0 the text is first split on the specials (encode path).
+//   bmask: document boundaries of bpe_encode_batch (flag_words(n) words, or null): every set bit is a one-byte occurrence of
+//          class B, like a special token -- the text before it sees the end of a text, the text after it the start of one.
 // Leaves ctx->flags holding the start bitmask.  Synchronises the stream once (error words).
 int ctx_run_flags(bpe_ctx *ctx, u64 *n_io, bool translate_newlines, const uint8_t *sp_blob_dev, const u32 *sp_offs_dev,
-                  int n_sp, u32 sp_max_len, u64 err_lo, u64 err_hi) {
+                  int n_sp, u32 sp_max_len, u64 err_lo, u64 err_hi, const u32 *bmask) {
     u64 n = *n_io;
     cudaStream_t st = ctx->stream;
     u64 *scr = (u64 *)ctx->scratch.p;
@@ -224,12 +226,18 @@ int ctx_run_flags(bpe_ctx *ctx, u64 *n_io, bool translate_newlines, const uint8_
             BPE_TRY(bpe_buf_reserve(ctx, ctx->spmask, fw * sizeof(u32)));
             BPE_TRY(bpe_buf_reserve(ctx, ctx->spstart, fw * sizeof(u32)));
             BPE_TRY(bpe_buf_reserve(ctx, ctx->tmp0, fw * sizeof(u32)));
-            CUDA_TRY(ctx, cudaMemsetAsync(ctx->spmask.p, 0, fw * sizeof(u32), st));
-            CUDA_TRY(ctx, cudaMemsetAsync(ctx->spstart.p, 0, fw * sizeof(u32), st));
+            if (bmask) {                         // the special-token kernels OR their occurrences into the boundaries
+                launch_copy_words2(bmask, (u32 *)ctx->spmask.p, (u32 *)ctx->spstart.p, fw, ctx->sm_count, st);
+            } else {
+                CUDA_TRY(ctx, cudaMemsetAsync(ctx->spmask.p, 0, fw * sizeof(u32), st));
+                CUDA_TRY(ctx, cudaMemsetAsync(ctx->spstart.p, 0, fw * sizeof(u32), st));
+            }
             CUDA_TRY(ctx, cudaMemsetAsync(ctx->tmp0.p, 0, fw * sizeof(u32), st));
             launch_special_split(text, n, sp_blob_dev, sp_offs_dev, n_sp, sp_max_len, (u32 *)ctx->tmp0.p,
                                  (u32 *)ctx->spstart.p, (u32 *)ctx->spmask.p, (n + 31) / 32, ctx->sm_count, st);
             spmask = (const u32 *)ctx->spmask.p; spstart = (const u32 *)ctx->spstart.p;
+        } else if (bmask) {                      // boundaries only: they are both the occurrences and their first bytes
+            spmask = bmask; spstart = bmask;
         }
         // words past the last tile stay zero
         u64 tiles_words = ((n + 4095) / 4096) * (4096 / 32);

@@ -46,6 +46,7 @@ struct bpe_ctx {
     std::vector<uint8_t> sp_cache_blob; std::vector<uint32_t> sp_cache_offs;
     // double buffering of the host-side entry points: second text arena / output buffers, copy streams, events
     DevBuf text_alt, out_a, out_b;
+    DevBuf doc_bmask, doc_offs, doc_stage;   // bpe_encode_batch: boundary bitmask; document / id offsets; second upload buffer
     cudaStream_t s_in = nullptr, s_out = nullptr;
     cudaEvent_t ev_in[2] = {}, ev_out[2] = {}, ev_done = nullptr;
     void *pinned = nullptr; size_t pinned_cap = 0;   // small pinned staging for scalar readbacks

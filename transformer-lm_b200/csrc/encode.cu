@@ -38,6 +38,7 @@
 //   0..3   that many ids inline, 20 bits each at bits 0, 20, 40
 //   4      ids in the id pool: bits 59..24 = offset, bits 23..0 = count
 //   5      KeyError: bits 31..0 = offending symbol (bit 31 set: index of a special token instead)
+//   13     (per-occurrence array only, bpe_encode_batch) document boundary: bits 39..0 = index of the document it ends, in the chunk
 //   14     (per-occurrence array only) not computed when looked up: bits 31..0 = cache slot reference
 //   15     not computed yet
 #define VAL_NONE 0xFFFFFFFFFFFFFFFFull
@@ -45,6 +46,8 @@
 #define VAL_TAG(v) ((u32)((v) >> 60))
 #define VAL_EXT 4ull
 #define VAL_ERR 5ull
+#define VAL_DOC 13ull
+#define VAL_DOC_MASK ((1ull << 40) - 1)
 #define INLINE_ID_LIMIT (1u << 20)
 #define RANK_NONE 0xFFFFFFFFFFFFFFFFull
 #define MKEY_EMPTY 0xFFFFFFFFFFFFFFFFull
@@ -72,6 +75,9 @@ struct EncTables {
     // [0]=n_short [1]=n_long [2]=todo count [3]=table overflow [4]=kpool cursor [5]=ipool cursor [6]=pretoken too long
     // [7]=smallest ordinal (in the text of the call) of a pretoken whose value is a KeyError  [8]=n_medium  [9]=step tickets of the lookup kernel
     u64 *ctr;
+    // document boundaries of bpe_encode_batch (all null for bpe_encode): bit per arena byte, boundaries before every 512-byte group,
+    // id_offs[j] = index of the first id after document j of the chunk (id_base + its offset in the chunk's output)
+    const u32 *bmask; const u64 *bpre; u64 *id_offs; u64 id_base;
 };
 
 __device__ __forceinline__ const uint8_t *enc_rep_ptr(const EncTables &t, u64 meta) {
@@ -293,6 +299,9 @@ __device__ __forceinline__ void lookup_drain(const EncTables &t, LookupQueues &q
 
 // chunks [c_lo, c_hi) (16 bytes each, absolute positions 16 c; c_lo a multiple of 32); pre[g] = ordinal of the first pretoken of the
 // g-th group of 32 chunks (absolute), ord0 = ordinal of the batch's first pretoken, base = 16 c_lo
+// DOCS (bpe_encode_batch): a pretoken that starts on a boundary bit is a document boundary, value VAL_DOC | document index (boundary
+// bits before the step's group + the warp's lanes before this one + the chunk's bits before the pretoken); it never touches the cache.
+template <bool DOCS>
 __global__ void __launch_bounds__(LK_NT, 1) k_enc_lookup(EncTables t, const u32 *__restrict__ flags, const u64 *__restrict__ pre, u64 ord0,
                                                         u64 c_lo, u64 c_hi, u64 n, u64 base, u64 *__restrict__ vals) {
     extern __shared__ __align__(16) unsigned char lk_smem[];
@@ -318,12 +327,20 @@ __global__ void __launch_bounds__(LK_NT, 1) k_enc_lookup(EncTables t, const u32 
         const u64 c = c_lo + (tk * LK_TICKET + sub) * 32u + lane;
         const bool live = c < c_hi;
         const u64 p0 = c * 16u;
-        uint4 A = make_uint4(0, 0, 0, 0), B = A; u32 f0 = 0, f1 = 0;
+        uint4 A = make_uint4(0, 0, 0, 0), B = A; u32 f0 = 0, f1 = 0, bm = 0;
         const u64 ordg = __ldcs(pre + ((c - lane) >> 5));            // (one word per step, the same for all lanes)
         if (live) {
             const uint4 *tp = reinterpret_cast<const uint4 *>(t.text + p0);
             A = __ldcs(tp); B = __ldcs(tp + 1);
             const u64 w = c >> 1; f0 = __ldcs(flags + w); f1 = w + 1 < n_fw ? __ldcs(flags + w + 1) : 0u;
+            if (DOCS) bm = (__ldcs(t.bmask + w) >> (u32)(p0 & 16u)) & 0xFFFFu;
+        }
+        u64 docc = 0;                            // index of the first document boundary of the chunk
+        if (DOCS) {
+            u32 bi = __popc(bm);
+#pragma unroll
+            for (u32 d = 1; d < 32; d <<= 1) { const u32 o = __shfl_up_sync(0xffffffffu, bi, d); if (lane >= d) bi += o; }
+            docc = __ldcs(t.bpre + ((c - lane) >> 5)) + bi - __popc(bm);
         }
         const u32 W0 = A.x, W1 = A.y, W2 = A.z, W3 = A.w, W4 = B.x, W5 = B.y, W6 = B.z, W7 = B.w;
         u64 F = (((u64)f1 << 32) | f0) >> (u32)(p0 & 16u);           // bit i: a pretoken starts at byte p0 + i (>= 48 bits)
@@ -342,7 +359,9 @@ __global__ void __launch_bounds__(LK_NT, 1) k_enc_lookup(EncTables t, const u32 
             const u32 ord = ordc + __popc(mall & ((1u << j) - 1u));
             const u64 rest = F >> (j + 1u);
             u32 len = (u32)__ffsll((long long)rest);
-            if (act && len == 0) {               // no further start in the window: a long pretoken, or the last one of the text
+            const bool isb = DOCS && act && ((bm >> j) & 1u);
+            if (isb) __stcs(&vals[ord], (VAL_DOC << 60) | (docc + __popc(bm & ((1u << j) - 1u))));
+            if (act && !isb && len == 0) {               // no further start in the window: a long pretoken, or the last one of the text
                 const u64 e = flags_next_start(flags, p0 + j + 1, n) - (p0 + j);
                 if (e > MAX_TOKEN_LEN) { t.ctr[6] = 1; len = MAX_TOKEN_LEN; } else len = (u32)e;
             }
@@ -353,8 +372,8 @@ __global__ void __launch_bounds__(LK_NT, 1) k_enc_lookup(EncTables t, const u32 
             const u32 Y0 = q1 ? X1 : X0, Y1 = q1 ? X2 : X1, Y2 = q1 ? X3 : X2, Y3 = q1 ? X4 : X3, Y4 = q1 ? X5 : X4;
             const u64 k0 = (u64)__funnelshift_r(Y0, Y1, sh) | ((u64)__funnelshift_r(Y1, Y2, sh) << 32);
             const u64 k1 = (u64)__funnelshift_r(Y2, Y3, sh) | ((u64)__funnelshift_r(Y3, Y4, sh) << 32);
-            bool q_s = act && len <= SHORT_MAX;
-            const bool q_m = act && len > SHORT_MAX && len <= 15u, q_l = act && len > 15u;
+            bool q_s = act && !isb && len <= SHORT_MAX;
+            const bool q_m = act && !isb && len > SHORT_MAX && len <= 15u, q_l = act && !isb && len > 15u;
             const u64 key = (k0 & low_bytes_mask(len)) | ((u64)len << 56);               // (short pretokens)
             if (q_s) {
                 u32 slot = enc_sm_slot(key);
@@ -713,6 +732,14 @@ __global__ void __launch_bounds__(SE_NT) k_enc_scan_emit(EncTables t, const u64 
         if (staged) stage_ids();
     }
     __syncthreads();
+    if (t.id_offs) {                             // bpe_encode_batch: a document boundary holds where the next document's ids start
+        u64 o = t.id_base + out_base + s_prefix + ex;
+#pragma unroll
+        for (u32 k = 0; k < SE_ITEMS; k++) {
+            if (VAL_TAG(v[k]) == VAL_DOC) t.id_offs[v[k] & VAL_DOC_MASK] = o;
+            o += value_count(v[k]);
+        }
+    }
     if (!kEmit) return;
     const u64 tile_dst = out_base + s_prefix;
     if (staged) {
@@ -955,6 +982,7 @@ struct bpe_tok {
     u64 hot_nb = 0;
     bool hot_built = false, sampling = false;
     std::vector<uint8_t> key_error;              // bytes of the last KeyError key
+    int doc_sep = -1;                            // boundary byte of bpe_encode_batch (-1: every candidate occurs in a special)
 };
 
 static int alloc_exact_e(bpe_ctx *ctx, DevBuf &b, size_t bytes) { return bpe_buf_alloc(ctx, b, bytes ? bytes : 256); }
@@ -986,6 +1014,7 @@ static EncTables enc_tables(bpe_tok *tok) {
     t.hot = (const ulonglong2 *)tok->hot.p; t.hot_nb = tok->hot_nb; t.hval = (const u64 *)((const ulonglong2 *)tok->hot.p + 2 * tok->hot_nb);
     t.sm_img = tok->hot_built ? (const ulonglong2 *)tok->sm_img.p : nullptr;
     t.scnt = tok->sampling ? (u32 *)tok->samp.p : nullptr; t.mcnt = tok->sampling ? (u32 *)tok->samp.p + tok->scap : nullptr;
+    t.bmask = nullptr; t.bpre = nullptr; t.id_offs = nullptr; t.id_base = 0;
     return t;
 }
 
@@ -1168,6 +1197,14 @@ BPE_API int bpe_tok_create(bpe_ctx *ctx, const int32_t *merge_pairs, const int32
         CUDA_TRY(ctx, cudaMemcpyAsync(tok->sp_ids.p, special_ids, (size_t)n_specials * 8, cudaMemcpyHostToDevice, st));
     }
     tok->max_id = max_id;
+    // bpe_encode_batch's boundary byte: an ASCII value that occurs in no special token, so that no special-token match can cross a
+    // boundary (it would have to contain the byte); never '\r', which the flags kernel reports as a carriage return
+    {
+        bool used[128] = {false};
+        used['\r'] = true;
+        for (uint8_t b : tok->sp_blob_h) if (b < 128) used[b] = true;
+        for (int b = 0; b < 128 && tok->doc_sep < 0; b++) if (!used[b]) tok->doc_sep = b;
+    }
     // decode tables: dense id -> (offset, length)
     long long n_dense = 0;
     for (int64_t i = 0; i < n_vocab; i++) {
@@ -1228,9 +1265,14 @@ BPE_API int bpe_tok_key_error(bpe_tok *tok, uint8_t *buf, uint64_t cap, uint64_t
 #define ENC_BATCH_BYTES (256ull << 20)
 #define ENC_CACHE_MAX_ENTRIES (384ull << 20)
 
+// Document boundaries of a bpe_encode_batch chunk: bit per arena byte; id_offs[j] gets id_base + the offset of the first id after
+// the chunk's document j.
+struct DocBounds { const u32 *bmask; u64 *id_offs; u64 id_base; };
+
 // Encode the n bytes in the context's text arena into out_dev (device pointer, may be null: count only).
 // *n_out = number of tokens (may exceed dev_cap; only dev_cap are written).  stats, when given, are ADDED to.
-static int encode_core(bpe_tok *tok, u64 n, int out_dtype, void *out_dev, u64 dev_cap, uint64_t *n_out, bpe_encode_stats *stats) {
+static int encode_core(bpe_tok *tok, u64 n, int out_dtype, void *out_dev, u64 dev_cap, uint64_t *n_out, bpe_encode_stats *stats,
+                       const DocBounds *docs = nullptr) {
     bpe_ctx *ctx = tok->ctx;
     cudaStream_t st = ctx->stream;
     *n_out = 0;
@@ -1239,18 +1281,24 @@ static int encode_core(bpe_tok *tok, u64 n, int out_dtype, void *out_dev, u64 de
     const uint8_t *spb; const u32 *spo; u32 spmax;
     BPE_TRY(ctx_upload_specials(ctx, tok->sp_blob_h.data(), tok->sp_offs_h.data(), tok->n_sp, &spb, &spo, &spmax));
     u64 nn = n;
-    BPE_TRY(ctx_run_flags(ctx, &nn, false, spb, spo, tok->n_sp, spmax));
+    BPE_TRY(ctx_run_flags(ctx, &nn, false, spb, spo, tok->n_sp, spmax, 0, ~0ull, docs ? docs->bmask : nullptr));
     ctx->saw_cr_encode |= ctx->saw_cr;
     // ordinal of the first pretoken of every GROUP of 16 flag words (512 bytes of text = one warp step of the lookup kernel, which
     // gets the ordinals inside a step from a warp scan): a scan over N / 512 entries instead of N / 32
     const u64 nw = (n + 31) / 32, ng = (nw + 15) / 16;
     size_t cnt_b = round_up((ng + 1) * sizeof(u32), 256), pre_b = round_up((ng + 2) * sizeof(u64), 256);
-    BPE_TRY(bpe_buf_reserve(ctx, ctx->tmp0, cnt_b + pre_b + scan_tmp_elems_host(ng) * sizeof(u64)));
+    const size_t bpre_b = docs ? pre_b : 0;
+    BPE_TRY(bpe_buf_reserve(ctx, ctx->tmp0, cnt_b + pre_b + bpre_b + scan_tmp_elems_host(ng) * sizeof(u64)));
     u32 *cnt = (u32 *)ctx->tmp0.p;
     u64 *pre = (u64 *)((uint8_t *)ctx->tmp0.p + cnt_b);
-    u64 *scan_tmp = (u64 *)((uint8_t *)ctx->tmp0.p + cnt_b + pre_b);
+    u64 *bpre = (u64 *)((uint8_t *)ctx->tmp0.p + cnt_b + pre_b);
+    u64 *scan_tmp = (u64 *)((uint8_t *)ctx->tmp0.p + cnt_b + pre_b + bpre_b);
     launch_popc_words16((const u32 *)ctx->flags.p, ng, cnt, ctx->sm_count, st);
     launch_scan_u32(cnt, ng, pre, scan_tmp, st);
+    if (docs) {                                  // the same per group for the boundary bits: document index of a boundary
+        launch_popc_words16(docs->bmask, ng, cnt, ctx->sm_count, st);
+        launch_scan_u32(cnt, ng, bpre, scan_tmp, st);
+    }
     CUDA_TRY(ctx, cudaGetLastError());
     // (test knobs: BPE_ENC_BATCH_KB = batch size, BPE_ENC_HOT_MIN = pretokens a batch needs to be sampled for the hot table)
     static const u64 batch_bytes = getenv("BPE_ENC_BATCH_KB") ? std::max<u64>(1, (u64)atoll(getenv("BPE_ENC_BATCH_KB"))) << 10 : ENC_BATCH_BYTES;
@@ -1309,6 +1357,7 @@ static int encode_core(bpe_tok *tok, u64 n, int out_dtype, void *out_dev, u64 de
             tok->sampling = true;
         }
         EncTables t = enc_tables(tok);
+        if (docs) { t.bmask = docs->bmask; t.bpre = bpre; t.id_offs = docs->id_offs; t.id_base = docs->id_base; }
         const u64 base = b_lo * 32;
         CUDA_TRY(ctx, cudaEventRecord(evs[0], st));
         if (bound) {
@@ -1316,9 +1365,14 @@ static int encode_core(bpe_tok *tok, u64 n, int out_dtype, void *out_dev, u64 de
             const u64 steps = (c_hi - c_lo + 32 * LK_WARPS * LK_TICKET - 1) / (32 * LK_WARPS * LK_TICKET);
             CUDA_TRY(ctx, cudaMemsetAsync((u64 *)tok->ctr.p + 9, 0, 8, st));
             static bool attr_set = false;
-            if (!attr_set) { CUDA_TRY(ctx, cudaFuncSetAttribute((void *)k_enc_lookup, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LK_DYN_SMEM)); attr_set = true; }
+            if (!attr_set) {
+                CUDA_TRY(ctx, cudaFuncSetAttribute((void *)k_enc_lookup<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LK_DYN_SMEM));
+                CUDA_TRY(ctx, cudaFuncSetAttribute((void *)k_enc_lookup<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LK_DYN_SMEM));
+                attr_set = true;
+            }
             const unsigned lgrid = (unsigned)std::max<u64>(1, std::min<u64>((u64)ctx->sm_count, steps));
-            KLAUNCH(k_enc_lookup, lgrid, LK_NT, LK_DYN_SMEM, st, t, (const u32 *)ctx->flags.p, pre, ord[b], c_lo, c_hi, n, base, vals);
+            if (docs) KLAUNCH(k_enc_lookup<true>, lgrid, LK_NT, LK_DYN_SMEM, st, t, (const u32 *)ctx->flags.p, pre, ord[b], c_lo, c_hi, n, base, vals);
+            else KLAUNCH(k_enc_lookup<false>, lgrid, LK_NT, LK_DYN_SMEM, st, t, (const u32 *)ctx->flags.p, pre, ord[b], c_lo, c_hi, n, base, vals);
         }
         CUDA_TRY(ctx, cudaGetLastError());
         CUDA_TRY(ctx, cudaEventRecord(evs[1], st));
@@ -1427,8 +1481,6 @@ static int encode_check_args(bpe_tok *tok, const uint8_t *text, u64 n, int out_d
     return BPE_OK;
 }
 
-// ---- host entry point: chunks cut at exact boundaries, double-buffered so that the upload of chunk k+1 and the download
-// of chunk k-1 run while chunk k is encoded ----------------------------------------------------------------------------
 #define ENC_PIPE_CHUNK (256ull << 20)
 #define ENC_PIPE_MIN (96ull << 20)
 #define ENC_CUT_WINDOW (8ull << 20)
@@ -1463,67 +1515,168 @@ static u64 find_exact_cut(const bpe_tok *tok, const uint8_t *t, u64 n, u64 nomin
     return 0;
 }
 
-BPE_API int bpe_encode(bpe_tok *tok, const uint8_t *text_host, uint64_t n, int out_dtype, void *out, uint64_t cap, uint64_t *n_out,
-                       bpe_encode_stats *stats) {
+// ---- bpe_encode_batch: a chunk of documents into the text arena, one boundary byte after every document that ends in it ----------
+// ends[j] - lo = where document j ends in the chunk (ascending, 0..len).  Byte i of the chunk goes to i + #{j : ends[j] - lo <= i},
+// the boundary after document j to ends[j] - lo + j, which also sets its bit in bmask (zeroed by the caller).  A warp takes 512
+// bytes at a time, 32 consecutive bytes per instruction; the boundaries inside them (usually none) come from a binary search.
+__device__ __forceinline__ u64 ends_lower_bound(const u64 *__restrict__ e, u64 lo, u64 hi, u64 x) {      // first index with e >= x
+    while (lo < hi) { const u64 m = (lo + hi) >> 1; if (__ldg(&e[m]) < x) lo = m + 1; else hi = m; }
+    return lo;
+}
+__global__ void __launch_bounds__(256) k_enc_expand_docs(const uint8_t *__restrict__ src, u64 len, const u64 *__restrict__ ends, u64 n_ends,
+                                                        u64 lo, uint8_t *__restrict__ arena, u32 *__restrict__ bmask, uint8_t sep) {
+    const u32 lane = lane_id();
+    const u64 gw = ((u64)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nw = ((u64)gridDim.x * blockDim.x) >> 5;
+    for (u64 w0 = gw * 512; w0 < len; w0 += nw * 512) {
+        const u64 r = ends_lower_bound(ends, 0, n_ends, lo + w0), r1 = ends_lower_bound(ends, r, n_ends, lo + w0 + 512);
+        for (u32 k = 0; k < 16; k++) {
+            const u64 i = w0 + k * 32 + lane;
+            if (i >= len) break;
+            const u64 rank = r1 > r ? ends_lower_bound(ends, r, r1, lo + i + 1) : r;
+            arena[i + rank] = src[i];
+        }
+    }
+    for (u64 j = (u64)blockIdx.x * blockDim.x + threadIdx.x; j < n_ends; j += (u64)gridDim.x * blockDim.x) {
+        const u64 p = ends[j] - lo + j;
+        arena[p] = sep;
+        atomicOr(&bmask[p >> 5], 1u << (p & 31));
+    }
+}
+
+// A pipeline chunk: bytes [lo, hi) of the caller's text; bpe_encode_batch: documents [da, db) end inside it.
+struct EncChunk { u64 lo, hi, da, db; };
+
+// bpe_encode_batch's chunks: cut at a document end near every multiple of the nominal size; a document that runs well past it is cut
+// at an exact boundary inside it (find_exact_cut on the document alone), or else stays whole.
+static std::vector<EncChunk> doc_chunks(const bpe_tok *tok, const uint8_t *t, u64 n, const uint64_t *doc_offs, u64 n_docs, u64 chunk) {
+    std::vector<EncChunk> out;
+    u64 lo = 0, d = 0;
+    while (n >= ENC_PIPE_MIN && n - lo > chunk + chunk / 2) {
+        const u64 target = lo + chunk;
+        const u64 j = (u64)(std::upper_bound(doc_offs + 1 + d, doc_offs + 1 + n_docs, target) - (doc_offs + 1));   // docs [d, j) end <= target
+        const u64 e = j > d ? doc_offs[j] : lo;
+        u64 hi, nd;
+        if (e >= lo + chunk / 2) { hi = e; nd = j; }
+        else {
+            const u64 ds = doc_offs[j], c = find_exact_cut(tok, t + ds, doc_offs[j + 1] - ds, target - ds);   // (ds < target: j does not end by it)
+            if (c && ds + c > lo) { hi = ds + c; nd = j; }
+            else if (e > lo) { hi = e; nd = j; }
+            else { hi = doc_offs[j + 1]; nd = j + 1; }
+        }
+        out.push_back({lo, hi, d, nd});
+        lo = hi; d = nd;
+    }
+    out.push_back({lo, n, d, n_docs});
+    return out;
+}
+
+// ---- host entry points: chunks cut at exact boundaries, double-buffered so that the upload of chunk k+1 and the download of
+// chunk k-1 run while chunk k is encoded.  doc_offs (bpe_encode_batch) or null (bpe_encode).
+//   bpe_encode:       a chunk is uploaded straight into the arena the kernels read next (the two arenas alternate)
+//   bpe_encode_batch: a chunk is uploaded as it is into one of two staging buffers; on the compute stream k_enc_expand_docs moves it
+//                     into the arena with a boundary byte after every document and sets the boundary bitmask
+static int encode_pipeline(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs, uint64_t n_docs, int out_dtype,
+                           void *out, uint64_t cap, uint64_t *n_out, uint64_t *id_offs_out, bpe_encode_stats *stats) {
     BPE_TRY(encode_check_args(tok, text_host, n, out_dtype, n_out));
     bpe_ctx *ctx = tok->ctx;
     cudaStream_t st = ctx->stream;
     ctx->saw_cr_encode = false;
     if (stats) memset(stats, 0, sizeof(*stats));
     const size_t esz = out_dtype == BPE_DTYPE_U16 ? 2 : 4;
-    // chunk boundaries
-    std::vector<u64> cut{0};
     u64 chunk = ENC_PIPE_CHUNK;
     if (const char *e = getenv("BPE_ENCODE_CHUNK_MB")) chunk = std::max<u64>(1, strtoull(e, nullptr, 10)) << 20;
-    if (n >= ENC_PIPE_MIN) {
-        for (u64 nominal = chunk; nominal + chunk / 2 < n; ) {
-            u64 c = find_exact_cut(tok, text_host, n, nominal);
-            if (!c || c <= cut.back()) break;     // no exact boundary nearby: the rest goes in one piece
-            cut.push_back(c);
-            nominal = c + chunk;
+    std::vector<EncChunk> chunks;
+    if (doc_offs) chunks = doc_chunks(tok, text_host, n, doc_offs, n_docs, chunk);
+    else {
+        std::vector<u64> cut{0};
+        if (n >= ENC_PIPE_MIN) {
+            for (u64 nominal = chunk; nominal + chunk / 2 < n; ) {
+                u64 c = find_exact_cut(tok, text_host, n, nominal);
+                if (!c || c <= cut.back()) break;     // no exact boundary nearby: the rest goes in one piece
+                cut.push_back(c);
+                nominal = c + chunk;
+            }
         }
+        cut.push_back(n);
+        for (size_t k = 0; k + 1 < cut.size(); k++) chunks.push_back({cut[k], cut[k + 1], 0, 0});
     }
-    cut.push_back(n);
-    const size_t m = cut.size() - 1;
+    const size_t m = chunks.size();
     BPE_TRY(ctx_pipeline_init(ctx));
+    u64 *id_dev = nullptr;
+    if (doc_offs) {                              // document offsets up; id offsets come back in the second half of the buffer
+        BPE_TRY(bpe_buf_reserve(ctx, ctx->doc_offs, (n_docs + 1) * 16));
+        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->doc_offs.p, doc_offs, (n_docs + 1) * 8, cudaMemcpyHostToDevice, st));
+        id_dev = (u64 *)ctx->doc_offs.p + (n_docs + 1);
+    }
     EvTimer tm(ctx);
     int e0 = tm.mark();
-    DevBuf *tbuf[2] = {&ctx->text, &ctx->text_alt};
+    DevBuf *tbuf[2] = {&ctx->text, &ctx->text_alt};     // bpe_encode: the two arenas
+    DevBuf *sbuf[2] = {&ctx->text_alt, &ctx->doc_stage};   // bpe_encode_batch: the two staging buffers (the arena is ctx->text)
     DevBuf *obuf[2] = {&ctx->out_a, &ctx->out_b};
     u64 max_chunk = 0;
-    for (size_t k = 0; k < m; k++) max_chunk = std::max(max_chunk, cut[k + 1] - cut[k]);
-    auto upload = [&](size_t k, DevBuf &dst) -> int {     // chunk k -> arena dst, on the copy-in stream
-        const u64 len = cut[k + 1] - cut[k];
-        BPE_TRY(ctx_prepare_arena(ctx, dst, m > 1 ? max_chunk : len, ctx->s_in));
-        if (m > 1 && len < max_chunk)             // bytes between this chunk's end and the arena padding must read as padding
-            CUDA_TRY(ctx, cudaMemsetAsync((uint8_t *)dst.p + BPE_PAD + len, BPE_BYTE_PAD, max_chunk - len, ctx->s_in));
-        if (len) CUDA_TRY(ctx, cudaMemcpyAsync((uint8_t *)dst.p + BPE_PAD, text_host + cut[k], len, cudaMemcpyHostToDevice, ctx->s_in));
+    for (const EncChunk &c : chunks) max_chunk = std::max(max_chunk, c.hi - c.lo);
+    auto upload = [&](size_t k, DevBuf &dst) -> int {     // chunk k -> arena (staging buffer) dst, on the copy-in stream
+        const u64 len = chunks[k].hi - chunks[k].lo;
+        if (doc_offs) BPE_TRY(bpe_buf_reserve(ctx, dst, std::max<u64>(max_chunk, 16)));
+        else {
+            BPE_TRY(ctx_prepare_arena(ctx, dst, m > 1 ? max_chunk : len, ctx->s_in));
+            if (m > 1 && len < max_chunk)         // bytes between this chunk's end and the arena padding must read as padding
+                CUDA_TRY(ctx, cudaMemsetAsync((uint8_t *)dst.p + BPE_PAD + len, BPE_BYTE_PAD, max_chunk - len, ctx->s_in));
+        }
+        uint8_t *p = (uint8_t *)dst.p + (doc_offs ? 0 : BPE_PAD);
+        if (len) CUDA_TRY(ctx, cudaMemcpyAsync(p, text_host + chunks[k].lo, len, cudaMemcpyHostToDevice, ctx->s_in));
         CUDA_TRY(ctx, cudaEventRecord(ctx->ev_in[k & 1], ctx->s_in));
         return BPE_OK;
     };
     // (the compute stream must not run ahead of pool (re)allocations done for the other buffer: everything below that
     // touches a buffer is ordered by events, and every chunk ends with a host-side synchronisation of the compute stream)
     CUDA_TRY(ctx, cudaStreamSynchronize(st));
-    BPE_TRY(upload(0, *tbuf[0]));
+    BPE_TRY(upload(0, doc_offs ? *sbuf[0] : *tbuf[0]));
     u64 total = 0;
     int rc = BPE_OK;
     for (size_t k = 0; k < m && rc == BPE_OK; k++) {
         const int cur = (int)(k & 1);
-        const u64 len = cut[k + 1] - cut[k];
-        if (k + 1 < m) { rc = upload(k + 1, *tbuf[cur ^ 1]); if (rc != BPE_OK) break; }
-        if (cur == 1) std::swap(ctx->text, ctx->text_alt);         // the arena the kernels read is always ctx->text
+        const EncChunk &ch = chunks[k];
+        const u64 len = ch.hi - ch.lo;
+        if (k + 1 < m) { rc = upload(k + 1, doc_offs ? *sbuf[cur ^ 1] : *tbuf[cur ^ 1]); if (rc != BPE_OK) break; }
+        const bool swap = !doc_offs && cur == 1;
+        if (swap) std::swap(ctx->text, ctx->text_alt);            // the arena the kernels read is always ctx->text
         CUDA_TRY(ctx, cudaStreamWaitEvent(st, ctx->ev_in[cur], 0));
         void *odev = nullptr;
         if (out) {
             rc = bpe_buf_reserve(ctx, *obuf[cur], std::max<size_t>((m > 1 ? max_chunk : len) * esz, 16));
-            if (rc != BPE_OK) { if (cur == 1) std::swap(ctx->text, ctx->text_alt); break; }
+            if (rc != BPE_OK) { if (swap) std::swap(ctx->text, ctx->text_alt); break; }
             CUDA_TRY(ctx, cudaStreamWaitEvent(st, ctx->ev_out[cur], 0));   // its previous download has finished
             odev = obuf[cur]->p;
         }
         uint64_t nt = 0;
-        rc = encode_core(tok, len, out_dtype, odev, len, &nt, stats);
-        if (cur == 1) std::swap(ctx->text, ctx->text_alt);
-        if (rc != BPE_OK) { ctx->err_detail += (int64_t)cut[k]; break; }
+        if (doc_offs) {
+            const u64 nb = ch.db - ch.da, an = len + nb;            // a boundary byte after each document that ends here
+            rc = ctx_prepare_arena(ctx, ctx->text, an);
+            if (rc == BPE_OK) rc = bpe_buf_reserve(ctx, ctx->doc_bmask, flag_words(an) * sizeof(u32));
+            if (rc != BPE_OK) break;
+            CUDA_TRY(ctx, cudaMemsetAsync(ctx->doc_bmask.p, 0, flag_words(an) * sizeof(u32), st));
+            const unsigned g = (unsigned)std::max<u64>(1, std::min<u64>((u64)ctx->sm_count * 16, std::max((len + 4095) / 4096, (nb + 255) / 256)));
+            KLAUNCH(k_enc_expand_docs, g, 256, 0, st, (const uint8_t *)sbuf[cur]->p, len, (const u64 *)ctx->doc_offs.p + ch.da + 1, nb, ch.lo,
+                    (uint8_t *)ctx->text.p + BPE_PAD, (u32 *)ctx->doc_bmask.p, (uint8_t)tok->doc_sep);
+            CUDA_TRY(ctx, cudaGetLastError());
+            const DocBounds db{(const u32 *)ctx->doc_bmask.p, id_dev + ch.da + 1, total};
+            rc = encode_core(tok, an, out_dtype, odev, len, &nt, stats, &db);
+            if (rc == BPE_ERR_UTF8 || rc == BPE_ERR_KEY) {      // arena offset -> offset in the caller's text: minus the boundaries before it
+                const u64 p = (u64)ctx->err_detail;
+                u64 a = 0, b = nb;                              // boundaries j < a lie before p (boundary j sits at ends[j] - lo + j)
+                while (a < b) { const u64 mid = (a + b) / 2; if (doc_offs[ch.da + 1 + mid] - ch.lo + mid < p) a = mid + 1; else b = mid; }
+                ctx->err_detail = (int64_t)(ch.lo + p - a);
+                bpe_set_error(ctx, rc, rc == BPE_ERR_UTF8 ? "invalid UTF-8 at byte offset %llu of the batch"
+                                                          : "KeyError: a token of the pretoken at byte %llu of the batch is not in the vocabulary",
+                              (unsigned long long)ctx->err_detail);
+            }
+            if (rc != BPE_OK) break;
+        } else {
+            rc = encode_core(tok, len, out_dtype, odev, len, &nt, stats);
+            if (swap) std::swap(ctx->text, ctx->text_alt);
+            if (rc != BPE_OK) { ctx->err_detail += (int64_t)ch.lo; break; }
+        }
         if (out && total < cap) {
             const u64 w = std::min<u64>(nt, cap - total);
             CUDA_TRY(ctx, cudaEventRecord(ctx->ev_done, st));
@@ -1539,9 +1692,40 @@ BPE_API int bpe_encode(bpe_tok *tok, const uint8_t *text_host, uint64_t n, int o
     int e1 = tm.mark();
     CUDA_TRY(ctx, cudaStreamSynchronize(st));
     *n_out = total;
-    if (stats) { stats->ms_total = tm.ms(e0, e1); stats->ms_h2d = 0; stats->ms_d2h = 0; }
+    if (doc_offs) {
+        id_offs_out[0] = 0;
+        if (n_docs) CUDA_TRY(ctx, cudaMemcpy(id_offs_out + 1, id_dev + 1, n_docs * 8, cudaMemcpyDeviceToHost));
+    }
+    if (stats) {
+        stats->ms_total = tm.ms(e0, e1); stats->ms_h2d = 0; stats->ms_d2h = 0;
+        stats->n_bytes -= n_docs; stats->n_pretokens -= n_docs;     // (the boundaries)
+    }
     if (out && total > cap) return bpe_set_error(ctx, BPE_ERR_TOO_SMALL, "need room for %llu ids", (unsigned long long)total);
     return BPE_OK;
+}
+
+BPE_API int bpe_encode(bpe_tok *tok, const uint8_t *text_host, uint64_t n, int out_dtype, void *out, uint64_t cap, uint64_t *n_out,
+                       bpe_encode_stats *stats) {
+    return encode_pipeline(tok, text_host, n, nullptr, 0, out_dtype, out, cap, n_out, nullptr, stats);
+}
+
+BPE_API int bpe_encode_batch(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
+                             int out_dtype, void *out, uint64_t cap, uint64_t *n_out, uint64_t *id_offs_out, bpe_encode_stats *stats) {
+    if (!tok || !n_out || !id_offs_out || (n_docs && !doc_offs_host)) return BPE_ERR_ARG;
+    bpe_ctx *ctx = tok->ctx;
+    for (uint64_t j = 0; j < n_docs; j++)
+        if (doc_offs_host[j] > doc_offs_host[j + 1]) return bpe_set_error(ctx, BPE_ERR_ARG, "bpe_encode_batch: document offsets must not decrease");
+    if (n_docs ? (doc_offs_host[0] != 0 || doc_offs_host[n_docs] != n) : n != 0)
+        return bpe_set_error(ctx, BPE_ERR_ARG, "bpe_encode_batch: document offsets must run from 0 to n");
+    if (n_docs && tok->doc_sep < 0)
+        return bpe_set_error(ctx, BPE_ERR_UNSUPPORTED, "bpe_encode_batch: every ASCII byte but '\\r' occurs in a special token (no boundary byte)");
+    if (n_docs == 0) {
+        BPE_TRY(encode_check_args(tok, text_host, 0, out_dtype, n_out));
+        if (stats) memset(stats, 0, sizeof(*stats));
+        id_offs_out[0] = 0;
+        return BPE_OK;
+    }
+    return encode_pipeline(tok, text_host, n, doc_offs_host, n_docs, out_dtype, out, cap, n_out, id_offs_out, stats);
 }
 
 BPE_API int bpe_encode_dev(bpe_tok *tok, const uint8_t *text_dev, uint64_t n, int out_dtype, void *out_dev, uint64_t cap, uint64_t *n_out,

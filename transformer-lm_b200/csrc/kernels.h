@@ -14,6 +14,7 @@ void launch_special_split(const uint8_t *text, u64 n, const uint8_t *sp_blob_dev
 void launch_popc_words(const u32 *flags, u64 n_words, u32 *cnt, int sm_count, cudaStream_t st);
 void launch_popc_words16(const u32 *flags, u64 n_groups, u32 *cnt, int sm_count, cudaStream_t st);
 void launch_flags_to_offsets(const u32 *flags, u64 n_words, const u64 *pre, u64 *out, u64 cap, int sm_count, cudaStream_t st);
+void launch_copy_words2(const u32 *src, u32 *a, u32 *b, u64 n_words, int sm_count, cudaStream_t st);   // a[i] = b[i] = src[i]
 void launch_scan_u32(const u32 *in, u64 n, u64 *out, u64 *tmp, cudaStream_t st);
 size_t scan_tmp_elems_host(u64 n);
 // Small control words WITHOUT the copy engines: while the pipelined entry points stream 256 MB chunks over PCIe, a 16-byte

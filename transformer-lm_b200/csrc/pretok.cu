@@ -405,5 +405,13 @@ void launch_flags_to_offsets(const u32 *flags, u64 n_words, const u64 *pre, u64 
     if (grid > capg) grid = capg;
     if (grid) KLAUNCH(k_flags_to_offsets, (unsigned)grid, 256, 0, st, flags, n_words, pre, out, cap);
 }
+__global__ void __launch_bounds__(256) k_copy_words2(const u32 *__restrict__ src, u32 *__restrict__ a, u32 *__restrict__ b, u64 n_words) {
+    for (u64 w = (u64)blockIdx.x * blockDim.x + threadIdx.x; w < n_words; w += (u64)gridDim.x * blockDim.x) { const u32 v = src[w]; a[w] = v; b[w] = v; }
+}
+void launch_copy_words2(const u32 *src, u32 *a, u32 *b, u64 n_words, int sm_count, cudaStream_t st) {
+    u64 grid = (n_words + 255) / 256, capg = (u64)sm_count * bpe_grid_mult(64);
+    if (grid > capg) grid = capg;
+    if (grid) KLAUNCH(k_copy_words2, (unsigned)grid, 256, 0, st, src, a, b, n_words);
+}
 void launch_scan_u32(const u32 *in, u64 n, u64 *out, u64 *tmp, cudaStream_t st) { launch_excl_scan_u32_to_u64(in, n, out, tmp, st); }
 size_t scan_tmp_elems_host(u64 n) { return scan_tmp_elems(n); }

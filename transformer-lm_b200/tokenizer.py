@@ -1,6 +1,7 @@
 """Tokenizer host: mirrors models/tokenizer/tokenizer.py:11-167 of the reference.
 
     Tokenizer(vocab, merges, special_tokens).encode(str) -> list[int]
+                                            .encode_batch(Sequence[str]) -> list[list[int]]
                                             .encode_iterable(Iterable[str]) -> Iterator[int]
                                             .decode(list[int]) -> str
 
@@ -13,7 +14,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import pickle
-from typing import Iterable, Iterator, List, Tuple
+from typing import Iterable, Iterator, List, Sequence, Tuple
 
 import numpy as np
 
@@ -21,6 +22,32 @@ from . import _lib
 from .train import train_bpe
 
 _CHUNK_CHARS = 1024 * 1024 * 2                   # tokenizer.py:145
+
+
+def _pack_documents(texts: list) -> Tuple[np.ndarray, np.ndarray, UnicodeEncodeError | None]:
+    """(UTF-8 bytes of all documents back to back as uint8, uint64 byte offsets (len + 1), None), or -- when item k is a str that
+    cannot be encoded (a lone surrogate) -- the packing of the items before it and the error."""
+    try:
+        joined = "".join(texts)
+    except TypeError:                            # some items are bytes
+        joined = None
+    if joined is not None and joined.isascii():  # one byte per character: no per-item encode
+        lens = np.fromiter(map(len, texts), dtype=np.uint64, count=len(texts))
+        parts, bad = [joined.encode("ascii")], None
+    else:
+        parts, bad = [], None
+        for t in texts:
+            if isinstance(t, str):
+                try:
+                    t = t.encode("utf-8")
+                except UnicodeEncodeError as e:
+                    bad = e
+                    break
+            parts.append(t)
+        lens = np.fromiter(map(len, parts), dtype=np.uint64, count=len(parts))
+    offs = np.zeros(lens.size + 1, dtype=np.uint64)
+    np.cumsum(lens, out=offs[1:])
+    return np.frombuffer(b"".join(parts), dtype=np.uint8), offs, bad
 
 
 class Tokenizer:
@@ -187,6 +214,51 @@ class Tokenizer:
 
     def encode(self, text: str) -> List[int]:
         return self.encode_to_numpy(text.encode("utf-8"), np.int32).tolist()
+
+    def encode_batch(self, texts: Sequence[str]) -> List[List[int]]:
+        """[self.encode(t) for t in texts] -- the same ids, split the same way, the same first exception -- with one device pass
+        over all documents (bpe_encode_batch) instead of one pipeline per document."""
+        ids, offs = self.encode_batch_to_numpy(texts, np.int32)
+        flat, o = ids.tolist(), offs.tolist()
+        return [flat[o[j]: o[j + 1]] for j in range(len(o) - 1)]
+
+    def encode_batch_to_numpy(self, texts: Sequence[str | bytes], dtype=np.int32) -> Tuple[np.ndarray, np.ndarray]:
+        """Ids of every document back to back (uint16 or int32) and int64 offsets (len(texts) + 1): document j's ids are
+        ids[offsets[j]:offsets[j + 1]].  A `bytes` item must be UTF-8; it fails as item.decode("utf-8") would.  Where several
+        documents would fail, the error is that of the first one in list order, as in a loop over encode_to_numpy."""
+        texts = list(texts)
+        blob, offs, bad = _pack_documents(texts)
+        if bad is not None:                      # a str that cannot be encoded: the documents before it fail first, if any does
+            self._encode_batch_packed(blob, offs, dtype)
+            raise bad
+        return self._encode_batch_packed(blob, offs, dtype, texts)
+
+    def _encode_batch_packed(self, blob: np.ndarray, offs: np.ndarray, dtype, texts=None):
+        tok = self._device_tok()
+        ctx = self._tok_ctx
+        L = _lib.lib()
+        code = {np.dtype(np.uint16): _lib.DTYPE_U16, np.dtype(np.int32): _lib.DTYPE_I32}[np.dtype(dtype)]
+        n_docs = offs.size - 1
+        out = np.empty(max(blob.size, 1), dtype=dtype)            # a token covers at least one byte
+        id_offs = np.zeros(n_docs + 1, dtype=np.uint64)
+        n_out = C.c_uint64(0)
+        stats = _lib.EncodeStats()
+        with ctx.lock:
+            rc = L.bpe_encode_batch(tok, _lib.ptr(blob) if blob.size else None, blob.size, _lib.ptr(offs), n_docs, code,
+                                    _lib.ptr(out), out.size, C.byref(n_out), _lib.ptr(id_offs), C.byref(stats))
+            detail = L.bpe_last_error_detail(ctx.handle)
+            if rc == _lib.ERR_UTF8 and texts is not None:
+                # the device reports invalid UTF-8 in a chunk before a KeyError in it: the documents before the invalid one
+                # go first, then that document fails as its decode does
+                k = int(np.searchsorted(offs, detail, side="right")) - 1
+                self._encode_batch_packed(blob[: int(offs[k])], offs[: k + 1], dtype)
+                item = texts[k]
+                if isinstance(item, (bytes, bytearray, memoryview)):
+                    bytes(item).decode("utf-8")
+            if rc != _lib.BPE_OK:
+                self._raise(ctx, rc)
+        self.last_stats = stats.as_dict()
+        return out[: n_out.value], id_offs.astype(np.int64)
 
     def encode_sharded(self, data, dtype=np.uint16, group=None):
         """Multi-GPU encode (one process per GPU, torch.distributed initialised): every rank passes the same UTF-8 `data`
