@@ -78,10 +78,12 @@ typedef struct bpe_train_stats {
     uint64_t n_unique;           /* unique pretokens (words) */
     uint64_t n_symbols;          /* total symbols over unique words at merge-loop start */
     uint64_t n_pairs_initial;    /* distinct adjacent byte pairs at start */
-    uint64_t n_pairs_final;      /* pair-table keys ever created */
+    uint64_t n_pairs_final;      /* distinct pair keys ever created (popped ones included); independent of the pair table's size and growth */
     uint64_t log_records;        /* inverted-index records written by the merge loop */
     uint64_t duplicate_tokens;   /* positive-count merges whose product bytes already existed (SURVEY A-6): provably 0, kept as an invariant check */
-    uint64_t sum_live_pairs;     /* sum over merges of the live pair-table keys (what the reference's max() scans) */
+    uint64_t sum_live_pairs;     /* sum over merges of the live pair-table keys (what the reference's max() scans), every merge of a
+                                    grid step charged the count at the start of the step (so it does not depend on the timing of
+                                    the step's own insertions, but does depend on how merges are batched into steps) */
     uint64_t merge_steps;        /* grid steps of the merge loop (a step applies up to 12 merges, see csrc/merge.cuh) */
     float ms_h2d;                /* host->device copy of the text */
     float ms_validate;           /* UTF-8 validation + CR scan */

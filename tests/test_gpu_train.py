@@ -253,15 +253,6 @@ def test_merges_do_not_depend_on_the_batch_limit(monkeypatch, batch):
     assert _train_bytes(fz, 5000, []) == oracle.train_bpe_on_bytes(fz, 5000, [])
 
 
-def test_merge_loop_survives_table_growth():
-    rnd = random.Random(77)
-    words = ["".join(rnd.choice("abcdefghijklmnopqrstuvwxyz") for _ in range(rnd.randint(2, 9))) for _ in range(6000)]
-    data = " ".join(rnd.choice(words) for _ in range(40000)).encode()
-    want = oracle.train_bpe_on_bytes(data, 2500, [])
-    got = _train_bytes(data, 2500, [])
-    assert got[1] == want[1] and got[0] == want[0]
-
-
 # ---- big host inputs: chunked, double-buffered upload (bpe_train) must equal the one-piece device path -----------------
 def test_pipelined_host_training_equals_one_piece():
     import numpy as np

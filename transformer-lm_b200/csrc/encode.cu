@@ -1300,9 +1300,12 @@ static int encode_core(bpe_tok *tok, u64 n, int out_dtype, void *out_dev, u64 de
         launch_scan_u32(cnt, ng, bpre, scan_tmp, st);
     }
     CUDA_TRY(ctx, cudaGetLastError());
-    // (test knobs: BPE_ENC_BATCH_KB = batch size, BPE_ENC_HOT_MIN = pretokens a batch needs to be sampled for the hot table)
+    // (test knobs: BPE_ENC_BATCH_KB = batch size, BPE_ENC_HOT_MIN = pretokens a batch needs to be sampled for the hot table,
+    // BPE_ENC_CACHE_MAX = cache entries above which the cache is dropped between two batches)
     static const u64 batch_bytes = getenv("BPE_ENC_BATCH_KB") ? std::max<u64>(1, (u64)atoll(getenv("BPE_ENC_BATCH_KB"))) << 10 : ENC_BATCH_BYTES;
     static const u64 hot_min_batch = getenv("BPE_ENC_HOT_MIN") ? (u64)atoll(getenv("BPE_ENC_HOT_MIN")) : ENC_HOT_MIN_BATCH;
+    static const u64 cache_max = getenv("BPE_ENC_CACHE_MAX") ? (u64)atoll(getenv("BPE_ENC_CACHE_MAX")) : ENC_CACHE_MAX_ENTRIES;
+    static const bool prof = getenv("BPE_ENC_PROFILE") != nullptr;
     const u64 words_per_batch = batch_bytes / 32;
     // batch boundaries (flag words).  While the hot table is still to be built the first batch is a small one (64 MB: enough pretokens
     // to sample), so that the cold start -- every lookup a probe of the big tables -- is over after a quarter of a normal batch.
@@ -1336,7 +1339,10 @@ static int encode_core(bpe_tok *tok, u64 n, int out_dtype, void *out_dev, u64 de
         const u64 bound = ord[b + 1] - ord[b];
         const u64 bytes = (b_hi - b_lo) * 32;
         BPE_TRY(cache_read_ctr(tok, c, 9));
-        if (c[0] + c[1] + c[8] + bound > ENC_CACHE_MAX_ENTRIES && c[0] + c[1] + c[8] > (u64)tok->n_sp) {
+        if (c[0] + c[1] + c[8] + bound > cache_max && c[0] + c[1] + c[8] > (u64)tok->n_sp) {
+            if (prof) fprintf(stderr, "  [encoder cache reset: %llu entries + up to %llu new > %llu, before batch %llu of %llu]\n",
+                              (unsigned long long)(c[0] + c[1] + c[8]), (unsigned long long)bound, (unsigned long long)cache_max,
+                              (unsigned long long)b, (unsigned long long)n_batches);
             BPE_TRY(cache_reset(tok));
             BPE_TRY(cache_read_ctr(tok, c, 9));
         }

@@ -131,9 +131,9 @@ struct MergeState {
     int32_t *merges_out; i64 *merge_cnt_out; int n_merges;
     int32_t *live_pairs; int live_cap;           // page-locked HOST memory (or null): the merges as they are made, for the host to follow (bpe_train_set_live)
     // [0]=log cursor [1]=n_done (next merge) [2]=pair keys created [3]=status flags [4]=tok bytes cursor
-    // [5]=keys popped since the table was last rebuilt [6]=number of keys still to be popped (the last step's winners, in [16..16+MG_BATCH))
+    // [5]=keys popped [6]=number of keys still to be popped (the last step's winners, in [16..16+MG_BATCH))
     // [7]=sum over merges of the live pair-table keys (the reference's max() scans that many dict entries, train.py:187-189;
-    //     merges of one step are all charged the table size at the start of the step)
+    //     merges of one step are all charged [2] - [5] at the start of the step)
     // [8]=words rewritten (all steps) [9]=bk_off pool cursor [10]=slices sorted
     // [12]=grid steps taken
     u64 *ctr;
@@ -812,7 +812,8 @@ __device__ __forceinline__ void grid_gather(BarSlot *slots, u32 *counter, u32 G,
 }
 
 // ---- token bookkeeping: bytes and prefix keys of the new tokens, outputs (one CTA, all its threads; warp j = merge j) ------
-__device__ __forceinline__ void token_bookkeeping(int step0, u32 nw0, const Batch *B, u32 *s_off) {
+// live: ctr[2] at the start of the step (the apply CTAs claim keys while this runs: reading ctr[2] here would depend on timing)
+__device__ __forceinline__ void token_bookkeeping(int step0, u32 nw0, const Batch *B, u32 *s_off, u64 live) {
     const u32 tid = threadIdx.x, lane = lane_id(), warp = tid >> 5;
     const u32 r = B->r;
     if (warp == 0) {
@@ -825,7 +826,6 @@ __device__ __forceinline__ void token_bookkeeping(int step0, u32 nw0, const Batc
         if (lane == r - 1) s_off[MG_BATCH] = inc;
     }
     const u64 cur = cM.ctr[4];
-    const u64 live = cM.ctr[2];
     __syncthreads();
     const u64 total = s_off[MG_BATCH];
     if (cur + total > cM.tok_bytes_cap) { if (tid == 0) cM.ctr[3] = 4; }
@@ -1043,8 +1043,21 @@ __global__ void __launch_bounds__(MG_NT) k_merge_loop() {
         if (r == 0) break;                       // len(byte_pair_frequencies) == 0 (train.py:184-185)
         const u32 nw0 = 256 + (u32)step;         // symbol ids of the new tokens: nw0 + j = a_j + b_j (train.py:190)
         const u64 n_rec = s_B.pre[r];
+        // Every key this step can create contains one of its new tokens: (x, nw0 + j) or (nw0 + j, y) with x, y < nw0 + r, and a
+        // site claims at most two of them.  When that bound could take the table past three quarters full, hand back to the host
+        // before anything is applied (the check at the start of the step leaves only the keys already in the table as headroom,
+        // and one step can claim more).  The winners of the previous step were popped in phase B, so none is left pending; the
+        // relaunch derives this step's merges again.
+        {
+            const u64 bound = min(2 * n_rec, 2ull * r * (nw0 + r));
+            if ((s_status[1] + bound) * 4 > cM.pcap * 3) {
+                __syncthreads();
+                if (tid == 0) { s_B.r = 0; if (blockIdx.x == 0) cM.ctr[3] = MG_NEED_GROW; }
+                break;
+            }
+        }
 
-        if (token_cta) token_bookkeeping(step, nw0, &s_B, s_off);
+        if (token_cta) token_bookkeeping(step, nw0, &s_B, s_off, s_status[1]);
         // Records are dealt to the warps of all apply CTAs R at a time, R as small as one pass over the slices allows (but not
         // below cM.min_rec): a step with a few hundred occurrences runs a few lanes on every SM instead of sixteen full warps on
         // one SM, with less divergence between the sites that share a warp.
@@ -1095,23 +1108,19 @@ __global__ void __launch_bounds__(256) k_insert_initial_pairs(const u64 *__restr
     if (p < 65536 && dense[p]) pair_add(p >> 8, p & 255u, (i64)dense[p]);
 }
 
-// Table growth: re-insert every live key of the old table (popped keys and the pending pops are dropped).
-struct PendingPops { u64 key[MG_BATCH]; u32 n; };
-__global__ void __launch_bounds__(256) k_pairs_rehash(const u64 *__restrict__ okey, const i64 *__restrict__ ocnt, u64 ocap, PendingPops pending) {
+// Table growth: copy every key of the old table with its count as it is.  Popped keys stay as tombstones (CNT_DEAD, or CNT_DEAD
+// plus later deltas, which the next rescan repairs) and the last step's winners stay pending (ctr[6]): the grown table holds
+// exactly the keys of the old one, ctr[2] and ctr[5] keep their meaning, and the relaunch -- which rescans every block in its
+// first step -- pops the pending winners like a launch on a table that never grew.
+__global__ void __launch_bounds__(256) k_pairs_rehash(const u64 *__restrict__ okey, const i64 *__restrict__ ocnt, u64 ocap) {
     for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < ocap; i += (u64)gridDim.x * blockDim.x) {
-        u64 k = okey[i];
+        const u64 k = okey[i];
         if (k == PAIR_EMPTY) continue;
-        bool popped = false;
-        for (u32 j = 0; j < pending.n; j++) popped |= k == pending.key[j];
-        if (popped) continue;
-        i64 c = ocnt[i];
-        if (c == CNT_DEAD) continue;
-        if (c < CNT_DEAD_LIMIT) c = (i64)((u64)c - (u64)CNT_DEAD);     // popped, then touched again
+        const i64 c = ocnt[i];
         u64 mask = cM.pcap - 1, s = pair_hash(k) & mask;
         for (;;) {
             if (cM.pkey[s] == PAIR_EMPTY && atomicCAS(&cM.pkey[s], PAIR_EMPTY, k) == PAIR_EMPTY) { cM.pcnt[s] = c; break; }
             s = (s + 1) & mask;
         }
-        atomicAdd(&cM.ctr[2], 1ull);
     }
 }

@@ -1283,7 +1283,9 @@ static int run_merges(bpe_ctx *ctx, const uint8_t *sp_blob, const u32 *sp_offs, 
     M.csr_off = (const u32 *)B.csr_off.p; M.csr_rec = (const Rec *)B.csr_rec.p;
     M.log = (Rec *)B.log.p; M.log_rng = (u64 *)B.log_rng.p; M.log_cap = log_cap;
     {
-        const u64 bk_cap = log_cap / 32 + (u64)(SORT_MAX_BK + 1) * 64 + 1024;
+        u64 bk_cap = log_cap / 32 + (u64)(SORT_MAX_BK + 1) * 64 + 1024;
+        // (test knob: a smaller pool of bucket offsets runs out within the run, and the later slices stay unsorted)
+        if (const char *e = getenv("BPE_MERGE_SORTPOOL")) bk_cap = std::min<u64>(bk_cap, std::max<u64>(1, strtoull(e, nullptr, 10)));
         BPE_TRY(alloc_exact(ctx, B.log2, log_cap * sizeof(Rec))); BPE_TRY(alloc_exact(ctx, B.bk_lg, ((u64)n_merges + 2) * 4));
         BPE_TRY(alloc_exact(ctx, B.bk_start, ((u64)n_merges + 2) * 8)); BPE_TRY(alloc_exact(ctx, B.bk_off, bk_cap * 4));
         BPE_TRY(alloc_exact(ctx, B.bk_scratch, (u64)4 * SORT_MAX_BK * 4));
@@ -1321,7 +1323,7 @@ static int run_merges(bpe_ctx *ctx, const uint8_t *sp_blob, const u32 *sp_offs, 
     BPE_TRY(alloc_exact(ctx, B.bar, bar_bytes));
     M.bar = (BarSlot *)B.bar.p; M.bar_ctr = (u32 *)(M.bar + MG_MAX_CTAS);
     u64 ctr[MG_CTR_WORDS] = {0};
-    u64 keys_created = 0;
+    static const bool verbose = getenv("BPE_MERGE_VERBOSE") != nullptr;
     M.stop_at = n_merges;
     for (int round = 0; n_merges > 0 && round < 64; round++) {
         CUDA_TRY(ctx, cudaMemcpyToSymbolAsync(cM, &M, sizeof(M), 0, cudaMemcpyHostToDevice, st));
@@ -1341,29 +1343,25 @@ static int run_merges(bpe_ctx *ctx, const uint8_t *sp_blob, const u32 *sp_offs, 
         CUDA_TRY(ctx, cudaStreamSynchronize(st));
         for (int i = 0; i < MG_CTR_WORDS; i++) ctr[i] = host[i];
         if (ctr[3] != MG_NEED_GROW) break;                            // done, pair table ran empty (train.py:184-185), or error
-        // grow x4 and re-insert the live keys; the pending pops (the last step's winners) are applied by dropping those keys
-        keys_created += ctr[2];
+        // grow x4: the new table holds the same keys with the same counts (k_pairs_rehash); the counters carry over, the pending
+        // pops (the last step's winners) included, and the relaunch rescans every block
         DevBuf okey = B.pkey, ocnt = B.pcnt;
         u64 ocap = M.pcap;
         B.pkey = DevBuf(); B.pcnt = DevBuf();
         int rc = alloc_pair_table(ocap * 4);
         if (rc != BPE_OK) { bpe_buf_free(ctx, okey); bpe_buf_free(ctx, ocnt); return rc; }
-        PendingPops pending;
-        pending.n = (u32)std::min<u64>(ctr[6], MG_BATCH);
-        for (u32 i = 0; i < MG_BATCH; i++) pending.key[i] = i < pending.n ? ctr[MG_CTR_PENDING + i] : PAIR_EMPTY;
-        host[2] = 0; host[3] = 0; host[5] = 0; host[6] = 0;
-        CUDA_TRY(ctx, cudaMemcpyAsync((u64 *)B.ctr.p + 2, host + 2, 16, cudaMemcpyHostToDevice, st));
-        CUDA_TRY(ctx, cudaMemcpyAsync((u64 *)B.ctr.p + 5, host + 5, 16, cudaMemcpyHostToDevice, st));
+        if (verbose) fprintf(stderr, "  [pair table: %llu -> %llu slots at merge %llu, %llu keys]\n", (unsigned long long)ocap,
+                             (unsigned long long)M.pcap, (unsigned long long)ctr[1], (unsigned long long)ctr[2]);
+        host[3] = 0;
+        CUDA_TRY(ctx, cudaMemcpyAsync((u64 *)B.ctr.p + 3, host + 3, 8, cudaMemcpyHostToDevice, st));
         ctr[3] = 0;
         unsigned rg = (unsigned)std::min<u64>((u64)ctx->sm_count * bpe_grid_mult(64), (ocap + 255) / 256);
         CUDA_TRY(ctx, cudaMemcpyToSymbolAsync(cM, &M, sizeof(M), 0, cudaMemcpyHostToDevice, st));
-        KLAUNCH(k_pairs_rehash, rg, 256, 0, st, (const u64 *)okey.p, (const i64 *)ocnt.p, ocap, pending);
+        KLAUNCH(k_pairs_rehash, rg, 256, 0, st, (const u64 *)okey.p, (const i64 *)ocnt.p, ocap);
         CUDA_TRY(ctx, cudaGetLastError());
         CUDA_TRY(ctx, cudaStreamSynchronize(st));
         bpe_buf_free(ctx, okey); bpe_buf_free(ctx, ocnt);
     }
-    keys_created += ctr[2];
-    ctr[2] = keys_created;
     int ev_merge1 = tm.mark();
     CUDA_TRY(ctx, cudaMemcpyAsync(g_merge_prof, B.prof.p, 256, cudaMemcpyDeviceToHost, st));
     if (M.cta_prof) {
