@@ -208,7 +208,33 @@ int bpe_encode(bpe_tok *tok, const uint8_t *text_host, uint64_t n, int out_dtype
  * token (the boundary byte between documents must occur in none).  bpe_tok_saw_cr afterwards: a '\r' in any document. */
 int bpe_encode_batch(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
                      int out_dtype, void *out, uint64_t cap, uint64_t *n_out, uint64_t *id_offs_out, bpe_encode_stats *stats);
-/* 1 if the text of the last bpe_encode / bpe_encode_dev / bpe_encode_batch call on this tokenizer's context held a carriage return (the flags kernel
+/* BPE-dropout (subword regularisation, Provilkov et al. 2020): bpe_encode / bpe_encode_batch where every pretoken occurrence gets its
+ * own random segmentation.  Same two-call idiom (out == NULL reports the same *n_out), dtypes, errors, error details and
+ * bpe_tok_saw_cr as the deterministic calls; BPE_ERR_ARG when p is outside [0, 1] or NaN.  The result is a pure function of
+ * (tokenizer, text, document split, p, seed): it does not depend on the pretoken cache or on how the library cuts the text.
+ *   mix(z): z += 0x9E3779B97F4A7C15; z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9; z = (z ^ (z >> 27)) * 0x94D049BB133111EB;
+ *           return z ^ (z >> 31)                                                         (splitmix64 finalizer, all mod 2^64)
+ *   u(seed, doc, off, t) = mix(mix(mix(mix(seed) ^ doc) ^ off) ^ t)
+ *   thr(p) = 2^32 if p == 1 else floor(p * 2^32)
+ *   dropped = (u(seed, doc, off, t) >> 32) < thr(p)
+ * doc = the document's index (0 for bpe_encode_dropout), off = byte offset in that document of the first byte of the candidate pair's
+ * left token, t = the 0-based merge round within the pretoken occurrence.  BPE of one occurrence (the merge loop of
+ * models/tokenizer/tokenizer.py:92-109,124-136 with candidates removed at random):
+ *   tokens = the pretoken's bytes; t = 0
+ *   loop: cand = { i : (tokens[i], tokens[i+1]) has a merge rank and not dropped(seed, doc, off_i, t) }
+ *         if cand is empty: stop
+ *         r = min rank over cand; scan i left to right: if i in cand and rank(i) == r: merge i, i+1 and i += 2, else i += 1
+ *         t += 1
+ *   ids = vocab_inv[token] for each token (a missing token is BPE_ERR_KEY, as in tokenizer.py:135)
+ * Special-token occurrences are one id and never split.  p = 0 gives exactly bpe_encode / bpe_encode_batch; p = 1 gives every
+ * pretoken as single bytes.  Dropout can emit tokens deterministic BPE never does, so with a vocabulary that lacks an intermediate
+ * merge product one of the two calls can raise a KeyError the other does not. */
+int bpe_encode_dropout(bpe_tok *tok, const uint8_t *text_host, uint64_t n, double p, uint64_t seed, int out_dtype,
+                       void *out, uint64_t cap, uint64_t *n_out, bpe_encode_stats *stats);
+int bpe_encode_batch_dropout(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
+                             double p, uint64_t seed, int out_dtype, void *out, uint64_t cap, uint64_t *n_out,
+                             uint64_t *id_offs_out, bpe_encode_stats *stats);
+/* 1 if the text of the last bpe_encode* call on this tokenizer's context held a carriage return (the flags kernel
  * sees every byte anyway).  Tokenizer.encode takes a str and keeps '\r' as it is; a caller that reads a FILE in text mode, like the
  * reference's bulk driver (models/tokenizer/encode.py:31-34, universal newlines), uses this instead of scanning the text on the host:
  * it translates and encodes the piece again in the rare case. */

@@ -13,6 +13,8 @@
 //   3. k_enc_bpe_short / k_enc_bpe   the queued (new unique) pretokens: the merges in rank order through the pair -> rank table
 //                     (repeatedly the lowest-ranked adjacent pair, all its non-overlapping occurrences left to right); one thread
 //                     per pretoken of <= 32 bytes, one warp per longer one
+//   (bpe_encode_dropout / bpe_encode_batch_dropout only: k_enc_drop_starts, k_enc_drop_short / k_enc_drop_warp replace the value of
+//                     every occurrence whose segmentation can change with its own BPE-dropout result, bypassing the cache)
 //   4. k_enc_scan_emit  tokens per pretoken -> exclusive offsets -> ids scattered to the uint16 / int32 output, in one
 //                     pass (single-pass scan with decoupled look-back)
 // The reference re-runs BPE for every occurrence (no memoisation, tokenizer.py:118-136); the result per
@@ -760,6 +762,189 @@ __global__ void __launch_bounds__(SE_NT) k_enc_scan_emit(EncTables t, const u64 
     }
 }
 
+// ---- BPE-dropout (bpe_encode_dropout / bpe_encode_batch_dropout): every pretoken occurrence gets its own random BPE ----------
+// Spec (include/bpe_sm100.h): candidate pair (i, i+1) of merge round t is dropped when (u(seed, doc, off_i, t) >> 32) < thr, with
+// u = mix(mix(mix(mix(seed) ^ doc) ^ off) ^ t), mix = the splitmix64 finalizer, off_i = byte offset in the document of token i's first
+// byte.  The round takes the lowest rank among the pairs that are left and merges, left to right and non-overlapping, exactly those of
+// its occurrences that were not dropped.  The result depends on the occurrence, so it never goes to the cache: the stage runs after the
+// cache BPE kernels and replaces vals[ordinal] of the batch, with ids (when they do not fit the value) in the id pool's unused tail.
+struct EncDrop {
+    u64 thr;                                     // 0 < thr <= 2^32
+    u64 seed_mix;                                // mix(seed)
+    u64 lo;                                      // where the chunk starts in the caller's text
+    const u64 *doffs; u64 da;                    // bpe_encode_batch: the caller's document offsets, the chunk's first document (else null, 0)
+    const u32 *skip;                             // special-token starts and document boundaries (or null): their values stay
+    const u64 *starts;                           // byte offset in the arena of every pretoken of the batch
+    u32 *loff;                                   // per byte from the batch start: token offsets of the warp kernel's pretokens
+    u64 ibase;                                   // id pool offset of the batch start's scratch (one id per byte)
+};
+
+__device__ __forceinline__ u64 splitmix64(u64 z) {
+    z += 0x9E3779B97F4A7C15ull;
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    return z ^ (z >> 31);
+}
+__device__ __forceinline__ bool drop_pair(u64 thr, u64 h_doc, u64 off, u32 round) {
+    return (splitmix64(splitmix64(h_doc ^ off) ^ round) >> 32) < thr;
+}
+// mix(mix(seed) ^ doc) and the offset in its document of the pretoken at arena byte p
+__device__ __forceinline__ void drop_doc(const EncTables &t, const EncDrop &d, u64 p, u64 *h_doc, u64 *off) {
+    if (!d.doffs) { *h_doc = splitmix64(d.seed_mix); *off = d.lo + p; return; }
+    const u64 w = p >> 5;
+    u64 j = t.bpre[w >> 4];                      // boundaries before p: before its 512-byte group, then the words of the group
+    for (u64 k = w & ~15ull; k < w; k++) j += __popc(t.bmask[k]);
+    j += __popc(t.bmask[w] & ((1u << (p & 31)) - 1u));
+    *h_doc = splitmix64(d.seed_mix ^ (d.da + j));
+    *off = d.lo + p - j - d.doffs[d.da + j];     // (arena -> caller position: minus the boundary bytes before it)
+}
+
+// starts[ordinal - ord0] = arena offset of every pretoken starting in flag words [w_lo, w_hi)
+__global__ void __launch_bounds__(256) k_enc_drop_starts(const u32 *__restrict__ flags, const u64 *__restrict__ pre, u64 ord0, u64 w_lo, u64 w_hi,
+                                                        u64 *__restrict__ starts) {
+    for (u64 w = w_lo + (u64)blockIdx.x * blockDim.x + threadIdx.x; w < w_hi; w += (u64)gridDim.x * blockDim.x) {
+        u32 bits = flags[w];
+        if (!bits) continue;
+        u64 o = pre[w >> 4] - ord0;
+        for (u64 k = w & ~15ull; k < w; k++) o += __popc(flags[k]);
+        while (bits) { const u32 j = __ffs(bits) - 1; bits &= bits - 1; starts[o++] = w * 32 + j; }
+    }
+}
+
+// One thread per occurrence of <= 32 bytes (the row layout of k_enc_bpe_short, plus each token's byte offset); longer ones that need
+// redoing are queued (t.todo, count in ctr[10]) for k_enc_drop_warp.  An occurrence keeps its cached value when it is a special token or
+// a document boundary, or when that value already has one token per byte: no pair had a rank, and dropout only removes candidates.
+__global__ void __launch_bounds__(BPT_NT) k_enc_drop_short(EncTables t, EncDrop d, const u32 *__restrict__ flags, u64 n, u64 base, u64 bound,
+                                                          u64 *__restrict__ vals) {
+    __shared__ u32 s_sym[BPT_NT][BPT_MAX + 1];
+    __shared__ u32 s_rk[BPT_NT][BPT_MAX + 1];
+    __shared__ uint8_t s_off[BPT_NT][BPT_MAX + 1];
+    u32 *sym = s_sym[threadIdx.x], *rk = s_rk[threadIdx.x];
+    uint8_t *to = s_off[threadIdx.x];
+    for (u64 q = (u64)blockIdx.x * blockDim.x + threadIdx.x; q < bound; q += (u64)gridDim.x * blockDim.x) {
+        u64 v = vals[q];
+        if (VAL_TAG(v) == VAL_DOC) continue;
+        const u64 p = d.starts[q];
+        if (d.skip && ((d.skip[p >> 5] >> (p & 31)) & 1u)) continue;
+        const u64 e = q + 1 < bound ? d.starts[q + 1] : flags_next_start(flags, p + 1, n);
+        const u32 len = (u32)(e - p);
+        if (VAL_TAG(v) == VAL_FWD) v = enc_value(t, (u32)v);
+        if (VAL_TAG(v) != VAL_ERR && value_count(v) == len) continue;
+        if (len > BPT_MAX) { const u64 k = atomicAdd(&t.ctr[10], 1ull); t.todo[k] = (u32)q; continue; }
+        u64 h_doc, off0;
+        drop_doc(t, d, p, &h_doc, &off0);
+        u32 nt = len;
+        for (u32 i = 0; i < nt; i++) { sym[i] = t.text[p + i]; to[i] = (uint8_t)i; }
+        for (u32 i = 0; i + 1 < nt; i++) rk[i] = (u32)(rank_lookup(t, sym[i], sym[i + 1]) >> 32);
+        for (u32 round = 0; nt > 1; round++) {
+            // lowest rank among the pairs this round keeps; cand = the kept ones
+            u32 best = 0xFFFFFFFFu, cand = 0;
+            for (u32 i = 0; i + 1 < nt; i++) {
+                if (rk[i] == 0xFFFFFFFFu || drop_pair(d.thr, h_doc, off0 + to[i], round)) continue;
+                cand |= 1u << i;
+                if (rk[i] < best) best = rk[i];
+            }
+            if (best == 0xFFFFFFFFu) break;
+            u32 bi = __ffs(cand & ~0u) - 1;
+            while (rk[bi] != best) { cand &= ~(1u << bi); bi = __ffs(cand) - 1; }
+            const u32 res = (u32)rank_lookup(t, sym[bi], sym[bi + 1]);
+            u32 o = 0, merged = 0;
+            for (u32 i = 0; i < nt; o++) {
+                if (i + 1 < nt && ((cand >> i) & 1u) && rk[i] == best) { sym[o] = res; to[o] = to[i]; merged |= 1u << o; i += 2; }
+                else { sym[o] = sym[i]; rk[o] = rk[i]; to[o] = to[i]; i += 1; }
+            }
+            nt = o;
+            for (u32 i = 0; i + 1 < nt; i++)
+                if ((merged >> i) & 3u) rk[i] = (u32)(rank_lookup(t, sym[i], sym[i + 1]) >> 32);
+        }
+        u64 value = 0;
+        bool bad = false, big = false;
+        for (u32 i = 0; i < nt && !bad; i++) {
+            const int32_t id = t.sym_to_id[sym[i]];
+            if (id < 0) { bad = true; value = (VAL_ERR << 60) | sym[i]; }
+            else { big |= (u32)id >= INLINE_ID_LIMIT; rk[i] = (u32)id; }
+        }
+        if (!bad) {
+            if (nt <= 3 && !big) {
+                value = (u64)nt << 60;
+                if (nt > 0) value |= (u64)rk[0];
+                if (nt > 1) value |= (u64)rk[1] << 20;
+                if (nt > 2) value |= (u64)rk[2] << 40;
+            } else {
+                const u64 io = d.ibase + (p - base);
+                for (u32 i = 0; i < nt; i++) t.ipool[io + i] = rk[i];
+                value = (VAL_EXT << 60) | (io << 24) | nt;
+            }
+        }
+        vals[q] = value;
+    }
+}
+
+// The queued occurrences of > 32 bytes: one warp each, symbols in place in the id pool scratch, token offsets beside them in d.loff
+// (the long path of k_enc_bpe with the dropped candidates taken out of the minimum and of the merge).
+__global__ void __launch_bounds__(256) k_enc_drop_warp(EncTables t, EncDrop d, const u32 *__restrict__ flags, u64 n, u64 base, u64 bound,
+                                                      u64 *__restrict__ vals) {
+    const u32 lane = lane_id();
+    const u64 gwarp = ((u64)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = ((u64)gridDim.x * blockDim.x) >> 5;
+    const u64 n_q = t.ctr[10];
+    for (u64 k = gwarp; k < n_q; k += nwarps) {
+        const u64 q = t.todo[k];
+        const u64 p = d.starts[q];
+        const u64 e = q + 1 < bound ? d.starts[q + 1] : flags_next_start(flags, p + 1, n);
+        const u32 len = (u32)(e - p);
+        u64 h_doc, off0;
+        drop_doc(t, d, p, &h_doc, &off0);
+        const u64 io = d.ibase + (p - base);
+        u32 *w = t.ipool + io, *to = d.loff + (p - base);
+        for (u32 i = lane; i < len; i += 32) { w[i] = t.text[p + i]; to[i] = i; }
+        __syncwarp();
+        u32 nt = len;
+        for (u32 round = 0; nt > 1; round++) {
+            u64 best = RANK_NONE;
+            for (u32 b0 = 0; b0 + 1 < nt; b0 += 32) {
+                const u32 i = b0 + lane;
+                if (i + 1 < nt) {
+                    const u64 r = rank_lookup(t, w[i], w[i + 1]);
+                    if (r < best && !drop_pair(d.thr, h_doc, off0 + to[i], round)) best = r;
+                }
+            }
+            best = warp_min_u64(best);
+            if (best == RANK_NONE) break;
+            const u32 j = (u32)(best >> 32), res = (u32)best;
+            const u32 a = (u32)t.mpairs[2 * j], b = (u32)t.mpairs[2 * j + 1];
+            u32 out = 0, carry = 0;
+            for (u32 b0 = 0; b0 < nt; b0 += 32) {
+                const u32 i = b0 + lane;
+                const u32 cur = i < nt ? w[i] : 0xFFFFFFFFu, nx = i + 1 < nt ? w[i + 1] : 0xFFFFFFFFu, ci = i < nt ? to[i] : 0u;
+                const bool hit = cur == a && nx == b && !drop_pair(d.thr, h_doc, off0 + ci, round);
+                const u32 m = __ballot_sync(0xffffffffu, hit);
+                const u32 heads = resolve_heads_same(m, carry);      // (left to right, non-overlapping: only (a, a) can overlap)
+                const u32 valid = __ballot_sync(0xffffffffu, i < nt);
+                const u32 kept = valid & ~((heads << 1) | carry);
+                carry = heads >> 31;
+                const u32 val = ((heads >> lane) & 1u) ? res : cur;
+                const u32 pos = out + __popc(kept & ((1u << lane) - 1u));
+                __syncwarp();
+                if ((kept >> lane) & 1u) { w[pos] = val; to[pos] = ci; }
+                out += __popc(kept);
+                __syncwarp();
+            }
+            nt = out;
+        }
+        u32 bad_idx = 0xFFFFFFFFu;
+        for (u32 i = lane; i < nt; i += 32) if (t.sym_to_id[w[i]] < 0 && i < bad_idx) bad_idx = i;
+        for (int dd = 16; dd; dd >>= 1) { const u32 o = __shfl_xor_sync(0xffffffffu, bad_idx, dd); bad_idx = o < bad_idx ? o : bad_idx; }
+        u64 value;
+        if (bad_idx != 0xFFFFFFFFu) value = (VAL_ERR << 60) | w[bad_idx];
+        else {
+            for (u32 i = lane; i < nt; i += 32) w[i] = (u32)t.sym_to_id[w[i]];
+            value = (VAL_EXT << 60) | (io << 24) | nt;
+        }
+        __syncwarp();
+        if (lane == 0) vals[q] = value;
+    }
+}
+
 // ---- hot table: histogram of the sampled hit counts, build ----------------------------------------------------------
 #define ENC_HOT_HIST 64
 __global__ void __launch_bounds__(256) k_enc_hot_hist(EncTables t, u64 *__restrict__ hist /* [ENC_HOT_HIST] */) {
@@ -982,6 +1167,7 @@ struct bpe_tok {
     u64 hot_nb = 0;
     bool hot_built = false, sampling = false;
     std::vector<uint8_t> key_error;              // bytes of the last KeyError key
+    DevBuf drop;                                 // BPE-dropout scratch of a batch: pretoken offsets, token offsets of long pretokens
     int doc_sep = -1;                            // boundary byte of bpe_encode_batch (-1: every candidate occurs in a special)
 };
 
@@ -1240,7 +1426,7 @@ BPE_API void bpe_tok_destroy(bpe_tok *tok) {
     if (!tok) return;
     if (tok->ctx) { cudaSetDevice(tok->ctx->device); cudaStreamSynchronize(tok->ctx->stream); }
     for (DevBuf *b : {&tok->mtab, &tok->mpairs, &tok->sym_to_id, &tok->vlen, &tok->voff, &tok->vblob, &tok->sp_offs, &tok->sp_ids,
-                      &tok->stab, &tok->medtab, &tok->ltab, &tok->kpool, &tok->ipool, &tok->todo, &tok->ctr, &tok->hot, &tok->samp, &tok->sm_img})
+                      &tok->stab, &tok->medtab, &tok->ltab, &tok->kpool, &tok->ipool, &tok->todo, &tok->ctr, &tok->hot, &tok->samp, &tok->sm_img, &tok->drop})
         bpe_buf_free(tok->ctx, *b);
     delete tok;
 }
@@ -1271,8 +1457,9 @@ struct DocBounds { const u32 *bmask; u64 *id_offs; u64 id_base; };
 
 // Encode the n bytes in the context's text arena into out_dev (device pointer, may be null: count only).
 // *n_out = number of tokens (may exceed dev_cap; only dev_cap are written).  stats, when given, are ADDED to.
+// drop (BPE-dropout, or null): its thr, seed_mix, lo, doffs and da; the rest is filled in per batch.
 static int encode_core(bpe_tok *tok, u64 n, int out_dtype, void *out_dev, u64 dev_cap, uint64_t *n_out, bpe_encode_stats *stats,
-                       const DocBounds *docs = nullptr) {
+                       const DocBounds *docs = nullptr, const EncDrop *drop = nullptr) {
     bpe_ctx *ctx = tok->ctx;
     cudaStream_t st = ctx->stream;
     *n_out = 0;
@@ -1396,6 +1583,27 @@ static int encode_core(bpe_tok *tok, u64 n, int out_dtype, void *out_dev, u64 de
             CUDA_TRY(ctx, cudaGetLastError());
         }
         if (tok->sampling) BPE_TRY(cache_build_hot(tok));
+        if (drop && bound) {                     // BPE-dropout: every occurrence's own BPE replaces its cached value
+            BPE_TRY(cache_read_ctr(tok, c, 6));  // id pool cursor after the cache BPE: the batch's id scratch starts there
+            const u64 span = std::min<u64>(n - base, bytes + MAX_TOKEN_LEN);      // (the batch's last pretoken may run past its end)
+            BPE_TRY(grow_keep(ctx, tok->ipool, (c[5] + span) * 4, c[5] * 4));
+            t.ipool = (u32 *)tok->ipool.p;
+            const size_t starts_b = round_up(bound * 8, 256);
+            BPE_TRY(bpe_buf_reserve(ctx, tok->drop, starts_b + span * 4));
+            EncDrop d = *drop;
+            d.skip = tok->n_sp > 0 && spmax > 0 ? (const u32 *)ctx->spstart.p : docs ? docs->bmask : nullptr;
+            d.starts = (const u64 *)tok->drop.p;
+            d.loff = (u32 *)((uint8_t *)tok->drop.p + starts_b);
+            d.ibase = c[5];
+            CUDA_TRY(ctx, cudaMemsetAsync((u64 *)tok->ctr.p + 10, 0, 8, st));
+            const unsigned gmax = (unsigned)((u64)ctx->sm_count * bpe_grid_mult(64));
+            KLAUNCH(k_enc_drop_starts, (unsigned)std::min<u64>(gmax, (b_hi - b_lo + 255) / 256), 256, 0, st, (const u32 *)ctx->flags.p, pre, ord[b],
+                    b_lo, b_hi, (u64 *)tok->drop.p);
+            KLAUNCH(k_enc_drop_short, (unsigned)std::min<u64>(gmax, (bound + BPT_NT - 1) / BPT_NT), BPT_NT, 0, st, t, d, (const u32 *)ctx->flags.p,
+                    n, base, bound, vals);
+            KLAUNCH(k_enc_drop_warp, (unsigned)ctx->sm_count * 8, 256, 0, st, t, d, (const u32 *)ctx->flags.p, n, base, bound, vals);
+            CUDA_TRY(ctx, cudaGetLastError());
+        }
         CUDA_TRY(ctx, cudaEventRecord(evs[2], st));
         // tokens per pretoken -> offsets -> ids, one pass
         u64 *host = (u64 *)ctx->pinned;
@@ -1581,8 +1789,10 @@ static std::vector<EncChunk> doc_chunks(const bpe_tok *tok, const uint8_t *t, u6
 //   bpe_encode:       a chunk is uploaded straight into the arena the kernels read next (the two arenas alternate)
 //   bpe_encode_batch: a chunk is uploaded as it is into one of two staging buffers; on the compute stream k_enc_expand_docs moves it
 //                     into the arena with a boundary byte after every document and sets the boundary bitmask
+// drop: BPE-dropout (thr and seed_mix set), or null.
 static int encode_pipeline(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs, uint64_t n_docs, int out_dtype,
-                           void *out, uint64_t cap, uint64_t *n_out, uint64_t *id_offs_out, bpe_encode_stats *stats) {
+                           void *out, uint64_t cap, uint64_t *n_out, uint64_t *id_offs_out, bpe_encode_stats *stats,
+                           const EncDrop *drop = nullptr) {
     BPE_TRY(encode_check_args(tok, text_host, n, out_dtype, n_out));
     bpe_ctx *ctx = tok->ctx;
     cudaStream_t st = ctx->stream;
@@ -1656,6 +1866,9 @@ static int encode_pipeline(bpe_tok *tok, const uint8_t *text_host, uint64_t n, c
             odev = obuf[cur]->p;
         }
         uint64_t nt = 0;
+        EncDrop dch{};                           // the chunk's place in the caller's text, for the dropout offsets
+        if (drop) { dch = *drop; dch.lo = ch.lo; dch.da = ch.da; dch.doffs = doc_offs ? (const u64 *)ctx->doc_offs.p : nullptr; }
+        const EncDrop *dp = drop ? &dch : nullptr;
         if (doc_offs) {
             const u64 nb = ch.db - ch.da, an = len + nb;            // a boundary byte after each document that ends here
             rc = ctx_prepare_arena(ctx, ctx->text, an);
@@ -1667,7 +1880,7 @@ static int encode_pipeline(bpe_tok *tok, const uint8_t *text_host, uint64_t n, c
                     (uint8_t *)ctx->text.p + BPE_PAD, (u32 *)ctx->doc_bmask.p, (uint8_t)tok->doc_sep);
             CUDA_TRY(ctx, cudaGetLastError());
             const DocBounds db{(const u32 *)ctx->doc_bmask.p, id_dev + ch.da + 1, total};
-            rc = encode_core(tok, an, out_dtype, odev, len, &nt, stats, &db);
+            rc = encode_core(tok, an, out_dtype, odev, len, &nt, stats, &db, dp);
             if (rc == BPE_ERR_UTF8 || rc == BPE_ERR_KEY) {      // arena offset -> offset in the caller's text: minus the boundaries before it
                 const u64 p = (u64)ctx->err_detail;
                 u64 a = 0, b = nb;                              // boundaries j < a lie before p (boundary j sits at ends[j] - lo + j)
@@ -1679,7 +1892,7 @@ static int encode_pipeline(bpe_tok *tok, const uint8_t *text_host, uint64_t n, c
             }
             if (rc != BPE_OK) break;
         } else {
-            rc = encode_core(tok, len, out_dtype, odev, len, &nt, stats);
+            rc = encode_core(tok, len, out_dtype, odev, len, &nt, stats, nullptr, dp);
             if (swap) std::swap(ctx->text, ctx->text_alt);
             if (rc != BPE_OK) { ctx->err_detail += (int64_t)ch.lo; break; }
         }
@@ -1715,8 +1928,9 @@ BPE_API int bpe_encode(bpe_tok *tok, const uint8_t *text_host, uint64_t n, int o
     return encode_pipeline(tok, text_host, n, nullptr, 0, out_dtype, out, cap, n_out, nullptr, stats);
 }
 
-BPE_API int bpe_encode_batch(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
-                             int out_dtype, void *out, uint64_t cap, uint64_t *n_out, uint64_t *id_offs_out, bpe_encode_stats *stats) {
+static int encode_batch_impl(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
+                             int out_dtype, void *out, uint64_t cap, uint64_t *n_out, uint64_t *id_offs_out, bpe_encode_stats *stats,
+                             const EncDrop *drop) {
     if (!tok || !n_out || !id_offs_out || (n_docs && !doc_offs_host)) return BPE_ERR_ARG;
     bpe_ctx *ctx = tok->ctx;
     for (uint64_t j = 0; j < n_docs; j++)
@@ -1731,7 +1945,42 @@ BPE_API int bpe_encode_batch(bpe_tok *tok, const uint8_t *text_host, uint64_t n,
         id_offs_out[0] = 0;
         return BPE_OK;
     }
-    return encode_pipeline(tok, text_host, n, doc_offs_host, n_docs, out_dtype, out, cap, n_out, id_offs_out, stats);
+    return encode_pipeline(tok, text_host, n, doc_offs_host, n_docs, out_dtype, out, cap, n_out, id_offs_out, stats, drop);
+}
+
+BPE_API int bpe_encode_batch(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
+                             int out_dtype, void *out, uint64_t cap, uint64_t *n_out, uint64_t *id_offs_out, bpe_encode_stats *stats) {
+    return encode_batch_impl(tok, text_host, n, doc_offs_host, n_docs, out_dtype, out, cap, n_out, id_offs_out, stats, nullptr);
+}
+
+// BPE-dropout: thr(p) = 2^32 for p = 1, else floor(p * 2^32) (exact in binary64); p outside [0, 1] or NaN is BPE_ERR_ARG.
+// p = 0 drops nothing: the deterministic pipeline runs.
+static int dropout_args(bpe_tok *tok, double p, uint64_t seed, EncDrop *d) {
+    if (!(p >= 0.0 && p <= 1.0)) return tok ? bpe_set_error(tok->ctx, BPE_ERR_ARG, "dropout probability must be in [0, 1]") : BPE_ERR_ARG;
+    memset(d, 0, sizeof(*d));
+    d->thr = p == 1.0 ? (1ull << 32) : (u64)(p * 4294967296.0);
+    u64 z = seed + 0x9E3779B97F4A7C15ull;        // mix(seed), as splitmix64 on the device
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    d->seed_mix = z ^ (z >> 31);
+    return BPE_OK;
+}
+
+BPE_API int bpe_encode_dropout(bpe_tok *tok, const uint8_t *text_host, uint64_t n, double p, uint64_t seed, int out_dtype, void *out,
+                               uint64_t cap, uint64_t *n_out, bpe_encode_stats *stats) {
+    if (!tok) return BPE_ERR_ARG;
+    EncDrop d;
+    BPE_TRY(dropout_args(tok, p, seed, &d));
+    return encode_pipeline(tok, text_host, n, nullptr, 0, out_dtype, out, cap, n_out, nullptr, stats, d.thr ? &d : nullptr);
+}
+
+BPE_API int bpe_encode_batch_dropout(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
+                                     double p, uint64_t seed, int out_dtype, void *out, uint64_t cap, uint64_t *n_out,
+                                     uint64_t *id_offs_out, bpe_encode_stats *stats) {
+    if (!tok) return BPE_ERR_ARG;
+    EncDrop d;
+    BPE_TRY(dropout_args(tok, p, seed, &d));
+    return encode_batch_impl(tok, text_host, n, doc_offs_host, n_docs, out_dtype, out, cap, n_out, id_offs_out, stats, d.thr ? &d : nullptr);
 }
 
 BPE_API int bpe_encode_dev(bpe_tok *tok, const uint8_t *text_dev, uint64_t n, int out_dtype, void *out_dev, uint64_t cap, uint64_t *n_out,

@@ -1,6 +1,6 @@
 """Tokenizer host: mirrors models/tokenizer/tokenizer.py:11-167 of the reference.
 
-    Tokenizer(vocab, merges, special_tokens).encode(str) -> list[int]
+    Tokenizer(vocab, merges, special_tokens).encode(str, *, dropout=0.0, seed=0) -> list[int]
                                             .encode_batch(Sequence[str]) -> list[list[int]]
                                             .encode_iterable(Iterable[str]) -> Iterator[int]
                                             .decode(list[int]) -> str
@@ -48,6 +48,16 @@ def _pack_documents(texts: list) -> Tuple[np.ndarray, np.ndarray, UnicodeEncodeE
     offs = np.zeros(lens.size + 1, dtype=np.uint64)
     np.cumsum(lens, out=offs[1:])
     return np.frombuffer(b"".join(parts), dtype=np.uint8), offs, bad
+
+
+def _check_dropout(dropout, seed) -> Tuple[float, int]:
+    """BPE-dropout arguments: a probability in [0, 1] and a seed in [0, 2**64)."""
+    p = float(dropout)
+    if not 0.0 <= p <= 1.0:                      # (also rejects NaN)
+        raise ValueError("dropout must be a probability in [0, 1], got %r" % (dropout,))
+    if isinstance(seed, bool) or not isinstance(seed, (int, np.integer)) or not 0 <= int(seed) < 2**64:
+        raise ValueError("seed must be an integer in [0, 2**64), got %r" % (seed,))
+    return p, int(seed)
 
 
 class Tokenizer:
@@ -178,8 +188,11 @@ class Tokenizer:
         ctx.check(rc)
 
     # ---- encode (tokenizer.py:111-138) -------------------------------------------------------------
-    def encode_to_numpy(self, data, dtype=np.int32) -> np.ndarray:
-        """Token ids of UTF-8 `data` (bytes / uint8 array) as a numpy array of `dtype` (uint16 or int32)."""
+    def encode_to_numpy(self, data, dtype=np.int32, *, dropout: float = 0.0, seed: int = 0) -> np.ndarray:
+        """Token ids of UTF-8 `data` (bytes / uint8 array) as a numpy array of `dtype` (uint16 or int32).  dropout > 0: BPE-dropout
+        (every pretoken occurrence merged with each candidate pair of each round dropped with that probability; a pure function of
+        the text, dropout and seed -- see bpe_encode_dropout in include/bpe_sm100.h)."""
+        dropout, seed = _check_dropout(dropout, seed)
         tok = self._device_tok()
         ctx = self._tok_ctx
         L = _lib.lib()
@@ -189,7 +202,11 @@ class Tokenizer:
         n_out = C.c_uint64(0)
         stats = _lib.EncodeStats()
         with ctx.lock:
-            rc = L.bpe_encode(tok, _lib.ptr(arr) if arr.size else None, arr.size, code, _lib.ptr(out), out.size, C.byref(n_out), C.byref(stats))
+            if dropout:
+                rc = L.bpe_encode_dropout(tok, _lib.ptr(arr) if arr.size else None, arr.size, dropout, seed, code, _lib.ptr(out), out.size,
+                                          C.byref(n_out), C.byref(stats))
+            else:
+                rc = L.bpe_encode(tok, _lib.ptr(arr) if arr.size else None, arr.size, code, _lib.ptr(out), out.size, C.byref(n_out), C.byref(stats))
             if rc != _lib.BPE_OK:
                 self._raise(ctx, rc, arr)
         self.last_stats = stats.as_dict()
@@ -212,28 +229,35 @@ class Tokenizer:
         self.last_saw_cr = bool(L.bpe_tok_saw_cr(tok))
         return int(n_out.value)
 
-    def encode(self, text: str) -> List[int]:
-        return self.encode_to_numpy(text.encode("utf-8"), np.int32).tolist()
+    def encode(self, text: str, *, dropout: float = 0.0, seed: int = 0) -> List[int]:
+        """Token ids of `text`; dropout > 0 samples a BPE-dropout segmentation (see encode_to_numpy)."""
+        dropout, seed = _check_dropout(dropout, seed)
+        return self.encode_to_numpy(text.encode("utf-8"), np.int32, dropout=dropout, seed=seed).tolist()
 
-    def encode_batch(self, texts: Sequence[str]) -> List[List[int]]:
+    def encode_batch(self, texts: Sequence[str], *, dropout: float = 0.0, seed: int = 0) -> List[List[int]]:
         """[self.encode(t) for t in texts] -- the same ids, split the same way, the same first exception -- with one device pass
-        over all documents (bpe_encode_batch) instead of one pipeline per document."""
-        ids, offs = self.encode_batch_to_numpy(texts, np.int32)
+        over all documents (bpe_encode_batch) instead of one pipeline per document.  With dropout > 0, document j is sampled as
+        document j of the batch: encode(d, dropout=p, seed=s) == encode_batch([d], dropout=p, seed=s)[0]."""
+        ids, offs = self.encode_batch_to_numpy(texts, np.int32, dropout=dropout, seed=seed)
         flat, o = ids.tolist(), offs.tolist()
         return [flat[o[j]: o[j + 1]] for j in range(len(o) - 1)]
 
-    def encode_batch_to_numpy(self, texts: Sequence[str | bytes], dtype=np.int32) -> Tuple[np.ndarray, np.ndarray]:
+    def encode_batch_to_numpy(self, texts: Sequence[str | bytes], dtype=np.int32, *, dropout: float = 0.0,
+                              seed: int = 0) -> Tuple[np.ndarray, np.ndarray]:
         """Ids of every document back to back (uint16 or int32) and int64 offsets (len(texts) + 1): document j's ids are
         ids[offsets[j]:offsets[j + 1]].  A `bytes` item must be UTF-8; it fails as item.decode("utf-8") would.  Where several
-        documents would fail, the error is that of the first one in list order, as in a loop over encode_to_numpy."""
+        documents would fail, the error is that of the first one in list order, as in a loop over encode_to_numpy.  dropout > 0:
+        BPE-dropout with the document's index in `texts` as its `doc` (bpe_encode_batch_dropout)."""
+        drop = _check_dropout(dropout, seed)
+        kw = {"drop": drop} if drop[0] else {}
         texts = list(texts)
         blob, offs, bad = _pack_documents(texts)
         if bad is not None:                      # a str that cannot be encoded: the documents before it fail first, if any does
-            self._encode_batch_packed(blob, offs, dtype)
+            self._encode_batch_packed(blob, offs, dtype, **kw)
             raise bad
-        return self._encode_batch_packed(blob, offs, dtype, texts)
+        return self._encode_batch_packed(blob, offs, dtype, texts, **kw)
 
-    def _encode_batch_packed(self, blob: np.ndarray, offs: np.ndarray, dtype, texts=None):
+    def _encode_batch_packed(self, blob: np.ndarray, offs: np.ndarray, dtype, texts=None, drop=(0.0, 0)):
         tok = self._device_tok()
         ctx = self._tok_ctx
         L = _lib.lib()
@@ -244,14 +268,18 @@ class Tokenizer:
         n_out = C.c_uint64(0)
         stats = _lib.EncodeStats()
         with ctx.lock:
-            rc = L.bpe_encode_batch(tok, _lib.ptr(blob) if blob.size else None, blob.size, _lib.ptr(offs), n_docs, code,
-                                    _lib.ptr(out), out.size, C.byref(n_out), _lib.ptr(id_offs), C.byref(stats))
+            if drop[0]:
+                rc = L.bpe_encode_batch_dropout(tok, _lib.ptr(blob) if blob.size else None, blob.size, _lib.ptr(offs), n_docs, drop[0], drop[1],
+                                                code, _lib.ptr(out), out.size, C.byref(n_out), _lib.ptr(id_offs), C.byref(stats))
+            else:
+                rc = L.bpe_encode_batch(tok, _lib.ptr(blob) if blob.size else None, blob.size, _lib.ptr(offs), n_docs, code,
+                                        _lib.ptr(out), out.size, C.byref(n_out), _lib.ptr(id_offs), C.byref(stats))
             detail = L.bpe_last_error_detail(ctx.handle)
             if rc == _lib.ERR_UTF8 and texts is not None:
                 # the device reports invalid UTF-8 in a chunk before a KeyError in it: the documents before the invalid one
                 # go first, then that document fails as its decode does
                 k = int(np.searchsorted(offs, detail, side="right")) - 1
-                self._encode_batch_packed(blob[: int(offs[k])], offs[: k + 1], dtype)
+                self._encode_batch_packed(blob[: int(offs[k])], offs[: k + 1], dtype, **({"drop": drop} if drop[0] else {}))
                 item = texts[k]
                 if isinstance(item, (bytes, bytearray, memoryview)):
                     bytes(item).decode("utf-8")
