@@ -48,6 +48,11 @@ def gpt2():
 def _texts():
     out = {name: (FIXTURES_PATH / name).read_bytes() for name in ["corpus.en", "tinystories_sample.txt", "german.txt"]}
     out["synth_owt"] = synth_host("owt", 3, 3 << 20).tobytes().decode("utf-8", errors="ignore").encode()
+    # pretokens at and around the row limits of the per-thread kernel (15 / 16 and 32 / 33 bytes) and long runs of one repeated
+    # byte for the per-warp kernel; joined by spaces, every part but the first is a pretoken one byte longer (" " + the part)
+    parts = ["a" * 33, "a" * 1000, " " * 777 + "x", "ab" * 500, "=" * 4097, "é" * 700, "x" * 32, "y" * 31, "z" * 64, "w" * 65,
+             "q" * 14, "r" * 15, "s" * 16]
+    out["long_pretokens"] = " ".join(parts).encode()
     return out
 
 

@@ -12,9 +12,10 @@
 //                     medium and long tables); unseen pretokens claim a slot there and are queued
 //   3. k_enc_bpe_short / k_enc_bpe   the queued (new unique) pretokens: the merges in rank order through the pair -> rank table
 //                     (repeatedly the lowest-ranked adjacent pair, all its non-overlapping occurrences left to right); one thread
-//                     per pretoken of <= 32 bytes, one warp per longer one
-//   (bpe_encode_dropout / bpe_encode_batch_dropout only: k_enc_drop_starts, k_enc_drop_short / k_enc_drop_warp replace the value of
-//                     every occurrence whose segmentation can change with its own BPE-dropout result, bypassing the cache)
+//                     per pretoken of <= 32 bytes (row_bpe), one warp per longer one (warp_bpe)
+//   (bpe_encode_dropout / bpe_encode_batch_dropout only: k_enc_drop_starts, then k_enc_drop_short / k_enc_drop_warp -- row_bpe and
+//                     warp_bpe with dropped candidates -- replace the value of every occurrence whose segmentation can change with its
+//                     own BPE-dropout result, bypassing the cache)
 //   4. k_enc_scan_emit  tokens per pretoken -> exclusive offsets -> ids scattered to the uint16 / int32 output, in one
 //                     pass (single-pass scan with decoupled look-back)
 // The reference re-runs BPE for every occurrence (no memoisation, tokenizer.py:118-136); the result per
@@ -400,7 +401,25 @@ __global__ void __launch_bounds__(LK_NT, 1) k_enc_lookup(EncTables t, const u32 
     lookup_drain(t, q, base, vals, lane, true);
 }
 
-// ---- BPE of the queued pretokens: one warp each ----------------------------------------------------------
+// ---- BPE of one pretoken: the rank loop, shared by the cache kernels and the BPE-dropout kernels -------------------------------
+// Repeatedly the lowest-ranked adjacent pair through the pair -> rank table (tokenizer.py:128-131), and every non-overlapping
+// occurrence of it, left to right (Tokenizer.merge, tokenizer.py:92-109).  Two forms: row_bpe, one thread over a shared-memory row
+// (pretokens of <= 32 bytes), and warp_bpe, one warp over the tokens in place in the id pool (longer ones).
+// DROP (BPE-dropout, spec below at EncDrop): a round also leaves out the candidate pairs that DropOcc::drops, takes the lowest rank
+// among the pairs that are left and merges exactly those of its occurrences; for that every token carries the byte offset of its
+// first byte in the occurrence (to[]).  The deterministic instances have neither the test nor the offsets.
+__device__ __forceinline__ u64 splitmix64(u64 z) {
+    z += 0x9E3779B97F4A7C15ull;
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    return z ^ (z >> 31);
+}
+struct DropOcc {                                 // BPE-dropout of one occurrence (see drop_occ)
+    u64 thr, h_doc, off0;                        // threshold, mix(mix(seed) ^ doc), the occurrence's byte offset in its document
+    // is the pair whose left token starts at byte o of the occurrence dropped in merge round `round`?
+    __device__ __forceinline__ bool drops(u64 o, u32 round) const { return (splitmix64(splitmix64(h_doc ^ (off0 + o)) ^ round) >> 32) < thr; }
+};
+
 __device__ __forceinline__ u64 warp_min_u64(u64 v) {
 #pragma unroll
     for (int d = 16; d; d >>= 1) { u64 o = __shfl_xor_sync(0xffffffffu, v, d); v = o < v ? o : v; }
@@ -418,27 +437,117 @@ __device__ __forceinline__ u32 resolve_heads_same(u32 m, u32 prev_head) {
     return heads;
 }
 
-__device__ __forceinline__ u64 make_value(const EncTables &t, u32 n, int32_t id, u32 sym, u32 lane) {
-    // n <= 32 tokens, lane i holds id / sym of token i
-    u32 bad = __ballot_sync(0xffffffffu, lane < n && id < 0);
-    if (bad) {
-        u32 first = __ffs(bad) - 1;
-        u32 s = __shfl_sync(0xffffffffu, sym, first);
-        return (VAL_ERR << 60) | s;
+// One thread: the n (<= 32) symbols in sym[], the ranks of the adjacent pairs kept up to date in rk[] (after a merge only the pairs
+// next to a merged token change).  Returns the number of tokens left in sym[].
+template <bool DROP>
+__device__ __forceinline__ u32 row_bpe(const EncTables &t, u32 *sym, u32 *rk, uint8_t *to, u32 n, const DropOcc &x) {
+    if constexpr (DROP) for (u32 i = 0; i < n; i++) to[i] = (uint8_t)i;
+    for (u32 i = 0; i + 1 < n; i++) rk[i] = (u32)(rank_lookup(t, sym[i], sym[i + 1]) >> 32);
+    for (u32 round = 0; n > 1; round++) {
+        // the lowest-ranked candidate pair; cand = the candidates (DROP only: otherwise every pair is one)
+        u32 best = 0xFFFFFFFFu, bi = 0, cand = 0;
+        for (u32 i = 0; i + 1 < n; i++) {
+            if constexpr (DROP) {
+                if (rk[i] == 0xFFFFFFFFu || x.drops(to[i], round)) continue;
+                cand |= 1u << i;
+            }
+            if (rk[i] < best) { best = rk[i]; bi = i; }
+        }
+        if (best == 0xFFFFFFFFu) break;
+        const u32 a = sym[bi], b = sym[bi + 1], res = (u32)rank_lookup(t, a, b);
+        // its candidates, left to right, non-overlapping (equal rank <=> same pair)
+        u32 o = 0, merged = 0;
+        for (u32 i = 0; i < n; o++) {
+            if (i + 1 < n && rk[i] == best && (!DROP || ((cand >> i) & 1u))) {
+                sym[o] = res; merged |= 1u << o;
+                if constexpr (DROP) to[o] = to[i];
+                i += 2;
+            } else {
+                sym[o] = sym[i]; rk[o] = rk[i];
+                if constexpr (DROP) to[o] = to[i];
+                i += 1;
+            }
+        }
+        n = o;
+        for (u32 i = 0; i + 1 < n; i++)
+            if ((merged >> i) & 3u) rk[i] = (u32)(rank_lookup(t, sym[i], sym[i + 1]) >> 32);
     }
-    u32 big = __ballot_sync(0xffffffffu, lane < n && (u32)id >= INLINE_ID_LIMIT);
-    if (n <= 3 && !big) {
-        u64 i0 = (u32)__shfl_sync(0xffffffffu, id, 0), i1 = (u32)__shfl_sync(0xffffffffu, id, 1), i2 = (u32)__shfl_sync(0xffffffffu, id, 2);
-        u64 v = (u64)n << 60;
-        if (n > 0) v |= i0;
-        if (n > 1) v |= i1 << 20;
-        if (n > 2) v |= i2 << 40;
-        return v;
+    return n;
+}
+
+// The value of the n tokens in sym[] (their ids go through rk[]); a token missing from the vocabulary is a KeyError
+// (tokenizer.py:135).  Up to 3 ids below INLINE_ID_LIMIT go into the value, more go to the id pool at pool_off(n).
+template <typename PoolOff>
+__device__ __forceinline__ u64 row_value(const EncTables &t, const u32 *sym, u32 *rk, u32 n, PoolOff pool_off) {
+    u64 value = 0;
+    bool bad = false, big = false;
+    for (u32 i = 0; i < n && !bad; i++) {
+        const int32_t id = t.sym_to_id[sym[i]];
+        if (id < 0) { bad = true; value = (VAL_ERR << 60) | sym[i]; }
+        else { big |= (u32)id >= INLINE_ID_LIMIT; rk[i] = (u32)id; }
     }
-    u64 off = 0;
-    if (lane == 0) off = atomicAdd(&t.ctr[5], (u64)n);
-    off = __shfl_sync(0xffffffffu, off, 0);
-    if (lane < n) t.ipool[off + lane] = (u32)id;
+    if (!bad) {
+        if (n <= 3 && !big) {
+            value = (u64)n << 60;
+            if (n > 0) value |= (u64)rk[0];
+            if (n > 1) value |= (u64)rk[1] << 20;
+            if (n > 2) value |= (u64)rk[2] << 40;
+        } else {
+            const u64 off = pool_off(n);
+            for (u32 i = 0; i < n; i++) t.ipool[off + i] = rk[i];
+            value = (VAL_EXT << 60) | (off << 24) | n;
+        }
+    }
+    return value;
+}
+
+// One warp: the n bytes at src, as tokens in place in w = t.ipool + off, which holds their ids at the end; to[] (DROP only) sits
+// beside w.  Returns the value.
+template <bool DROP>
+__device__ __forceinline__ u64 warp_bpe(const EncTables &t, const uint8_t *src, u32 *w, u32 *to, u32 n, u64 off, const DropOcc &x, u32 lane) {
+    for (u32 i = lane; i < n; i += 32) {
+        w[i] = src[i];
+        if constexpr (DROP) to[i] = i;
+    }
+    __syncwarp();
+    for (u32 round = 0; n > 1; round++) {
+        u64 best = RANK_NONE;
+        for (u32 b0 = 0; b0 + 1 < n; b0 += 32) {
+            u32 i = b0 + lane;
+            if (i + 1 < n) { u64 r = rank_lookup(t, w[i], w[i + 1]); if (r < best && !(DROP && x.drops(to[i], round))) best = r; }
+        }
+        best = warp_min_u64(best);
+        if (best == RANK_NONE) break;
+        const u32 j = (u32)(best >> 32), res = (u32)best;
+        const u32 a = (u32)t.mpairs[2 * j], b = (u32)t.mpairs[2 * j + 1];
+        u32 out = 0, carry = 0;
+        for (u32 b0 = 0; b0 < n; b0 += 32) {
+            u32 i = b0 + lane;
+            u32 cur = i < n ? w[i] : 0xFFFFFFFFu, nx = i + 1 < n ? w[i + 1] : 0xFFFFFFFFu, ci = DROP && i < n ? to[i] : 0u;
+            u32 m = __ballot_sync(0xffffffffu, cur == a && nx == b && !(DROP && x.drops(ci, round)));
+            // only the matches of (a, a) can overlap: a match of (a, b), a != b, ends in b, which starts no match
+            u32 heads = a == b ? resolve_heads_same(m, carry) : m;
+            u32 valid = __ballot_sync(0xffffffffu, i < n);
+            u32 kept = valid & ~((heads << 1) | carry);
+            carry = heads >> 31;
+            u32 val = ((heads >> lane) & 1u) ? res : cur;
+            u32 pos = out + __popc(kept & ((1u << lane) - 1u));
+            __syncwarp();
+            if ((kept >> lane) & 1u) {
+                w[pos] = val;
+                if constexpr (DROP) to[pos] = ci;
+            }
+            out += __popc(kept);
+            __syncwarp();
+        }
+        n = out;
+    }
+    // ids in place; a token missing from the vocabulary is a KeyError (tokenizer.py:135)
+    u32 bad_idx = 0xFFFFFFFFu;
+    for (u32 i = lane; i < n; i += 32) if (t.sym_to_id[w[i]] < 0 && i < bad_idx) bad_idx = i;
+    for (int d = 16; d; d >>= 1) { u32 o = __shfl_xor_sync(0xffffffffu, bad_idx, d); bad_idx = o < bad_idx ? o : bad_idx; }
+    if (bad_idx != 0xFFFFFFFFu) return (VAL_ERR << 60) | w[bad_idx];
+    for (u32 i = lane; i < n; i += 32) w[i] = (u32)t.sym_to_id[w[i]];
     return (VAL_EXT << 60) | (off << 24) | n;
 }
 
@@ -479,147 +588,37 @@ __global__ void __launch_bounds__(BPT_NT) k_enc_bpe_short(EncTables t, u64 n_tod
             n = (u32)(k >> 56);
             for (u32 i = 0; i < n; i++) sym[i] = (u32)((k >> (8 * i)) & 0xFFu);
         }
-        // ranks of the adjacent pairs, kept up to date: after a merge only the pairs next to a merged token change
-        for (u32 i = 0; i + 1 < n; i++) rk[i] = (u32)(rank_lookup(t, sym[i], sym[i + 1]) >> 32);
-        while (n > 1) {
-            // lowest-ranked adjacent pair (tokenizer.py:128-131)
-            u32 best = 0xFFFFFFFFu, bi = 0;
-            for (u32 i = 0; i + 1 < n; i++) if (rk[i] < best) { best = rk[i]; bi = i; }
-            if (best == 0xFFFFFFFFu) break;
-            const u32 a = sym[bi], b = sym[bi + 1], res = (u32)rank_lookup(t, a, b);
-            // Tokenizer.merge (tokenizer.py:92-109): every non-overlapping occurrence, left to right (equal rank <=> same pair)
-            u32 o = 0, merged = 0;
-            for (u32 i = 0; i < n; o++) {
-                if (i + 1 < n && rk[i] == best) { sym[o] = res; merged |= 1u << o; i += 2; }
-                else { sym[o] = sym[i]; rk[o] = rk[i]; i += 1; }
-            }
-            n = o;
-            for (u32 i = 0; i + 1 < n; i++)
-                if ((merged >> i) & 3u) rk[i] = (u32)(rank_lookup(t, sym[i], sym[i + 1]) >> 32);
-        }
-        // ids; a token missing from the vocabulary is a KeyError (tokenizer.py:135)
-        u64 value = 0;
-        bool bad = false, big = false;
-        for (u32 i = 0; i < n && !bad; i++) {
-            const int32_t id = t.sym_to_id[sym[i]];
-            if (id < 0) { bad = true; value = (VAL_ERR << 60) | sym[i]; }
-            else { big |= (u32)id >= INLINE_ID_LIMIT; rk[i] = (u32)id; }
-        }
-        if (!bad) {
-            if (n <= 3 && !big) {
-                value = (u64)n << 60;
-                if (n > 0) value |= (u64)rk[0];
-                if (n > 1) value |= (u64)rk[1] << 20;
-                if (n > 2) value |= (u64)rk[2] << 40;
-            } else {
-                const u64 off = atomicAdd(&t.ctr[5], (u64)n);
-                for (u32 i = 0; i < n; i++) t.ipool[off + i] = rk[i];
-                value = (VAL_EXT << 60) | (off << 24) | n;
-            }
-        }
+        n = row_bpe<false>(t, sym, rk, nullptr, n, DropOcc{});
+        const u64 value = row_value(t, sym, rk, n, [&](u32 c) { return (u64)atomicAdd(&t.ctr[5], (u64)c); });
         if (is_med) t.medtab[slot].val = value; else if (is_long) t.ltab[slot].val = value; else t.stab[slot].val = value;
     }
 }
 
-// ---- the same for pretokens longer than 32 bytes: one warp each, tokens in place in the id pool ----
+// ---- the long-table entries of more than BPT_MAX bytes: one warp each, tokens in place in the id pool ----
+// (every entry of up to BPT_MAX bytes, short and medium ones included, is k_enc_bpe_short's)
 __global__ void __launch_bounds__(256) k_enc_bpe(EncTables t, u64 n_todo) {
     const u32 lane = lane_id();
     const u64 gwarp = ((u64)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = ((u64)gridDim.x * blockDim.x) >> 5;
     for (u64 q = gwarp; q < n_todo; q += nwarps) {
         const u32 ref = t.todo[q];
-        const bool is_long = ref & REF_LONG;
+        if (!(ref & REF_LONG)) continue;
         const u32 slot = REF_SLOT(ref);
-        u32 len; const uint8_t *p = nullptr; u64 skey = 0;
-        if (!is_long) continue;                  // (<= 15 bytes: k_enc_bpe_short)
-        if (is_long) {
-            u64 m = t.ltab[slot].meta;
-            len = (u32)(m & META_LEN_MASK);
-            if (len <= BPT_MAX) continue;        // k_enc_bpe_short
-            const uint8_t *src = enc_rep_ptr(t, m);
-            // move the key bytes out of the (transient) text arena into the persistent key pool
-            u64 ko = 0;
-            if (lane == 0) ko = atomicAdd(&t.ctr[4], (u64)len);
-            ko = __shfl_sync(0xffffffffu, ko, 0);
-            for (u32 i = lane; i < len; i += 32) t.kpool[ko + i] = src[i];
-            __syncwarp();
-            if (lane == 0) t.ltab[slot].meta = ((ko | META_POOL_BIT) << META_LEN_BITS) | len;
-            p = t.kpool + ko;
-        } else {
-            skey = t.stab[slot].key;
-            len = (u32)(skey >> 56);
-        }
-        u64 value;
-        if (len <= 32) {
-            // ---- register path: lane i holds token i ----
-            u32 s = 0;
-            if (lane < len) s = is_long ? p[lane] : (u32)((skey >> (8 * lane)) & 0xFFu);
-            u32 n = len;
-            while (n > 1) {
-                u32 nxt = __shfl_down_sync(0xffffffffu, s, 1);
-                u64 r = lane + 1 < n ? rank_lookup(t, s, nxt) : RANK_NONE;
-                u64 best = warp_min_u64(r);
-                if (best == RANK_NONE) break;
-                u32 m = __ballot_sync(0xffffffffu, r == best);
-                u32 j = (u32)(best >> 32);
-                u32 heads = (t.mpairs[2 * j] == t.mpairs[2 * j + 1]) ? resolve_heads_same(m, 0) : m;
-                u32 valid = n == 32 ? 0xFFFFFFFFu : ((1u << n) - 1u);
-                u32 kept = valid & ~(heads << 1);
-                u32 val = ((heads >> lane) & 1u) ? (u32)best : s;
-                u32 src = __fns(kept, 0, lane + 1);              // lane of the (lane+1)-th kept token
-                u32 got = __shfl_sync(0xffffffffu, val, src & 31u);
-                n = __popc(kept);
-                s = lane < n ? got : 0;
-            }
-            int32_t id = lane < n ? t.sym_to_id[s] : 0;
-            value = make_value(t, n, id, s, lane);
-        } else {
-            // ---- long path: tokens in place in the id pool ----
-            u64 off = 0;
-            if (lane == 0) off = atomicAdd(&t.ctr[5], (u64)len);
-            off = __shfl_sync(0xffffffffu, off, 0);
-            u32 *w = t.ipool + off;
-            for (u32 i = lane; i < len; i += 32) w[i] = p[i];
-            __syncwarp();
-            u32 n = len;
-            while (n > 1) {
-                u64 best = RANK_NONE;
-                for (u32 base = 0; base + 1 < n; base += 32) {
-                    u32 i = base + lane;
-                    if (i + 1 < n) { u64 r = rank_lookup(t, w[i], w[i + 1]); best = r < best ? r : best; }
-                }
-                best = warp_min_u64(best);
-                if (best == RANK_NONE) break;
-                const u32 j = (u32)(best >> 32), res = (u32)best;
-                const u32 a = (u32)t.mpairs[2 * j], b = (u32)t.mpairs[2 * j + 1];
-                u32 out = 0, carry = 0;
-                for (u32 base = 0; base < n; base += 32) {
-                    u32 i = base + lane;
-                    u32 cur = i < n ? w[i] : 0xFFFFFFFFu, nx = i + 1 < n ? w[i + 1] : 0xFFFFFFFFu;
-                    u32 m = __ballot_sync(0xffffffffu, cur == a && nx == b);
-                    u32 heads = a == b ? resolve_heads_same(m, carry) : m;
-                    u32 valid = __ballot_sync(0xffffffffu, i < n);
-                    u32 kept = valid & ~((heads << 1) | carry);
-                    carry = heads >> 31;
-                    u32 val = ((heads >> lane) & 1u) ? res : cur;
-                    u32 pos = out + __popc(kept & ((1u << lane) - 1u));
-                    __syncwarp();
-                    if ((kept >> lane) & 1u) w[pos] = val;
-                    out += __popc(kept);
-                    __syncwarp();
-                }
-                n = out;
-            }
-            // ids in place; a token missing from the vocabulary is a KeyError (tokenizer.py:135)
-            u32 bad_idx = 0xFFFFFFFFu;
-            for (u32 i = lane; i < n; i += 32) if (t.sym_to_id[w[i]] < 0 && i < bad_idx) bad_idx = i;
-            for (int d = 16; d; d >>= 1) { u32 o = __shfl_xor_sync(0xffffffffu, bad_idx, d); bad_idx = o < bad_idx ? o : bad_idx; }
-            if (bad_idx != 0xFFFFFFFFu) value = (VAL_ERR << 60) | w[bad_idx];
-            else {
-                for (u32 i = lane; i < n; i += 32) w[i] = (u32)t.sym_to_id[w[i]];
-                value = (VAL_EXT << 60) | (off << 24) | n;
-            }
-        }
-        if (lane == 0) { if (is_long) t.ltab[slot].val = value; else t.stab[slot].val = value; }
+        const u64 m = t.ltab[slot].meta;
+        const u32 len = (u32)(m & META_LEN_MASK);
+        if (len <= BPT_MAX) continue;
+        const uint8_t *src = enc_rep_ptr(t, m);
+        // move the key bytes out of the (transient) text arena into the persistent key pool
+        u64 ko = 0;
+        if (lane == 0) ko = atomicAdd(&t.ctr[4], (u64)len);
+        ko = __shfl_sync(0xffffffffu, ko, 0);
+        for (u32 i = lane; i < len; i += 32) t.kpool[ko + i] = src[i];
+        __syncwarp();
+        if (lane == 0) t.ltab[slot].meta = ((ko | META_POOL_BIT) << META_LEN_BITS) | len;
+        u64 off = 0;
+        if (lane == 0) off = atomicAdd(&t.ctr[5], (u64)len);
+        off = __shfl_sync(0xffffffffu, off, 0);
+        const u64 value = warp_bpe<false>(t, t.kpool + ko, t.ipool + off, nullptr, len, off, DropOcc{}, lane);
+        if (lane == 0) t.ltab[slot].val = value;
     }
 }
 
@@ -779,24 +778,14 @@ struct EncDrop {
     u64 ibase;                                   // id pool offset of the batch start's scratch (one id per byte)
 };
 
-__device__ __forceinline__ u64 splitmix64(u64 z) {
-    z += 0x9E3779B97F4A7C15ull;
-    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-    return z ^ (z >> 31);
-}
-__device__ __forceinline__ bool drop_pair(u64 thr, u64 h_doc, u64 off, u32 round) {
-    return (splitmix64(splitmix64(h_doc ^ off) ^ round) >> 32) < thr;
-}
 // mix(mix(seed) ^ doc) and the offset in its document of the pretoken at arena byte p
-__device__ __forceinline__ void drop_doc(const EncTables &t, const EncDrop &d, u64 p, u64 *h_doc, u64 *off) {
-    if (!d.doffs) { *h_doc = splitmix64(d.seed_mix); *off = d.lo + p; return; }
+__device__ __forceinline__ DropOcc drop_occ(const EncTables &t, const EncDrop &d, u64 p) {
+    if (!d.doffs) return {d.thr, splitmix64(d.seed_mix), d.lo + p};
     const u64 w = p >> 5;
     u64 j = t.bpre[w >> 4];                      // boundaries before p: before its 512-byte group, then the words of the group
     for (u64 k = w & ~15ull; k < w; k++) j += __popc(t.bmask[k]);
     j += __popc(t.bmask[w] & ((1u << (p & 31)) - 1u));
-    *h_doc = splitmix64(d.seed_mix ^ (d.da + j));
-    *off = d.lo + p - j - d.doffs[d.da + j];     // (arena -> caller position: minus the boundary bytes before it)
+    return {d.thr, splitmix64(d.seed_mix ^ (d.da + j)), d.lo + p - j - d.doffs[d.da + j]};   // (arena -> caller position: minus the boundary bytes before it)
 }
 
 // starts[ordinal - ord0] = arena offset of every pretoken starting in flag words [w_lo, w_hi)
@@ -811,16 +800,15 @@ __global__ void __launch_bounds__(256) k_enc_drop_starts(const u32 *__restrict__
     }
 }
 
-// One thread per occurrence of <= 32 bytes (the row layout of k_enc_bpe_short, plus each token's byte offset); longer ones that need
-// redoing are queued (t.todo, count in ctr[10]) for k_enc_drop_warp.  An occurrence keeps its cached value when it is a special token or
-// a document boundary, or when that value already has one token per byte: no pair had a rank, and dropout only removes candidates.
+// One thread per occurrence of <= 32 bytes (row_bpe in the row layout of k_enc_bpe_short, plus each token's byte offset); longer ones
+// that need redoing are queued (t.todo, count in ctr[10]) for k_enc_drop_warp.  An occurrence keeps its cached value when it is a special
+// token or a document boundary, or when that value already has one token per byte: no pair had a rank, and dropout only removes candidates.
 __global__ void __launch_bounds__(BPT_NT) k_enc_drop_short(EncTables t, EncDrop d, const u32 *__restrict__ flags, u64 n, u64 base, u64 bound,
                                                           u64 *__restrict__ vals) {
     __shared__ u32 s_sym[BPT_NT][BPT_MAX + 1];
     __shared__ u32 s_rk[BPT_NT][BPT_MAX + 1];
     __shared__ uint8_t s_off[BPT_NT][BPT_MAX + 1];
     u32 *sym = s_sym[threadIdx.x], *rk = s_rk[threadIdx.x];
-    uint8_t *to = s_off[threadIdx.x];
     for (u64 q = (u64)blockIdx.x * blockDim.x + threadIdx.x; q < bound; q += (u64)gridDim.x * blockDim.x) {
         u64 v = vals[q];
         if (VAL_TAG(v) == VAL_DOC) continue;
@@ -831,57 +819,14 @@ __global__ void __launch_bounds__(BPT_NT) k_enc_drop_short(EncTables t, EncDrop 
         if (VAL_TAG(v) == VAL_FWD) v = enc_value(t, (u32)v);
         if (VAL_TAG(v) != VAL_ERR && value_count(v) == len) continue;
         if (len > BPT_MAX) { const u64 k = atomicAdd(&t.ctr[10], 1ull); t.todo[k] = (u32)q; continue; }
-        u64 h_doc, off0;
-        drop_doc(t, d, p, &h_doc, &off0);
-        u32 nt = len;
-        for (u32 i = 0; i < nt; i++) { sym[i] = t.text[p + i]; to[i] = (uint8_t)i; }
-        for (u32 i = 0; i + 1 < nt; i++) rk[i] = (u32)(rank_lookup(t, sym[i], sym[i + 1]) >> 32);
-        for (u32 round = 0; nt > 1; round++) {
-            // lowest rank among the pairs this round keeps; cand = the kept ones
-            u32 best = 0xFFFFFFFFu, cand = 0;
-            for (u32 i = 0; i + 1 < nt; i++) {
-                if (rk[i] == 0xFFFFFFFFu || drop_pair(d.thr, h_doc, off0 + to[i], round)) continue;
-                cand |= 1u << i;
-                if (rk[i] < best) best = rk[i];
-            }
-            if (best == 0xFFFFFFFFu) break;
-            u32 bi = __ffs(cand & ~0u) - 1;
-            while (rk[bi] != best) { cand &= ~(1u << bi); bi = __ffs(cand) - 1; }
-            const u32 res = (u32)rank_lookup(t, sym[bi], sym[bi + 1]);
-            u32 o = 0, merged = 0;
-            for (u32 i = 0; i < nt; o++) {
-                if (i + 1 < nt && ((cand >> i) & 1u) && rk[i] == best) { sym[o] = res; to[o] = to[i]; merged |= 1u << o; i += 2; }
-                else { sym[o] = sym[i]; rk[o] = rk[i]; to[o] = to[i]; i += 1; }
-            }
-            nt = o;
-            for (u32 i = 0; i + 1 < nt; i++)
-                if ((merged >> i) & 3u) rk[i] = (u32)(rank_lookup(t, sym[i], sym[i + 1]) >> 32);
-        }
-        u64 value = 0;
-        bool bad = false, big = false;
-        for (u32 i = 0; i < nt && !bad; i++) {
-            const int32_t id = t.sym_to_id[sym[i]];
-            if (id < 0) { bad = true; value = (VAL_ERR << 60) | sym[i]; }
-            else { big |= (u32)id >= INLINE_ID_LIMIT; rk[i] = (u32)id; }
-        }
-        if (!bad) {
-            if (nt <= 3 && !big) {
-                value = (u64)nt << 60;
-                if (nt > 0) value |= (u64)rk[0];
-                if (nt > 1) value |= (u64)rk[1] << 20;
-                if (nt > 2) value |= (u64)rk[2] << 40;
-            } else {
-                const u64 io = d.ibase + (p - base);
-                for (u32 i = 0; i < nt; i++) t.ipool[io + i] = rk[i];
-                value = (VAL_EXT << 60) | (io << 24) | nt;
-            }
-        }
-        vals[q] = value;
+        for (u32 i = 0; i < len; i++) sym[i] = t.text[p + i];
+        const u32 nt = row_bpe<true>(t, sym, rk, s_off[threadIdx.x], len, drop_occ(t, d, p));
+        vals[q] = row_value(t, sym, rk, nt, [&](u32) { return d.ibase + (p - base); });
     }
 }
 
-// The queued occurrences of > 32 bytes: one warp each, symbols in place in the id pool scratch, token offsets beside them in d.loff
-// (the long path of k_enc_bpe with the dropped candidates taken out of the minimum and of the merge).
+// The queued occurrences of > 32 bytes: warp_bpe, one warp each, symbols in place in the id pool scratch, token offsets beside them
+// in d.loff.
 __global__ void __launch_bounds__(256) k_enc_drop_warp(EncTables t, EncDrop d, const u32 *__restrict__ flags, u64 n, u64 base, u64 bound,
                                                       u64 *__restrict__ vals) {
     const u32 lane = lane_id();
@@ -891,56 +836,8 @@ __global__ void __launch_bounds__(256) k_enc_drop_warp(EncTables t, EncDrop d, c
         const u64 q = t.todo[k];
         const u64 p = d.starts[q];
         const u64 e = q + 1 < bound ? d.starts[q + 1] : flags_next_start(flags, p + 1, n);
-        const u32 len = (u32)(e - p);
-        u64 h_doc, off0;
-        drop_doc(t, d, p, &h_doc, &off0);
         const u64 io = d.ibase + (p - base);
-        u32 *w = t.ipool + io, *to = d.loff + (p - base);
-        for (u32 i = lane; i < len; i += 32) { w[i] = t.text[p + i]; to[i] = i; }
-        __syncwarp();
-        u32 nt = len;
-        for (u32 round = 0; nt > 1; round++) {
-            u64 best = RANK_NONE;
-            for (u32 b0 = 0; b0 + 1 < nt; b0 += 32) {
-                const u32 i = b0 + lane;
-                if (i + 1 < nt) {
-                    const u64 r = rank_lookup(t, w[i], w[i + 1]);
-                    if (r < best && !drop_pair(d.thr, h_doc, off0 + to[i], round)) best = r;
-                }
-            }
-            best = warp_min_u64(best);
-            if (best == RANK_NONE) break;
-            const u32 j = (u32)(best >> 32), res = (u32)best;
-            const u32 a = (u32)t.mpairs[2 * j], b = (u32)t.mpairs[2 * j + 1];
-            u32 out = 0, carry = 0;
-            for (u32 b0 = 0; b0 < nt; b0 += 32) {
-                const u32 i = b0 + lane;
-                const u32 cur = i < nt ? w[i] : 0xFFFFFFFFu, nx = i + 1 < nt ? w[i + 1] : 0xFFFFFFFFu, ci = i < nt ? to[i] : 0u;
-                const bool hit = cur == a && nx == b && !drop_pair(d.thr, h_doc, off0 + ci, round);
-                const u32 m = __ballot_sync(0xffffffffu, hit);
-                const u32 heads = resolve_heads_same(m, carry);      // (left to right, non-overlapping: only (a, a) can overlap)
-                const u32 valid = __ballot_sync(0xffffffffu, i < nt);
-                const u32 kept = valid & ~((heads << 1) | carry);
-                carry = heads >> 31;
-                const u32 val = ((heads >> lane) & 1u) ? res : cur;
-                const u32 pos = out + __popc(kept & ((1u << lane) - 1u));
-                __syncwarp();
-                if ((kept >> lane) & 1u) { w[pos] = val; to[pos] = ci; }
-                out += __popc(kept);
-                __syncwarp();
-            }
-            nt = out;
-        }
-        u32 bad_idx = 0xFFFFFFFFu;
-        for (u32 i = lane; i < nt; i += 32) if (t.sym_to_id[w[i]] < 0 && i < bad_idx) bad_idx = i;
-        for (int dd = 16; dd; dd >>= 1) { const u32 o = __shfl_xor_sync(0xffffffffu, bad_idx, dd); bad_idx = o < bad_idx ? o : bad_idx; }
-        u64 value;
-        if (bad_idx != 0xFFFFFFFFu) value = (VAL_ERR << 60) | w[bad_idx];
-        else {
-            for (u32 i = lane; i < nt; i += 32) w[i] = (u32)t.sym_to_id[w[i]];
-            value = (VAL_EXT << 60) | (io << 24) | nt;
-        }
-        __syncwarp();
+        const u64 value = warp_bpe<true>(t, t.text + p, t.ipool + io, d.loff + (p - base), (u32)(e - p), io, drop_occ(t, d, p), lane);
         if (lane == 0) vals[q] = value;
     }
 }
@@ -1757,11 +1654,11 @@ __global__ void __launch_bounds__(256) k_enc_expand_docs(const uint8_t *__restri
     }
 }
 
-// A pipeline chunk: bytes [lo, hi) of the caller's text; bpe_encode_batch: documents [da, db) end inside it.
+// A pipeline chunk: bytes [lo, hi) of the caller's text; documents [da, db) end inside it.
 struct EncChunk { u64 lo, hi, da, db; };
 
-// bpe_encode_batch's chunks: cut at a document end near every multiple of the nominal size; a document that runs well past it is cut
-// at an exact boundary inside it (find_exact_cut on the document alone), or else stays whole.
+// The pipeline's chunks: cut at a document end near every multiple of the nominal size; a document that runs well past it is cut
+// at an exact boundary inside it (find_exact_cut on the document alone), or else stays whole.  bpe_encode: one document.
 static std::vector<EncChunk> doc_chunks(const bpe_tok *tok, const uint8_t *t, u64 n, const uint64_t *doc_offs, u64 n_docs, u64 chunk) {
     std::vector<EncChunk> out;
     u64 lo = 0, d = 0;
@@ -1775,6 +1672,7 @@ static std::vector<EncChunk> doc_chunks(const bpe_tok *tok, const uint8_t *t, u6
             const u64 ds = doc_offs[j], c = find_exact_cut(tok, t + ds, doc_offs[j + 1] - ds, target - ds);   // (ds < target: j does not end by it)
             if (c && ds + c > lo) { hi = ds + c; nd = j; }
             else if (e > lo) { hi = e; nd = j; }
+            else if (doc_offs[j + 1] == n) break;    // the rest is this document: one piece
             else { hi = doc_offs[j + 1]; nd = j + 1; }
         }
         out.push_back({lo, hi, d, nd});
@@ -1801,21 +1699,9 @@ static int encode_pipeline(bpe_tok *tok, const uint8_t *text_host, uint64_t n, c
     const size_t esz = out_dtype == BPE_DTYPE_U16 ? 2 : 4;
     u64 chunk = ENC_PIPE_CHUNK;
     if (const char *e = getenv("BPE_ENCODE_CHUNK_MB")) chunk = std::max<u64>(1, strtoull(e, nullptr, 10)) << 20;
-    std::vector<EncChunk> chunks;
-    if (doc_offs) chunks = doc_chunks(tok, text_host, n, doc_offs, n_docs, chunk);
-    else {
-        std::vector<u64> cut{0};
-        if (n >= ENC_PIPE_MIN) {
-            for (u64 nominal = chunk; nominal + chunk / 2 < n; ) {
-                u64 c = find_exact_cut(tok, text_host, n, nominal);
-                if (!c || c <= cut.back()) break;     // no exact boundary nearby: the rest goes in one piece
-                cut.push_back(c);
-                nominal = c + chunk;
-            }
-        }
-        cut.push_back(n);
-        for (size_t k = 0; k + 1 < cut.size(); k++) chunks.push_back({cut[k], cut[k + 1], 0, 0});
-    }
+    const uint64_t one_doc[2] = {0, n};
+    const std::vector<EncChunk> chunks = doc_offs ? doc_chunks(tok, text_host, n, doc_offs, n_docs, chunk)
+                                                  : doc_chunks(tok, text_host, n, one_doc, 1, chunk);
     const size_t m = chunks.size();
     BPE_TRY(ctx_pipeline_init(ctx));
     u64 *id_dev = nullptr;
