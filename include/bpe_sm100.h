@@ -234,6 +234,33 @@ int bpe_encode_dropout(bpe_tok *tok, const uint8_t *text_host, uint64_t n, doubl
 int bpe_encode_batch_dropout(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
                              double p, uint64_t seed, int out_dtype, void *out, uint64_t cap, uint64_t *n_out,
                              uint64_t *id_offs_out, bpe_encode_stats *stats);
+/* Token offsets: the ids of bpe_encode / bpe_encode_batch / bpe_encode_dropout / bpe_encode_batch_dropout with the same arguments, and
+ * for every token i its span [start_i, end_i) of the input, offs_out[2 i], offs_out[2 i + 1] (int64, cap x 2 entries).  Same two-call
+ * idiom (out == NULL reports *n_out and writes no offsets; otherwise offs_out must be given), dtypes, errors in the same order and error
+ * details; BPE_ERR_ARG for an unknown unit.
+ *   BPE_OFF_BYTES  the bytes token i was produced from.  The spans tile the document in order (start_0 = 0, end_i = start_{i+1}, the last
+ *                  end = its length).  The tokens of a pretoken occurrence tile it; each but its last is as long as its vocabulary entry
+ *                  and the last ends where the pretoken ends.  So data[start:end] == vocab[id] for an ordinary token, and a special-token
+ *                  occurrence spans the special's bytes whatever its id (also an id missing from the vocabulary or shared with another
+ *                  token, SURVEY A-12).
+ *   BPE_OFF_CHARS  Python str indices: start = index of the character that holds the token's first byte, end = one past the index of the
+ *                  character that holds its last byte.  A token that splits a multi-byte character maps to the whole character, so the
+ *                  spans of the tokens that share it overlap by one (as HF byte-level offsets do): text[start:end].encode() always
+ *                  contains the token's bytes, and equals them when no character is split.
+ * Batch calls: spans are relative to each document's start, as if it were encoded on its own.  The spans depend only on the text, the
+ * document split, p and seed: not on the pretoken cache, how the library cuts the text, or the batch size. */
+#define BPE_OFF_BYTES 0
+#define BPE_OFF_CHARS 1
+int bpe_encode_offsets(bpe_tok *tok, const uint8_t *text_host, uint64_t n, int out_dtype, void *out, uint64_t cap, uint64_t *n_out,
+                       int unit, int64_t *offs_out, bpe_encode_stats *stats);
+int bpe_encode_batch_offsets(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
+                             int out_dtype, void *out, uint64_t cap, uint64_t *n_out, uint64_t *id_offs_out, int unit, int64_t *offs_out,
+                             bpe_encode_stats *stats);
+int bpe_encode_dropout_offsets(bpe_tok *tok, const uint8_t *text_host, uint64_t n, double p, uint64_t seed, int out_dtype, void *out,
+                               uint64_t cap, uint64_t *n_out, int unit, int64_t *offs_out, bpe_encode_stats *stats);
+int bpe_encode_batch_dropout_offsets(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
+                                     double p, uint64_t seed, int out_dtype, void *out, uint64_t cap, uint64_t *n_out,
+                                     uint64_t *id_offs_out, int unit, int64_t *offs_out, bpe_encode_stats *stats);
 /* 1 if the text of the last bpe_encode* call on this tokenizer's context held a carriage return (the flags kernel
  * sees every byte anyway).  Tokenizer.encode takes a str and keeps '\r' as it is; a caller that reads a FILE in text mode, like the
  * reference's bulk driver (models/tokenizer/encode.py:31-34, universal newlines), uses this instead of scanning the text on the host:

@@ -17,6 +17,7 @@ BPE_OK = 0
 (ERR_ARG, ERR_CUDA, ERR_OOM, ERR_UTF8, ERR_KEY, ERR_CAPACITY, ERR_TOO_SMALL, ERR_UNSUPPORTED, ERR_NO_DEVICE, ERR_HALO,
  ERR_NEWLINE) = range(-1, -12, -1)
 DTYPE_U16, DTYPE_I32 = 0, 1
+OFF_BYTES, OFF_CHARS = 0, 1
 SYNTH_TINYSTORIES, SYNTH_OWT = 0, 1
 
 
@@ -53,7 +54,8 @@ EXPORTS = [
     "bpe_last_error_detail", "bpe_device_sync", "bpe_utf8_validate", "bpe_pretokenize", "bpe_train", "bpe_train_dev",
     "bpe_count_begin", "bpe_count_add_shard", "bpe_count_add_shard_dev", "bpe_count_export_size", "bpe_count_export",
     "bpe_count_export_dev", "bpe_count_import", "bpe_count_import_dev", "bpe_count_pair_table",
-    "bpe_train_from_counts", "bpe_last_pair_table", "bpe_train_set_live", "bpe_tok_create", "bpe_tok_destroy", "bpe_encode", "bpe_encode_batch", "bpe_encode_dropout", "bpe_encode_batch_dropout", "bpe_encode_dev", "bpe_tok_key_error", "bpe_tok_saw_cr",
+    "bpe_train_from_counts", "bpe_last_pair_table", "bpe_train_set_live", "bpe_tok_create", "bpe_tok_destroy", "bpe_encode", "bpe_encode_batch", "bpe_encode_dropout", "bpe_encode_batch_dropout", "bpe_encode_offsets",
+    "bpe_encode_batch_offsets", "bpe_encode_dropout_offsets", "bpe_encode_batch_dropout_offsets", "bpe_encode_dev", "bpe_tok_key_error", "bpe_tok_saw_cr",
     "bpe_tok_cache_reset", "bpe_decode", "bpe_decode_batch", "bpe_batch_windows_dev", "bpe_synth_dev", "bpe_synth_host", "bpe_synth_dev_at", "bpe_synth_host_at", "bpe_ctx_set_stream", "bpe_host_alloc", "bpe_host_free", "bpe_launch_count",
 ]
 
@@ -99,6 +101,13 @@ def lib():
             L.bpe_encode_dropout.argtypes = [vp, vp, C.c_uint64, C.c_double, C.c_uint64, C.c_int, vp, C.c_uint64, u64p, C.POINTER(EncodeStats)]
             L.bpe_encode_batch_dropout.argtypes = [vp, vp, C.c_uint64, vp, C.c_uint64, C.c_double, C.c_uint64, C.c_int, vp, C.c_uint64, u64p, vp,
                                                    C.POINTER(EncodeStats)]
+            L.bpe_encode_offsets.argtypes = [vp, vp, C.c_uint64, C.c_int, vp, C.c_uint64, u64p, C.c_int, vp, C.POINTER(EncodeStats)]
+            L.bpe_encode_batch_offsets.argtypes = [vp, vp, C.c_uint64, vp, C.c_uint64, C.c_int, vp, C.c_uint64, u64p, vp, C.c_int, vp,
+                                                   C.POINTER(EncodeStats)]
+            L.bpe_encode_dropout_offsets.argtypes = [vp, vp, C.c_uint64, C.c_double, C.c_uint64, C.c_int, vp, C.c_uint64, u64p, C.c_int, vp,
+                                                     C.POINTER(EncodeStats)]
+            L.bpe_encode_batch_dropout_offsets.argtypes = [vp, vp, C.c_uint64, vp, C.c_uint64, C.c_double, C.c_uint64, C.c_int, vp,
+                                                           C.c_uint64, u64p, vp, C.c_int, vp, C.POINTER(EncodeStats)]
             L.bpe_tok_key_error.argtypes = [vp, vp, C.c_uint64, u64p]
             L.bpe_tok_cache_reset.argtypes = [vp]
             L.bpe_tok_saw_cr.argtypes = [vp]

@@ -778,13 +778,19 @@ struct EncDrop {
     u64 ibase;                                   // id pool offset of the batch start's scratch (one id per byte)
 };
 
+// set bits before arena byte p of a bitmask with one bit per byte, from its counts before every 512-byte group (pre) and the words of
+// p's group; mask needs the word that holds p
+__device__ __forceinline__ u64 bits_before(const u32 *__restrict__ mask, const u64 *__restrict__ pre, u64 p) {
+    const u64 w = p >> 5;
+    u64 j = pre[w >> 4];
+    for (u64 k = w & ~15ull; k < w; k++) j += __popc(mask[k]);
+    return j + __popc(mask[w] & ((1u << (p & 31)) - 1u));
+}
+
 // mix(mix(seed) ^ doc) and the offset in its document of the pretoken at arena byte p
 __device__ __forceinline__ DropOcc drop_occ(const EncTables &t, const EncDrop &d, u64 p) {
     if (!d.doffs) return {d.thr, splitmix64(d.seed_mix), d.lo + p};
-    const u64 w = p >> 5;
-    u64 j = t.bpre[w >> 4];                      // boundaries before p: before its 512-byte group, then the words of the group
-    for (u64 k = w & ~15ull; k < w; k++) j += __popc(t.bmask[k]);
-    j += __popc(t.bmask[w] & ((1u << (p & 31)) - 1u));
+    const u64 j = bits_before(t.bmask, t.bpre, p);   // document boundaries before p
     return {d.thr, splitmix64(d.seed_mix ^ (d.da + j)), d.lo + p - j - d.doffs[d.da + j]};   // (arena -> caller position: minus the boundary bytes before it)
 }
 
@@ -840,6 +846,100 @@ __global__ void __launch_bounds__(256) k_enc_drop_warp(EncTables t, EncDrop d, c
         const u64 value = warp_bpe<true>(t, t.text + p, t.ipool + io, d.loff + (p - base), (u32)(e - p), io, drop_occ(t, d, p), lane);
         if (lane == 0) vals[q] = value;
     }
+}
+
+// ---- token offsets (bpe_encode_offsets and the other *_offsets calls): a span of the input for every token --------------------------
+// Spec (include/bpe_sm100.h): the tokens of a pretoken occurrence tile its bytes in order; each but the last is as long as its vocabulary
+// entry (tok->vlen), the last ends where the pretoken ends.  So a special-token occurrence -- one id, whatever that id is -- spans the
+// special's bytes.  Per batch, after the emit kernel: the pretoken starts (k_enc_drop_starts), the token count of every pretoken and its
+// exclusive scan (the index of its first token), then one thread per pretoken writes {start, end} of its tokens next to their ids.
+// Characters: lead bytes ((b & 0xC0) != 0x80) before a byte, counted from a bit per arena byte and its count per 512-byte group;
+// a token's start is the index of the character holding its first byte, its end one past that of the character holding its last byte.
+struct EncOffs {
+    int chars;                                   // BPE_OFF_CHARS: character indices, else byte offsets
+    long long *out;                              // {start, end} of every token of the chunk, in the order of its ids
+    u64 lo;                                      // where the chunk starts in the caller's text
+    const u64 *doffs; u64 da;                    // bpe_encode_batch*: the caller's document offsets, the chunk's first document (else null, 0)
+    u64 carry;                                   // characters of the chunk's first document before lo
+    const u32 *lmask; const u64 *lpre;           // lead-byte bit per arena byte (words up to 16 (groups + 1)), count before every 512-byte group
+    const u32 *vlen; u64 n_dense;                // byte length of every vocabulary id
+    const u64 *starts, *tpre;                    // per batch: arena offset of every pretoken, index of its first token in the batch
+};
+
+// lmask[w] = lead-byte bits of arena bytes 32 w .. 32 w + 31 (none past n), for w < n_words
+__global__ void __launch_bounds__(256) k_enc_lead_bits(const uint8_t *__restrict__ text, u64 n, u64 n_words, u32 *__restrict__ lmask) {
+    for (u64 w = (u64)blockIdx.x * blockDim.x + threadIdx.x; w < n_words; w += (u64)gridDim.x * blockDim.x) {
+        u32 m = 0;
+        if (w * 32 < n) {
+            const uint4 *p = reinterpret_cast<const uint4 *>(text + w * 32);
+            const uint4 a = p[0], b = p[1];
+            const u32 x[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+#pragma unroll
+            for (int k = 0; k < 8; k++) {
+                const u32 l = ~((x[k] >> 7) & ~(x[k] >> 6)) & 0x01010101u;      // bit 0 of every byte: not a continuation byte 10xxxxxx
+                m |= ((l | (l >> 7) | (l >> 14) | (l >> 21)) & 0xFu) << (4 * k);
+            }
+            if (n - w * 32 < 32) m &= (1u << (n - w * 32)) - 1u;
+        }
+        lmask[w] = m;
+    }
+}
+
+// cnt[q] = tokens of pretoken q of the batch; forward references are resolved in vals (the emit kernel has read them)
+__global__ void __launch_bounds__(256) k_enc_off_count(EncTables t, u64 *__restrict__ vals, u64 bound, u32 *__restrict__ cnt) {
+    for (u64 q = (u64)blockIdx.x * blockDim.x + threadIdx.x; q < bound; q += (u64)gridDim.x * blockDim.x) {
+        u64 v = vals[q];
+        if (VAL_TAG(v) == VAL_FWD) { v = enc_value(t, (u32)v); vals[q] = v; }
+        cnt[q] = value_count(v);
+    }
+}
+
+// o.out[out_base + o.tpre[q] + k] = span of token k of pretoken q (below cap); n = arena bytes, flags = pretoken starts
+template <bool CHARS>
+__global__ void __launch_bounds__(256) k_enc_offsets(EncTables t, EncOffs o, const u32 *__restrict__ flags, const u64 *__restrict__ vals, u64 n,
+                                                    u64 bound, u64 out_base, u64 cap) {
+    longlong2 *out = reinterpret_cast<longlong2 *>(o.out);
+    for (u64 q = (u64)blockIdx.x * blockDim.x + threadIdx.x; q < bound; q += (u64)gridDim.x * blockDim.x) {
+        const u64 v = vals[q];
+        const u32 c = value_count(v);
+        if (!c) continue;                        // a document boundary (or a KeyError: the call fails)
+        const u64 p = o.starts[q], e = q + 1 < bound ? o.starts[q + 1] : flags_next_start(flags, p + 1, n);
+        // its document: j boundaries before p; arena -> document coordinates (all mod 2^64)
+        const u64 j = t.bmask ? bits_before(t.bmask, t.bpre, p) : 0;
+        const u64 bbase = o.lo - j - (o.doffs ? o.doffs[o.da + j] : 0);
+        u64 cbase = 0, lc = 0;                   // lc = lead bytes before the token
+        if (CHARS) {
+            cbase = j ? 0 - bits_before(o.lmask, o.lpre, o.doffs[o.da + j] - o.lo + j) : o.carry;
+            lc = bits_before(o.lmask, o.lpre, p);
+        }
+        const u32 *pool = t.ipool + ((v >> 24) & 0xFFFFFFFFFull);
+        const u64 dst = out_base + o.tpre[q];
+        u64 s = p;
+        for (u32 k = 0; k < c; k++) {
+            u64 end = e;
+            if (k + 1 < c) {
+                const u32 id = VAL_TAG(v) <= 3 ? (u32)((v >> (20 * k)) & 0xFFFFFu) : pool[k];
+                end = min(e, s + (id < o.n_dense ? o.vlen[id] : 1u));
+            }
+            longlong2 span;
+            if (CHARS) {
+                const u64 le = bits_before(o.lmask, o.lpre, end);
+                const u64 lead = (o.lmask[s >> 5] >> (s & 31)) & 1u;
+                span = make_longlong2((long long)(lc + lead - 1 + cbase), (long long)(le + cbase));
+                lc = le;
+            } else {
+                span = make_longlong2((long long)(s + bbase), (long long)(end + bbase));
+            }
+            if (dst + k < cap) out[dst + k] = span;
+            s = end;
+        }
+    }
+}
+
+// *host = lead bytes in arena bytes [a, b)
+__global__ void k_enc_lead_span(const u32 *__restrict__ lmask, const u64 *__restrict__ lpre, u64 a, u64 b, u64 *host) {
+    *host = bits_before(lmask, lpre, b) - bits_before(lmask, lpre, a);
+    __threadfence_system();
 }
 
 // ---- hot table: histogram of the sampled hit counts, build ----------------------------------------------------------
@@ -1065,6 +1165,7 @@ struct bpe_tok {
     bool hot_built = false, sampling = false;
     std::vector<uint8_t> key_error;              // bytes of the last KeyError key
     DevBuf drop;                                 // BPE-dropout scratch of a batch: pretoken offsets, token offsets of long pretokens
+    DevBuf offs_text, offs_batch, offs_out[2];   // token offsets: lead-byte bits of a chunk; pretoken starts and token scan of a batch; spans of a chunk
     int doc_sep = -1;                            // boundary byte of bpe_encode_batch (-1: every candidate occurs in a special)
 };
 
@@ -1323,7 +1424,8 @@ BPE_API void bpe_tok_destroy(bpe_tok *tok) {
     if (!tok) return;
     if (tok->ctx) { cudaSetDevice(tok->ctx->device); cudaStreamSynchronize(tok->ctx->stream); }
     for (DevBuf *b : {&tok->mtab, &tok->mpairs, &tok->sym_to_id, &tok->vlen, &tok->voff, &tok->vblob, &tok->sp_offs, &tok->sp_ids,
-                      &tok->stab, &tok->medtab, &tok->ltab, &tok->kpool, &tok->ipool, &tok->todo, &tok->ctr, &tok->hot, &tok->samp, &tok->sm_img, &tok->drop})
+                      &tok->stab, &tok->medtab, &tok->ltab, &tok->kpool, &tok->ipool, &tok->todo, &tok->ctr, &tok->hot, &tok->samp, &tok->sm_img, &tok->drop,
+                      &tok->offs_text, &tok->offs_batch, &tok->offs_out[0], &tok->offs_out[1]})
         bpe_buf_free(tok->ctx, *b);
     delete tok;
 }
@@ -1355,8 +1457,11 @@ struct DocBounds { const u32 *bmask; u64 *id_offs; u64 id_base; };
 // Encode the n bytes in the context's text arena into out_dev (device pointer, may be null: count only).
 // *n_out = number of tokens (may exceed dev_cap; only dev_cap are written).  stats, when given, are ADDED to.
 // drop (BPE-dropout, or null): its thr, seed_mix, lo, doffs and da; the rest is filled in per batch.
+// offs (token offsets, or null; needs out_dev): its chars, out, lo, doffs, da and carry; on return carry = that of the next chunk, whose first
+// document starts at arena byte next_ds (next_keep: it is this chunk's first one, which continues).
 static int encode_core(bpe_tok *tok, u64 n, int out_dtype, void *out_dev, u64 dev_cap, uint64_t *n_out, bpe_encode_stats *stats,
-                       const DocBounds *docs = nullptr, const EncDrop *drop = nullptr) {
+                       const DocBounds *docs = nullptr, const EncDrop *drop = nullptr, EncOffs *offs = nullptr, u64 next_ds = 0,
+                       bool next_keep = false) {
     bpe_ctx *ctx = tok->ctx;
     cudaStream_t st = ctx->stream;
     *n_out = 0;
@@ -1382,6 +1487,20 @@ static int encode_core(bpe_tok *tok, u64 n, int out_dtype, void *out_dev, u64 de
     if (docs) {                                  // the same per group for the boundary bits: document index of a boundary
         launch_popc_words16(docs->bmask, ng, cnt, ctx->sm_count, st);
         launch_scan_u32(cnt, ng, bpre, scan_tmp, st);
+    }
+    EncOffs o{};
+    if (offs) {                                  // lead-byte bits and their count per group: character indices
+        o = *offs;
+        const u64 lw = 16 * (ng + 1);
+        BPE_TRY(bpe_buf_reserve(ctx, tok->offs_text, lw * sizeof(u32) + (ng + 2) * sizeof(u64)));
+        u32 *lmask = (u32 *)tok->offs_text.p;
+        u64 *lpre = (u64 *)(lmask + lw);
+        KLAUNCH(k_enc_lead_bits, (unsigned)std::min<u64>((u64)ctx->sm_count * 16, (lw + 255) / 256), 256, 0, st,
+                (const uint8_t *)ctx->text.p + BPE_PAD, n, lw, lmask);
+        launch_popc_words16(lmask, ng, cnt, ctx->sm_count, st);
+        launch_scan_u32(cnt, ng, lpre, scan_tmp, st);
+        o.lmask = lmask; o.lpre = lpre;
+        o.vlen = (const u32 *)tok->vlen.p; o.n_dense = (u64)tok->n_dense;
     }
     CUDA_TRY(ctx, cudaGetLastError());
     // (test knobs: BPE_ENC_BATCH_KB = batch size, BPE_ENC_HOT_MIN = pretokens a batch needs to be sampled for the hot table,
@@ -1517,6 +1636,23 @@ static int encode_core(bpe_tok *tok, u64 n, int out_dtype, void *out_dev, u64 de
             CUDA_TRY(ctx, cudaGetLastError());
             launch_peek(host, total_dev, 1, st);
         }
+        if (offs && bound) {                     // token offsets, while the batch's values are resident
+            const size_t starts_b = round_up(bound * 8, 256), cnt_b2 = round_up(bound * 4, 256), tpre_b = round_up((bound + 1) * 8, 256);
+            BPE_TRY(bpe_buf_reserve(ctx, tok->offs_batch, starts_b + cnt_b2 + tpre_b + scan_tmp_elems_host(bound) * sizeof(u64)));
+            uint8_t *ob = (uint8_t *)tok->offs_batch.p;
+            u64 *starts = (u64 *)ob, *tpre = (u64 *)(ob + starts_b + cnt_b2), *otmp = (u64 *)(ob + starts_b + cnt_b2 + tpre_b);
+            u32 *ocnt = (u32 *)(ob + starts_b);
+            const unsigned gmax = (unsigned)((u64)ctx->sm_count * bpe_grid_mult(64));
+            const unsigned gq = (unsigned)std::min<u64>(gmax, (bound + 255) / 256);
+            KLAUNCH(k_enc_drop_starts, (unsigned)std::min<u64>(gmax, (b_hi - b_lo + 255) / 256), 256, 0, st, (const u32 *)ctx->flags.p, pre, ord[b],
+                    b_lo, b_hi, starts);
+            KLAUNCH(k_enc_off_count, gq, 256, 0, st, t, vals, bound, ocnt);
+            launch_scan_u32(ocnt, bound, tpre, otmp, st);
+            o.starts = starts; o.tpre = tpre;
+            if (o.chars) KLAUNCH(k_enc_offsets<true>, gq, 256, 0, st, t, o, (const u32 *)ctx->flags.p, vals, n, bound, total_tokens, dev_cap);
+            else KLAUNCH(k_enc_offsets<false>, gq, 256, 0, st, t, o, (const u32 *)ctx->flags.p, vals, n, bound, total_tokens, dev_cap);
+            CUDA_TRY(ctx, cudaGetLastError());
+        }
         launch_peek(host + 1, (u64 *)tok->ctr.p + 7, 1, st);
         CUDA_TRY(ctx, cudaStreamSynchronize(st));
         const u64 batch_tokens = host[0], err_ord = host[1];
@@ -1570,6 +1706,13 @@ static int encode_core(bpe_tok *tok, u64 n, int out_dtype, void *out_dev, u64 de
         cudaEventElapsedTime(&f, evs[1], evs[2]); ms_bpe += f;
         cudaEventElapsedTime(&f, evs[2], evs[3]); ms_emit += f;
         total_tokens += batch_tokens;
+    }
+    if (offs) {                                  // characters of the next chunk's first document in this one
+        u64 *host = (u64 *)ctx->pinned;
+        KLAUNCH(k_enc_lead_span, 1, 1, 0, st, o.lmask, o.lpre, next_keep ? 0 : std::min(next_ds, n), n, host);
+        CUDA_TRY(ctx, cudaGetLastError());
+        CUDA_TRY(ctx, cudaStreamSynchronize(st));
+        offs->carry = (next_keep ? offs->carry : 0) + host[0];
     }
     int e3 = tm.mark();
     *n_out = total_tokens;
@@ -1687,10 +1830,10 @@ static std::vector<EncChunk> doc_chunks(const bpe_tok *tok, const uint8_t *t, u6
 //   bpe_encode:       a chunk is uploaded straight into the arena the kernels read next (the two arenas alternate)
 //   bpe_encode_batch: a chunk is uploaded as it is into one of two staging buffers; on the compute stream k_enc_expand_docs moves it
 //                     into the arena with a boundary byte after every document and sets the boundary bitmask
-// drop: BPE-dropout (thr and seed_mix set), or null.
+// drop: BPE-dropout (thr and seed_mix set), or null.  offs_out (with out): the tokens' spans in `unit` (BPE_OFF_*), downloaded with the ids.
 static int encode_pipeline(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs, uint64_t n_docs, int out_dtype,
                            void *out, uint64_t cap, uint64_t *n_out, uint64_t *id_offs_out, bpe_encode_stats *stats,
-                           const EncDrop *drop = nullptr) {
+                           const EncDrop *drop = nullptr, int unit = BPE_OFF_BYTES, int64_t *offs_out = nullptr) {
     BPE_TRY(encode_check_args(tok, text_host, n, out_dtype, n_out));
     bpe_ctx *ctx = tok->ctx;
     cudaStream_t st = ctx->stream;
@@ -1734,8 +1877,9 @@ static int encode_pipeline(bpe_tok *tok, const uint8_t *text_host, uint64_t n, c
     // touches a buffer is ordered by events, and every chunk ends with a host-side synchronisation of the compute stream)
     CUDA_TRY(ctx, cudaStreamSynchronize(st));
     BPE_TRY(upload(0, doc_offs ? *sbuf[0] : *tbuf[0]));
-    u64 total = 0;
+    u64 total = 0, char_carry = 0;
     int rc = BPE_OK;
+    const bool want_offs = out && offs_out;
     for (size_t k = 0; k < m && rc == BPE_OK; k++) {
         const int cur = (int)(k & 1);
         const EncChunk &ch = chunks[k];
@@ -1748,9 +1892,21 @@ static int encode_pipeline(bpe_tok *tok, const uint8_t *text_host, uint64_t n, c
         if (out) {
             rc = bpe_buf_reserve(ctx, *obuf[cur], std::max<size_t>((m > 1 ? max_chunk : len) * esz, 16));
             if (rc != BPE_OK) { if (swap) std::swap(ctx->text, ctx->text_alt); break; }
+            if (want_offs) rc = bpe_buf_reserve(ctx, tok->offs_out[cur], std::max<size_t>((m > 1 ? max_chunk : len) * 16, 16));
+            if (rc != BPE_OK) { if (swap) std::swap(ctx->text, ctx->text_alt); break; }
             CUDA_TRY(ctx, cudaStreamWaitEvent(st, ctx->ev_out[cur], 0));   // its previous download has finished
             odev = obuf[cur]->p;
         }
+        // token offsets: the chunk's place in the caller's text; the next chunk's first document (ch.db) starts in this one unless none ends here
+        EncOffs och{};
+        const uint64_t *dofs = doc_offs ? doc_offs : one_doc;
+        if (want_offs) {
+            och.chars = unit == BPE_OFF_CHARS; och.out = (long long *)tok->offs_out[cur].p; och.lo = ch.lo; och.da = ch.da; och.carry = char_carry;
+            och.doffs = doc_offs ? (const u64 *)ctx->doc_offs.p : nullptr;
+        }
+        EncOffs *op = want_offs ? &och : nullptr;
+        const bool next_keep = ch.db == ch.da;
+        const u64 next_ds = next_keep ? 0 : dofs[ch.db] - ch.lo + (doc_offs ? ch.db - ch.da : 0);
         uint64_t nt = 0;
         EncDrop dch{};                           // the chunk's place in the caller's text, for the dropout offsets
         if (drop) { dch = *drop; dch.lo = ch.lo; dch.da = ch.da; dch.doffs = doc_offs ? (const u64 *)ctx->doc_offs.p : nullptr; }
@@ -1766,7 +1922,7 @@ static int encode_pipeline(bpe_tok *tok, const uint8_t *text_host, uint64_t n, c
                     (uint8_t *)ctx->text.p + BPE_PAD, (u32 *)ctx->doc_bmask.p, (uint8_t)tok->doc_sep);
             CUDA_TRY(ctx, cudaGetLastError());
             const DocBounds db{(const u32 *)ctx->doc_bmask.p, id_dev + ch.da + 1, total};
-            rc = encode_core(tok, an, out_dtype, odev, len, &nt, stats, &db, dp);
+            rc = encode_core(tok, an, out_dtype, odev, len, &nt, stats, &db, dp, op, next_ds, next_keep);
             if (rc == BPE_ERR_UTF8 || rc == BPE_ERR_KEY) {      // arena offset -> offset in the caller's text: minus the boundaries before it
                 const u64 p = (u64)ctx->err_detail;
                 u64 a = 0, b = nb;                              // boundaries j < a lie before p (boundary j sits at ends[j] - lo + j)
@@ -1778,7 +1934,7 @@ static int encode_pipeline(bpe_tok *tok, const uint8_t *text_host, uint64_t n, c
             }
             if (rc != BPE_OK) break;
         } else {
-            rc = encode_core(tok, len, out_dtype, odev, len, &nt, stats, nullptr, dp);
+            rc = encode_core(tok, len, out_dtype, odev, len, &nt, stats, nullptr, dp, op, next_ds, next_keep);
             if (swap) std::swap(ctx->text, ctx->text_alt);
             if (rc != BPE_OK) { ctx->err_detail += (int64_t)ch.lo; break; }
         }
@@ -1787,9 +1943,11 @@ static int encode_pipeline(bpe_tok *tok, const uint8_t *text_host, uint64_t n, c
             CUDA_TRY(ctx, cudaEventRecord(ctx->ev_done, st));
             CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->s_out, ctx->ev_done, 0));
             if (w) CUDA_TRY(ctx, cudaMemcpyAsync((uint8_t *)out + total * esz, odev, w * esz, cudaMemcpyDeviceToHost, ctx->s_out));
+            if (w && want_offs) CUDA_TRY(ctx, cudaMemcpyAsync(offs_out + 2 * total, och.out, w * 16, cudaMemcpyDeviceToHost, ctx->s_out));
             CUDA_TRY(ctx, cudaEventRecord(ctx->ev_out[cur], ctx->s_out));
         }
         total += nt;
+        char_carry = och.carry;
     }
     cudaStreamSynchronize(ctx->s_in);
     cudaStreamSynchronize(ctx->s_out);
@@ -1816,7 +1974,7 @@ BPE_API int bpe_encode(bpe_tok *tok, const uint8_t *text_host, uint64_t n, int o
 
 static int encode_batch_impl(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
                              int out_dtype, void *out, uint64_t cap, uint64_t *n_out, uint64_t *id_offs_out, bpe_encode_stats *stats,
-                             const EncDrop *drop) {
+                             const EncDrop *drop, int unit = BPE_OFF_BYTES, int64_t *offs_out = nullptr) {
     if (!tok || !n_out || !id_offs_out || (n_docs && !doc_offs_host)) return BPE_ERR_ARG;
     bpe_ctx *ctx = tok->ctx;
     for (uint64_t j = 0; j < n_docs; j++)
@@ -1831,7 +1989,7 @@ static int encode_batch_impl(bpe_tok *tok, const uint8_t *text_host, uint64_t n,
         id_offs_out[0] = 0;
         return BPE_OK;
     }
-    return encode_pipeline(tok, text_host, n, doc_offs_host, n_docs, out_dtype, out, cap, n_out, id_offs_out, stats, drop);
+    return encode_pipeline(tok, text_host, n, doc_offs_host, n_docs, out_dtype, out, cap, n_out, id_offs_out, stats, drop, unit, offs_out);
 }
 
 BPE_API int bpe_encode_batch(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
@@ -1867,6 +2025,45 @@ BPE_API int bpe_encode_batch_dropout(bpe_tok *tok, const uint8_t *text_host, uin
     EncDrop d;
     BPE_TRY(dropout_args(tok, p, seed, &d));
     return encode_batch_impl(tok, text_host, n, doc_offs_host, n_docs, out_dtype, out, cap, n_out, id_offs_out, stats, d.thr ? &d : nullptr);
+}
+
+// ---- token offsets: the ids of the four calls above and a span of the input for every token -------------------------------------
+static int offsets_args(bpe_tok *tok, int unit, const void *out, const int64_t *offs_out) {
+    if (!tok) return BPE_ERR_ARG;
+    if (unit != BPE_OFF_BYTES && unit != BPE_OFF_CHARS) return bpe_set_error(tok->ctx, BPE_ERR_ARG, "unknown offset unit %d", unit);
+    if (out && !offs_out) return bpe_set_error(tok->ctx, BPE_ERR_ARG, "offs_out is null");
+    return BPE_OK;
+}
+
+BPE_API int bpe_encode_offsets(bpe_tok *tok, const uint8_t *text_host, uint64_t n, int out_dtype, void *out, uint64_t cap, uint64_t *n_out,
+                               int unit, int64_t *offs_out, bpe_encode_stats *stats) {
+    BPE_TRY(offsets_args(tok, unit, out, offs_out));
+    return encode_pipeline(tok, text_host, n, nullptr, 0, out_dtype, out, cap, n_out, nullptr, stats, nullptr, unit, offs_out);
+}
+
+BPE_API int bpe_encode_batch_offsets(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
+                                     int out_dtype, void *out, uint64_t cap, uint64_t *n_out, uint64_t *id_offs_out, int unit,
+                                     int64_t *offs_out, bpe_encode_stats *stats) {
+    BPE_TRY(offsets_args(tok, unit, out, offs_out));
+    return encode_batch_impl(tok, text_host, n, doc_offs_host, n_docs, out_dtype, out, cap, n_out, id_offs_out, stats, nullptr, unit, offs_out);
+}
+
+BPE_API int bpe_encode_dropout_offsets(bpe_tok *tok, const uint8_t *text_host, uint64_t n, double p, uint64_t seed, int out_dtype, void *out,
+                                       uint64_t cap, uint64_t *n_out, int unit, int64_t *offs_out, bpe_encode_stats *stats) {
+    BPE_TRY(offsets_args(tok, unit, out, offs_out));
+    EncDrop d;
+    BPE_TRY(dropout_args(tok, p, seed, &d));
+    return encode_pipeline(tok, text_host, n, nullptr, 0, out_dtype, out, cap, n_out, nullptr, stats, d.thr ? &d : nullptr, unit, offs_out);
+}
+
+BPE_API int bpe_encode_batch_dropout_offsets(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
+                                             double p, uint64_t seed, int out_dtype, void *out, uint64_t cap, uint64_t *n_out,
+                                             uint64_t *id_offs_out, int unit, int64_t *offs_out, bpe_encode_stats *stats) {
+    BPE_TRY(offsets_args(tok, unit, out, offs_out));
+    EncDrop d;
+    BPE_TRY(dropout_args(tok, p, seed, &d));
+    return encode_batch_impl(tok, text_host, n, doc_offs_host, n_docs, out_dtype, out, cap, n_out, id_offs_out, stats, d.thr ? &d : nullptr,
+                             unit, offs_out);
 }
 
 BPE_API int bpe_encode_dev(bpe_tok *tok, const uint8_t *text_dev, uint64_t n, int out_dtype, void *out_dev, uint64_t cap, uint64_t *n_out,

@@ -3,6 +3,7 @@
     Tokenizer(vocab, merges, special_tokens).encode(str, *, dropout=0.0, seed=0) -> list[int]
                                             .encode_batch(Sequence[str]) -> list[list[int]]
                                             .encode_iterable(Iterable[str]) -> Iterator[int]
+                                            .encode_with_offsets(str) -> (list[int], list[(start, end)])
                                             .decode(list[int]) -> str
 
 encode / decode run on the GPU through the C ABI (bpe_tok_create / bpe_encode / bpe_decode in
@@ -58,6 +59,16 @@ def _check_dropout(dropout, seed) -> Tuple[float, int]:
     if isinstance(seed, bool) or not isinstance(seed, (int, np.integer)) or not 0 <= int(seed) < 2**64:
         raise ValueError("seed must be an integer in [0, 2**64), got %r" % (seed,))
     return p, int(seed)
+
+
+_UNITS = {"byte": _lib.OFF_BYTES, "char": _lib.OFF_CHARS}
+
+
+def _check_unit(unit) -> int:
+    """Offset unit of the *_offsets calls: "byte" (offsets into the UTF-8 bytes) or "char" (Python str indices)."""
+    if not isinstance(unit, str) or unit not in _UNITS:
+        raise ValueError("unit must be 'byte' or 'char', got %r" % (unit,))
+    return _UNITS[unit]
 
 
 class Tokenizer:
@@ -212,6 +223,39 @@ class Tokenizer:
         self.last_stats = stats.as_dict()
         return out[: n_out.value]
 
+    def encode_offsets_to_numpy(self, data, dtype=np.int32, *, unit: str = "byte", dropout: float = 0.0,
+                                seed: int = 0) -> Tuple[np.ndarray, np.ndarray]:
+        """encode_to_numpy's ids and int64 spans [n, 2] of `data` in `unit` ("byte" or "char"), computed on the device in the same pass:
+        token i came from data[start:end] ("byte"), or text[start:end] holds its bytes ("char"; a character that several tokens split
+        belongs to each of them).  See bpe_encode_offsets in include/bpe_sm100.h."""
+        code_unit = _check_unit(unit)
+        dropout, seed = _check_dropout(dropout, seed)
+        tok = self._device_tok()
+        ctx = self._tok_ctx
+        L = _lib.lib()
+        arr = _lib.as_u8(data)
+        code = {np.dtype(np.uint16): _lib.DTYPE_U16, np.dtype(np.int32): _lib.DTYPE_I32}[np.dtype(dtype)]
+        out = np.empty(max(arr.size, 1), dtype=dtype)             # a token covers at least one byte
+        spans = np.empty((out.size, 2), dtype=np.int64)
+        n_out = C.c_uint64(0)
+        stats = _lib.EncodeStats()
+        src = (tok, _lib.ptr(arr) if arr.size else None, arr.size)
+        with ctx.lock:
+            if dropout:
+                rc = L.bpe_encode_dropout_offsets(*src, dropout, seed, code, _lib.ptr(out), out.size, C.byref(n_out), code_unit, _lib.ptr(spans),
+                                                  C.byref(stats))
+            else:
+                rc = L.bpe_encode_offsets(*src, code, _lib.ptr(out), out.size, C.byref(n_out), code_unit, _lib.ptr(spans), C.byref(stats))
+            if rc != _lib.BPE_OK:
+                self._raise(ctx, rc, arr)
+        self.last_stats = stats.as_dict()
+        return out[: n_out.value], spans[: n_out.value]
+
+    def encode_with_offsets(self, text: str, *, dropout: float = 0.0, seed: int = 0) -> Tuple[List[int], List[Tuple[int, int]]]:
+        """encode(text)'s ids and the character span (start, end) of every token in `text` (encode_offsets_to_numpy, unit="char")."""
+        ids, spans = self.encode_offsets_to_numpy(text.encode("utf-8"), np.int32, unit="char", dropout=dropout, seed=seed)
+        return ids.tolist(), list(map(tuple, spans.tolist()))
+
     def encode_into(self, data, out: np.ndarray) -> int:
         """encode_to_numpy into a caller-owned array (uint16 or int32; page-locked for PCIe-speed downloads).  Returns the count."""
         tok = self._device_tok()
@@ -257,7 +301,30 @@ class Tokenizer:
             raise bad
         return self._encode_batch_packed(blob, offs, dtype, texts, **kw)
 
-    def _encode_batch_packed(self, blob: np.ndarray, offs: np.ndarray, dtype, texts=None, drop=(0.0, 0)):
+    def encode_batch_offsets_to_numpy(self, texts: Sequence[str | bytes], dtype=np.int32, *, unit: str = "byte", dropout: float = 0.0,
+                                      seed: int = 0) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """encode_batch_to_numpy's ids and document offsets with the int64 span [n, 2] of every token in `unit` ("byte" / "char"),
+        relative to its document's start: (ids, spans, offsets), and document j's tokens are [offsets[j], offsets[j + 1]).  Document j's
+        spans are those of encode_offsets_to_numpy(texts[j]); the errors are those of encode_batch_to_numpy."""
+        code_unit = _check_unit(unit)
+        drop = _check_dropout(dropout, seed)
+        kw = {"drop": drop} if drop[0] else {}
+        texts = list(texts)
+        blob, offs, bad = _pack_documents(texts)
+        if bad is not None:                      # as in encode_batch_to_numpy
+            self._encode_batch_packed(blob, offs, dtype, **kw)
+            raise bad
+        return self._encode_batch_packed(blob, offs, dtype, texts, unit=code_unit, **kw)
+
+    def encode_batch_with_offsets(self, texts: Sequence[str], *, dropout: float = 0.0,
+                                  seed: int = 0) -> List[Tuple[List[int], List[Tuple[int, int]]]]:
+        """[self.encode_with_offsets(t) for t in texts] in one device pass (encode_batch_offsets_to_numpy, unit="char")."""
+        ids, spans, o = self.encode_batch_offsets_to_numpy(texts, np.int32, unit="char", dropout=dropout, seed=seed)
+        flat, sp, o = ids.tolist(), list(map(tuple, spans.tolist())), o.tolist()
+        return [(flat[o[j]: o[j + 1]], sp[o[j]: o[j + 1]]) for j in range(len(o) - 1)]
+
+    def _encode_batch_packed(self, blob: np.ndarray, offs: np.ndarray, dtype, texts=None, drop=(0.0, 0), unit=None):
+        """(ids, id offsets), or with an offset unit (_lib.OFF_*) (ids, spans, id offsets)."""
         tok = self._device_tok()
         ctx = self._tok_ctx
         L = _lib.lib()
@@ -268,7 +335,15 @@ class Tokenizer:
         n_out = C.c_uint64(0)
         stats = _lib.EncodeStats()
         with ctx.lock:
-            if drop[0]:
+            if unit is not None:
+                spans = np.empty((out.size, 2), dtype=np.int64)
+                args = (tok, _lib.ptr(blob) if blob.size else None, blob.size, _lib.ptr(offs), n_docs)
+                tail = (code, _lib.ptr(out), out.size, C.byref(n_out), _lib.ptr(id_offs), unit, _lib.ptr(spans), C.byref(stats))
+                if drop[0]:
+                    rc = L.bpe_encode_batch_dropout_offsets(*args, drop[0], drop[1], *tail)
+                else:
+                    rc = L.bpe_encode_batch_offsets(*args, *tail)
+            elif drop[0]:
                 rc = L.bpe_encode_batch_dropout(tok, _lib.ptr(blob) if blob.size else None, blob.size, _lib.ptr(offs), n_docs, drop[0], drop[1],
                                                 code, _lib.ptr(out), out.size, C.byref(n_out), _lib.ptr(id_offs), C.byref(stats))
             else:
@@ -286,6 +361,8 @@ class Tokenizer:
             if rc != _lib.BPE_OK:
                 self._raise(ctx, rc)
         self.last_stats = stats.as_dict()
+        if unit is not None:
+            return out[: n_out.value], spans[: n_out.value], id_offs.astype(np.int64)
         return out[: n_out.value], id_offs.astype(np.int64)
 
     def encode_sharded(self, data, dtype=np.uint16, group=None):
