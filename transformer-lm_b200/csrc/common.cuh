@@ -64,6 +64,7 @@ int bpe_set_error(bpe_ctx *ctx, int code, const char *fmt, ...);
 // synchronise the device, and every call of the library asks for the same sizes again.
 int bpe_buf_reserve(bpe_ctx *ctx, DevBuf &b, size_t bytes);       // grow-only, contents NOT preserved
 int bpe_buf_alloc(bpe_ctx *ctx, DevBuf &b, size_t bytes);         // (re)size to about `bytes` (may shrink), contents NOT preserved
+static inline int alloc_exact(bpe_ctx *ctx, DevBuf &b, size_t bytes) { return bpe_buf_alloc(ctx, b, bytes ? bytes : 256); }   // (0 bytes: still a buffer)
 void bpe_buf_free(bpe_ctx *ctx, DevBuf &b);                       // back to the pool
 void bpe_pool_trim(bpe_ctx *ctx);                                 // cudaFree everything cached
 

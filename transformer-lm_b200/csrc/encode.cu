@@ -26,12 +26,6 @@
 #include "hashtab.cuh"
 #include "scan.cuh"
 
-#define SHORT_MAX 7u
-#define META_EMPTY 0xFFFFFFFFFFFFFFFFull
-#define META_LEN_BITS 24
-#define META_LEN_MASK ((1ull << META_LEN_BITS) - 1)
-#define META_POOL_BIT (1ull << 39)
-#define MAX_TOKEN_LEN ((1u << META_LEN_BITS) - 2)
 #define REF_LONG 0x80000000u
 #define REF_MED 0x40000000u
 #define REF_SLOT(r) ((r) & 0x3FFFFFFFu)
@@ -55,38 +49,25 @@
 #define RANK_NONE 0xFFFFFFFFFFFFFFFFull
 #define MKEY_EMPTY 0xFFFFFFFFFFFFFFFFull
 
-struct __align__(16) SSlot { u64 key, val; };
-struct __align__(32) LSlot { u64 meta, hash, val, pad; };
-struct __align__(32) MSlot { u64 k0, k1, val, pad; };     // pretokens of 8..15 bytes: the 16-byte key IS the token (k0 = bytes 0-7, k1 = bytes 8-14 | len << 56)
-
-struct EncTables {
+// the pretoken cache: the tables of hashtab.cuh, payload = the cached value (VAL_NONE in an empty slot).  Key and value share a slot,
+// so a lookup brings the value in with the key (one 32-byte sector); pool = persistent key bytes of long pretokens.
+struct EncTables : PtTables {
     const ulonglong2 *mtab; u64 mmask;           // pair -> {key = a<<32|b, (rank << 32) | result symbol}
     const int32_t *mpairs;                       // operand symbols of merge j
     const int32_t *sym_to_id;
-    // key and cached value share a slot, so the lookup brings the value in with the key (one 32-byte sector)
-    SSlot *stab; u64 scap;                       // pretokens of <= 7 bytes: the key is the token (bytes | len << 56)
-    MSlot *medtab; u64 medcap;                   // 8..15 bytes: one sector per lookup, claimed and published by one 128-bit CAS (as in training)
-    LSlot *ltab; u64 lcap;                       // >= 16 bytes: (offset:40 | len:24) of the bytes, 64-bit hash filter
-    const uint8_t *text;                         // payload of the current text arena
-    uint8_t *kpool;                              // persistent key bytes of long pretokens
     u32 *ipool;                                  // token ids of pretokens with more than 3 tokens
     u32 *todo;                                   // slots claimed in this batch (REF_LONG = long table)
     // hot table (see k_enc_hot_build): hot_nb buckets of two 16-byte keys (one sector), their cached values in hval; 0 = none
     const ulonglong2 *hot; const u64 *hval; u64 hot_nb;
     const ulonglong2 *sm_img;                    // LK_SM_SLOTS x {key, value}: image of the lookup kernel's shared-memory value cache (or null)
     u32 *scnt, *mcnt;                            // per-slot hit counters (short, medium) while the cache is being sampled for the hot table (else null)
-    // [0]=n_short [1]=n_long [2]=todo count [3]=table overflow [4]=kpool cursor [5]=ipool cursor [6]=pretoken too long
+    // [0]=n_short [1]=n_long [2]=todo count [3]=table overflow [4]=key pool cursor [5]=ipool cursor [6]=pretoken too long
     // [7]=smallest ordinal (in the text of the call) of a pretoken whose value is a KeyError  [8]=n_medium  [9]=step tickets of the lookup kernel
     u64 *ctr;
     // document boundaries of bpe_encode_batch (all null for bpe_encode): bit per arena byte, boundaries before every 512-byte group,
     // id_offs[j] = index of the first id after document j of the chunk (id_base + its offset in the chunk's output)
     const u32 *bmask; const u64 *bpre; u64 *id_offs; u64 id_base;
 };
-
-__device__ __forceinline__ const uint8_t *enc_rep_ptr(const EncTables &t, u64 meta) {
-    u64 off = meta >> META_LEN_BITS;
-    return (off & META_POOL_BIT) ? t.kpool + (off & ~META_POOL_BIT) : t.text + off;
-}
 
 // ---- pair -> rank ---------------------------------------------------------------------------------
 __device__ __forceinline__ u64 rank_lookup(const EncTables &t, u32 a, u32 b) {
@@ -116,89 +97,37 @@ __global__ void __launch_bounds__(256) k_enc_build_ranks(ulonglong2 *__restrict_
 }
 
 // ---- pretoken cache: lookup or claim -----------------------------------------------------------------
-// Returns the cached value of the pretoken, or (VAL_FWD << 60 | slot reference) when it is not computed yet.
+// Returns the cached value of the pretoken, or (VAL_FWD << 60 | slot reference) when it is not computed yet (a value read early can
+// only be "not computed yet", which yields a forward reference that is resolved after the BPE kernels: correct either way).  A claim
+// counts the new key and queues its slot for the BPE kernels; a sampled lookup (scnt / mcnt set) bumps the slot's hit counter.
 __device__ __forceinline__ u64 enc_short_get(const EncTables &t, u64 key) {
-    u64 mask = t.scap - 1;
-    u64 s = mix64(key) & mask;
-    for (u64 probes = 0; probes < t.scap; probes++) {
-        const ulonglong2 kv = *reinterpret_cast<const ulonglong2 *>(&t.stab[s]);
-        u64 k = kv.x;
-        if (k == 0) {
-            u64 old = atomicCAS(&t.stab[s].key, 0ull, key);
-            if (old == 0) {
-                atomicAdd(&t.ctr[0], 1ull);
-                u64 q = atomicAdd(&t.ctr[2], 1ull);
-                t.todo[q] = (u32)s;
-                if (t.scnt) atomicAdd(&t.scnt[s], 1u);
-                return (VAL_FWD << 60) | (u32)s;
-            }
-            k = old;
-            if (k == key) { if (t.scnt) atomicAdd(&t.scnt[s], 1u); return (VAL_FWD << 60) | (u32)s; }   // inserted by another thread just now: not computed yet
-        }
-        if (k == key) { if (t.scnt) atomicAdd(&t.scnt[s], 1u); return kv.y != VAL_NONE ? kv.y : ((VAL_FWD << 60) | (u32)s); }
-        s = (s + 1) & mask;
-    }
-    t.ctr[3] = 1;
-    return 0;
+    return short_find_or_claim<true>(t, key, t.ctr,
+        [&](u64 s) {
+            atomicAdd(&t.ctr[0], 1ull);
+            t.todo[atomicAdd(&t.ctr[2], 1ull)] = (u32)s;
+            if (t.scnt) atomicAdd(&t.scnt[s], 1u);
+            return (VAL_FWD << 60) | (u32)s;
+        },
+        [&](u64 s, u64 v) { if (t.scnt) atomicAdd(&t.scnt[s], 1u); return v != VAL_NONE ? v : ((VAL_FWD << 60) | (u32)s); });
 }
-
 __device__ __forceinline__ u64 enc_med_get(const EncTables &t, u64 k0, u64 k1) {
-    const u64 mask = t.medcap - 1;
-    u64 s = mix64(k0 ^ (k1 * 0x9E3779B97F4A7C15ull)) & mask;
-    for (u64 probes = 0; probes < t.medcap; probes++) {
-        const ulonglong2 kk = *reinterpret_cast<const ulonglong2 *>(&t.medtab[s]);
-        const u64 vv = t.medtab[s].val;          // (same sector; a value read early can only be "not computed yet")
-        u64 a = kk.x, b = kk.y;
-        if ((a | b) == 0) {                      // (k1 carries the length: a real key is never all zero)
-            asm volatile("{\n .reg .b128 c, n, d;\n mov.b128 c, {%3, %4};\n mov.b128 n, {%5, %6};\n atom.global.cas.b128 d, [%2], c, n;\n mov.b128 {%0, %1}, d;\n}"
-                         : "=l"(a), "=l"(b) : "l"(&t.medtab[s]), "l"(0ull), "l"(0ull), "l"(k0), "l"(k1) : "memory");
-            if ((a | b) == 0) {
-                atomicAdd(&t.ctr[8], 1ull);
-                u64 q = atomicAdd(&t.ctr[2], 1ull);
-                t.todo[q] = (u32)s | REF_MED;
-                if (t.mcnt) atomicAdd(&t.mcnt[s], 1u);
-                return (VAL_FWD << 60) | (u32)s | REF_MED;
-            }
-            if (a == k0 && b == k1) { if (t.mcnt) atomicAdd(&t.mcnt[s], 1u); return (VAL_FWD << 60) | (u32)s | REF_MED; }
-        }
-        if (a == k0 && b == k1) { if (t.mcnt) atomicAdd(&t.mcnt[s], 1u); return vv != VAL_NONE ? vv : ((VAL_FWD << 60) | (u32)s | REF_MED); }
-        s = (s + 1) & mask;
-    }
-    t.ctr[3] = 1;
-    return 0;
+    return medium_find_or_claim<true>(t, k0, k1, t.ctr,
+        [&](u64 s) {
+            atomicAdd(&t.ctr[8], 1ull);
+            t.todo[atomicAdd(&t.ctr[2], 1ull)] = (u32)s | REF_MED;
+            if (t.mcnt) atomicAdd(&t.mcnt[s], 1u);
+            return (VAL_FWD << 60) | (u32)s | REF_MED;
+        },
+        [&](u64 s, u64 v) { if (t.mcnt) atomicAdd(&t.mcnt[s], 1u); return v != VAL_NONE ? v : ((VAL_FWD << 60) | (u32)s | REF_MED); });
 }
-
 __device__ __forceinline__ u64 enc_long_get(const EncTables &t, const uint8_t *p, u32 len, u64 off_meta) {
-    u64 h = hash_long(p, len);
-    u64 mask = t.lcap - 1;
-    u64 s = h & mask;
-    u64 mine = (off_meta << META_LEN_BITS) | len;
-    for (u64 probes = 0; probes < t.lcap; probes++) {
-        // the whole 32-byte slot in one round trip (a value read early can only be "not computed yet", which yields a forward
-        // reference that is resolved after the BPE kernel: correct either way)
-        const ulonglong2 mh = *reinterpret_cast<const ulonglong2 *>(&t.ltab[s]);
-        const ulonglong2 vp = *(reinterpret_cast<const ulonglong2 *>(&t.ltab[s]) + 1);
-        u64 m = mh.x, hh = mh.y;
-        if (m == META_EMPTY) {
-            u64 old = atomicCAS(&t.ltab[s].meta, META_EMPTY, mine);
-            if (old == META_EMPTY) {
-                t.ltab[s].hash = h;
-                atomicAdd(&t.ctr[1], 1ull);
-                u64 q = atomicAdd(&t.ctr[2], 1ull);
-                t.todo[q] = (u32)s | REF_LONG;
-                return (VAL_FWD << 60) | (u32)s | REF_LONG;
-            }
-            m = old;
-            hh = *((volatile u64 *)&t.ltab[s].hash);
-        }
-        if ((m & META_LEN_MASK) == len && (hh == 0 || hh == h) && bytes_equal(enc_rep_ptr(t, m), p, len)) {
-            const u64 v = vp.x;
-            return v != VAL_NONE ? v : ((VAL_FWD << 60) | (u32)s | REF_LONG);
-        }
-        s = (s + 1) & mask;
-    }
-    t.ctr[3] = 1;
-    return 0;
+    return long_find_or_claim<true>(t, p, len, off_meta, t.ctr,
+        [&](u64 s) {
+            atomicAdd(&t.ctr[1], 1ull);
+            t.todo[atomicAdd(&t.ctr[2], 1ull)] = (u32)s | REF_LONG;
+            return (VAL_FWD << 60) | (u32)s | REF_LONG;
+        },
+        [&](u64 s, u64 v) { return v != VAL_NONE ? v : ((VAL_FWD << 60) | (u32)s | REF_LONG); });
 }
 
 // ---- hot table ---------------------------------------------------------------------------------------------------------
@@ -209,7 +138,6 @@ __device__ __forceinline__ u64 enc_long_get(const EncTables &t, const uint8_t *p
 // stays in L2: a bucket is one sector holding two 16-byte keys (k0 = bytes 0-7, k1 = bytes 8-14 | len << 56; k1 = 0 and k0 = the
 // short-table key for <= 7 bytes), the values sit in an array beside it.  A key whose bucket is full simply stays with the big
 // tables, so a probe is exactly one sector.  Values are immutable once computed, so the copy never goes stale.
-__device__ __forceinline__ u64 enc_hot_bucket(u64 nb, u64 k0, u64 k1) { return ((mix64(k0 ^ (k1 * 0x9E3779B97F4A7C15ull)) >> 32) * nb) >> 32; }
 
 // ---- lookup: straight from the text and its start bits -------------------------------------------------------------------
 // vals[ordinal of the pretoken in the batch] = its cached value when the cache has it, else a forward reference to its slot
@@ -264,18 +192,10 @@ __device__ __forceinline__ void lookup_drain(const EncTables &t, LookupQueues &q
         bool ta = ha, tb = hb;                   // still to be looked up in the big tables
         u64 va = 0, vb = 0;
         if (t.hot_nb) {
-            const u64 ba = enc_hot_bucket(t.hot_nb, ka.x, ka.y), bb = enc_hot_bucket(t.hot_nb, kb.x, kb.y);
-            ulonglong2 a0 = make_ulonglong2(0, 0), a1 = a0, b0 = a0, b1 = a0;
-            if (ha) { a0 = __ldg(&t.hot[2 * ba]); a1 = __ldg(&t.hot[2 * ba + 1]); }
-            if (hb) { b0 = __ldg(&t.hot[2 * bb]); b1 = __ldg(&t.hot[2 * bb + 1]); }
-            if (ha) {
-                const bool m0 = a0.x == ka.x && a0.y == ka.y, m1 = a1.x == ka.x && a1.y == ka.y;
-                if (m0 || m1) { va = __ldg(&t.hval[2 * ba + (m1 ? 1 : 0)]); ta = false; }
-            }
-            if (hb) {
-                const bool m0 = b0.x == kb.x && b0.y == kb.y, m1 = b1.x == kb.x && b1.y == kb.y;
-                if (m0 || m1) { vb = __ldg(&t.hval[2 * bb + (m1 ? 1 : 0)]); tb = false; }
-            }
+            const u64 ba = hot_bucket(t.hot_nb, ka.x, ka.y), bb = hot_bucket(t.hot_nb, kb.x, kb.y);
+            const int ia = ha ? hot_find(t.hot, ba, ka.x, ka.y) : -1, ib = hb ? hot_find(t.hot, bb, kb.x, kb.y) : -1;
+            if (ia >= 0) { va = __ldg(&t.hval[2 * ba + ia]); ta = false; }
+            if (ib >= 0) { vb = __ldg(&t.hval[2 * bb + ib]); tb = false; }
         }
         if (ta) va = enc_queued_get(t, ka, xa, base);
         if (tb) vb = enc_queued_get(t, kb, xb, base);
@@ -376,7 +296,7 @@ __global__ void __launch_bounds__(LK_NT, 1) k_enc_lookup(EncTables t, const u32 
             const u64 k0 = (u64)__funnelshift_r(Y0, Y1, sh) | ((u64)__funnelshift_r(Y1, Y2, sh) << 32);
             const u64 k1 = (u64)__funnelshift_r(Y2, Y3, sh) | ((u64)__funnelshift_r(Y3, Y4, sh) << 32);
             bool q_s = act && !isb && len <= SHORT_MAX;
-            const bool q_m = act && !isb && len > SHORT_MAX && len <= 15u, q_l = act && !isb && len > 15u;
+            const bool q_m = act && !isb && len > SHORT_MAX && len <= MED_MAX, q_l = act && !isb && len > MED_MAX;
             const u64 key = (k0 & low_bytes_mask(len)) | ((u64)len << 56);               // (short pretokens)
             if (q_s) {
                 u32 slot = enc_sm_slot(key);
@@ -578,10 +498,10 @@ __global__ void __launch_bounds__(BPT_NT) k_enc_bpe_short(EncTables t, u64 n_tod
             const u64 m = t.ltab[slot].meta;
             n = (u32)(m & META_LEN_MASK);
             if (n > BPT_MAX) continue;           // the warp kernel's
-            const uint8_t *src = enc_rep_ptr(t, m);
+            const uint8_t *src = rep_ptr(t, m);
             // move the key bytes out of the (transient) text arena into the persistent key pool
             const u64 ko = atomicAdd(&t.ctr[4], (u64)n);
-            for (u32 i = 0; i < n; i++) { const u32 b = src[i]; t.kpool[ko + i] = (uint8_t)b; sym[i] = b; }
+            for (u32 i = 0; i < n; i++) { const u32 b = src[i]; t.pool[ko + i] = (uint8_t)b; sym[i] = b; }
             t.ltab[slot].meta = ((ko | META_POOL_BIT) << META_LEN_BITS) | n;
         } else {
             const u64 k = t.stab[slot].key;
@@ -606,18 +526,18 @@ __global__ void __launch_bounds__(256) k_enc_bpe(EncTables t, u64 n_todo) {
         const u64 m = t.ltab[slot].meta;
         const u32 len = (u32)(m & META_LEN_MASK);
         if (len <= BPT_MAX) continue;
-        const uint8_t *src = enc_rep_ptr(t, m);
+        const uint8_t *src = rep_ptr(t, m);
         // move the key bytes out of the (transient) text arena into the persistent key pool
         u64 ko = 0;
         if (lane == 0) ko = atomicAdd(&t.ctr[4], (u64)len);
         ko = __shfl_sync(0xffffffffu, ko, 0);
-        for (u32 i = lane; i < len; i += 32) t.kpool[ko + i] = src[i];
+        for (u32 i = lane; i < len; i += 32) t.pool[ko + i] = src[i];
         __syncwarp();
         if (lane == 0) t.ltab[slot].meta = ((ko | META_POOL_BIT) << META_LEN_BITS) | len;
         u64 off = 0;
         if (lane == 0) off = atomicAdd(&t.ctr[5], (u64)len);
         off = __shfl_sync(0xffffffffu, off, 0);
-        const u64 value = warp_bpe<false>(t, t.kpool + ko, t.ipool + off, nullptr, len, off, DropOcc{}, lane);
+        const u64 value = warp_bpe<false>(t, t.pool + ko, t.ipool + off, nullptr, len, off, DropOcc{}, lane);
         if (lane == 0) t.ltab[slot].val = value;
     }
 }
@@ -970,16 +890,9 @@ __global__ void __launch_bounds__(256) k_enc_hot_build(EncTables t, ulonglong2 *
             if ((k0 | k1) == 0) continue;
         }
         if (v == VAL_NONE || VAL_TAG(v) == VAL_FWD) continue;
-        const u64 b = enc_hot_bucket(nb, k0, k1);
-        u64 x, y; u32 w = 0;
-        asm volatile("{\n .reg .b128 c, n, d;\n mov.b128 c, {%3, %4};\n mov.b128 n, {%5, %6};\n atom.global.cas.b128 d, [%2], c, n;\n mov.b128 {%0, %1}, d;\n}"
-                     : "=l"(x), "=l"(y) : "l"(&hot[2 * b]), "l"(0ull), "l"(0ull), "l"(k0), "l"(k1) : "memory");
-        if ((x | y) != 0) {
-            w = 1;
-            asm volatile("{\n .reg .b128 c, n, d;\n mov.b128 c, {%3, %4};\n mov.b128 n, {%5, %6};\n atom.global.cas.b128 d, [%2], c, n;\n mov.b128 {%0, %1}, d;\n}"
-                         : "=l"(x), "=l"(y) : "l"(&hot[2 * b + 1]), "l"(0ull), "l"(0ull), "l"(k0), "l"(k1) : "memory");
-        }
-        if ((x | y) == 0) hval[2 * b + w] = v;
+        const u64 b = hot_bucket(nb, k0, k1);
+        const int w = hot_claim(hot, b, k0, k1);
+        if (w >= 0) hval[2 * b + w] = v;
     }
 }
 
@@ -1015,45 +928,18 @@ __global__ void __launch_bounds__(256) k_enc_sm_build(EncTables t, ulonglong2 *_
 }
 
 // ---- cache maintenance ---------------------------------------------------------------------------------
+// growth: every key of an old table into the bigger one
 __global__ void __launch_bounds__(256) k_enc_rehash_short(const SSlot *__restrict__ otab, u64 ocap, EncTables t) {
-    u64 mask = t.scap - 1;
-    for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < ocap; i += (u64)gridDim.x * blockDim.x) {
-        u64 k = otab[i].key;
-        if (!k) continue;
-        u64 s = mix64(k) & mask;
-        for (;;) {
-            if (t.stab[s].key == 0 && atomicCAS(&t.stab[s].key, 0ull, k) == 0) { t.stab[s].val = otab[i].val; break; }
-            s = (s + 1) & mask;
-        }
-    }
+    for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < ocap; i += (u64)gridDim.x * blockDim.x)
+        if (otab[i].key) short_insert_unique(t, otab[i].key, otab[i].val);
 }
 __global__ void __launch_bounds__(256) k_enc_rehash_long(const LSlot *__restrict__ otab, u64 ocap, EncTables t) {
-    u64 mask = t.lcap - 1;
-    for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < ocap; i += (u64)gridDim.x * blockDim.x) {
-        u64 m = otab[i].meta;
-        if (m == META_EMPTY) continue;
-        u64 s = otab[i].hash & mask;
-        for (;;) {
-            if (t.ltab[s].meta == META_EMPTY && atomicCAS(&t.ltab[s].meta, META_EMPTY, m) == META_EMPTY) {
-                t.ltab[s].hash = otab[i].hash; t.ltab[s].val = otab[i].val;
-                break;
-            }
-            s = (s + 1) & mask;
-        }
-    }
+    for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < ocap; i += (u64)gridDim.x * blockDim.x)
+        if (otab[i].meta != META_EMPTY) long_insert_unique(t, otab[i].meta, otab[i].hash, otab[i].val);
 }
-
 __global__ void __launch_bounds__(256) k_enc_rehash_med(const MSlot *__restrict__ otab, u64 ocap, EncTables t) {
-    const u64 mask = t.medcap - 1;
-    for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < ocap; i += (u64)gridDim.x * blockDim.x) {
-        const u64 k0 = otab[i].k0, k1 = otab[i].k1;
-        if ((k0 | k1) == 0) continue;
-        u64 s = mix64(k0 ^ (k1 * 0x9E3779B97F4A7C15ull)) & mask;
-        for (;;) {                               // keys are unique: claim the k1 word (never 0 for a real key), then fill in
-            if (t.medtab[s].k1 == 0 && atomicCAS(&t.medtab[s].k1, 0ull, k1) == 0ull) { t.medtab[s].k0 = k0; t.medtab[s].val = otab[i].val; break; }
-            s = (s + 1) & mask;
-        }
-    }
+    for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < ocap; i += (u64)gridDim.x * blockDim.x)
+        if ((otab[i].k0 | otab[i].k1) != 0) medium_insert_unique(t, otab[i].k0, otab[i].k1, otab[i].val);
 }
 
 // empty tables: short {0, VAL_NONE}, medium {0, 0, VAL_NONE, 0}, long {META_EMPTY, 0, VAL_NONE, 0}
@@ -1071,52 +957,29 @@ __global__ void __launch_bounds__(256) k_enc_clear_tables(EncTables t) {
     }
 }
 
-// Special tokens are pretokens of their own (tokenizer.py:119-122): pre-insert them with their id.
-// Their bytes sit at the start of the key pool (sp_offs are offsets into it).
+// Special tokens are pretokens of their own (tokenizer.py:119-122): pre-insert them with their id into the empty tables.
+// Their bytes sit at the start of the key pool (sp_offs are offsets into it).  Of specials with the same bytes the first one counts.
 __global__ void k_enc_insert_specials(EncTables t, const u32 *__restrict__ sp_offs, const long long *__restrict__ sp_ids, int n_sp) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_sp) return;
     u32 o = sp_offs[i], len = sp_offs[i + 1] - o;
     if (len == 0) return;
-    const uint8_t *p = t.kpool + o;
+    const uint8_t *p = t.pool + o;
+    for (int j = 0; j < i; j++)
+        if (sp_offs[j + 1] - sp_offs[j] == len && bytes_equal(t.pool + sp_offs[j], p, len)) return;
     long long id = sp_ids[i];
     u64 v;
     if (id < 0) v = (VAL_ERR << 60) | 0x80000000ull | (u32)i;
     else if ((u64)id < INLINE_ID_LIMIT) v = (1ull << 60) | (u64)id;
     else { u64 q = atomicAdd(&t.ctr[5], 1ull); t.ipool[q] = (u32)id; v = (VAL_EXT << 60) | (q << 24) | 1ull; }
-    if (len <= SHORT_MAX) {
-        u64 key = 0;
-        for (u32 k = 0; k < len; k++) key |= (u64)p[k] << (8 * k);
-        key |= (u64)len << 56;
-        u64 mask = t.scap - 1, s = mix64(key) & mask;
-        for (;;) {
-            u64 old = atomicCAS(&t.stab[s].key, 0ull, key);
-            if (old == 0) { atomicAdd(&t.ctr[0], 1ull); t.stab[s].val = v; return; }
-            if (old == key) return;              // duplicate special
-            s = (s + 1) & mask;
-        }
-    } else if (len <= 15) {
-        u64 k0 = 0, k1 = (u64)len << 56;
-        for (u32 k = 0; k < len; k++) { if (k < 8) k0 |= (u64)p[k] << (8 * k); else k1 |= (u64)p[k] << (8 * (k - 8)); }
-        const u64 mask = t.medcap - 1;
-        u64 s = mix64(k0 ^ (k1 * 0x9E3779B97F4A7C15ull)) & mask;
-        for (;;) {
-            u64 a, b;
-            asm volatile("{\n .reg .b128 c, n, d;\n mov.b128 c, {%3, %4};\n mov.b128 n, {%5, %6};\n atom.global.cas.b128 d, [%2], c, n;\n mov.b128 {%0, %1}, d;\n}"
-                         : "=l"(a), "=l"(b) : "l"(&t.medtab[s]), "l"(0ull), "l"(0ull), "l"(k0), "l"(k1) : "memory");
-            if ((a | b) == 0) { atomicAdd(&t.ctr[8], 1ull); t.medtab[s].val = v; return; }
-            if (a == k0 && b == k1) return;      // duplicate special
-            s = (s + 1) & mask;
-        }
+    if (len <= MED_MAX) {
+        u64 k0, k1;
+        pretoken_key(p, len, k0, k1);
+        if (k1 == 0) { short_insert_unique(t, k0, v); atomicAdd(&t.ctr[0], 1ull); }
+        else { medium_insert_unique(t, k0, k1, v); atomicAdd(&t.ctr[8], 1ull); }
     } else {
-        u64 h = hash_long(p, len), mask = t.lcap - 1, s = h & mask;
-        u64 mine = (((u64)o | META_POOL_BIT) << META_LEN_BITS) | len;
-        for (;;) {
-            u64 old = atomicCAS(&t.ltab[s].meta, META_EMPTY, mine);
-            if (old == META_EMPTY) { t.ltab[s].hash = h; atomicAdd(&t.ctr[1], 1ull); t.ltab[s].val = v; return; }
-            if ((old & META_LEN_MASK) == len && bytes_equal(enc_rep_ptr(t, old), p, len)) return;
-            s = (s + 1) & mask;
-        }
+        long_insert_unique(t, (((u64)o | META_POOL_BIT) << META_LEN_BITS) | len, hash_long(p, len), v);
+        atomicAdd(&t.ctr[1], 1ull);
     }
 }
 
@@ -1169,7 +1032,6 @@ struct bpe_tok {
     int doc_sep = -1;                            // boundary byte of bpe_encode_batch (-1: every candidate occurs in a special)
 };
 
-static int alloc_exact_e(bpe_ctx *ctx, DevBuf &b, size_t bytes) { return bpe_buf_alloc(ctx, b, bytes ? bytes : 256); }
 // grow keeping the first `used` bytes
 static int grow_keep(bpe_ctx *ctx, DevBuf &b, size_t need, size_t used) {
     if (need <= b.cap) return BPE_OK;
@@ -1193,7 +1055,7 @@ static EncTables enc_tables(bpe_tok *tok) {
     t.medtab = (MSlot *)tok->medtab.p; t.medcap = tok->medcap;
     t.ltab = (LSlot *)tok->ltab.p; t.lcap = tok->lcap;
     t.text = tok->ctx->text.p ? (const uint8_t *)tok->ctx->text.p + BPE_PAD : nullptr;
-    t.kpool = (uint8_t *)tok->kpool.p; t.ipool = (u32 *)tok->ipool.p; t.todo = (u32 *)tok->todo.p;
+    t.pool = (uint8_t *)tok->kpool.p; t.ipool = (u32 *)tok->ipool.p; t.todo = (u32 *)tok->todo.p;
     t.ctr = (u64 *)tok->ctr.p;
     t.hot = (const ulonglong2 *)tok->hot.p; t.hot_nb = tok->hot_nb; t.hval = (const u64 *)((const ulonglong2 *)tok->hot.p + 2 * tok->hot_nb);
     t.sm_img = tok->hot_built ? (const ulonglong2 *)tok->sm_img.p : nullptr;
@@ -1202,11 +1064,12 @@ static EncTables enc_tables(bpe_tok *tok) {
     return t;
 }
 
-static int cache_tables_alloc(bpe_tok *tok, u64 scap, u64 medcap, u64 lcap) {
+static int cache_tables_alloc(bpe_tok *tok, PtCaps cap) {
     bpe_ctx *ctx = tok->ctx;
-    BPE_TRY(alloc_exact_e(ctx, tok->stab, scap * sizeof(SSlot)));
-    BPE_TRY(alloc_exact_e(ctx, tok->medtab, medcap * sizeof(MSlot)));
-    BPE_TRY(alloc_exact_e(ctx, tok->ltab, lcap * sizeof(LSlot)));
+    const u64 scap = cap.s, medcap = cap.m, lcap = cap.l;
+    BPE_TRY(alloc_exact(ctx, tok->stab, scap * sizeof(SSlot)));
+    BPE_TRY(alloc_exact(ctx, tok->medtab, medcap * sizeof(MSlot)));
+    BPE_TRY(alloc_exact(ctx, tok->ltab, lcap * sizeof(LSlot)));
     tok->scap = scap; tok->medcap = medcap; tok->lcap = lcap;
     EncTables t = enc_tables(tok);
     KLAUNCH(k_enc_clear_tables, (unsigned)std::min<u64>((u64)ctx->sm_count * bpe_grid_mult(64), (std::max(scap, std::max(medcap, lcap)) + 255) / 256), 256, 0, ctx->stream, t);
@@ -1219,7 +1082,7 @@ static int cache_reset(bpe_tok *tok) {
     bpe_ctx *ctx = tok->ctx;
     cudaStream_t st = ctx->stream;
     BPE_TRY(bpe_buf_reserve(ctx, tok->ctr, 64 * sizeof(u64)));
-    BPE_TRY(cache_tables_alloc(tok, 1 << 16, 1 << 14, 1 << 14));
+    BPE_TRY(cache_tables_alloc(tok, pt_caps(0, 0, 0, 0, 0)));
     size_t spb = tok->sp_blob_h.size();
     BPE_TRY(bpe_buf_reserve(ctx, tok->kpool, std::max<size_t>(spb, 1) + (1 << 20)));
     BPE_TRY(bpe_buf_reserve(ctx, tok->ipool, ((size_t)tok->n_sp + (1 << 18)) * 4));
@@ -1255,12 +1118,12 @@ static int cache_build_hot(bpe_tok *tok) {
     u64 *host = (u64 *)ctx->pinned;
     CUDA_TRY(ctx, cudaMemcpyAsync(host, hist, ENC_HOT_HIST * sizeof(u64), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(ctx, cudaStreamSynchronize(st));
-    u64 n_hot = 0, thresh = ENC_HOT_HIST;
-    for (int k = ENC_HOT_HIST - 1; k >= 2; k--) { if (n_hot + host[k] > hot_max) break; n_hot += host[k]; thresh = (u64)k; }
+    u64 n_hot;
+    const u64 thresh = fit_threshold(host, ENC_HOT_HIST, hot_max, &n_hot);
     static const bool hot_test = getenv("BPE_ENC_HOT_TEST") != nullptr;       // test knob: build it however few pretokens qualify
     if (thresh < ENC_HOT_HIST && (hot_test || n_hot >= 1024)) {
         const u64 nb = n_hot + 64;
-        BPE_TRY(alloc_exact_e(ctx, tok->hot, nb * 48));
+        BPE_TRY(alloc_exact(ctx, tok->hot, nb * 48));
         CUDA_TRY(ctx, cudaMemsetAsync(tok->hot.p, 0, nb * 48, st));
         KLAUNCH(k_enc_hot_build, grid, 256, 0, st, t, (ulonglong2 *)tok->hot.p, (u64 *)((ulonglong2 *)tok->hot.p + 2 * nb), nb, (u32)thresh);
         CUDA_TRY(ctx, cudaGetLastError());
@@ -1276,9 +1139,9 @@ static int cache_build_hot(bpe_tok *tok) {
         KLAUNCH(k_enc_sm_hist, g, 256, 0, st, t, h2);
         CUDA_TRY(ctx, cudaMemcpyAsync(host, h2, 256 * sizeof(u64), cudaMemcpyDeviceToHost, st));
         CUDA_TRY(ctx, cudaStreamSynchronize(st));
-        u64 acc = 0; u32 min_bucket = 256;
-        for (int k = 255; k >= 2; k--) { if (acc + host[k] > LK_SM_SLOTS * LK_SM_FILL_NUM / 8) break; acc += host[k]; min_bucket = (u32)k; }
-        BPE_TRY(alloc_exact_e(ctx, tok->sm_img, (size_t)LK_SM_SLOTS * 16));
+        u64 acc;
+        const u32 min_bucket = (u32)fit_threshold(host, 256, LK_SM_SLOTS * LK_SM_FILL_NUM / 8, &acc);
+        BPE_TRY(alloc_exact(ctx, tok->sm_img, (size_t)LK_SM_SLOTS * 16));
         CUDA_TRY(ctx, cudaMemsetAsync(tok->sm_img.p, 0, (size_t)LK_SM_SLOTS * 16, st));
         if (min_bucket < 256) KLAUNCH(k_enc_sm_build, g, 256, 0, st, t, (ulonglong2 *)tok->sm_img.p, min_bucket);
         CUDA_TRY(ctx, cudaGetLastError());
@@ -1300,18 +1163,13 @@ static int cache_read_ctr(bpe_tok *tok, u64 *out, int k) {
 // c = the counters (cache_read_ctr(tok, c, 9)); the batch can add up to new_short pretokens of <= 7 bytes and new_long longer ones
 static int cache_ensure_capacity(bpe_tok *tok, const u64 *c, u64 new_short, u64 new_long) {
     bpe_ctx *ctx = tok->ctx;
-    const u64 n_short = c[0], n_long = c[1], n_med = c[8];
-    u64 need_s = next_pow2(std::max<u64>(1 << 16, (n_short + new_short) * 8 / 7 + 64));
-    u64 need_m = next_pow2(std::max<u64>(1 << 14, (n_med + new_long) * 8 / 7 + 64));
-    // pretokens of >= 16 bytes: at most bytes / 16 of them in a batch, i.e. half of the bound for >= 8 bytes
-    u64 need_l = next_pow2(std::max<u64>(1 << 14, (n_long + (new_long + 1) / 2) * 8 / 7 + 64));
-    if (need_s >= (1ull << 30) || need_m >= (1ull << 30) || need_l >= (1ull << 30)) return bpe_set_error(ctx, BPE_ERR_CAPACITY, "pretoken cache would exceed 2^30 slots");
-    if (need_s <= tok->scap && need_m <= tok->medcap && need_l <= tok->lcap) return BPE_OK;
-    need_s = std::max(need_s, tok->scap); need_m = std::max(need_m, tok->medcap); need_l = std::max(need_l, tok->lcap);
+    const PtCaps need = pt_caps(c[0], c[8], c[1], new_short, new_long);
+    if (need.s >= (1ull << 30) || need.m >= (1ull << 30) || need.l >= (1ull << 30)) return bpe_set_error(ctx, BPE_ERR_CAPACITY, "pretoken cache would exceed 2^30 slots");
+    if (need.s <= tok->scap && need.m <= tok->medcap && need.l <= tok->lcap) return BPE_OK;
     DevBuf ostab = tok->stab, omtab = tok->medtab, oltab = tok->ltab;
     u64 oscap = tok->scap, omcap = tok->medcap, olcap = tok->lcap;
     tok->stab = DevBuf(); tok->medtab = DevBuf(); tok->ltab = DevBuf();
-    int rc = cache_tables_alloc(tok, need_s, need_m, need_l);
+    int rc = cache_tables_alloc(tok, {std::max(need.s, tok->scap), std::max(need.m, tok->medcap), std::max(need.l, tok->lcap)});
     if (rc == BPE_OK) {
         EncTables t = enc_tables(tok);
         auto grid_for = [&](u64 cap) { return (unsigned)std::min<u64>((u64)ctx->sm_count * bpe_grid_mult(64), (cap + 255) / 256); };

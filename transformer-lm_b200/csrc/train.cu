@@ -15,52 +15,19 @@
 // =============================================================================================
 // 1. Pretoken counting  (extract_subword_frequencies, train.py:16-28)
 //
-// Two open-addressing tables in HBM:
-//   short table: pretokens of <= 7 bytes.  The key IS the token: bytes packed little-endian in the
-//                low 56 bits, length in the top byte, so one 64-bit CAS claims and publishes a slot
-//                and equality is an integer compare (exact, no fingerprints).
-//   long table:  pretokens of >= 8 bytes.  meta = (offset:40 | len:24) of a representative occurrence,
-//                claimed by CAS; a 64-bit hash is kept beside it as a filter and every hash hit is
-//                confirmed by comparing the bytes (exact).
-//   medium table: pretokens of 8..15 bytes -- a sixth of all occurrences of English-like text and nearly all of those with more
-//                than 7 bytes.  32-byte slots {bytes 0-7, bytes 8-14 | len << 56, count, -}: the 16-byte key IS the token,
-//                claimed and published by one 128-bit CAS, so an occurrence costs one 32-byte sector like a short one (through
-//                the long table it cost the slot, the bytes of the stored representative and a second look at the text).
-// Counts are 64-bit atomics.  Offsets with bit 39 set address the persistent pool (imported /
-// re-homed words), others the text arena of the current shard.
+// The short, medium and long pretoken tables of hashtab.cuh in HBM, payload = the count (64-bit atomics).  Long keys with
+// META_POOL_BIT address the persistent pool (imported / re-homed words), others the text arena of the current shard.
 // =============================================================================================
-#define SHORT_MAX 7u
-#define MED_MAX 15u
-#define META_EMPTY 0ull                          // a real meta word has len >= 8, never 0: empty tables are all-zero memory
-#define META_LEN_BITS 24
-#define META_LEN_MASK ((1ull << META_LEN_BITS) - 1)
-#define META_POOL_BIT (1ull << 39)
-#define MAX_TOKEN_LEN ((1u << META_LEN_BITS) - 2)
-
-struct CountTables {
-    u64 *stab; u64 scap;                         // short: slots of {key, count}            (16 B)
-    u64 *mtab; u64 mcap;                         // medium: slots of {k0, k1, count, pad}    (32 B, one sector)
-    u64 *ltab; u64 lcap;                         // long:  slots of {meta, hash, count, pad} (32 B, one sector)
-    // slot of the k-th unique short / long word (k = value of counters[0] / [1] when it was claimed): everything that walks the
-    // words (re-homing, export, word list, table growth) walks these lists instead of scanning the tables' capacity, which is
-    // sized for the worst case (every pretoken of a batch new) and mostly empty
+struct CountTables : PtTables {
+    // slot of the k-th unique short / medium / long word (k = value of counters[0] / [7] / [1] when it was claimed): everything that
+    // walks the words (re-homing, export, word list, table growth) walks these lists instead of scanning the tables' capacity, which
+    // is sized for the worst case (every pretoken of a batch new) and mostly empty
     u32 *slist, *mlist, *llist;
     ulonglong2 *hot; u64 *hcnt; u64 hot_nb;      // hot table (see below): hot_nb buckets of two 16-byte keys, counts apart; 0 = none
-    const uint8_t *text;                         // payload of the current text arena
-    const uint8_t *pool;                         // persistent bytes of long words
     u64 *counters;                               // [0]=n_short [1]=n_long [2]=long_bytes [3]=overflow [4]=n_pretokens [5]=too_long
                                                  // [6]=an owned pretoken ran past the trusted part of the right halo [7]=n_medium
 };
 struct WordCounts { u64 n_short, n_medium, n_long; };
-
-#define SKEY(t, s) ((t).stab[2 * (s)])
-#define SCNT(t, s) ((t).stab[2 * (s) + 1])
-#define MK0(t, s) ((t).mtab[4 * (s)])
-#define MK1(t, s) ((t).mtab[4 * (s) + 1])
-#define MCNT(t, s) ((t).mtab[4 * (s) + 2])
-#define LMETA(t, s) ((t).ltab[4 * (s)])
-#define LHASH(t, s) ((t).ltab[4 * (s) + 1])
-#define LCNT(t, s) ((t).ltab[4 * (s) + 2])
 
 struct CountState {
     DevBuf stab, mtab, ltab, slist, mlist, llist, pool, counters, hot;
@@ -72,78 +39,25 @@ struct CountState {
     u64 n_rehomed = 0;                           // long words [0, n_rehomed) of the list have their bytes in the pool
 };
 
-__device__ __forceinline__ const uint8_t *rep_ptr(const CountTables &t, u64 meta) {
-    u64 off = meta >> META_LEN_BITS;
-    return (off & META_POOL_BIT) ? t.pool + (off & ~META_POOL_BIT) : t.text + off;
-}
-
+// count `delta` more occurrences of a word: a claim appends the slot to the tier's list; the count is never read
 __device__ __forceinline__ void short_add(const CountTables &t, u64 key, u64 delta) {
-    u64 mask = t.scap - 1;
-    u64 s = mix64(key) & mask;
-    for (u64 probes = 0; probes < t.scap; probes++) {
-        u64 k = SKEY(t, s);
-        if (k == 0) {
-            u64 old = atomicCAS(&SKEY(t, s), 0ull, key);
-            if (old == 0) { t.slist[atomicAdd(&t.counters[0], 1ull)] = (u32)s; k = key; }
-            else k = old;
-        }
-        if (k == key) { atomicAdd(&SCNT(t, s), delta); return; }
-        s = (s + 1) & mask;
-    }
-    t.counters[3] = 1;
-}
-
-// 128-bit compare-and-swap on a 16-byte aligned address: returns the old value in (lo, hi)
-__device__ __forceinline__ void cas128(u64 *addr, u64 cmp_lo, u64 cmp_hi, u64 new_lo, u64 new_hi, u64 &lo, u64 &hi) {
-    asm volatile("{\n .reg .b128 c, n, d;\n mov.b128 c, {%3, %4};\n mov.b128 n, {%5, %6};\n atom.global.cas.b128 d, [%2], c, n;\n mov.b128 {%0, %1}, d;\n}"
-                 : "=l"(lo), "=l"(hi) : "l"(addr), "l"(cmp_lo), "l"(cmp_hi), "l"(new_lo), "l"(new_hi) : "memory");
-}
-// key of a pretoken of 8..15 bytes: k0 = bytes 0-7, k1 = bytes 8-14 (little-endian) | len << 56
-__device__ __forceinline__ void medium_key(const uint8_t *p, u32 len, u64 &k0, u64 &k1) {
-    k0 = load8_unaligned(p);
-    k1 = (len > 8 ? load8_unaligned(p + 8) & low_bytes_mask(len - 8) : 0ull) | ((u64)len << 56);
+    short_find_or_claim<false>(t, key, t.counters,
+        [&](u64 s) { t.slist[atomicAdd(&t.counters[0], 1ull)] = (u32)s; atomicAdd(&t.stab[s].val, delta); },
+        [&](u64 s, u64) { atomicAdd(&t.stab[s].val, delta); });
 }
 __device__ __forceinline__ void medium_add(const CountTables &t, u64 k0, u64 k1, u64 delta) {
-    u64 mask = t.mcap - 1;
-    u64 s = mix64(k0 ^ (k1 * 0x9E3779B97F4A7C15ull)) & mask;
-    for (u64 probes = 0; probes < t.mcap; probes++) {
-        const ulonglong2 kv = *reinterpret_cast<const ulonglong2 *>(&MK0(t, s));
-        u64 a = kv.x, b = kv.y;
-        if (a == 0 && b == 0) {                  // (k1 carries the length: a real key is never all zero)
-            cas128(&MK0(t, s), 0, 0, k0, k1, a, b);
-            if (a == 0 && b == 0) { t.mlist[atomicAdd(&t.counters[7], 1ull)] = (u32)s; a = k0; b = k1; }
-        }
-        if (a == k0 && b == k1) { atomicAdd(&MCNT(t, s), delta); return; }
-        s = (s + 1) & mask;
-    }
-    t.counters[3] = 1;
+    medium_find_or_claim<false>(t, k0, k1, t.counters,
+        [&](u64 s) { t.mlist[atomicAdd(&t.counters[7], 1ull)] = (u32)s; atomicAdd(&t.medtab[s].val, delta); },
+        [&](u64 s, u64) { atomicAdd(&t.medtab[s].val, delta); });
 }
-
-// p = bytes of the occurrence, off_meta = its offset in the space META addresses (text or pool bit set)
 __device__ __forceinline__ void long_add(const CountTables &t, const uint8_t *p, u32 len, u64 off_meta, u64 delta) {
-    u64 h = hash_long(p, len);
-    u64 mask = t.lcap - 1;
-    u64 s = h & mask;
-    u64 mine = (off_meta << META_LEN_BITS) | len;
-    for (u64 probes = 0; probes < t.lcap; probes++) {
-        const ulonglong2 mh = *reinterpret_cast<const ulonglong2 *>(&LMETA(t, s));   // meta and hash: one 16-byte load, one round trip
-        u64 m = mh.x, hh = mh.y;
-        if (m == META_EMPTY) {
-            u64 old = atomicCAS(&LMETA(t, s), META_EMPTY, mine);
-            if (old == META_EMPTY) {
-                LHASH(t, s) = h;
-                t.llist[atomicAdd(&t.counters[1], 1ull)] = (u32)s;
-                atomicAdd(&t.counters[2], (u64)len);
-                atomicAdd(&LCNT(t, s), delta);
-                return;
-            }
-            m = old;
-            hh = *((volatile u64 *)&LHASH(t, s));
-        }
-        if ((m & META_LEN_MASK) == len && (hh == 0 || hh == h) && bytes_equal(rep_ptr(t, m), p, len)) { atomicAdd(&LCNT(t, s), delta); return; }
-        s = (s + 1) & mask;
-    }
-    t.counters[3] = 1;
+    long_find_or_claim<false>(t, p, len, off_meta, t.counters,
+        [&](u64 s) {
+            t.llist[atomicAdd(&t.counters[1], 1ull)] = (u32)s;
+            atomicAdd(&t.counters[2], (u64)len);
+            atomicAdd(&t.ltab[s].val, delta);
+        },
+        [&](u64 s, u64) { atomicAdd(&t.ltab[s].val, delta); });
 }
 
 // Counting straight from the text and its start bits (no per-pretoken offset array, no scan).  A warp takes 32 consecutive 16-byte
@@ -194,9 +108,6 @@ struct CountQueues { ulonglong2 *qe; u64 *ql; u32 n, nl; };
 // one), the counts sit in an array beside it -- at most ~1 M words, 50 MB: it stays in L2.  A word whose bucket is full stays with
 // the big tables, so a probe is exactly one sector: no chains, no claims, all lanes of a warp finish together.  The counts are added
 // back to the big tables whenever somebody needs those (count_hot_flush).
-__device__ __forceinline__ u64 hot_bucket_of(const CountTables &t, u64 k0, u64 k1) {
-    return ((mix64(k0 ^ (k1 * 0x9E3779B97F4A7C15ull)) >> 32) * t.hot_nb) >> 32;
-}
 
 // Drain the warp's queues: whole groups of 64 keys (everything when `all`), two per lane with their probes in flight together;
 // every long entry.
@@ -210,18 +121,10 @@ __device__ __forceinline__ void count_drain(const CountTables &t, CountQueues &q
         if (hb) kb = q.qe[e0 + 32u + lane];
         bool ta = ha, tb = hb;                   // still to be added to the big tables
         if (t.hot_nb) {
-            const u64 ba = hot_bucket_of(t, ka.x, ka.y), bb = hot_bucket_of(t, kb.x, kb.y);
-            ulonglong2 a0 = make_ulonglong2(0, 0), a1 = a0, b0 = a0, b1 = a0;
-            if (ha) { a0 = t.hot[2 * ba]; a1 = t.hot[2 * ba + 1]; }
-            if (hb) { b0 = t.hot[2 * bb]; b1 = t.hot[2 * bb + 1]; }
-            if (ha) {
-                const bool m0 = a0.x == ka.x && a0.y == ka.y, m1 = a1.x == ka.x && a1.y == ka.y;
-                if (m0 || m1) { atomicAdd(&t.hcnt[2 * ba + (m1 ? 1 : 0)], 1ull); ta = false; }
-            }
-            if (hb) {
-                const bool m0 = b0.x == kb.x && b0.y == kb.y, m1 = b1.x == kb.x && b1.y == kb.y;
-                if (m0 || m1) { atomicAdd(&t.hcnt[2 * bb + (m1 ? 1 : 0)], 1ull); tb = false; }
-            }
+            const u64 ba = hot_bucket(t.hot_nb, ka.x, ka.y), bb = hot_bucket(t.hot_nb, kb.x, kb.y);
+            const int ia = ha ? hot_find(t.hot, ba, ka.x, ka.y) : -1, ib = hb ? hot_find(t.hot, bb, kb.x, kb.y) : -1;
+            if (ia >= 0) { atomicAdd(&t.hcnt[2 * ba + ia], 1ull); ta = false; }
+            if (ib >= 0) { atomicAdd(&t.hcnt[2 * bb + ib], 1ull); tb = false; }
         }
         if (ta) { if (ka.y == 0) short_add(t, ka.x, 1); else medium_add(t, ka.x, ka.y, 1); }
         if (tb) { if (kb.y == 0) short_add(t, kb.x, 1); else medium_add(t, kb.x, kb.y, 1); }
@@ -405,26 +308,21 @@ __global__ void __launch_bounds__(256) k_hot_hist(CountTables t, u64 n_short, u6
     if (threadIdx.x < HOT_HIST) s_h[threadIdx.x] = 0;
     __syncthreads();
     for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n_short + n_medium; i += (u64)gridDim.x * blockDim.x) {
-        const u64 c = i < n_short ? SCNT(t, t.slist[i]) : MCNT(t, t.mlist[i - n_short]);
+        const u64 c = i < n_short ? t.stab[t.slist[i]].val : t.medtab[t.mlist[i - n_short]].val;
         atomicAdd(&s_h[c < HOT_HIST ? (u32)c : HOT_HIST - 1], 1u);
     }
     __syncthreads();
     if (threadIdx.x < HOT_HIST && s_h[threadIdx.x]) atomicAdd(&hist[threadIdx.x], (u64)s_h[threadIdx.x]);
 }
 // every short / medium word counted at least `thresh` times is placed in its bucket if one of the two slots is free
-// (the keys are distinct: no comparison)
 __global__ void __launch_bounds__(256) k_hot_build(CountTables t, u64 n_short, u64 n_medium, u64 thresh, u64 *__restrict__ placed) {
     u64 np = 0;
     for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n_short + n_medium; i += (u64)gridDim.x * blockDim.x) {
         u64 k0, k1, c;
-        if (i < n_short) { const u64 s = t.slist[i]; k0 = SKEY(t, s); k1 = 0; c = SCNT(t, s); }
-        else { const u64 s = t.mlist[i - n_short]; k0 = MK0(t, s); k1 = MK1(t, s); c = MCNT(t, s); }
+        if (i < n_short) { const SSlot &e = t.stab[t.slist[i]]; k0 = e.key; k1 = 0; c = e.val; }
+        else { const MSlot &e = t.medtab[t.mlist[i - n_short]]; k0 = e.k0; k1 = e.k1; c = e.val; }
         if (c < thresh) continue;
-        const u64 b = hot_bucket_of(t, k0, k1);
-        u64 x, y;
-        cas128(reinterpret_cast<u64 *>(&t.hot[2 * b]), 0, 0, k0, k1, x, y);
-        if ((x | y) != 0) cas128(reinterpret_cast<u64 *>(&t.hot[2 * b + 1]), 0, 0, k0, k1, x, y);
-        if ((x | y) == 0) np++;
+        if (hot_claim(t.hot, hot_bucket(t.hot_nb, k0, k1), k0, k1) >= 0) np++;
     }
     for (int d = 16; d; d >>= 1) np += __shfl_down_sync(0xffffffffu, np, d);
     if (lane_id() == 0 && np) atomicAdd(placed, np);
@@ -440,34 +338,24 @@ __global__ void __launch_bounds__(256) k_hot_flush(CountTables t) {
     }
 }
 
-// ---- table growth: re-insert every entry of an old table into a bigger one -------------------
-__global__ void __launch_bounds__(256) k_rehash_short(const u64 *__restrict__ otab, const u32 *__restrict__ olist, u64 n_old, CountTables t) {
+// ---- table growth: re-insert every word of an old table's list into a bigger table, at the same position of the new list ------
+// (so counters[0], [7], [1] and [2] stay as they are)
+__global__ void __launch_bounds__(256) k_rehash_short(const SSlot *__restrict__ otab, const u32 *__restrict__ olist, u64 n_old, CountTables t) {
     for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n_old; i += (u64)gridDim.x * blockDim.x) {
-        const u64 o = olist[i];
-        short_add(t, otab[2 * o], otab[2 * o + 1]);          // (claims a slot and appends it to the new list: counters[0] was reset)
+        const SSlot &o = otab[olist[i]];
+        t.slist[i] = (u32)short_insert_unique(t, o.key, o.val);
     }
 }
-__global__ void __launch_bounds__(256) k_rehash_long(const u64 *__restrict__ otab, const u32 *__restrict__ olist, u64 n_old, CountTables t) {
-    u64 mask = t.lcap - 1;
+__global__ void __launch_bounds__(256) k_rehash_medium(const MSlot *__restrict__ otab, const u32 *__restrict__ olist, u64 n_old, CountTables t) {
     for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n_old; i += (u64)gridDim.x * blockDim.x) {
-        const u64 o = olist[i];
-        u64 m = otab[4 * o];
-        u64 s = otab[4 * o + 1] & mask;          // keys are unique: no comparison needed, just find a hole
-        for (;;) {
-            if (LMETA(t, s) == META_EMPTY && atomicCAS(&LMETA(t, s), META_EMPTY, m) == META_EMPTY) {
-                LHASH(t, s) = otab[4 * o + 1]; LCNT(t, s) = otab[4 * o + 2];
-                t.llist[i] = (u32)s;             // same position in the list: counters[1] / [2] stay as they are
-                break;
-            }
-            s = (s + 1) & mask;
-        }
+        const MSlot &o = otab[olist[i]];
+        t.mlist[i] = (u32)medium_insert_unique(t, o.k0, o.k1, o.val);
     }
 }
-
-__global__ void __launch_bounds__(256) k_rehash_medium(const u64 *__restrict__ otab, const u32 *__restrict__ olist, u64 n_old, CountTables t) {
+__global__ void __launch_bounds__(256) k_rehash_long(const LSlot *__restrict__ otab, const u32 *__restrict__ olist, u64 n_old, CountTables t) {
     for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n_old; i += (u64)gridDim.x * blockDim.x) {
-        const u64 o = olist[i];
-        medium_add(t, otab[4 * o], otab[4 * o + 1], otab[4 * o + 2]);   // (claims a slot and appends it to the new list: counters[7] was reset)
+        const LSlot &o = otab[olist[i]];
+        t.llist[i] = (u32)long_insert_unique(t, o.meta, o.hash, o.val);
     }
 }
 
@@ -476,7 +364,7 @@ __global__ void __launch_bounds__(256) k_rehash_medium(const u64 *__restrict__ o
 __global__ void __launch_bounds__(256) k_rehome_sizes(CountTables t, u64 first, u64 n_long, u64 *__restrict__ need /* [0] */) {
     u64 c = 0;
     for (u64 i = first + (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n_long; i += (u64)gridDim.x * blockDim.x) {
-        u64 m = LMETA(t, t.llist[i]);
+        u64 m = t.ltab[t.llist[i]].meta;
         if (!((m >> META_LEN_BITS) & META_POOL_BIT)) c += m & META_LEN_MASK;
     }
     for (int d = 16; d; d >>= 1) c += __shfl_down_sync(0xffffffffu, c, d);
@@ -485,13 +373,13 @@ __global__ void __launch_bounds__(256) k_rehome_sizes(CountTables t, u64 first, 
 __global__ void __launch_bounds__(256) k_rehome_copy(CountTables t, u64 first, u64 n_long, uint8_t *__restrict__ pool, u64 *__restrict__ cursor) {
     for (u64 i = first + (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n_long; i += (u64)gridDim.x * blockDim.x) {
         const u64 s = t.llist[i];
-        u64 m = LMETA(t, s);
+        u64 m = t.ltab[s].meta;
         if ((m >> META_LEN_BITS) & META_POOL_BIT) continue;
         u32 len = (u32)(m & META_LEN_MASK);
         u64 o = atomicAdd(cursor, (u64)len);
         const uint8_t *src = t.text + (m >> META_LEN_BITS);
         for (u32 k = 0; k < len; k++) pool[o + k] = src[k];
-        LMETA(t, s) = ((o | META_POOL_BIT) << META_LEN_BITS) | len;
+        t.ltab[s].meta = ((o | META_POOL_BIT) << META_LEN_BITS) | len;
     }
 }
 
@@ -502,16 +390,10 @@ __global__ void __launch_bounds__(256) k_import_words(CountTables t, const uint8
         u64 o = offs[i]; u64 len = offs[i + 1] - o;
         const uint8_t *p = blob_in_pool + o;
         if (len == 0) continue;
-        if (len <= SHORT_MAX) {
-            u64 key = 0;
-            for (u32 k = 0; k < (u32)len; k++) key |= (u64)p[k] << (8 * k);
-            key |= len << 56;
-            short_add(t, key, (u64)counts[i]);
-        } else if (len <= MED_MAX) {
-            u64 k0 = 0, k1 = len << 56;
-            for (u32 k = 0; k < 8; k++) k0 |= (u64)p[k] << (8 * k);
-            for (u32 k = 8; k < (u32)len; k++) k1 |= (u64)p[k] << (8 * (k - 8));
-            medium_add(t, k0, k1, (u64)counts[i]);
+        if (len <= MED_MAX) {
+            u64 k0, k1;
+            pretoken_key(p, (u32)len, k0, k1);
+            if (k1 == 0) short_add(t, k0, (u64)counts[i]); else medium_add(t, k0, k1, (u64)counts[i]);
         } else if (len <= MAX_TOKEN_LEN) {
             long_add(t, p, (u32)len, (pool_base + o) | META_POOL_BIT, (u64)counts[i]);
         } else t.counters[5] = 1;
@@ -522,24 +404,27 @@ __global__ void __launch_bounds__(256) k_import_words(CountTables t, const uint8
 struct WordRef { u32 len; u64 cnt; const uint8_t *src; uint8_t tmp[16]; };
 __device__ __forceinline__ void word_at(const CountTables &t, const WordCounts &wc, u64 i, WordRef &w) {
     if (i < wc.n_short) {
-        const u64 sl = t.slist[i], k = SKEY(t, sl);
-        w.len = (u32)(k >> 56); w.cnt = SCNT(t, sl);
+        const SSlot &e = t.stab[t.slist[i]];
+        const u64 k = e.key;
+        w.len = (u32)(k >> 56); w.cnt = e.val;
         for (u32 j = 0; j < 8; j++) w.tmp[j] = (uint8_t)(k >> (8 * j));
         w.src = w.tmp;
     } else if (i < wc.n_short + wc.n_medium) {
-        const u64 sl = t.mlist[i - wc.n_short], k0 = MK0(t, sl), k1 = MK1(t, sl);
-        w.len = (u32)(k1 >> 56); w.cnt = MCNT(t, sl);
+        const MSlot &e = t.medtab[t.mlist[i - wc.n_short]];
+        const u64 k0 = e.k0, k1 = e.k1;
+        w.len = (u32)(k1 >> 56); w.cnt = e.val;
         for (u32 j = 0; j < 8; j++) { w.tmp[j] = (uint8_t)(k0 >> (8 * j)); w.tmp[8 + j] = (uint8_t)(k1 >> (8 * j)); }
         w.src = w.tmp;
     } else {
-        const u64 sl = t.llist[i - wc.n_short - wc.n_medium], m = LMETA(t, sl);
-        w.len = (u32)(m & META_LEN_MASK); w.cnt = LCNT(t, sl); w.src = rep_ptr(t, m);
+        const LSlot &e = t.ltab[t.llist[i - wc.n_short - wc.n_medium]];
+        const u64 m = e.meta;
+        w.len = (u32)(m & META_LEN_MASK); w.cnt = e.val; w.src = rep_ptr(t, m);
     }
 }
 __device__ __forceinline__ u32 word_len_at(const CountTables &t, const WordCounts &wc, u64 i) {
-    if (i < wc.n_short) return (u32)(SKEY(t, t.slist[i]) >> 56);
-    if (i < wc.n_short + wc.n_medium) return (u32)(MK1(t, t.mlist[i - wc.n_short]) >> 56);
-    return (u32)(LMETA(t, t.llist[i - wc.n_short - wc.n_medium]) & META_LEN_MASK);
+    if (i < wc.n_short) return (u32)(t.stab[t.slist[i]].key >> 56);
+    if (i < wc.n_short + wc.n_medium) return (u32)(t.medtab[t.mlist[i - wc.n_short]].k1 >> 56);
+    return (u32)(t.ltab[t.llist[i - wc.n_short - wc.n_medium]].meta & META_LEN_MASK);
 }
 
 // ---- export: (bytes, offs, counts) of every word ----------------------------------------------------------------------
@@ -727,13 +612,13 @@ struct TrainBufs {
 static CountTables count_tables(bpe_ctx *ctx) {
     CountState *cs = ctx->count;
     CountTables t;
-    t.stab = (u64 *)cs->stab.p; t.scap = cs->scap;
-    t.mtab = (u64 *)cs->mtab.p; t.mcap = cs->mcap;
-    t.ltab = (u64 *)cs->ltab.p; t.lcap = cs->lcap;
+    t.stab = (SSlot *)cs->stab.p; t.scap = cs->scap;
+    t.medtab = (MSlot *)cs->mtab.p; t.medcap = cs->mcap;
+    t.ltab = (LSlot *)cs->ltab.p; t.lcap = cs->lcap;
     t.slist = (u32 *)cs->slist.p; t.mlist = (u32 *)cs->mlist.p; t.llist = (u32 *)cs->llist.p;
     t.hot = (ulonglong2 *)cs->hot.p; t.hot_nb = cs->hot_nb; t.hcnt = (u64 *)((ulonglong2 *)cs->hot.p + 2 * cs->hot_nb);
     t.text = ctx->text.p ? (const uint8_t *)ctx->text.p + BPE_PAD : nullptr;
-    t.pool = (const uint8_t *)cs->pool.p;
+    t.pool = (uint8_t *)cs->pool.p;
     t.counters = (u64 *)cs->counters.p;
     return t;
 }
@@ -746,9 +631,8 @@ void count_state_free(bpe_ctx *ctx) {
     ctx->count = nullptr;
 }
 
-static int alloc_exact(bpe_ctx *ctx, DevBuf &b, size_t bytes) { return bpe_buf_alloc(ctx, b, bytes ? bytes : 256); }
-
-static int count_tables_alloc(bpe_ctx *ctx, u64 scap, u64 mcap, u64 lcap) {
+static int count_tables_alloc(bpe_ctx *ctx, PtCaps cap) {
+    const u64 scap = cap.s, mcap = cap.m, lcap = cap.l;
     CountState *cs = ctx->count;
     BPE_TRY(alloc_exact(ctx, cs->stab, scap * 16)); BPE_TRY(alloc_exact(ctx, cs->mtab, mcap * 32)); BPE_TRY(alloc_exact(ctx, cs->ltab, lcap * 32));
     BPE_TRY(alloc_exact(ctx, cs->slist, scap * 4)); BPE_TRY(alloc_exact(ctx, cs->mlist, mcap * 4)); BPE_TRY(alloc_exact(ctx, cs->llist, lcap * 4));   // (written before read: no clearing)
@@ -766,7 +650,7 @@ BPE_API int bpe_count_begin(bpe_ctx *ctx) {
     CountState *cs = ctx->count;
     BPE_TRY(bpe_buf_reserve(ctx, cs->counters, 64 * sizeof(u64)));
     CUDA_TRY(ctx, cudaMemsetAsync(cs->counters.p, 0, 64 * sizeof(u64), ctx->stream));
-    BPE_TRY(count_tables_alloc(ctx, 1 << 16, 1 << 14, 1 << 14));
+    BPE_TRY(count_tables_alloc(ctx, pt_caps(0, 0, 0, 0, 0)));
     cs->pool_used = 0; cs->active = true; cs->n_pretokens = 0; cs->n_rehomed = 0;
     bpe_buf_free(ctx, cs->hot); cs->hot_nb = 0; cs->hot_seen = 0; cs->hot_builds = 0;
     return BPE_OK;
@@ -780,30 +664,24 @@ static int read_counters(bpe_ctx *ctx, u64 *out, int k) {
     return BPE_OK;
 }
 
-// Make sure the tables can absorb `new_short` / `new_long` more unique words (of <= 7 / >= 8 bytes) without exceeding 7/8 load.
+// Make sure the tables can absorb `new_short` more unique words of <= 7 bytes and `new_long` of >= 8 bytes (medium and long tables
+// together) without exceeding 7/8 load.
 // c = the counters as read by read_counters(ctx, c, 8).
 static int count_ensure_capacity(bpe_ctx *ctx, const u64 *c, u64 new_short, u64 new_long) {
     CountState *cs = ctx->count;
     const u64 n_short = c[0], n_long = c[1], n_medium = c[7];
-    u64 need_s = next_pow2(std::max<u64>(1 << 16, (n_short + new_short) * 8 / 7 + 64));
-    u64 need_m = next_pow2(std::max<u64>(1 << 14, (n_medium + new_long) * 8 / 7 + 64));
-    // pretokens of >= 16 bytes: at most bytes / 16 of them in a batch, i.e. half of the bound for >= 8 bytes
-    u64 need_l = next_pow2(std::max<u64>(1 << 14, (n_long + (new_long + 1) / 2) * 8 / 7 + 64));
-    if (need_s <= cs->scap && need_m <= cs->mcap && need_l <= cs->lcap) return BPE_OK;
-    need_s = std::max(need_s, cs->scap); need_m = std::max(need_m, cs->mcap); need_l = std::max(need_l, cs->lcap);
+    const PtCaps need = pt_caps(n_short, n_medium, n_long, new_short, new_long);
+    if (need.s <= cs->scap && need.m <= cs->mcap && need.l <= cs->lcap) return BPE_OK;
     // grow: move old tables aside, allocate, re-insert the words of the old lists
     CountState old_view = *cs;                   // shallow copy of the DevBufs
     cs->stab = DevBuf(); cs->mtab = DevBuf(); cs->ltab = DevBuf(); cs->slist = DevBuf(); cs->mlist = DevBuf(); cs->llist = DevBuf();
-    int rc = count_tables_alloc(ctx, need_s, need_m, need_l);
+    int rc = count_tables_alloc(ctx, {std::max(need.s, cs->scap), std::max(need.m, cs->mcap), std::max(need.l, cs->lcap)});
     if (rc != BPE_OK) return rc;
-    // the short and medium rehashes re-count their uniques through short_add / medium_add: reset [0] and [7]; [1],[2] (long) are untouched
-    CUDA_TRY(ctx, cudaMemsetAsync(cs->counters.p, 0, sizeof(u64), ctx->stream));
-    CUDA_TRY(ctx, cudaMemsetAsync((u64 *)cs->counters.p + 7, 0, sizeof(u64), ctx->stream));
     CountTables t = count_tables(ctx);
     auto grid_for = [&](u64 n) { return (unsigned)std::min<u64>((u64)ctx->sm_count * bpe_grid_mult(64), (n + 255) / 256); };
-    if (n_short) KLAUNCH(k_rehash_short, grid_for(n_short), 256, 0, ctx->stream, (const u64 *)old_view.stab.p, (const u32 *)old_view.slist.p, n_short, t);
-    if (n_medium) KLAUNCH(k_rehash_medium, grid_for(n_medium), 256, 0, ctx->stream, (const u64 *)old_view.mtab.p, (const u32 *)old_view.mlist.p, n_medium, t);
-    if (n_long) KLAUNCH(k_rehash_long, grid_for(n_long), 256, 0, ctx->stream, (const u64 *)old_view.ltab.p, (const u32 *)old_view.llist.p, n_long, t);
+    if (n_short) KLAUNCH(k_rehash_short, grid_for(n_short), 256, 0, ctx->stream, (const SSlot *)old_view.stab.p, (const u32 *)old_view.slist.p, n_short, t);
+    if (n_medium) KLAUNCH(k_rehash_medium, grid_for(n_medium), 256, 0, ctx->stream, (const MSlot *)old_view.mtab.p, (const u32 *)old_view.mlist.p, n_medium, t);
+    if (n_long) KLAUNCH(k_rehash_long, grid_for(n_long), 256, 0, ctx->stream, (const LSlot *)old_view.ltab.p, (const u32 *)old_view.llist.p, n_long, t);
     CUDA_TRY(ctx, cudaGetLastError());
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     for (DevBuf *b : {&old_view.stab, &old_view.mtab, &old_view.ltab, &old_view.slist, &old_view.mlist, &old_view.llist}) bpe_buf_free(ctx, *b);
@@ -840,8 +718,8 @@ static int count_hot_rebuild(bpe_ctx *ctx, const u64 *c) {
     u64 *host = (u64 *)ctx->pinned;
     CUDA_TRY(ctx, cudaMemcpyAsync(host, hist, HOT_HIST * sizeof(u64), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(ctx, cudaStreamSynchronize(st));
-    u64 n_hot = 0, thresh = HOT_HIST;
-    for (int k = HOT_HIST - 1; k >= 2; k--) { if (n_hot + host[k] > hot_max) break; n_hot += host[k]; thresh = (u64)k; }
+    u64 n_hot;
+    const u64 thresh = fit_threshold(host, HOT_HIST, hot_max, &n_hot);
     if (thresh >= HOT_HIST || (!hot_test && n_hot < 1024)) return BPE_OK;
     const u64 nb = n_hot + 64;                   // one bucket (two slots) per selected word: ~10 % of them find theirs full
     BPE_TRY(alloc_exact(ctx, cs->hot, nb * 48));
@@ -1091,7 +969,7 @@ static int count_import(bpe_ctx *ctx, const uint8_t *blob, const uint64_t *offs,
     cudaStream_t st = ctx->stream;
     const cudaMemcpyKind kind = from_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
     // blob goes straight into the pool (long words keep pointing at it)
-    if (cs->pool_used + nb > cs->pool.cap) {
+    if (cs->pool_used + nb + 16 > cs->pool.cap) {  // (+ 16: the key loads read up to 15 bytes past a word)
         DevBuf nbuf;
         BPE_TRY(bpe_buf_reserve(ctx, nbuf, (cs->pool_used + nb) * 2 + (1 << 20)));
         if (cs->pool_used) CUDA_TRY(ctx, cudaMemcpyAsync(nbuf.p, cs->pool.p, cs->pool_used, cudaMemcpyDeviceToDevice, st));
