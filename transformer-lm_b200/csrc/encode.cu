@@ -1181,6 +1181,12 @@ static int cache_ensure_capacity(bpe_tok *tok, const u64 *c, u64 new_short, u64 
         if (e != cudaSuccess) rc = bpe_set_error(ctx, BPE_ERR_CUDA, "cache rehash: %s", cudaGetErrorString(e));
     }
     for (DevBuf *b : {&ostab, &omtab, &oltab}) bpe_buf_free(ctx, *b);
+    static const bool prof = getenv("BPE_ENC_PROFILE") != nullptr;       // (the growth tests read these notes)
+    if (prof && rc == BPE_OK)
+        fprintf(stderr, "  [encoder cache grow: short %llu -> %llu slots (%llu entries), medium %llu -> %llu (%llu), long %llu -> %llu (%llu)]\n",
+                (unsigned long long)oscap, (unsigned long long)tok->scap, (unsigned long long)c[0], (unsigned long long)omcap,
+                (unsigned long long)tok->medcap, (unsigned long long)c[8], (unsigned long long)olcap, (unsigned long long)tok->lcap,
+                (unsigned long long)c[1]);
     return rc;
 }
 

@@ -685,6 +685,11 @@ static int count_ensure_capacity(bpe_ctx *ctx, const u64 *c, u64 new_short, u64 
     CUDA_TRY(ctx, cudaGetLastError());
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     for (DevBuf *b : {&old_view.stab, &old_view.mtab, &old_view.ltab, &old_view.slist, &old_view.mlist, &old_view.llist}) bpe_buf_free(ctx, *b);
+    static const bool prof = getenv("BPE_COUNT_PROFILE") != nullptr;     // (the growth tests read these notes)
+    if (prof) fprintf(stderr, "  [count tables grow: short %llu -> %llu slots (%llu entries), medium %llu -> %llu (%llu), long %llu -> %llu (%llu)]\n",
+                      (unsigned long long)old_view.scap, (unsigned long long)cs->scap, (unsigned long long)n_short,
+                      (unsigned long long)old_view.mcap, (unsigned long long)cs->mcap, (unsigned long long)n_medium,
+                      (unsigned long long)old_view.lcap, (unsigned long long)cs->lcap, (unsigned long long)n_long);
     return BPE_OK;
 }
 
@@ -834,7 +839,7 @@ static int count_rehome(bpe_ctx *ctx) {
     u64 need = host[0];
     cs->n_rehomed = n_long;
     if (!need) return BPE_OK;
-    if (cs->pool_used + need > cs->pool.cap) {
+    if (cs->pool_used + need + 16 > cs->pool.cap) {  // (+ 16: the key loads read up to 15 bytes past a word)
         DevBuf nb;
         BPE_TRY(bpe_buf_reserve(ctx, nb, (cs->pool_used + need) * 2 + (1 << 20)));
         if (cs->pool_used) CUDA_TRY(ctx, cudaMemcpyAsync(nb.p, cs->pool.p, cs->pool_used, cudaMemcpyDeviceToDevice, st));
