@@ -112,6 +112,30 @@ int bpe_train_dev(bpe_ctx *ctx, const uint8_t *text_dev, uint64_t n,
                   const uint8_t *specials_blob, const uint32_t *special_offs, int n_specials,
                   int n_merges, int32_t *merge_pairs_out, int *n_done, bpe_train_stats *stats);
 
+/* Training options of the _ex entry points (an unknown bit is BPE_ERR_ARG).
+ * BPE_TRAIN_SPLIT_SPECIALS (train_bpe(..., split_special_tokens=True)): training splits the text on the special tokens before
+ * counting, the way the tokenizer splits it before encoding.  Without it training is bpe_train exactly (SURVEY A-1).
+ *   1. The input is validated as strict UTF-8 over all of it (same BPE_ERR_UTF8 and detail = the first invalid byte of the whole
+ *      input), then universal newlines are translated (A-2).
+ *   2. The translated text is split on the special-token occurrences as Tokenizer.segment splits it: leftmost match, longest
+ *      special first (re.split on the escaped alternation sorted by length, descending; the order of the caller's list does not
+ *      matter).  A special containing '\r' never matches: the text holds no '\r' after translation.  An empty special matches
+ *      nothing (empty specials are unsupported, DESIGN.md section 8).
+ *   3. Every piece between occurrences is pretokenised on its own with the GPT-2 pattern, as a whole text (\s+(?!\S) sees the
+ *      end of the text before an occurrence).
+ *   4. Occurrences are counted nowhere: they add no word and no pair, and no word or merge crosses one.  stats->n_pretokens
+ *      counts the ordinary pretokens only.
+ *   5. The merge loop and everything after it are unchanged (vocab layout A-3, dedupe A-5, tie-break A-10, zero-count tail A-7).
+ * Consequences: no learned token contains a special token (a piece holds no whole occurrence of one), and a text in which no
+ * special occurs trains exactly as without the flag. */
+#define BPE_TRAIN_SPLIT_SPECIALS 1
+int bpe_train_ex(bpe_ctx *ctx, const uint8_t *text_host, uint64_t n,
+                 const uint8_t *specials_blob, const uint32_t *special_offs, int n_specials,
+                 int n_merges, int32_t *merge_pairs_out, int *n_done, bpe_train_stats *stats, int flags);
+int bpe_train_dev_ex(bpe_ctx *ctx, const uint8_t *text_dev, uint64_t n,
+                     const uint8_t *specials_blob, const uint32_t *special_offs, int n_specials,
+                     int n_merges, int32_t *merge_pairs_out, int *n_done, bpe_train_stats *stats, int flags);
+
 /* Sharded training (one process per GPU; SURVEY 8e).  A rank counts the pretokens that START in its
  * byte range of the file, exports its (word, count) table, the host exchanges tables (NCCL all-gather
  * via torch.distributed), every rank imports the other ranks' tables and runs the replicated merge
@@ -128,6 +152,17 @@ int bpe_count_add_shard(bpe_ctx *ctx, const uint8_t *text_host, uint64_t n,
                         uint64_t own_begin, uint64_t own_end, int at_file_start, int at_file_end);
 int bpe_count_add_shard_dev(bpe_ctx *ctx, const uint8_t *text_dev, uint64_t n,
                             uint64_t own_begin, uint64_t own_end, int at_file_start, int at_file_end);
+/* Same with the training options.  flags == 0 is bpe_count_add_shard (the specials are unused).  With BPE_TRAIN_SPLIT_SPECIALS
+ * the shard is split on the specials (bpe_train_ex) and counted as one whole text: the host cuts the file only at exact
+ * boundaries (the start of a special-token occurrence that no occurrence covers from the left, or a single U+0020 between two
+ * ASCII non-space bytes that no occurrence covers), where splitting and pretokenisation on both sides do not depend on the other.
+ * own_begin must be 0 and own_end n (BPE_ERR_ARG otherwise); there is no halo, BPE_ERR_HALO cannot occur. */
+int bpe_count_add_shard_ex(bpe_ctx *ctx, const uint8_t *text_host, uint64_t n,
+                           uint64_t own_begin, uint64_t own_end, int at_file_start, int at_file_end,
+                           const uint8_t *specials_blob, const uint32_t *special_offs, int n_specials, int flags);
+int bpe_count_add_shard_dev_ex(bpe_ctx *ctx, const uint8_t *text_dev, uint64_t n,
+                               uint64_t own_begin, uint64_t own_end, int at_file_start, int at_file_end,
+                               const uint8_t *specials_blob, const uint32_t *special_offs, int n_specials, int flags);
 /* Export sizes, then the table itself: blob = concatenated word bytes, offs[n_words+1], counts[n_words]. */
 int bpe_count_export_size(bpe_ctx *ctx, uint64_t *n_words, uint64_t *blob_bytes);
 int bpe_count_export(bpe_ctx *ctx, uint8_t *blob, uint64_t *offs, int64_t *counts);

@@ -17,6 +17,7 @@ BPE_OK = 0
 (ERR_ARG, ERR_CUDA, ERR_OOM, ERR_UTF8, ERR_KEY, ERR_CAPACITY, ERR_TOO_SMALL, ERR_UNSUPPORTED, ERR_NO_DEVICE, ERR_HALO,
  ERR_NEWLINE) = range(-1, -12, -1)
 DTYPE_U16, DTYPE_I32 = 0, 1
+TRAIN_SPLIT_SPECIALS = 1
 OFF_BYTES, OFF_CHARS = 0, 1
 SYNTH_TINYSTORIES, SYNTH_OWT = 0, 1
 
@@ -52,7 +53,8 @@ _lock = threading.Lock()
 EXPORTS = [
     "bpe_version", "bpe_unicode_table_source", "bpe_ctx_create", "bpe_ctx_destroy", "bpe_last_error",
     "bpe_last_error_detail", "bpe_device_sync", "bpe_utf8_validate", "bpe_pretokenize", "bpe_train", "bpe_train_dev",
-    "bpe_count_begin", "bpe_count_add_shard", "bpe_count_add_shard_dev", "bpe_count_export_size", "bpe_count_export",
+    "bpe_train_ex", "bpe_train_dev_ex", "bpe_count_begin", "bpe_count_add_shard", "bpe_count_add_shard_dev",
+    "bpe_count_add_shard_ex", "bpe_count_add_shard_dev_ex", "bpe_count_export_size", "bpe_count_export",
     "bpe_count_export_dev", "bpe_count_import", "bpe_count_import_dev", "bpe_count_pair_table",
     "bpe_train_from_counts", "bpe_last_pair_table", "bpe_train_set_live", "bpe_tok_create", "bpe_tok_destroy", "bpe_encode", "bpe_encode_batch", "bpe_encode_dropout", "bpe_encode_batch_dropout", "bpe_encode_offsets",
     "bpe_encode_batch_offsets", "bpe_encode_dropout_offsets", "bpe_encode_batch_dropout_offsets", "bpe_encode_dev", "bpe_tok_key_error", "bpe_tok_saw_cr",
@@ -81,9 +83,13 @@ def lib():
             L.bpe_pretokenize.argtypes = [vp, vp, C.c_uint64, vp, vp, C.c_int, vp, C.c_uint64, u64p]
             L.bpe_train.argtypes = [vp, vp, C.c_uint64, vp, vp, C.c_int, C.c_int, vp, C.POINTER(C.c_int), C.POINTER(TrainStats)]
             L.bpe_train_dev.argtypes = L.bpe_train.argtypes
+            L.bpe_train_ex.argtypes = L.bpe_train.argtypes + [C.c_int]
+            L.bpe_train_dev_ex.argtypes = L.bpe_train_ex.argtypes
             L.bpe_count_begin.argtypes = [vp]
             L.bpe_count_add_shard.argtypes = [vp, vp, C.c_uint64, C.c_uint64, C.c_uint64, C.c_int, C.c_int]
             L.bpe_count_add_shard_dev.argtypes = L.bpe_count_add_shard.argtypes
+            L.bpe_count_add_shard_ex.argtypes = L.bpe_count_add_shard.argtypes + [vp, vp, C.c_int, C.c_int]
+            L.bpe_count_add_shard_dev_ex.argtypes = L.bpe_count_add_shard_ex.argtypes
             L.bpe_count_export_dev.argtypes = [vp, vp, vp, vp]
             L.bpe_count_import_dev.argtypes = [vp, vp, vp, vp, C.c_uint64, C.c_uint64]
             L.bpe_count_pair_table.argtypes = [vp, vp, vp, C.c_int, vp]

@@ -1,4 +1,5 @@
 // api.cu -- context management and the pretokenizer entry points of the C ABI (include/bpe_sm100.h).
+#include <algorithm>
 #include "kernels.h"
 #include "ctx.h"
 #include "unicode_tables.h"
@@ -201,6 +202,35 @@ int ctx_upload_specials(bpe_ctx *ctx, const uint8_t *blob, const u32 *offs, int 
     *blob_dev = (const uint8_t *)ctx->sp_dev.p;
     *offs_dev = (const u32 *)((uint8_t *)ctx->sp_dev.p + offs_at);
     return BPE_OK;
+}
+
+static u32 special_len_at(const uint8_t *t, u64 n, u64 i, const uint8_t *sp_blob, const u32 *sp_offs, int n_sp) {
+    for (int s = 0; s < n_sp; s++) {             // longest special matching at i, or 0
+        u32 o = sp_offs[s], l = sp_offs[s + 1] - o;
+        if (l && i + l <= n && memcmp(t + i, sp_blob + o, l) == 0) return l;
+    }
+    return 0;
+}
+static bool covered_by_special_from_left(const uint8_t *t, u64 n, u64 i, const uint8_t *sp_blob, const u32 *sp_offs, int n_sp, u64 ml) {
+    for (u64 q = i >= ml ? i - ml + 1 : 0; q < i; q++) { u32 l = special_len_at(t, n, q, sp_blob, sp_offs, n_sp); if (l && q + l > i) return true; }
+    return false;
+}
+u64 exact_cut_host(const uint8_t *t, u64 n, u64 nominal, u64 window, const uint8_t *sp_blob, const u32 *sp_offs, int n_sp) {
+    const u64 end = std::min(n, nominal + window);
+    u64 ml = 0;
+    for (int s = 0; s < n_sp; s++) ml = std::max<u64>(ml, sp_offs[s + 1] - sp_offs[s]);
+    auto covered = [&](u64 i) { return covered_by_special_from_left(t, n, i, sp_blob, sp_offs, n_sp, ml); };
+    if (n_sp > 0) {
+        bool first[256] = {false};
+        for (int s = 0; s < n_sp; s++) if (sp_offs[s + 1] > sp_offs[s]) first[sp_blob[sp_offs[s]]] = true;
+        for (u64 i = nominal; i < end; i++)
+            if (first[t[i]] && special_len_at(t, n, i, sp_blob, sp_offs, n_sp) && !covered(i)) return i;
+    }
+    auto plain = [](uint8_t b) { return b > 0x20 && b < 0x7F; };
+    for (u64 i = std::max<u64>(nominal, 1); i + 1 < end; i++)
+        if (t[i] == ' ' && plain(t[i - 1]) && plain(t[i + 1]) && !(n_sp > 0 && (covered(i) || covered(i + 1))))
+            return i;
+    return 0;
 }
 
 // Run validation + flags over the text currently in the arena (payload length *n).

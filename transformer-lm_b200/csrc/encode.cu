@@ -1603,34 +1603,8 @@ static int encode_check_args(bpe_tok *tok, const uint8_t *text, u64 n, int out_d
 #define ENC_PIPE_MIN (96ull << 20)
 #define ENC_CUT_WINDOW (8ull << 20)
 
-static u32 special_len_at(const bpe_tok *tok, const uint8_t *t, u64 n, u64 i) {     // longest special matching at i, or 0
-    for (int s = 0; s < tok->n_sp; s++) {
-        u32 o = tok->sp_offs_h[s], l = tok->sp_offs_h[s + 1] - o;
-        if (l && i + l <= n && memcmp(t + i, tok->sp_blob_h.data() + o, l) == 0) return l;
-    }
-    return 0;
-}
-static bool covered_by_special_from_left(const bpe_tok *tok, const uint8_t *t, u64 n, u64 i) {
-    const u64 ml = tok->sp_max_len;
-    for (u64 q = i >= ml ? i - ml + 1 : 0; q < i; q++) { u32 l = special_len_at(tok, t, n, q); if (l && q + l > i) return true; }
-    return false;
-}
-// A position >= nominal where cutting the text changes nothing: the start of a special-token occurrence (segment()
-// splits there, tokenizer.py:63-66), or a single U+0020 between two ASCII non-space characters (SURVEY B.2).  0 = none.
 static u64 find_exact_cut(const bpe_tok *tok, const uint8_t *t, u64 n, u64 nominal) {
-    const u64 end = std::min(n, nominal + ENC_CUT_WINDOW);
-    if (tok->n_sp > 0) {
-        bool first[256] = {false};
-        for (int s = 0; s < tok->n_sp; s++) if (tok->sp_offs_h[s + 1] > tok->sp_offs_h[s]) first[tok->sp_blob_h[tok->sp_offs_h[s]]] = true;
-        for (u64 i = nominal; i < end; i++)
-            if (first[t[i]] && special_len_at(tok, t, n, i) && !covered_by_special_from_left(tok, t, n, i)) return i;
-    }
-    auto plain = [](uint8_t b) { return b > 0x20 && b < 0x7F; };
-    for (u64 i = std::max<u64>(nominal, 1); i + 1 < end; i++)
-        if (t[i] == ' ' && plain(t[i - 1]) && plain(t[i + 1]) && !(tok->n_sp > 0 && (covered_by_special_from_left(tok, t, n, i) ||
-                                                                                     covered_by_special_from_left(tok, t, n, i + 1))))
-            return i;
-    return 0;
+    return exact_cut_host(t, n, nominal, ENC_CUT_WINDOW, tok->sp_blob_h.data(), tok->sp_offs_h.data(), tok->n_sp);
 }
 
 // ---- bpe_encode_batch: a chunk of documents into the text arena, one boundary byte after every document that ends in it ----------

@@ -160,8 +160,11 @@ __device__ __forceinline__ void count_drain(const CountTables &t, CountQueues &q
 #define CNT_STAGE_POS 520u                       // up to 512 starts + the sentinel (first start after the step), 16-bit each
 #define CNT_POS_OWNED 0x8000u                    // the pretoken starts inside [own_begin, own_end) of this launch's chunks
 #define CNT_POS_UNKNOWN 0xFFFFu                  // sentinel: no start within the bits the last lane holds
-__global__ void __launch_bounds__(CNT_NT, 1024 / CNT_NT) k_count_pretokens(CountTables t, const u32 *__restrict__ flags, u64 c_lo, u64 c_hi, u64 n, u64 base,
-                                                              u64 own_begin, u64 own_end, u64 trust_end) {
+// SKIP_SP (training with split_special_tokens): spstart marks the first byte of every special-token occurrence.  Such a start
+// still ends the pretoken before it, but is not counted itself: the occurrence is no word.
+template <bool SKIP_SP>
+__device__ __forceinline__ void count_pretokens(const CountTables &t, const u32 *__restrict__ flags, const u32 *__restrict__ spstart,
+                                                u64 c_lo, u64 c_hi, u64 n, u64 base, u64 own_begin, u64 own_end, u64 trust_end) {
     extern __shared__ __align__(16) unsigned char cnt_smem[];
     const u32 lane = lane_id(), warp = threadIdx.x >> 5;
     u64 *s_key = reinterpret_cast<u64 *>(cnt_smem);                                        // shared-memory table: keys ...
@@ -188,11 +191,12 @@ __global__ void __launch_bounds__(CNT_NT, 1024 / CNT_NT) k_count_pretokens(Count
     u64 c = c_lo + (tk_cur * CNT_TICKET) * 32u + lane;
     // loads of a step: the chunk (lane 31: also the 16 bytes after it; the arena is padded), the two flag words that hold its
     // 48..64-bit window.  Chunks past c_hi are loaded as well while they are text: their start bits end the last pretokens of the range
-    uint4 A = make_uint4(0, 0, 0, 0), B = A; u32 f0 = 0, f1 = 0;
+    uint4 A = make_uint4(0, 0, 0, 0), B = A; u32 f0 = 0, f1 = 0, g0 = 0;
     if (tk_cur * CNT_TICKET < n_steps && c * 16u < n) {
         const uint4 *tp = reinterpret_cast<const uint4 *>(t.text + c * 16u);
         A = __ldcs(tp); if (lane == 31) B = __ldcs(tp + 1);
         const u64 w = c >> 1; f0 = __ldcs(flags + w); f1 = w + 1 < n_fw ? __ldcs(flags + w + 1) : 0u;
+        if (SKIP_SP) g0 = __ldcs(spstart + w);
     }
     while (tk_cur * CNT_TICKET + sub < n_steps) {
         c = c_lo + (tk_cur * CNT_TICKET + sub) * 32u + lane;
@@ -207,6 +211,7 @@ __global__ void __launch_bounds__(CNT_NT, 1024 / CNT_NT) k_count_pretokens(Count
         }
         const u64 p0 = c * 16u, step_p0 = (c - lane) * 16u;
         u64 F = (((u64)f1 << 32) | f0) >> (u32)(p0 & 16u);           // bit i: a pretoken starts at byte p0 + i (>= 48 bits)
+        const u32 sp = SKIP_SP ? g0 >> (u32)(p0 & 16u) : 0u;          // bit i: a special-token occurrence starts at byte p0 + i
         reinterpret_cast<uint4 *>(s_text)[lane] = A;
         if (lane == 31) reinterpret_cast<uint4 *>(s_text)[32] = B;
         // the next step's loads
@@ -215,12 +220,14 @@ __global__ void __launch_bounds__(CNT_NT, 1024 / CNT_NT) k_count_pretokens(Count
                 const uint4 *tp = reinterpret_cast<const uint4 *>(t.text + cn * 16u);
                 A = __ldcs(tp); if (lane == 31) B = __ldcs(tp + 1);
                 const u64 w = cn >> 1; f0 = __ldcs(flags + w); f1 = w + 1 < n_fw ? __ldcs(flags + w + 1) : 0u;
+                if (SKIP_SP) g0 = __ldcs(spstart + w);
             } else { f0 = 0; f1 = 0; }
         }
         if (p0 + 64 > n) F = p0 < n ? F & ((1ull << (n - p0)) - 1ull) : 0ull;   // bits past the end of the text do not count
         const u32 mall = (u32)F & 0xFFFFu;       // every start of the chunk
-        // the starts this launch counts: chunks of the range, positions inside [own_begin, own_end)
+        // the starts this launch counts: chunks of the range, positions inside [own_begin, own_end), no special occurrence
         u32 m = c < c_hi ? mall : 0u;
+        if (SKIP_SP) m &= ~sp;
         if (p0 < own_begin) m = own_begin - p0 >= 16 ? 0u : m & ~((1u << (u32)(own_begin - p0)) - 1u);
         if (p0 + 16 > own_end) m = own_end <= p0 ? 0u : m & ((1u << (u32)(own_end - p0)) - 1u);
         n_tok += __popc(m);
@@ -287,6 +294,14 @@ __global__ void __launch_bounds__(CNT_NT, 1024 / CNT_NT) k_count_pretokens(Count
     __syncthreads();
     for (u32 i = threadIdx.x; i < CNT_SMEM_SLOTS; i += CNT_NT)
         if (s_cnt[i]) short_add(t, s_key[i], (u64)s_cnt[i]);
+}
+__global__ void __launch_bounds__(CNT_NT, 1024 / CNT_NT) k_count_pretokens(CountTables t, const u32 *__restrict__ flags, u64 c_lo, u64 c_hi, u64 n, u64 base,
+                                                              u64 own_begin, u64 own_end, u64 trust_end) {
+    count_pretokens<false>(t, flags, nullptr, c_lo, c_hi, n, base, own_begin, own_end, trust_end);
+}
+__global__ void __launch_bounds__(CNT_NT, 1024 / CNT_NT) k_count_pretokens_split(CountTables t, const u32 *__restrict__ flags, const u32 *__restrict__ spstart,
+                                                                    u64 c_lo, u64 c_hi, u64 n, u64 base, u64 own_begin, u64 own_end, u64 trust_end) {
+    count_pretokens<true>(t, flags, spstart, c_lo, c_hi, n, base, own_begin, own_end, trust_end);
 }
 
 // upper bound of new unique words a range of flag words can create: its number of start bits
@@ -748,8 +763,8 @@ static double now_ms() { return std::chrono::duration<double, std::milli>(std::c
 #define COUNT_BATCH_BYTES (256ull << 20)
 
 // Count the pretokens whose start lies in [own_begin, own_end) of the text currently in the arena
-// (flags already computed).
-static int count_current_text(bpe_ctx *ctx, u64 n, u64 own_begin, u64 own_end, u64 trust_end) {
+// (flags already computed).  spstart (split_special_tokens): the first bytes of the special-token occurrences, which are not counted.
+static int count_current_text(bpe_ctx *ctx, u64 n, u64 own_begin, u64 own_end, u64 trust_end, const u32 *spstart = nullptr) {
     CountState *cs = ctx->count;
     cudaStream_t st = ctx->stream;
     if (own_end > n) own_end = n;
@@ -799,8 +814,15 @@ static int count_current_text(bpe_ctx *ctx, u64 n, u64 own_begin, u64 own_end, u
             unsigned g2 = (unsigned)std::min<u64>((u64)ctx->sm_count * cnt_ctas_per_sm, std::max<u64>(steps, 1));
             CUDA_TRY(ctx, cudaMemsetAsync(t.counters + 16, 0, 8, st));
             static bool attr_set = false;
-            if (!attr_set) { CUDA_TRY(ctx, cudaFuncSetAttribute((void *)k_count_pretokens, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CNT_DYN_SMEM)); attr_set = true; }
-            KLAUNCH(k_count_pretokens, g2, CNT_NT, CNT_DYN_SMEM, st, t, (const u32 *)ctx->flags.p, c_lo, c_hi, n, b_lo * 32, own_begin, own_end, trust_end);
+            if (!attr_set) {
+                CUDA_TRY(ctx, cudaFuncSetAttribute((void *)k_count_pretokens, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CNT_DYN_SMEM));
+                CUDA_TRY(ctx, cudaFuncSetAttribute((void *)k_count_pretokens_split, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CNT_DYN_SMEM));
+                attr_set = true;
+            }
+            if (spstart)
+                KLAUNCH(k_count_pretokens_split, g2, CNT_NT, CNT_DYN_SMEM, st, t, (const u32 *)ctx->flags.p, spstart, c_lo, c_hi, n, b_lo * 32, own_begin, own_end, trust_end);
+            else
+                KLAUNCH(k_count_pretokens, g2, CNT_NT, CNT_DYN_SMEM, st, t, (const u32 *)ctx->flags.p, c_lo, c_hi, n, b_lo * 32, own_begin, own_end, trust_end);
         }
         CUDA_TRY(ctx, cudaGetLastError());
         if (bi + 1 < n_batches) {
@@ -857,8 +879,49 @@ static int count_rehome(bpe_ctx *ctx) {
     return BPE_OK;
 }
 
-static int count_add_shard(bpe_ctx *ctx, const uint8_t *text, u64 n, bool on_device, u64 own_begin, u64 own_end, int at_file_end) {
+// ---- split_special_tokens (BPE_TRAIN_SPLIT_SPECIALS) ----------------------------------------------------------------------
+// The text is split on the special-token occurrences as Tokenizer.segment splits it (leftmost match, longest special first: the
+// encoder's k_special_candidates / k_special_resolve inside ctx_run_flags), every piece is pretokenised as a whole text, and the
+// occurrences themselves are counted nowhere (k_count_pretokens_split).  The specials, longest first, on the host (exact cuts) and
+// on the device.
+struct SplitSpecials {
+    std::vector<uint8_t> blob; std::vector<u32> offs{0};
+    const uint8_t *blob_dev = nullptr; const u32 *offs_dev = nullptr; u32 max_len = 0;
+    int n() const { return (int)offs.size() - 1; }
+};
+static int split_specials_upload(bpe_ctx *ctx, const uint8_t *blob, const u32 *offs, int n_sp, SplitSpecials &sp) {
+    std::vector<int> order;
+    for (int i = 0; i < n_sp; i++) order.push_back(i);
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return offs[a + 1] - offs[a] > offs[b + 1] - offs[b]; });
+    for (int i : order) { sp.blob.insert(sp.blob.end(), blob + offs[i], blob + offs[i + 1]); sp.offs.push_back((u32)sp.blob.size()); }
+    return ctx_upload_specials(ctx, sp.blob.data(), sp.offs.data(), sp.n(), &sp.blob_dev, &sp.offs_dev, &sp.max_len);
+}
+// flags of the text in the arena with the specials split out (sp null: the default mode); the special starts the count skips, or null
+static int run_flags_for_training(bpe_ctx *ctx, u64 *n_io, bool translate, const SplitSpecials *sp, const u32 **spstart,
+                                  u64 err_lo = 0, u64 err_hi = ~0ull) {
+    *spstart = nullptr;
+    if (!sp) return ctx_run_flags(ctx, n_io, translate, nullptr, nullptr, 0, 0, err_lo, err_hi);
+    BPE_TRY(ctx_run_flags(ctx, n_io, translate, sp->blob_dev, sp->offs_dev, sp->n(), sp->max_len, err_lo, err_hi));
+    if (sp->max_len) *spstart = (const u32 *)ctx->spstart.p;
+    return BPE_OK;
+}
+// flags & BPE_TRAIN_SPLIT_SPECIALS: the specials uploaded into `split`, which the counting paths then use; BPE_ERR_ARG for unknown bits
+static int split_from_flags(bpe_ctx *ctx, int flags, const uint8_t *specials_blob, const uint32_t *special_offs, int n_specials,
+                            SplitSpecials &split, const SplitSpecials **use) {
+    *use = nullptr;
+    if (!ctx || (flags & ~BPE_TRAIN_SPLIT_SPECIALS) || (n_specials > 0 && (!specials_blob || !special_offs))) return BPE_ERR_ARG;
+    if (!(flags & BPE_TRAIN_SPLIT_SPECIALS)) return BPE_OK;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    BPE_TRY(split_specials_upload(ctx, specials_blob, special_offs, n_specials, split));
+    *use = &split;
+    return BPE_OK;
+}
+
+// sp (split mode): the shard is one whole text, cut from the file at exact boundaries (own range = all of it, no halo).
+static int count_add_shard(bpe_ctx *ctx, const uint8_t *text, u64 n, bool on_device, u64 own_begin, u64 own_end, int at_file_end,
+                           const SplitSpecials *sp = nullptr) {
     if (!ctx || !ctx->count || !ctx->count->active || (!text && n) || own_begin > own_end || own_end > n) return BPE_ERR_ARG;
+    if (sp && (own_begin != 0 || own_end != n)) return bpe_set_error(ctx, BPE_ERR_ARG, "with BPE_TRAIN_SPLIT_SPECIALS a shard is counted whole");
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     static const bool prof = getenv("BPE_COUNT_PROFILE") != nullptr;     // debug aid: host-side wall time of the phases (synchronising)
     double t0 = 0, t1 = 0, t2 = 0, t3 = 0;
@@ -866,12 +929,13 @@ static int count_add_shard(bpe_ctx *ctx, const uint8_t *text, u64 n, bool on_dev
     BPE_TRY(ctx_load_text(ctx, text, n, on_device));
     u64 nn = n;
     // only ill-formed sequences that start in the owned range are this shard's to report
-    BPE_TRY(ctx_run_flags(ctx, &nn, false, nullptr, nullptr, 0, 0, own_begin, own_end));
+    const u32 *spstart;
+    BPE_TRY(run_flags_for_training(ctx, &nn, false, sp, &spstart, own_begin, own_end));
     if (ctx->saw_cr) return bpe_set_error(ctx, BPE_ERR_NEWLINE, "the shard contains a carriage return");
     if (prof) { cudaStreamSynchronize(ctx->stream); t1 = now_ms(); }
     // start bits in the last 16 bytes of a shard that is cut mid-file lack their right context
-    u64 trust_end = at_file_end ? n : (n >= 16 ? n - 16 : 0);
-    BPE_TRY(count_current_text(ctx, n, own_begin, own_end, trust_end));
+    u64 trust_end = at_file_end || sp ? n : (n >= 16 ? n - 16 : 0);
+    BPE_TRY(count_current_text(ctx, n, own_begin, own_end, trust_end, spstart));
     if (prof) { cudaStreamSynchronize(ctx->stream); t2 = now_ms(); }
     int rc = count_rehome(ctx);
     if (prof) { cudaStreamSynchronize(ctx->stream); t3 = now_ms(); fprintf(stderr, "[count_add_shard %.2f GB] load+flags %.2f ms, count %.2f ms, rehome %.2f ms\n", n / 1e9, t1 - t0, t2 - t1, t3 - t2); }
@@ -886,6 +950,24 @@ BPE_API int bpe_count_add_shard_dev(bpe_ctx *ctx, const uint8_t *text_dev, uint6
                                     int at_file_start, int at_file_end) {
     (void)at_file_start;
     return count_add_shard(ctx, text_dev, n, true, own_begin, own_end, at_file_end);
+}
+static int count_add_shard_ex(bpe_ctx *ctx, const uint8_t *text, u64 n, bool on_device, u64 own_begin, u64 own_end, int at_file_end,
+                              const uint8_t *specials_blob, const uint32_t *special_offs, int n_specials, int flags) {
+    SplitSpecials sp; const SplitSpecials *split;
+    BPE_TRY(split_from_flags(ctx, flags, specials_blob, special_offs, n_specials, sp, &split));
+    return count_add_shard(ctx, text, n, on_device, own_begin, own_end, at_file_end, split);
+}
+BPE_API int bpe_count_add_shard_ex(bpe_ctx *ctx, const uint8_t *text_host, uint64_t n, uint64_t own_begin, uint64_t own_end,
+                                   int at_file_start, int at_file_end, const uint8_t *specials_blob, const uint32_t *special_offs,
+                                   int n_specials, int flags) {
+    (void)at_file_start;
+    return count_add_shard_ex(ctx, text_host, n, false, own_begin, own_end, at_file_end, specials_blob, special_offs, n_specials, flags);
+}
+BPE_API int bpe_count_add_shard_dev_ex(bpe_ctx *ctx, const uint8_t *text_dev, uint64_t n, uint64_t own_begin, uint64_t own_end,
+                                       int at_file_start, int at_file_end, const uint8_t *specials_blob, const uint32_t *special_offs,
+                                       int n_specials, int flags) {
+    (void)at_file_start;
+    return count_add_shard_ex(ctx, text_dev, n, true, own_begin, own_end, at_file_end, specials_blob, special_offs, n_specials, flags);
 }
 
 // lens[] and the byte offsets of the export live in tmp1 between export_size and export (n_words entries, not table capacity)
@@ -1299,7 +1381,7 @@ static int run_merges(bpe_ctx *ctx, const uint8_t *sp_blob, const u32 *sp_offs, 
 }
 
 static int train_impl(bpe_ctx *ctx, const uint8_t *text, u64 n, bool text_is_device, const uint8_t *sp_blob, const u32 *sp_offs,
-                      int n_sp, int n_merges, int32_t *merge_pairs_out, int *n_done, bpe_train_stats *stats) {
+                      int n_sp, int n_merges, int32_t *merge_pairs_out, int *n_done, bpe_train_stats *stats, const SplitSpecials *split = nullptr) {
     if (!ctx || (!text && n) || !n_done || (n_merges > 0 && !merge_pairs_out) || (n_sp > 0 && (!sp_blob || !sp_offs))) return BPE_ERR_ARG;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     *n_done = 0;
@@ -1310,10 +1392,11 @@ static int train_impl(bpe_ctx *ctx, const uint8_t *text, u64 n, bool text_is_dev
     BPE_TRY(ctx_load_text(ctx, text, n, text_is_device));
     int e1 = tm.mark();
     u64 nn = n;
-    BPE_TRY(ctx_run_flags(ctx, &nn, true, nullptr, nullptr, 0, 0));
+    const u32 *spstart;
+    BPE_TRY(run_flags_for_training(ctx, &nn, true, split, &spstart));
     int e2 = tm.mark();
     BPE_TRY(bpe_count_begin(ctx));
-    BPE_TRY(count_current_text(ctx, nn, 0, nn, nn));
+    BPE_TRY(count_current_text(ctx, nn, 0, nn, nn, spstart));
     int e3 = tm.mark();
     int rc = run_merges(ctx, sp_blob, sp_offs, n_sp, n_merges, merge_pairs_out, n_done, stats, tm, e0);
     if (stats) {
@@ -1336,14 +1419,24 @@ static u64 align_cut_host(const uint8_t *t, u64 n, u64 pos) {       // largest p
     for (int k = 0; k < 3 && pos > 0 && (t[pos] & 0xC0u) == 0x80u; k++) pos--;
     return pos;
 }
-static int count_host_pipelined(bpe_ctx *ctx, const uint8_t *text, u64 n, bpe_train_stats *stats, float *ms_pretok, float *ms_count) {
+// Split mode (split != null): special-token resolution at a cut can depend on context further left than any fixed halo (chains of
+// overlapping candidates), so the chunks are cut only at exact boundaries (exact_cut_host, as the encoder's pipeline) and each one is
+// counted as a whole text.  A nominal cut with no exact boundary within TRAIN_CUT_WINDOW after it is skipped: that chunk grows.
+#define TRAIN_CUT_WINDOW (8ull << 20)
+static int count_host_pipelined(bpe_ctx *ctx, const uint8_t *text, u64 n, bpe_train_stats *stats, float *ms_pretok, float *ms_count,
+                                const SplitSpecials *split = nullptr) {
     BPE_TRY(ctx_pipeline_init(ctx));
     cudaStream_t st = ctx->stream;
     std::vector<u64> cut{0};
-    for (u64 p = TRAIN_PIPE_CHUNK; p + TRAIN_PIPE_CHUNK / 2 < n; p += TRAIN_PIPE_CHUNK) cut.push_back(align_cut_host(text, n, p));
+    for (u64 p = TRAIN_PIPE_CHUNK; p + TRAIN_PIPE_CHUNK / 2 < n; p += TRAIN_PIPE_CHUNK) {
+        if (!split) { cut.push_back(align_cut_host(text, n, p)); continue; }
+        const u64 c = exact_cut_host(text, n, p, TRAIN_CUT_WINDOW, split->blob.data(), split->offs.data(), split->n());
+        if (c) cut.push_back(c);
+    }
     cut.push_back(n);
     const size_t m = cut.size() - 1;
     auto range = [&](size_t k, u64 *rlo, u64 *rhi) {
+        if (split) { *rlo = cut[k]; *rhi = cut[k + 1]; return; }
         *rlo = align_cut_host(text, n, cut[k] > TRAIN_HALO_LEFT ? cut[k] - TRAIN_HALO_LEFT : 0);
         *rhi = align_cut_host(text, n, std::min(n, cut[k + 1] + TRAIN_HALO_RIGHT));
     };
@@ -1370,11 +1463,12 @@ static int count_host_pipelined(bpe_ctx *ctx, const uint8_t *text, u64 n, bpe_tr
         EvTimer tm(ctx, 8);
         int e0 = tm.mark();
         u64 nn = b - a;
-        rc = ctx_run_flags(ctx, &nn, false, nullptr, nullptr, 0, 0, cut[k] - a, cut[k + 1] - a);
+        const u32 *spstart;
+        rc = run_flags_for_training(ctx, &nn, false, split, &spstart, cut[k] - a, cut[k + 1] - a);
         int e1 = tm.mark();
         if (rc == BPE_OK && ctx->saw_cr) rc = 1;
         if (rc == BPE_OK) {
-            rc = count_current_text(ctx, b - a, cut[k] - a, cut[k + 1] - a, b == n ? b - a : (b - a >= 16 ? b - a - 16 : 0));
+            rc = count_current_text(ctx, b - a, cut[k] - a, cut[k + 1] - a, b == n || split ? b - a : (b - a >= 16 ? b - a - 16 : 0), spstart);
             if (rc == BPE_ERR_HALO) rc = 1;
         }
         int e2 = tm.mark();
@@ -1388,9 +1482,8 @@ static int count_host_pipelined(bpe_ctx *ctx, const uint8_t *text, u64 n, bpe_tr
     return rc;
 }
 
-BPE_API int bpe_train(bpe_ctx *ctx, const uint8_t *text_host, uint64_t n, const uint8_t *specials_blob,
-                      const uint32_t *special_offs, int n_specials, int n_merges, int32_t *merge_pairs_out, int *n_done,
-                      bpe_train_stats *stats) {
+static int train_host(bpe_ctx *ctx, const uint8_t *text_host, uint64_t n, const uint8_t *specials_blob, const uint32_t *special_offs,
+                      int n_specials, int n_merges, int32_t *merge_pairs_out, int *n_done, bpe_train_stats *stats, const SplitSpecials *split) {
     if (n >= TRAIN_PIPE_MIN && ctx && text_host && n_done && (n_merges <= 0 || merge_pairs_out) && (n_specials <= 0 || (specials_blob && special_offs))) {
         CUDA_TRY(ctx, cudaSetDevice(ctx->device));
         *n_done = 0;
@@ -1400,7 +1493,7 @@ BPE_API int bpe_train(bpe_ctx *ctx, const uint8_t *text_host, uint64_t n, const 
         int e0 = tm.mark();
         BPE_TRY(bpe_count_begin(ctx));
         float ms_pretok = 0, ms_count = 0;
-        int rc = count_host_pipelined(ctx, text_host, n, stats, &ms_pretok, &ms_count);
+        int rc = count_host_pipelined(ctx, text_host, n, stats, &ms_pretok, &ms_count, split);
         if (rc == BPE_OK) {
             rc = run_merges(ctx, specials_blob, special_offs, n_specials, n_merges, merge_pairs_out, n_done, stats, tm, e0);
             if (stats) { stats->n_bytes = n; stats->ms_h2d = 0; stats->ms_pretok = ms_pretok; stats->ms_count = ms_count; }
@@ -1410,12 +1503,31 @@ BPE_API int bpe_train(bpe_ctx *ctx, const uint8_t *text_host, uint64_t n, const 
         ctx->count->active = false;
         if (rc != 1) return rc;                   // (1 = needs the one-piece path below)
     }
-    return train_impl(ctx, text_host, n, false, specials_blob, special_offs, n_specials, n_merges, merge_pairs_out, n_done, stats);
+    return train_impl(ctx, text_host, n, false, specials_blob, special_offs, n_specials, n_merges, merge_pairs_out, n_done, stats, split);
+}
+BPE_API int bpe_train(bpe_ctx *ctx, const uint8_t *text_host, uint64_t n, const uint8_t *specials_blob,
+                      const uint32_t *special_offs, int n_specials, int n_merges, int32_t *merge_pairs_out, int *n_done,
+                      bpe_train_stats *stats) {
+    return train_host(ctx, text_host, n, specials_blob, special_offs, n_specials, n_merges, merge_pairs_out, n_done, stats, nullptr);
 }
 BPE_API int bpe_train_dev(bpe_ctx *ctx, const uint8_t *text_dev, uint64_t n, const uint8_t *specials_blob,
                           const uint32_t *special_offs, int n_specials, int n_merges, int32_t *merge_pairs_out, int *n_done,
                           bpe_train_stats *stats) {
     return train_impl(ctx, text_dev, n, true, specials_blob, special_offs, n_specials, n_merges, merge_pairs_out, n_done, stats);
+}
+BPE_API int bpe_train_ex(bpe_ctx *ctx, const uint8_t *text_host, uint64_t n, const uint8_t *specials_blob,
+                         const uint32_t *special_offs, int n_specials, int n_merges, int32_t *merge_pairs_out, int *n_done,
+                         bpe_train_stats *stats, int flags) {
+    SplitSpecials sp; const SplitSpecials *split;
+    BPE_TRY(split_from_flags(ctx, flags, specials_blob, special_offs, n_specials, sp, &split));
+    return train_host(ctx, text_host, n, specials_blob, special_offs, n_specials, n_merges, merge_pairs_out, n_done, stats, split);
+}
+BPE_API int bpe_train_dev_ex(bpe_ctx *ctx, const uint8_t *text_dev, uint64_t n, const uint8_t *specials_blob,
+                             const uint32_t *special_offs, int n_specials, int n_merges, int32_t *merge_pairs_out, int *n_done,
+                             bpe_train_stats *stats, int flags) {
+    SplitSpecials sp; const SplitSpecials *split;
+    BPE_TRY(split_from_flags(ctx, flags, specials_blob, special_offs, n_specials, sp, &split));
+    return train_impl(ctx, text_dev, n, true, specials_blob, special_offs, n_specials, n_merges, merge_pairs_out, n_done, stats, split);
 }
 BPE_API int bpe_train_from_counts(bpe_ctx *ctx, const uint8_t *specials_blob, const uint32_t *special_offs, int n_specials,
                                   int n_merges, int32_t *merge_pairs_out, int *n_done, bpe_train_stats *stats) {

@@ -70,10 +70,21 @@ class DeviceCounter:
         self.ctx.check(self.L.bpe_count_begin(self.ctx.handle))
         self._expected_pairs = None
 
-    # returns None, or ("utf8", offset within data) / ("halo", 0) / ("newline", 0)
+    # returns None, or ("utf8", offset within data) / ("halo", 0) / ("newline", 0).  split_specials (split_special_tokens): the
+    # special tokens; data is then one whole text cut at exact boundaries (bpe_count_add_shard_ex)
     def add(self, data, own_begin: int, own_end: int, at_file_start: bool, at_file_end: bool, device_ptr: int | None = None,
-            n_bytes: int | None = None):
-        if device_ptr is not None:
+            n_bytes: int | None = None, split_specials: List[str] | None = None):
+        if split_specials is not None:
+            sp_blob, sp_offs = _lib.pack_blobs([s.encode("utf-8") for s in split_specials])
+            sp = (_lib.ptr(sp_blob), _lib.ptr(sp_offs), len(split_specials), _lib.TRAIN_SPLIT_SPECIALS)
+            if device_ptr is not None:
+                rc = self.L.bpe_count_add_shard_dev_ex(self.ctx.handle, C.c_void_p(device_ptr), int(n_bytes), own_begin, own_end,
+                                                       int(at_file_start), int(at_file_end), *sp)
+            else:
+                arr = _lib.as_u8(data)
+                rc = self.L.bpe_count_add_shard_ex(self.ctx.handle, _lib.ptr(arr) if arr.size else None, arr.size, own_begin, own_end,
+                                                   int(at_file_start), int(at_file_end), *sp)
+        elif device_ptr is not None:
             rc = self.L.bpe_count_add_shard_dev(self.ctx.handle, C.c_void_p(device_ptr), int(n_bytes), own_begin, own_end,
                                                 int(at_file_start), int(at_file_end))
         else:
@@ -246,11 +257,21 @@ class FileShards:
     def raise_decode_error(self, offset: int):
         _raise_decode_error(self.peek, self.size, offset)
 
+    def load_exact(self, rank: int, world: int, special_tokens: List[str]):
+        """split_special_tokens: rank r's range between exact cuts (sharded_encode.shard_cuts: every rank computes the same list),
+        read without a halo and counted as one whole text."""
+        from .sharded_encode import shard_cuts
+        cuts = shard_cuts(self.peek, self.size, [s.encode("utf-8") for s in special_tokens], world)
+        lo, hi = cuts[rank], cuts[rank + 1]
+        return dict(data=self.peek(lo, hi), device_ptr=None, n_bytes=hi - lo, own_begin=0, own_end=hi - lo, at_start=True, at_end=True,
+                    base=lo)
 
-def sharded_count(counter, shards, special_tokens: List[str], group=None, verify: bool = True):
+
+def sharded_count(counter, shards, special_tokens: List[str], group=None, verify: bool = True, split_special_tokens: bool = False):
     """Count the pretokens of the corpus behind `shards` across the ranks of `group` into `counter` (every rank ends
     with the merged table).  Returns "ok", or "newline" when some shard contains a carriage return (the caller
-    then takes the unsharded path: universal-newline translation shifts byte offsets)."""
+    then takes the unsharded path: universal-newline translation shifts byte offsets).  split_special_tokens: the ranges are
+    cut at exact boundaries and split on the specials (FileShards.load_exact, DeviceCounter.add)."""
     dist = _dist()
     world, rank = dist.get_world_size(group), dist.get_rank(group)
     import time
@@ -258,6 +279,13 @@ def sharded_count(counter, shards, special_tokens: List[str], group=None, verify
     t0 = time.perf_counter()
     halo = HALO_RIGHT
     while True:
+        if split_special_tokens:
+            sh = shards.load_exact(rank, world, special_tokens)
+            status = None
+            if sh["n_bytes"]:                      # (a rank past the last exact cut has nothing to count)
+                status = counter.add(sh["data"], 0, sh["n_bytes"], True, True, device_ptr=sh["device_ptr"], n_bytes=sh["n_bytes"],
+                                     split_specials=list(special_tokens))
+            break
         sh = shards.load(rank, world, halo)
         status = counter.add(sh["data"], sh["own_begin"], sh["own_end"], sh["at_start"], sh["at_end"], device_ptr=sh["device_ptr"],
                              n_bytes=sh["n_bytes"])
@@ -319,18 +347,19 @@ def merges_digest(merges) -> int:
 
 
 def train_bpe_sharded(input_path, vocab_size: int, special_tokens: List[str] = [], *, group=None, ctx=None, verify: bool = True,
-                      return_stats: bool = False):
+                      return_stats: bool = False, split_special_tokens: bool = False):
     """train_bpe over the ranks of an initialised torch.distributed group (one process per GPU).  Every rank
-    returns the same (vocab, merges) as the single-GPU train_bpe / the reference."""
+    returns the same (vocab, merges) as the single-GPU train_bpe / the reference (with split_special_tokens, as train_bpe's)."""
     dist = _dist()
     size = os.path.getsize(input_path)
     peek, f = _file_peek(input_path)
     try:
         counter = DeviceCounter(ctx)
-        outcome = sharded_count(counter, FileShards(peek, size), special_tokens, group, verify)
+        outcome = sharded_count(counter, FileShards(peek, size), special_tokens, group, verify, split_special_tokens)
         if outcome == "newline":
             from .train import train_bpe
-            return train_bpe(input_path, vocab_size, special_tokens, ctx=ctx, return_stats=return_stats)
+            return train_bpe(input_path, vocab_size, special_tokens, ctx=ctx, return_stats=return_stats,
+                             split_special_tokens=split_special_tokens)
         res = counter.finish(vocab_size, special_tokens, return_stats=return_stats)
     finally:
         f.close()

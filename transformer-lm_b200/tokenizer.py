@@ -91,13 +91,14 @@ class Tokenizer:
 
     # ---- constructors (tokenizer.py:40-61) -------------------------------------------------------
     @classmethod
-    def train_from_file(cls, filepath: str, vocab_size: int, special_tokens: List[str]):
-        vocab, merges = train_bpe(filepath, vocab_size, special_tokens)
+    def train_from_file(cls, filepath: str, vocab_size: int, special_tokens: List[str], *, split_special_tokens: bool = False):
+        """split_special_tokens=True trains on the text split at the special tokens, as encode splits it (train.train_bpe)."""
+        vocab, merges = train_bpe(filepath, vocab_size, special_tokens, split_special_tokens=split_special_tokens)
         return cls(vocab, merges, special_tokens)
 
     @classmethod
-    def fit(cls, input_path: str, vocab_size: int, special_tokens: List[str]):
-        vocab, merges = train_bpe(input_path, vocab_size, special_tokens)
+    def fit(cls, input_path: str, vocab_size: int, special_tokens: List[str], *, split_special_tokens: bool = False):
+        vocab, merges = train_bpe(input_path, vocab_size, special_tokens, split_special_tokens=split_special_tokens)
         return cls(vocab, merges, special_tokens)
 
     @classmethod

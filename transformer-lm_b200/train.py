@@ -153,8 +153,9 @@ def merges_to_python(vocab: Vocab, pairs: np.ndarray, n_done: int):
 
 
 def train_bpe_on_bytes(data, vocab_size: int, special_tokens: List[str] = [], *, ctx=None, return_stats: bool = False,
-                       device_ptr: int | None = None, n_bytes: int | None = None):
-    """train_bpe on an in-memory byte buffer (bytes / numpy uint8) or, with device_ptr, on text already in HBM."""
+                       device_ptr: int | None = None, n_bytes: int | None = None, split_special_tokens: bool = False):
+    """train_bpe on an in-memory byte buffer (bytes / numpy uint8) or, with device_ptr, on text already in HBM.
+    split_special_tokens: see train_bpe."""
     ctx = ctx or _lib.default_context()
     L = _lib.lib()
     vocab = Vocab(special_tokens=list(special_tokens))
@@ -166,7 +167,8 @@ def train_bpe_on_bytes(data, vocab_size: int, special_tokens: List[str] = [], *,
     live = LiveMerges(ctx, vocab, n_merges)
     rc = -1
     try:
-        rc = _call_train(L, ctx, data, device_ptr, n_bytes, sp_blob, sp_offs, special_tokens, n_merges, pairs, n_done, stats)
+        rc = _call_train(L, ctx, data, device_ptr, n_bytes, sp_blob, sp_offs, special_tokens, n_merges, pairs, n_done, stats,
+                         _lib.TRAIN_SPLIT_SPECIALS if split_special_tokens else 0)
     finally:
         res = live.finish(pairs, n_done.value if rc == _lib.BPE_OK else 0)
     arr = None if device_ptr is not None else _lib.as_u8(data)
@@ -183,14 +185,17 @@ def train_bpe_on_bytes(data, vocab_size: int, special_tokens: List[str] = [], *,
     return out + (stats.as_dict(),) if return_stats else out
 
 
-def _call_train(L, ctx, data, device_ptr, n_bytes, sp_blob, sp_offs, special_tokens, n_merges, pairs, n_done, stats):
+def _call_train(L, ctx, data, device_ptr, n_bytes, sp_blob, sp_offs, special_tokens, n_merges, pairs, n_done, stats, flags=0):
+    ex = (flags,) if flags else ()
     if device_ptr is not None:
-        rc = L.bpe_train_dev(ctx.handle, C.c_void_p(device_ptr), int(n_bytes), _lib.ptr(sp_blob), _lib.ptr(sp_offs),
-                             len(special_tokens), n_merges, _lib.ptr(pairs), C.byref(n_done), C.byref(stats))
+        fn = L.bpe_train_dev_ex if flags else L.bpe_train_dev
+        rc = fn(ctx.handle, C.c_void_p(device_ptr), int(n_bytes), _lib.ptr(sp_blob), _lib.ptr(sp_offs),
+                len(special_tokens), n_merges, _lib.ptr(pairs), C.byref(n_done), C.byref(stats), *ex)
     else:
         arr = _lib.as_u8(data)
-        rc = L.bpe_train(ctx.handle, _lib.ptr(arr) if arr.size else None, arr.size, _lib.ptr(sp_blob), _lib.ptr(sp_offs),
-                         len(special_tokens), n_merges, _lib.ptr(pairs), C.byref(n_done), C.byref(stats))
+        fn = L.bpe_train_ex if flags else L.bpe_train
+        rc = fn(ctx.handle, _lib.ptr(arr) if arr.size else None, arr.size, _lib.ptr(sp_blob), _lib.ptr(sp_offs),
+                len(special_tokens), n_merges, _lib.ptr(pairs), C.byref(n_done), C.byref(stats), *ex)
     return rc
 
 
@@ -238,13 +243,17 @@ def _open_for_read(path, direct: bool):
 
 
 def _train_bpe_streamed(input_path, size: int, vocab_size: int, special_tokens: List[str], ctx=None, return_stats: bool = False,
-                        direct_io: bool | None = None):
+                        direct_io: bool | None = None, split_special_tokens: bool = False):
     """Ingest path for big files (SURVEY 8f row 2): the file is read in 256 MB chunks, each with a small halo, by a few
     threads into page-locked buffers while the GPU pretokenises and counts the previous chunk (bpe_count_add_shard --
     the same shard contract as the multi-GPU path); then the merge loop runs on the counts.  Returns None when the file
-    needs the one-piece path (a carriage return: universal newlines shift offsets; or a pretoken longer than the halo)."""
+    needs the one-piece path (a carriage return: universal newlines shift offsets; or a pretoken longer than the halo).
+    split_special_tokens: the chunks are cut only at exact boundaries (sharded_encode.first_exact_cut) and each is counted whole,
+    with no halo: special-token resolution at a cut can depend on context further left than any fixed halo.  Where no exact
+    boundary follows a nominal cut the chunk grows to the next one."""
     import concurrent.futures as cf
     from .sharded import DeviceCounter, align_cut, _raise_decode_error
+    from .sharded_encode import first_exact_cut
     if direct_io is None:
         direct_io = os.environ.get("BPE_IO_DIRECT", "0") not in ("", "0")
     fd, direct = _open_for_read(input_path, direct_io)
@@ -255,17 +264,32 @@ def _train_bpe_streamed(input_path, size: int, vocab_size: int, special_tokens: 
     try:
         def peek(lo, hi):
             return os.pread(fd_peek, hi - lo, lo)
+        split = list(special_tokens) if split_special_tokens else None
+        specials_b = [s.encode("utf-8") for s in special_tokens]
         cuts = [0]
         p = _STREAM_CHUNK
         while p + _STREAM_CHUNK // 2 < size:
-            cuts.append(align_cut(peek, p, size))
+            if split is None:
+                cuts.append(align_cut(peek, p, size))
+            else:
+                try:
+                    c = first_exact_cut(peek, size, specials_b, max(p, cuts[-1] + 1))
+                except RuntimeError:
+                    break                                # no exact boundary from here on: the rest is one chunk
+                if c >= size:
+                    break
+                cuts.append(c)
+                p = max(p, c)
             p += _STREAM_CHUNK
         cuts.append(size)
         ranges = []
         for k in range(len(cuts) - 1):
             lo, hi = cuts[k], cuts[k + 1]
-            rlo = align_cut(peek, max(0, lo - _STREAM_HALO_LEFT), size)
-            rhi = align_cut(peek, min(size, hi + _STREAM_HALO_RIGHT), size)
+            if split is None:
+                rlo = align_cut(peek, max(0, lo - _STREAM_HALO_LEFT), size)
+                rhi = align_cut(peek, min(size, hi + _STREAM_HALO_RIGHT), size)
+            else:
+                rlo, rhi = lo, hi
             ranges.append((lo, hi, rlo, rhi))
         # with O_DIRECT a chunk is read as the block-aligned range around it (the page-locked buffers are page aligned); `skew` =
         # where the chunk starts inside its buffer
@@ -295,7 +319,8 @@ def _train_bpe_streamed(input_path, size: int, vocab_size: int, special_tokens: 
             for fut in pending.pop(k):
                 fut.result()
             skew = rlo - rlo // A * A
-            status = counter.add(bufs[k % len(bufs)].array[skew: skew + rhi - rlo], lo - rlo, hi - rlo, rlo == 0, rhi == size)
+            status = counter.add(bufs[k % len(bufs)].array[skew: skew + rhi - rlo], lo - rlo, hi - rlo, rlo == 0, rhi == size,
+                                 **({} if split is None else {"split_specials": split}))
             if status is not None:
                 if status[0] == "utf8":
                     _raise_decode_error(peek, size, rlo + status[1])      # what open(path, encoding="utf-8").read() raises
@@ -317,14 +342,18 @@ def _train_bpe_streamed(input_path, size: int, vocab_size: int, special_tokens: 
             os.close(fd_peek)
 
 
-def train_bpe(input_path, vocab_size: int, special_tokens: List[str] = [], *, distributed: bool = False, **kwargs):
+def train_bpe(input_path, vocab_size: int, special_tokens: List[str] = [], *, distributed: bool = False,
+              split_special_tokens: bool = False, **kwargs):
     """Drop-in for models/tokenizer/train.py:142 train_bpe.  Extra keyword arguments are ours (the reference's
     adapter never passes any): ctx=, return_stats=, direct_io= (files of >= 512 MB are streamed; True or BPE_IO_DIRECT=1 reads them
     with O_DIRECT), and distributed=True to shard the file over the ranks of the initialised torch.distributed group (one process
-    per GPU; see sharded.py)."""
+    per GPU; see sharded.py).
+    split_special_tokens=True splits the text on the special tokens before counting, as the tokenizer does before encoding: no
+    pretoken, pair or merge crosses an occurrence and the occurrences are not counted (BPE_TRAIN_SPLIT_SPECIALS in
+    include/bpe_sm100.h).  The default (False) counts the text whole, exactly as the reference does."""
     if distributed:
         from .sharded import train_bpe_sharded
-        return train_bpe_sharded(input_path, vocab_size, special_tokens, **kwargs)
+        return train_bpe_sharded(input_path, vocab_size, special_tokens, split_special_tokens=split_special_tokens, **kwargs)
     t0 = time.time()
     size = os.path.getsize(input_path)           # FileNotFoundError like open() in the reference
     kwargs = dict(kwargs)
@@ -332,10 +361,11 @@ def train_bpe(input_path, vocab_size: int, special_tokens: List[str] = [], *, di
     direct_io = kwargs.pop("direct_io", None)
     res = None
     if size >= _STREAM_MIN:
-        res = _train_bpe_streamed(input_path, size, vocab_size, special_tokens, return_stats=True, direct_io=direct_io, **kwargs)
+        res = _train_bpe_streamed(input_path, size, vocab_size, special_tokens, return_stats=True, direct_io=direct_io,
+                                  split_special_tokens=split_special_tokens, **kwargs)
     if res is None:
         arr, _keep = _read_file(input_path)
-        res = train_bpe_on_bytes(arr, vocab_size, special_tokens, return_stats=True, **kwargs)
+        res = train_bpe_on_bytes(arr, vocab_size, special_tokens, return_stats=True, split_special_tokens=split_special_tokens, **kwargs)
     _log_stages(res[2], time.time() - t0)
     return res if want_stats else res[:2]
 
