@@ -231,71 +231,73 @@ typedef struct bpe_encode_stats {
  * returns BPE_ERR_ARG (the reference's np.uint16 cast at models/tokenizer/encode.py:37 would wrap). */
 int bpe_encode(bpe_tok *tok, const uint8_t *text_host, uint64_t n, int out_dtype,
                void *out, uint64_t cap, uint64_t *n_out, bpe_encode_stats *stats);
-/* Replaces [Tokenizer.encode(d) for d in docs]: models/tokenizer/tokenizer.py:111-138 once per document.
- * text_host holds n_docs UTF-8 documents back to back, document j = text[doc_offs[j] .. doc_offs[j+1])
- * (doc_offs[0] = 0, doc_offs[n_docs] = n, non-decreasing).  Writes the ids of all documents back to back and
- * id_offs_out[j] (n_docs + 1 entries) = index of document j's first id.  Same size-query idiom, dtypes and errors as
- * bpe_encode; BPE_ERR_UTF8 / BPE_ERR_KEY detail = byte offset in text_host.  Every document is encoded on its own: no
- * pretoken or special-token occurrence spans two documents, and UTF-8 validity is per document.  The error reported is the
- * first one the device meets: an invalid UTF-8 sequence anywhere in a pipeline chunk (256 MB of documents) comes before a
- * KeyError in it, so a caller that needs the first failing document in list order re-encodes the documents before the
- * invalid one (Tokenizer.encode_batch does).  BPE_ERR_UNSUPPORTED when every ASCII byte but '\r' occurs in some special
- * token (the boundary byte between documents must occur in none).  bpe_tok_saw_cr afterwards: a '\r' in any document. */
-int bpe_encode_batch(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
-                     int out_dtype, void *out, uint64_t cap, uint64_t *n_out, uint64_t *id_offs_out, bpe_encode_stats *stats);
-/* BPE-dropout (subword regularisation, Provilkov et al. 2020): bpe_encode / bpe_encode_batch where every pretoken occurrence gets its
- * own random segmentation.  Same two-call idiom (out == NULL reports the same *n_out), dtypes, errors, error details and
- * bpe_tok_saw_cr as the deterministic calls; BPE_ERR_ARG when p is outside [0, 1] or NaN.  The result is a pure function of
- * (tokenizer, text, document split, p, seed): it does not depend on the pretoken cache or on how the library cuts the text.
- *   mix(z): z += 0x9E3779B97F4A7C15; z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9; z = (z ^ (z >> 27)) * 0x94D049BB133111EB;
- *           return z ^ (z >> 31)                                                         (splitmix64 finalizer, all mod 2^64)
- *   u(seed, doc, off, t) = mix(mix(mix(mix(seed) ^ doc) ^ off) ^ t)
- *   thr(p) = 2^32 if p == 1 else floor(p * 2^32)
- *   dropped = (u(seed, doc, off, t) >> 32) < thr(p)
- * doc = the document's index (0 for bpe_encode_dropout), off = byte offset in that document of the first byte of the candidate pair's
- * left token, t = the 0-based merge round within the pretoken occurrence.  BPE of one occurrence (the merge loop of
- * models/tokenizer/tokenizer.py:92-109,124-136 with candidates removed at random):
- *   tokens = the pretoken's bytes; t = 0
- *   loop: cand = { i : (tokens[i], tokens[i+1]) has a merge rank and not dropped(seed, doc, off_i, t) }
- *         if cand is empty: stop
- *         r = min rank over cand; scan i left to right: if i in cand and rank(i) == r: merge i, i+1 and i += 2, else i += 1
- *         t += 1
- *   ids = vocab_inv[token] for each token (a missing token is BPE_ERR_KEY, as in tokenizer.py:135)
- * Special-token occurrences are one id and never split.  p = 0 gives exactly bpe_encode / bpe_encode_batch; p = 1 gives every
- * pretoken as single bytes.  Dropout can emit tokens deterministic BPE never does, so with a vocabulary that lacks an intermediate
- * merge product one of the two calls can raise a KeyError the other does not. */
-int bpe_encode_dropout(bpe_tok *tok, const uint8_t *text_host, uint64_t n, double p, uint64_t seed, int out_dtype,
-                       void *out, uint64_t cap, uint64_t *n_out, bpe_encode_stats *stats);
-int bpe_encode_batch_dropout(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
-                             double p, uint64_t seed, int out_dtype, void *out, uint64_t cap, uint64_t *n_out,
-                             uint64_t *id_offs_out, bpe_encode_stats *stats);
-/* Token offsets: the ids of bpe_encode / bpe_encode_batch / bpe_encode_dropout / bpe_encode_batch_dropout with the same arguments, and
- * for every token i its span [start_i, end_i) of the input, offs_out[2 i], offs_out[2 i + 1] (int64, cap x 2 entries).  Same two-call
- * idiom (out == NULL reports *n_out and writes no offsets; otherwise offs_out must be given), dtypes, errors in the same order and error
- * details; BPE_ERR_ARG for an unknown unit.
- *   BPE_OFF_BYTES  the bytes token i was produced from.  The spans tile the document in order (start_0 = 0, end_i = start_{i+1}, the last
- *                  end = its length).  The tokens of a pretoken occurrence tile it; each but its last is as long as its vocabulary entry
- *                  and the last ends where the pretoken ends.  So data[start:end] == vocab[id] for an ordinary token, and a special-token
- *                  occurrence spans the special's bytes whatever its id (also an id missing from the vocabulary or shared with another
- *                  token, SURVEY A-12).
- *   BPE_OFF_CHARS  Python str indices: start = index of the character that holds the token's first byte, end = one past the index of the
- *                  character that holds its last byte.  A token that splits a multi-byte character maps to the whole character, so the
- *                  spans of the tokens that share it overlap by one (as HF byte-level offsets do): text[start:end].encode() always
- *                  contains the token's bytes, and equals them when no character is split.
- * Batch calls: spans are relative to each document's start, as if it were encoded on its own.  The spans depend only on the text, the
- * document split, p and seed: not on the pretoken cache, how the library cuts the text, or the batch size. */
+/* bpe_encode_ex: bpe_encode with options -- documents, BPE-dropout and token offsets, each independent of the others; opts == NULL,
+ * or a zero-filled struct, is bpe_encode exactly.  BPE_ERR_ARG, checked in this order: a null tokenizer, an unknown offset_unit (with
+ * offsets), a null offs_out (with offsets and out != NULL), dropout outside [0, 1] or NaN, then document offsets that are not as
+ * described below (BPE_ERR_UNSUPPORTED after them when there is no boundary byte). */
+typedef struct bpe_encode_opts {
+    /* Documents: replaces [Tokenizer.encode(d) for d in docs]: models/tokenizer/tokenizer.py:111-138 once per document.
+     * doc_offs == NULL: the text is one document (bpe_encode), n_docs must be 0 and id_offs_out is unused.  Otherwise
+     * text_host holds n_docs UTF-8 documents back to back, document j = text[doc_offs[j] .. doc_offs[j+1])
+     * (doc_offs[0] = 0, doc_offs[n_docs] = n, non-decreasing); an empty batch passes the one-element array {0}.  Writes the ids of
+     * all documents back to back and id_offs_out[j] (n_docs + 1 entries, required) = index of document j's first id.  Same
+     * size-query idiom, dtypes and errors as bpe_encode; BPE_ERR_UTF8 / BPE_ERR_KEY detail = byte offset in text_host.  Every
+     * document is encoded on its own: no pretoken or special-token occurrence spans two documents, and UTF-8 validity is per
+     * document.  The error reported is the first one the device meets: an invalid UTF-8 sequence anywhere in a pipeline chunk
+     * (256 MB of documents) comes before a KeyError in it, so a caller that needs the first failing document in list order
+     * re-encodes the documents before the invalid one (Tokenizer.encode_batch does).  BPE_ERR_UNSUPPORTED when every ASCII byte
+     * but '\r' occurs in some special token (the boundary byte between documents must occur in none).  bpe_tok_saw_cr afterwards:
+     * a '\r' in any document. */
+    const uint64_t *doc_offs;
+    uint64_t n_docs;
+    uint64_t *id_offs_out;
+    /* BPE-dropout (subword regularisation, Provilkov et al. 2020): dropout = p in (0, 1], the encode where every pretoken occurrence
+     * gets its own random segmentation; p = 0 is the deterministic encode.  Same two-call idiom (out == NULL reports the same
+     * *n_out), dtypes, errors, error details and bpe_tok_saw_cr as the deterministic calls; BPE_ERR_ARG when p is outside [0, 1] or
+     * NaN.  The result is a pure function of (tokenizer, text, document split, p, seed): it does not depend on the pretoken cache or
+     * on how the library cuts the text.
+     *   mix(z): z += 0x9E3779B97F4A7C15; z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9; z = (z ^ (z >> 27)) * 0x94D049BB133111EB;
+     *           return z ^ (z >> 31)                                                         (splitmix64 finalizer, all mod 2^64)
+     *   u(seed, doc, off, t) = mix(mix(mix(mix(seed) ^ doc) ^ off) ^ t)
+     *   thr(p) = 2^32 if p == 1 else floor(p * 2^32)
+     *   dropped = (u(seed, doc, off, t) >> 32) < thr(p)
+     * doc = the document's index (0 when doc_offs == NULL), off = byte offset in that document of the first byte of the candidate
+     * pair's left token, t = the 0-based merge round within the pretoken occurrence.  BPE of one occurrence (the merge loop of
+     * models/tokenizer/tokenizer.py:92-109,124-136 with candidates removed at random):
+     *   tokens = the pretoken's bytes; t = 0
+     *   loop: cand = { i : (tokens[i], tokens[i+1]) has a merge rank and not dropped(seed, doc, off_i, t) }
+     *         if cand is empty: stop
+     *         r = min rank over cand; scan i left to right: if i in cand and rank(i) == r: merge i, i+1 and i += 2, else i += 1
+     *         t += 1
+     *   ids = vocab_inv[token] for each token (a missing token is BPE_ERR_KEY, as in tokenizer.py:135)
+     * Special-token occurrences are one id and never split.  p = 0 gives exactly the deterministic encode; p = 1 gives every
+     * pretoken as single bytes.  Dropout can emit tokens deterministic BPE never does, so with a vocabulary that lacks an
+     * intermediate merge product one of the two calls can raise a KeyError the other does not. */
+    double dropout;
+    uint64_t seed;
+    /* Token offsets (with_offsets != 0): the ids of the same call without offsets, and for every token i its span [start_i, end_i)
+     * of the input, offs_out[2 i], offs_out[2 i + 1] (int64, cap x 2 entries).  Same two-call idiom (out == NULL reports *n_out and
+     * writes no offsets; otherwise offs_out must be given), dtypes, errors in the same order and error details; BPE_ERR_ARG for an
+     * unknown offset_unit.
+     *   BPE_OFF_BYTES  the bytes token i was produced from.  The spans tile the document in order (start_0 = 0, end_i = start_{i+1}, the last
+     *                  end = its length).  The tokens of a pretoken occurrence tile it; each but its last is as long as its vocabulary entry
+     *                  and the last ends where the pretoken ends.  So data[start:end] == vocab[id] for an ordinary token, and a special-token
+     *                  occurrence spans the special's bytes whatever its id (also an id missing from the vocabulary or shared with another
+     *                  token, SURVEY A-12).
+     *   BPE_OFF_CHARS  Python str indices: start = index of the character that holds the token's first byte, end = one past the index of the
+     *                  character that holds its last byte.  A token that splits a multi-byte character maps to the whole character, so the
+     *                  spans of the tokens that share it overlap by one (as HF byte-level offsets do): text[start:end].encode() always
+     *                  contains the token's bytes, and equals them when no character is split.
+     * With documents: spans are relative to each document's start, as if it were encoded on its own.  The spans depend only on the
+     * text, the document split, p and seed: not on the pretoken cache, how the library cuts the text, or the batch size. */
+    int with_offsets;
+    int offset_unit;
+    int64_t *offs_out;
+} bpe_encode_opts;
 #define BPE_OFF_BYTES 0
 #define BPE_OFF_CHARS 1
-int bpe_encode_offsets(bpe_tok *tok, const uint8_t *text_host, uint64_t n, int out_dtype, void *out, uint64_t cap, uint64_t *n_out,
-                       int unit, int64_t *offs_out, bpe_encode_stats *stats);
-int bpe_encode_batch_offsets(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
-                             int out_dtype, void *out, uint64_t cap, uint64_t *n_out, uint64_t *id_offs_out, int unit, int64_t *offs_out,
-                             bpe_encode_stats *stats);
-int bpe_encode_dropout_offsets(bpe_tok *tok, const uint8_t *text_host, uint64_t n, double p, uint64_t seed, int out_dtype, void *out,
-                               uint64_t cap, uint64_t *n_out, int unit, int64_t *offs_out, bpe_encode_stats *stats);
-int bpe_encode_batch_dropout_offsets(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
-                                     double p, uint64_t seed, int out_dtype, void *out, uint64_t cap, uint64_t *n_out,
-                                     uint64_t *id_offs_out, int unit, int64_t *offs_out, bpe_encode_stats *stats);
+int bpe_encode_ex(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const bpe_encode_opts *opts,
+                  int out_dtype, void *out, uint64_t cap, uint64_t *n_out, bpe_encode_stats *stats);
 /* 1 if the text of the last bpe_encode* call on this tokenizer's context held a carriage return (the flags kernel
  * sees every byte anyway).  Tokenizer.encode takes a str and keeps '\r' as it is; a caller that reads a FILE in text mode, like the
  * reference's bulk driver (models/tokenizer/encode.py:31-34, universal newlines), uses this instead of scanning the text on the host:

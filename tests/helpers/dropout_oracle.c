@@ -1,5 +1,5 @@
 /*
- * dropout_oracle.c -- CPU oracle of BPE-dropout (bpe_encode_dropout / bpe_encode_batch_dropout, spec in include/bpe_sm100.h).
+ * dropout_oracle.c -- CPU oracle of BPE-dropout (bpe_encode_ex with dropout > 0, spec at bpe_encode_opts in include/bpe_sm100.h).
  * TEST INFRASTRUCTURE ONLY, built at test time by tests/helpers/dropout_oracle.py.
  *
  * It compiles the CPU oracle (oracle/bpe_oracle.c) into the same unit and reuses its tokenizer tables, segmentation and GPT-2

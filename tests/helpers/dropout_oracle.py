@@ -1,7 +1,7 @@
 """CPU oracle of BPE-dropout (tests/helpers/dropout_oracle.c on top of oracle/bpe_oracle.c).  TEST INFRASTRUCTURE ONLY.
 
-DropoutOracle is oracle.OracleTokenizer with encode_bytes(data, *, dropout=, seed=, doc=): the spec of bpe_encode_dropout
-(include/bpe_sm100.h) for `data` as document `doc` of a batch; dropout = 0 is the oracle's plain encode.  The library is compiled
+DropoutOracle is oracle.OracleTokenizer with encode_bytes(data, *, dropout=, seed=, doc=): the spec of BPE-dropout
+(bpe_encode_opts in include/bpe_sm100.h) for `data` as document `doc` of a batch; dropout = 0 is the oracle's plain encode.  The library is compiled
 on first use into the temporary directory (the repository tree may be read-only), named by a hash of its sources."""
 from __future__ import annotations
 

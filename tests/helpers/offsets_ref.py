@@ -1,4 +1,4 @@
-"""Python reference of the token-offsets spec (bpe_encode_offsets, include/bpe_sm100.h).  TEST INFRASTRUCTURE ONLY.
+"""Python reference of the token-offsets spec (bpe_encode_opts, include/bpe_sm100.h).  TEST INFRASTRUCTURE ONLY.
 
 reference_offsets(otok, data, unit, ids=None) -> (ids, spans[n, 2]): segment `data` on the special tokens (leftmost, longest first), GPT-2
 pretokens in between; the tokens of an occurrence tile it, each but the last as long as its vocabulary entry and the last up to the

@@ -1,6 +1,6 @@
 """Host logic of Tokenizer.encode_batch / encode_batch_to_numpy without a device: packing the documents into one buffer with byte
 offsets, the order of exceptions (the first failing document in list order), splitting the ids by the offsets, argument checks
-of bpe_encode_batch."""
+of bpe_encode_ex with document offsets."""
 import ctypes as C
 
 import numpy as np
@@ -41,25 +41,25 @@ def test_pack_stops_at_a_lone_surrogate():
 
 
 class _FakeDevice:
-    """_encode_batch_packed stand-in: ids = the bytes of each document; a document holding b"K" is a KeyError."""
+    """_encode_ex stand-in for a batch: ids = the bytes of each document; a document holding b"K" is a KeyError."""
 
-    def __call__(self, blob, offs, dtype, texts=None):
-        docs = _unpack(blob, offs)
-        for d in docs:
+    def __call__(self, blob, dtype, *, docs, texts=None, drop=(0.0, 0), unit=None):
+        parts = _unpack(blob, docs)
+        for d in parts:
             if b"K" in d:
                 raise KeyError(b"K")
-        ids = np.frombuffer(b"".join(docs), dtype=np.uint8).astype(dtype)
-        return ids, offs.astype(np.int64)
+        ids = np.frombuffer(b"".join(parts), dtype=np.uint8).astype(dtype)
+        return ids, None, docs.astype(np.int64)
 
 
 @pytest.fixture
 def fake_tok(monkeypatch):
     tok = Tokenizer({i: bytes([i]) for i in range(256)}, [], [])
-    monkeypatch.setattr(tok, "_encode_batch_packed", _FakeDevice())
+    monkeypatch.setattr(tok, "_encode_ex", _FakeDevice())
     return tok
 
 
-def test_first_failing_document_wins(fake_tok):
+def test_first_failing_document_in_list_order_raises(fake_tok):
     with pytest.raises(KeyError):
         fake_tok.encode_batch(["a", "K", "b \ud800"])             # the KeyError comes first in list order
     with pytest.raises(UnicodeEncodeError):
@@ -68,7 +68,7 @@ def test_first_failing_document_wins(fake_tok):
         fake_tok.encode_batch(["\ud800"])
 
 
-def test_split_by_offsets(fake_tok):
+def test_ids_split_by_document_offsets(fake_tok):
     docs = ["ab", "", "cde", "", "f"]
     assert fake_tok.encode_batch(docs) == [list(d.encode()) for d in docs]
     assert fake_tok.encode_batch([]) == []
@@ -77,10 +77,11 @@ def test_split_by_offsets(fake_tok):
     assert fake_tok.encode_batch(iter(["a", "b"])) == [[97], [98]]          # any iterable of documents
 
 
-def test_c_abi_argument_checks():
+def test_encode_ex_batch_rejects_null_tokenizer():
     L = _lib.lib()
     n_out = C.c_uint64(0)
     ids = np.zeros(2, dtype=np.uint64)
     offs = np.array([0, 3], dtype=np.uint64)
     blob = np.frombuffer(b"abc", dtype=np.uint8)
-    assert L.bpe_encode_batch(None, _lib.ptr(blob), 3, _lib.ptr(offs), 1, _lib.DTYPE_I32, None, 0, C.byref(n_out), _lib.ptr(ids), None) == _lib.ERR_ARG
+    opts = _lib.EncodeOpts(doc_offs=offs.ctypes.data, n_docs=1, id_offs_out=ids.ctypes.data)
+    assert L.bpe_encode_ex(None, _lib.ptr(blob), 3, C.byref(opts), _lib.DTYPE_I32, None, 0, C.byref(n_out), None) == _lib.ERR_ARG

@@ -1,4 +1,4 @@
-"""BPE-dropout spec (include/bpe_sm100.h, bpe_encode_dropout) on the CPU: its test vectors and worked example, the dropout oracle
+"""BPE-dropout spec (include/bpe_sm100.h, bpe_encode_opts) on the CPU: its test vectors and worked example, the dropout oracle
 (tests/helpers/dropout_oracle.c) against an independent Python restatement of the spec on fuzzed texts, and Tokenizer's argument
 checks."""
 import math

@@ -1,4 +1,4 @@
-"""Token-offsets spec (include/bpe_sm100.h, bpe_encode_offsets) on the CPU: the Python reference (tests/helpers/offsets_ref.py) against
+"""Token-offsets spec (include/bpe_sm100.h, bpe_encode_opts) on the CPU: the Python reference (tests/helpers/offsets_ref.py) against
 the spec's invariants on fuzzed text, hand-worked cases (split characters, special tokens missing from the vocabulary or sharing an id with
 an ordinary token, SURVEY A-12), and the argument checks of the Tokenizer methods and the C ABI."""
 import ctypes as C
@@ -125,13 +125,14 @@ def test_tokenizer_rejects_bad_dropout(kw):
             call()
 
 
-def test_c_abi_rejects_null_tokenizer():
+def test_encode_ex_offsets_reject_null_tokenizer():
     L = _lib.lib()
     n = C.c_uint64(0)
     buf = np.zeros(4, dtype=np.int64)
-    assert L.bpe_encode_offsets(None, None, 0, _lib.DTYPE_I32, None, 0, C.byref(n), _lib.OFF_BYTES, None, None) == _lib.ERR_ARG
-    assert L.bpe_encode_batch_offsets(None, None, 0, None, 0, _lib.DTYPE_I32, None, 0, C.byref(n), _lib.ptr(buf), _lib.OFF_CHARS, None,
-                                      None) == _lib.ERR_ARG
-    assert L.bpe_encode_dropout_offsets(None, None, 0, 0.5, 1, _lib.DTYPE_I32, None, 0, C.byref(n), _lib.OFF_BYTES, None, None) == _lib.ERR_ARG
-    assert L.bpe_encode_batch_dropout_offsets(None, None, 0, None, 0, 0.5, 1, _lib.DTYPE_I32, None, 0, C.byref(n), _lib.ptr(buf),
-                                              _lib.OFF_BYTES, None, None) == _lib.ERR_ARG
+    docs = np.zeros(1, dtype=np.uint64)                                   # an empty batch
+    batch = dict(doc_offs=docs.ctypes.data, n_docs=0, id_offs_out=buf.ctypes.data)
+    for opts in (_lib.EncodeOpts(with_offsets=1, offset_unit=_lib.OFF_BYTES),
+                 _lib.EncodeOpts(with_offsets=1, offset_unit=_lib.OFF_CHARS, **batch),
+                 _lib.EncodeOpts(dropout=0.5, seed=1, with_offsets=1, offset_unit=_lib.OFF_BYTES),
+                 _lib.EncodeOpts(dropout=0.5, seed=1, with_offsets=1, offset_unit=_lib.OFF_BYTES, **batch)):
+        assert L.bpe_encode_ex(None, None, 0, C.byref(opts), _lib.DTYPE_I32, None, 0, C.byref(n), None) == _lib.ERR_ARG

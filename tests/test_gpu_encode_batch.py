@@ -1,4 +1,4 @@
-"""GPU parity of Tokenizer.encode_batch / encode_batch_to_numpy (bpe_encode_batch): many documents in one device pass must give
+"""GPU parity of Tokenizer.encode_batch / encode_batch_to_numpy (bpe_encode_ex with document offsets): many documents in one device pass must give
 exactly [tok.encode(d) for d in docs] -- the same ids, the same split, the same first exception.  The expected value is the CPU
 oracle per document (and the encode loop); the documents are chosen so that encoding their concatenation would differ."""
 import ctypes as C
@@ -156,7 +156,7 @@ def test_surrogate_and_keyerror_ordering():
         tok.encode_batch(["ok", "bad \ud800", "zab"])
 
 
-def test_per_document_utf8_validity(gpt2):
+def test_utf8_validity_is_per_document(gpt2):
     tok, otok = gpt2
     docs = [b"ok ", b"abc\xe4\xb8", b"\xad rest"]                         # joined: valid ("abc" + U+4E2D + " rest")
     b"".join(docs).decode("utf-8")
@@ -178,8 +178,8 @@ def test_per_document_utf8_validity(gpt2):
     out = np.empty(blob.size, dtype=np.int32)
     id_offs = np.zeros(4, dtype=np.uint64)
     n_out = C.c_uint64(0)
-    rc = L.bpe_encode_batch(h, _lib.ptr(blob), blob.size, _lib.ptr(doc_offs), 3, _lib.DTYPE_I32, _lib.ptr(out), out.size,
-                            C.byref(n_out), _lib.ptr(id_offs), None)
+    opts = _lib.EncodeOpts(doc_offs=doc_offs.ctypes.data, n_docs=3, id_offs_out=id_offs.ctypes.data)
+    rc = L.bpe_encode_ex(h, _lib.ptr(blob), blob.size, C.byref(opts), _lib.DTYPE_I32, _lib.ptr(out), out.size, C.byref(n_out), None)
     assert rc == _lib.ERR_UTF8
     assert L.bpe_last_error_detail(tok._tok_ctx.handle) == 6
 
@@ -192,7 +192,7 @@ def test_keyerror_before_a_later_invalid_document():
         tok.encode_batch_to_numpy([b"ok", b"\xff", b"zab"])
 
 
-def test_c_abi_argument_checks(gpt2):
+def test_encode_ex_document_offset_checks(gpt2):
     tok, _ = gpt2
     L = _lib.lib()
     h = tok._device_tok()
@@ -200,14 +200,17 @@ def test_c_abi_argument_checks(gpt2):
     out = np.empty(8, dtype=np.int32)
     ids = np.zeros(3, dtype=np.uint64)
     n_out = C.c_uint64(0)
-    for offs in ([0, 4, 3], [1, 3, 6], [0, 3, 5]):
+
+    def encode_batch(offs, out, cap):
         o = np.array(offs, dtype=np.uint64)
-        assert L.bpe_encode_batch(h, _lib.ptr(blob), 6, _lib.ptr(o), 2, _lib.DTYPE_I32, _lib.ptr(out), 8, C.byref(n_out),
-                                  _lib.ptr(ids), None) == _lib.ERR_ARG
-    o = np.array([0, 3, 6], dtype=np.uint64)
-    assert L.bpe_encode_batch(h, _lib.ptr(blob), 6, _lib.ptr(o), 2, _lib.DTYPE_I32, _lib.ptr(out), 8, C.byref(n_out), _lib.ptr(ids), None) == 0
+        opts = _lib.EncodeOpts(doc_offs=o.ctypes.data, n_docs=2, id_offs_out=ids.ctypes.data)
+        return L.bpe_encode_ex(h, _lib.ptr(blob), 6, C.byref(opts), _lib.DTYPE_I32, out, cap, C.byref(n_out), None)
+
+    for offs in ([0, 4, 3], [1, 3, 6], [0, 3, 5]):
+        assert encode_batch(offs, _lib.ptr(out), 8) == _lib.ERR_ARG
+    assert encode_batch([0, 3, 6], _lib.ptr(out), 8) == 0
     assert ids.tolist()[0] == 0 and ids.tolist()[2] == n_out.value
-    assert L.bpe_encode_batch(h, _lib.ptr(blob), 6, _lib.ptr(o), 2, _lib.DTYPE_I32, None, 0, C.byref(n_out), _lib.ptr(ids), None) == 0
+    assert encode_batch([0, 3, 6], None, 0) == 0
     assert ids.tolist()[2] == n_out.value                                 # size query: the offsets too
 
 

@@ -1,4 +1,4 @@
-"""GPU parity of BPE-dropout (bpe_encode_dropout / bpe_encode_batch_dropout through Tokenizer.encode_to_numpy and
+"""GPU parity of BPE-dropout (bpe_encode_ex with dropout > 0, through Tokenizer.encode_to_numpy and
 encode_batch_to_numpy): exact equality with the CPU dropout oracle (tests/helpers/dropout_oracle.c), with doc = the document's index in the batch;
 independence from the pretoken cache, from batch and chunk boundaries; p = 0 is encode."""
 import os

@@ -1,4 +1,4 @@
-"""GPU token offsets (bpe_encode_offsets and the batch / dropout variants through Tokenizer.encode_offsets_to_numpy and
+"""GPU token offsets (bpe_encode_ex with offsets, alone or with documents and dropout, through Tokenizer.encode_offsets_to_numpy and
 encode_batch_offsets_to_numpy): exact equality of ids and spans, in bytes and in characters, with the Python reference of the spec
 (tests/helpers/offsets_ref.py) over the CPU oracles' ids; the ids equal those of the ids-only calls; batch spans equal the per-document
 ones; independence from pipeline chunks and the pretoken cache; the same errors as the ids-only calls.
@@ -184,7 +184,7 @@ def test_errors_match_ids_only_calls():
     assert _outcome(lambda: good.encode_to_numpy(data)) == _outcome(lambda: good.encode_offsets_to_numpy(data, unit="char"))
 
 
-def test_c_abi_unknown_unit_and_count_only(gpt2):
+def test_encode_ex_unknown_unit_and_count_only(gpt2):
     tok, _ = gpt2
     L = _lib.lib()
     h = tok._device_tok()
@@ -192,14 +192,17 @@ def test_c_abi_unknown_unit_and_count_only(gpt2):
     out = np.zeros(16, dtype=np.int32)
     spans = np.zeros((16, 2), dtype=np.int64)
     n = C.c_uint64(0)
+
+    def encode_offsets(out, cap, unit, offs_out):
+        opts = _lib.EncodeOpts(with_offsets=1, offset_unit=unit, offs_out=offs_out)
+        return L.bpe_encode_ex(h, _lib.ptr(data), data.size, C.byref(opts), _lib.DTYPE_I32, out, cap, C.byref(n), None)
+
     for unit in (-1, 2, 99):
-        assert L.bpe_encode_offsets(h, _lib.ptr(data), data.size, _lib.DTYPE_I32, _lib.ptr(out), 16, C.byref(n), unit, _lib.ptr(spans),
-                                    None) == _lib.ERR_ARG
-    assert L.bpe_encode_offsets(h, _lib.ptr(data), data.size, _lib.DTYPE_I32, _lib.ptr(out), 16, C.byref(n), 0, None, None) == _lib.ERR_ARG
-    assert L.bpe_encode_offsets(h, _lib.ptr(data), data.size, _lib.DTYPE_I32, None, 0, C.byref(n), 0, None, None) == _lib.BPE_OK
+        assert encode_offsets(_lib.ptr(out), 16, unit, spans.ctypes.data) == _lib.ERR_ARG
+    assert encode_offsets(_lib.ptr(out), 16, 0, None) == _lib.ERR_ARG
+    assert encode_offsets(None, 0, 0, None) == _lib.BPE_OK
     assert n.value == 2
-    assert L.bpe_encode_offsets(h, _lib.ptr(data), data.size, _lib.DTYPE_I32, _lib.ptr(out), 1, C.byref(n), 0, _lib.ptr(spans),
-                                None) == _lib.ERR_TOO_SMALL
+    assert encode_offsets(_lib.ptr(out), 1, 0, spans.ctypes.data) == _lib.ERR_TOO_SMALL
     assert spans[0].tolist() == [0, 5]
 
 

@@ -4,7 +4,7 @@ usage: python tools/time_encode_batch.py OUT.json [bytes=1.1e9] [loop_docs=10000
 
 Input: the TinyStories-shape synthetic corpus (seed 1234) split on <|endoftext|> into documents, GPT-2 fixture tokenizer.
 Reports, each the median of `reps` runs after one warm-up run:
-  (a) stats.ms_total (device timeline) of bpe_encode_batch on all documents against bpe_encode on the same bytes joined;
+  (a) stats.ms_total (device timeline) of the batch encode (bpe_encode_ex with document offsets) on all documents against bpe_encode on the same bytes joined;
   (b) wall time of encode_batch_to_numpy and of encode_batch from the list[str];
   (c) wall time of [tok.encode(d) for d in docs] over the first `loop_docs` documents, and encode_batch on the same documents.
 The card's name and power limit are read in the same run and stored with the numbers."""

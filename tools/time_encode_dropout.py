@@ -1,11 +1,11 @@
-"""GPU: BPE-dropout encode (bpe_encode_dropout / bpe_encode_batch_dropout) against the deterministic encode on the same bytes.
+"""GPU: BPE-dropout encode (bpe_encode_ex with dropout > 0) against the deterministic encode on the same bytes.
 
 usage: python tools/time_encode_dropout.py OUT.json [bytes=1.1e9] [reps=2]
 
 GPT-2 fixture tokenizer (with <|endoftext|>), synthetic TinyStories (seed 1234) and OWT (seed 4322) shapes of `bytes` each.  For each
 shape: bpe_encode, and dropout at p = 0.1 and p = 0.5, every one the median of `reps` runs after one warm-up run, with the device time
 per stage from bpe_encode_stats (ms_pretok, ms_lookup, ms_bpe -- the dropout stage is part of it --, ms_emit, ms_total).  Then the
-TinyStories text split on <|endoftext|> through bpe_encode_batch and bpe_encode_batch_dropout at p = 0.1.  For context, the CPU
+TinyStories text split on <|endoftext|> through the batch encode without and with dropout at p = 0.1.  For context, the CPU
 oracle (one core) on a 16 MB slice of each shape.  The card's name and power limit are read in the same run and stored with the numbers."""
 import json
 import os

@@ -1,12 +1,12 @@
-"""GPU: token offsets (bpe_encode_offsets / bpe_encode_batch_offsets) against the ids-only encode on the same bytes.
+"""GPU: token offsets (bpe_encode_ex with offsets) against the ids-only encode on the same bytes.
 
 usage: python tools/time_encode_offsets.py OUT.json [bytes=1.1e9] [reps=3]
 
 GPT-2 fixture tokenizer (with <|endoftext|>), synthetic TinyStories (seed 1234) and OWT (seed 4322) shapes of `bytes` each.  For each shape:
-bpe_encode and bpe_encode_offsets in bytes and in characters, alternated, each the median (and the range) of `reps` runs after one warm-up,
+bpe_encode and the encode with offsets in bytes and in characters, alternated, each the median (and the range) of `reps` runs after one warm-up,
 timed from host memory to the host arrays (bpe_encode_stats ms_total; the spans' download is part of it).  The device time of the offsets
 stage: one profiled run per unit (torch.profiler, CUDA kernels), the kernels only the stage launches plus the extra scans it adds over an
-ids-only run; and the device time of all kernels and copies of each call (the spans' download is most of the difference).  Then the TinyStories text split on <|endoftext|> through bpe_encode_batch and bpe_encode_batch_offsets.  For comparison, the
+ids-only run; and the device time of all kernels and copies of each call (the spans' download is most of the difference).  Then the TinyStories text split on <|endoftext|> through the batch encode without and with offsets.  For comparison, the
 same spans derived on the host with numpy from the ids (cumsum of the vocabulary lengths, and a cumulative lead-byte count for
 characters).  The card's name and power limit are read in the same run and stored with the numbers."""
 import json

@@ -46,6 +46,12 @@ class EncodeStats(C.Structure):
         return {n: getattr(self, n) for n, _ in self._fields_}
 
 
+class EncodeOpts(C.Structure):
+    """bpe_encode_opts: documents, BPE-dropout and token offsets of bpe_encode_ex (all zero: bpe_encode)."""
+    _fields_ = [("doc_offs", C.c_void_p), ("n_docs", C.c_uint64), ("id_offs_out", C.c_void_p), ("dropout", C.c_double),
+                ("seed", C.c_uint64), ("with_offsets", C.c_int), ("offset_unit", C.c_int), ("offs_out", C.c_void_p)]
+
+
 _lib = None
 _lock = threading.Lock()
 
@@ -56,8 +62,8 @@ EXPORTS = [
     "bpe_train_ex", "bpe_train_dev_ex", "bpe_count_begin", "bpe_count_add_shard", "bpe_count_add_shard_dev",
     "bpe_count_add_shard_ex", "bpe_count_add_shard_dev_ex", "bpe_count_export_size", "bpe_count_export",
     "bpe_count_export_dev", "bpe_count_import", "bpe_count_import_dev", "bpe_count_pair_table",
-    "bpe_train_from_counts", "bpe_last_pair_table", "bpe_train_set_live", "bpe_tok_create", "bpe_tok_destroy", "bpe_encode", "bpe_encode_batch", "bpe_encode_dropout", "bpe_encode_batch_dropout", "bpe_encode_offsets",
-    "bpe_encode_batch_offsets", "bpe_encode_dropout_offsets", "bpe_encode_batch_dropout_offsets", "bpe_encode_dev", "bpe_tok_key_error", "bpe_tok_saw_cr",
+    "bpe_train_from_counts", "bpe_last_pair_table", "bpe_train_set_live", "bpe_tok_create", "bpe_tok_destroy", "bpe_encode", "bpe_encode_ex",
+    "bpe_encode_dev", "bpe_tok_key_error", "bpe_tok_saw_cr",
     "bpe_tok_cache_reset", "bpe_decode", "bpe_decode_batch", "bpe_batch_windows_dev", "bpe_synth_dev", "bpe_synth_host", "bpe_synth_dev_at", "bpe_synth_host_at", "bpe_ctx_set_stream", "bpe_host_alloc", "bpe_host_free", "bpe_launch_count",
 ]
 
@@ -103,17 +109,7 @@ def lib():
             L.bpe_tok_destroy.restype = None
             L.bpe_encode.argtypes = [vp, vp, C.c_uint64, C.c_int, vp, C.c_uint64, u64p, C.POINTER(EncodeStats)]
             L.bpe_encode_dev.argtypes = L.bpe_encode.argtypes
-            L.bpe_encode_batch.argtypes = [vp, vp, C.c_uint64, vp, C.c_uint64, C.c_int, vp, C.c_uint64, u64p, vp, C.POINTER(EncodeStats)]
-            L.bpe_encode_dropout.argtypes = [vp, vp, C.c_uint64, C.c_double, C.c_uint64, C.c_int, vp, C.c_uint64, u64p, C.POINTER(EncodeStats)]
-            L.bpe_encode_batch_dropout.argtypes = [vp, vp, C.c_uint64, vp, C.c_uint64, C.c_double, C.c_uint64, C.c_int, vp, C.c_uint64, u64p, vp,
-                                                   C.POINTER(EncodeStats)]
-            L.bpe_encode_offsets.argtypes = [vp, vp, C.c_uint64, C.c_int, vp, C.c_uint64, u64p, C.c_int, vp, C.POINTER(EncodeStats)]
-            L.bpe_encode_batch_offsets.argtypes = [vp, vp, C.c_uint64, vp, C.c_uint64, C.c_int, vp, C.c_uint64, u64p, vp, C.c_int, vp,
-                                                   C.POINTER(EncodeStats)]
-            L.bpe_encode_dropout_offsets.argtypes = [vp, vp, C.c_uint64, C.c_double, C.c_uint64, C.c_int, vp, C.c_uint64, u64p, C.c_int, vp,
-                                                     C.POINTER(EncodeStats)]
-            L.bpe_encode_batch_dropout_offsets.argtypes = [vp, vp, C.c_uint64, vp, C.c_uint64, C.c_double, C.c_uint64, C.c_int, vp,
-                                                           C.c_uint64, u64p, vp, C.c_int, vp, C.POINTER(EncodeStats)]
+            L.bpe_encode_ex.argtypes = [vp, vp, C.c_uint64, C.POINTER(EncodeOpts), C.c_int, vp, C.c_uint64, u64p, C.POINTER(EncodeStats)]
             L.bpe_tok_key_error.argtypes = [vp, vp, C.c_uint64, u64p]
             L.bpe_tok_cache_reset.argtypes = [vp]
             L.bpe_tok_saw_cr.argtypes = [vp]

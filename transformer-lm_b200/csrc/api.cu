@@ -73,7 +73,7 @@ int bpe_buf_alloc(bpe_ctx *ctx, DevBuf &b, size_t bytes) {
     return pool_take(ctx, b, want);
 }
 
-BPE_API int bpe_version(void) { return 100; }
+BPE_API int bpe_version(void) { return 101; }
 BPE_API const char *bpe_unicode_table_source(void) { return BPE_UNICODE_TABLE_SOURCE; }
 
 BPE_API int bpe_ctx_create(int device, bpe_ctx **out) {
@@ -237,7 +237,7 @@ u64 exact_cut_host(const uint8_t *t, u64 n, u64 nominal, u64 window, const uint8
 //   translate_newlines: apply universal-newline translation when a '\r' is present (training path);
 //                       *n is updated to the translated length.
 //   specials: when n_sp > 0 the text is first split on the specials (encode path).
-//   bmask: document boundaries of bpe_encode_batch (flag_words(n) words, or null): every set bit is a one-byte occurrence of
+//   bmask: document boundaries of a batch encode (flag_words(n) words, or null): every set bit is a one-byte occurrence of
 //          class B, like a special token -- the text before it sees the end of a text, the text after it the start of one.
 // Leaves ctx->flags holding the start bitmask.  Synchronises the stream once (error words).
 int ctx_run_flags(bpe_ctx *ctx, u64 *n_io, bool translate_newlines, const uint8_t *sp_blob_dev, const u32 *sp_offs_dev,

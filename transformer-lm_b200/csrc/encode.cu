@@ -13,7 +13,7 @@
 //   3. k_enc_bpe_short / k_enc_bpe   the queued (new unique) pretokens: the merges in rank order through the pair -> rank table
 //                     (repeatedly the lowest-ranked adjacent pair, all its non-overlapping occurrences left to right); one thread
 //                     per pretoken of <= 32 bytes (row_bpe), one warp per longer one (warp_bpe)
-//   (bpe_encode_dropout / bpe_encode_batch_dropout only: k_enc_drop_starts, then k_enc_drop_short / k_enc_drop_warp -- row_bpe and
+//   (BPE-dropout only: k_enc_drop_starts, then k_enc_drop_short / k_enc_drop_warp -- row_bpe and
 //                     warp_bpe with dropped candidates -- replace the value of every occurrence whose segmentation can change with its
 //                     own BPE-dropout result, bypassing the cache)
 //   4. k_enc_scan_emit  tokens per pretoken -> exclusive offsets -> ids scattered to the uint16 / int32 output, in one
@@ -35,7 +35,7 @@
 //   0..3   that many ids inline, 20 bits each at bits 0, 20, 40
 //   4      ids in the id pool: bits 59..24 = offset, bits 23..0 = count
 //   5      KeyError: bits 31..0 = offending symbol (bit 31 set: index of a special token instead)
-//   13     (per-occurrence array only, bpe_encode_batch) document boundary: bits 39..0 = index of the document it ends, in the chunk
+//   13     (per-occurrence array only, batch encode) document boundary: bits 39..0 = index of the document it ends, in the chunk
 //   14     (per-occurrence array only) not computed when looked up: bits 31..0 = cache slot reference
 //   15     not computed yet
 #define VAL_NONE 0xFFFFFFFFFFFFFFFFull
@@ -64,7 +64,7 @@ struct EncTables : PtTables {
     // [0]=n_short [1]=n_long [2]=todo count [3]=table overflow [4]=key pool cursor [5]=ipool cursor [6]=pretoken too long
     // [7]=smallest ordinal (in the text of the call) of a pretoken whose value is a KeyError  [8]=n_medium  [9]=step tickets of the lookup kernel
     u64 *ctr;
-    // document boundaries of bpe_encode_batch (all null for bpe_encode): bit per arena byte, boundaries before every 512-byte group,
+    // document boundaries of a batch encode (all null for bpe_encode): bit per arena byte, boundaries before every 512-byte group,
     // id_offs[j] = index of the first id after document j of the chunk (id_base + its offset in the chunk's output)
     const u32 *bmask; const u64 *bpre; u64 *id_offs; u64 id_base;
 };
@@ -222,7 +222,7 @@ __device__ __forceinline__ void lookup_drain(const EncTables &t, LookupQueues &q
 
 // chunks [c_lo, c_hi) (16 bytes each, absolute positions 16 c; c_lo a multiple of 32); pre[g] = ordinal of the first pretoken of the
 // g-th group of 32 chunks (absolute), ord0 = ordinal of the batch's first pretoken, base = 16 c_lo
-// DOCS (bpe_encode_batch): a pretoken that starts on a boundary bit is a document boundary, value VAL_DOC | document index (boundary
+// DOCS (batch encode): a pretoken that starts on a boundary bit is a document boundary, value VAL_DOC | document index (boundary
 // bits before the step's group + the warp's lanes before this one + the chunk's bits before the pretoken); it never touches the cache.
 template <bool DOCS>
 __global__ void __launch_bounds__(LK_NT, 1) k_enc_lookup(EncTables t, const u32 *__restrict__ flags, const u64 *__restrict__ pre, u64 ord0,
@@ -653,7 +653,7 @@ __global__ void __launch_bounds__(SE_NT) k_enc_scan_emit(EncTables t, const u64 
         if (staged) stage_ids();
     }
     __syncthreads();
-    if (t.id_offs) {                             // bpe_encode_batch: a document boundary holds where the next document's ids start
+    if (t.id_offs) {                             // batch encode: a document boundary holds where the next document's ids start
         u64 o = t.id_base + out_base + s_prefix + ex;
 #pragma unroll
         for (u32 k = 0; k < SE_ITEMS; k++) {
@@ -681,7 +681,7 @@ __global__ void __launch_bounds__(SE_NT) k_enc_scan_emit(EncTables t, const u64 
     }
 }
 
-// ---- BPE-dropout (bpe_encode_dropout / bpe_encode_batch_dropout): every pretoken occurrence gets its own random BPE ----------
+// ---- BPE-dropout (bpe_encode_ex with dropout > 0): every pretoken occurrence gets its own random BPE ----------
 // Spec (include/bpe_sm100.h): candidate pair (i, i+1) of merge round t is dropped when (u(seed, doc, off_i, t) >> 32) < thr, with
 // u = mix(mix(mix(mix(seed) ^ doc) ^ off) ^ t), mix = the splitmix64 finalizer, off_i = byte offset in the document of token i's first
 // byte.  The round takes the lowest rank among the pairs that are left and merges, left to right and non-overlapping, exactly those of
@@ -691,7 +691,7 @@ struct EncDrop {
     u64 thr;                                     // 0 < thr <= 2^32
     u64 seed_mix;                                // mix(seed)
     u64 lo;                                      // where the chunk starts in the caller's text
-    const u64 *doffs; u64 da;                    // bpe_encode_batch: the caller's document offsets, the chunk's first document (else null, 0)
+    const u64 *doffs; u64 da;                    // batch encode: the caller's document offsets, the chunk's first document (else null, 0)
     const u32 *skip;                             // special-token starts and document boundaries (or null): their values stay
     const u64 *starts;                           // byte offset in the arena of every pretoken of the batch
     u32 *loff;                                   // per byte from the batch start: token offsets of the warp kernel's pretokens
@@ -768,7 +768,7 @@ __global__ void __launch_bounds__(256) k_enc_drop_warp(EncTables t, EncDrop d, c
     }
 }
 
-// ---- token offsets (bpe_encode_offsets and the other *_offsets calls): a span of the input for every token --------------------------
+// ---- token offsets (bpe_encode_ex with with_offsets): a span of the input for every token --------------------------
 // Spec (include/bpe_sm100.h): the tokens of a pretoken occurrence tile its bytes in order; each but the last is as long as its vocabulary
 // entry (tok->vlen), the last ends where the pretoken ends.  So a special-token occurrence -- one id, whatever that id is -- spans the
 // special's bytes.  Per batch, after the emit kernel: the pretoken starts (k_enc_drop_starts), the token count of every pretoken and its
@@ -779,7 +779,7 @@ struct EncOffs {
     int chars;                                   // BPE_OFF_CHARS: character indices, else byte offsets
     long long *out;                              // {start, end} of every token of the chunk, in the order of its ids
     u64 lo;                                      // where the chunk starts in the caller's text
-    const u64 *doffs; u64 da;                    // bpe_encode_batch*: the caller's document offsets, the chunk's first document (else null, 0)
+    const u64 *doffs; u64 da;                    // batch encode: the caller's document offsets, the chunk's first document (else null, 0)
     u64 carry;                                   // characters of the chunk's first document before lo
     const u32 *lmask; const u64 *lpre;           // lead-byte bit per arena byte (words up to 16 (groups + 1)), count before every 512-byte group
     const u32 *vlen; u64 n_dense;                // byte length of every vocabulary id
@@ -1029,7 +1029,7 @@ struct bpe_tok {
     std::vector<uint8_t> key_error;              // bytes of the last KeyError key
     DevBuf drop;                                 // BPE-dropout scratch of a batch: pretoken offsets, token offsets of long pretokens
     DevBuf offs_text, offs_batch, offs_out[2];   // token offsets: lead-byte bits of a chunk; pretoken starts and token scan of a batch; spans of a chunk
-    int doc_sep = -1;                            // boundary byte of bpe_encode_batch (-1: every candidate occurs in a special)
+    int doc_sep = -1;                            // boundary byte of the batch encode (-1: every candidate occurs in a special)
 };
 
 // grow keeping the first `used` bytes
@@ -1245,7 +1245,7 @@ BPE_API int bpe_tok_create(bpe_ctx *ctx, const int32_t *merge_pairs, const int32
         CUDA_TRY(ctx, cudaMemcpyAsync(tok->sp_ids.p, special_ids, (size_t)n_specials * 8, cudaMemcpyHostToDevice, st));
     }
     tok->max_id = max_id;
-    // bpe_encode_batch's boundary byte: an ASCII value that occurs in no special token, so that no special-token match can cross a
+    // the batch encode's boundary byte: an ASCII value that occurs in no special token, so that no special-token match can cross a
     // boundary (it would have to contain the byte); never '\r', which the flags kernel reports as a carriage return
     {
         bool used[128] = {false};
@@ -1314,7 +1314,7 @@ BPE_API int bpe_tok_key_error(bpe_tok *tok, uint8_t *buf, uint64_t cap, uint64_t
 #define ENC_BATCH_BYTES (256ull << 20)
 #define ENC_CACHE_MAX_ENTRIES (384ull << 20)
 
-// Document boundaries of a bpe_encode_batch chunk: bit per arena byte; id_offs[j] gets id_base + the offset of the first id after
+// Document boundaries of a batch encode's chunk: bit per arena byte; id_offs[j] gets id_base + the offset of the first id after
 // the chunk's document j.
 struct DocBounds { const u32 *bmask; u64 *id_offs; u64 id_base; };
 
@@ -1607,7 +1607,7 @@ static u64 find_exact_cut(const bpe_tok *tok, const uint8_t *t, u64 n, u64 nomin
     return exact_cut_host(t, n, nominal, ENC_CUT_WINDOW, tok->sp_blob_h.data(), tok->sp_offs_h.data(), tok->n_sp);
 }
 
-// ---- bpe_encode_batch: a chunk of documents into the text arena, one boundary byte after every document that ends in it ----------
+// ---- batch encode: a chunk of documents into the text arena, one boundary byte after every document that ends in it ----------
 // ends[j] - lo = where document j ends in the chunk (ascending, 0..len).  Byte i of the chunk goes to i + #{j : ends[j] - lo <= i},
 // the boundary after document j to ends[j] - lo + j, which also sets its bit in bmask (zeroed by the caller).  A warp takes 512
 // bytes at a time, 32 consecutive bytes per instruction; the boundaries inside them (usually none) come from a binary search.
@@ -1664,10 +1664,10 @@ static std::vector<EncChunk> doc_chunks(const bpe_tok *tok, const uint8_t *t, u6
 }
 
 // ---- host entry points: chunks cut at exact boundaries, double-buffered so that the upload of chunk k+1 and the download of
-// chunk k-1 run while chunk k is encoded.  doc_offs (bpe_encode_batch) or null (bpe_encode).
-//   bpe_encode:       a chunk is uploaded straight into the arena the kernels read next (the two arenas alternate)
-//   bpe_encode_batch: a chunk is uploaded as it is into one of two staging buffers; on the compute stream k_enc_expand_docs moves it
-//                     into the arena with a boundary byte after every document and sets the boundary bitmask
+// chunk k-1 run while chunk k is encoded.  doc_offs (batch encode) or null (one document).
+//   one document: a chunk is uploaded straight into the arena the kernels read next (the two arenas alternate)
+//   batch encode: a chunk is uploaded as it is into one of two staging buffers; on the compute stream k_enc_expand_docs moves it
+//                 into the arena with a boundary byte after every document and sets the boundary bitmask
 // drop: BPE-dropout (thr and seed_mix set), or null.  offs_out (with out): the tokens' spans in `unit` (BPE_OFF_*), downloaded with the ids.
 static int encode_pipeline(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs, uint64_t n_docs, int out_dtype,
                            void *out, uint64_t cap, uint64_t *n_out, uint64_t *id_offs_out, bpe_encode_stats *stats,
@@ -1693,8 +1693,8 @@ static int encode_pipeline(bpe_tok *tok, const uint8_t *text_host, uint64_t n, c
     }
     EvTimer tm(ctx);
     int e0 = tm.mark();
-    DevBuf *tbuf[2] = {&ctx->text, &ctx->text_alt};     // bpe_encode: the two arenas
-    DevBuf *sbuf[2] = {&ctx->text_alt, &ctx->doc_stage};   // bpe_encode_batch: the two staging buffers (the arena is ctx->text)
+    DevBuf *tbuf[2] = {&ctx->text, &ctx->text_alt};     // one document: the two arenas
+    DevBuf *sbuf[2] = {&ctx->text_alt, &ctx->doc_stage};   // batch encode: the two staging buffers (the arena is ctx->text)
     DevBuf *obuf[2] = {&ctx->out_a, &ctx->out_b};
     u64 max_chunk = 0;
     for (const EncChunk &c : chunks) max_chunk = std::max(max_chunk, c.hi - c.lo);
@@ -1807,101 +1807,47 @@ static int encode_pipeline(bpe_tok *tok, const uint8_t *text_host, uint64_t n, c
 
 BPE_API int bpe_encode(bpe_tok *tok, const uint8_t *text_host, uint64_t n, int out_dtype, void *out, uint64_t cap, uint64_t *n_out,
                        bpe_encode_stats *stats) {
-    return encode_pipeline(tok, text_host, n, nullptr, 0, out_dtype, out, cap, n_out, nullptr, stats);
+    return bpe_encode_ex(tok, text_host, n, nullptr, out_dtype, out, cap, n_out, stats);
 }
 
-static int encode_batch_impl(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
-                             int out_dtype, void *out, uint64_t cap, uint64_t *n_out, uint64_t *id_offs_out, bpe_encode_stats *stats,
-                             const EncDrop *drop, int unit = BPE_OFF_BYTES, int64_t *offs_out = nullptr) {
-    if (!tok || !n_out || !id_offs_out || (n_docs && !doc_offs_host)) return BPE_ERR_ARG;
+// Arguments are checked in the order include/bpe_sm100.h gives, every option's checks only when it is used.
+BPE_API int bpe_encode_ex(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const bpe_encode_opts *opts, int out_dtype, void *out,
+                          uint64_t cap, uint64_t *n_out, bpe_encode_stats *stats) {
+    if (!tok) return BPE_ERR_ARG;
     bpe_ctx *ctx = tok->ctx;
-    for (uint64_t j = 0; j < n_docs; j++)
-        if (doc_offs_host[j] > doc_offs_host[j + 1]) return bpe_set_error(ctx, BPE_ERR_ARG, "bpe_encode_batch: document offsets must not decrease");
-    if (n_docs ? (doc_offs_host[0] != 0 || doc_offs_host[n_docs] != n) : n != 0)
-        return bpe_set_error(ctx, BPE_ERR_ARG, "bpe_encode_batch: document offsets must run from 0 to n");
-    if (n_docs && tok->doc_sep < 0)
-        return bpe_set_error(ctx, BPE_ERR_UNSUPPORTED, "bpe_encode_batch: every ASCII byte but '\\r' occurs in a special token (no boundary byte)");
-    if (n_docs == 0) {
-        BPE_TRY(encode_check_args(tok, text_host, 0, out_dtype, n_out));
-        if (stats) memset(stats, 0, sizeof(*stats));
-        id_offs_out[0] = 0;
-        return BPE_OK;
+    const bpe_encode_opts o = opts ? *opts : bpe_encode_opts{};
+    if (o.with_offsets) {
+        if (o.offset_unit != BPE_OFF_BYTES && o.offset_unit != BPE_OFF_CHARS)
+            return bpe_set_error(ctx, BPE_ERR_ARG, "unknown offset unit %d", o.offset_unit);
+        if (out && !o.offs_out) return bpe_set_error(ctx, BPE_ERR_ARG, "offs_out is null");
     }
-    return encode_pipeline(tok, text_host, n, doc_offs_host, n_docs, out_dtype, out, cap, n_out, id_offs_out, stats, drop, unit, offs_out);
-}
-
-BPE_API int bpe_encode_batch(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
-                             int out_dtype, void *out, uint64_t cap, uint64_t *n_out, uint64_t *id_offs_out, bpe_encode_stats *stats) {
-    return encode_batch_impl(tok, text_host, n, doc_offs_host, n_docs, out_dtype, out, cap, n_out, id_offs_out, stats, nullptr);
-}
-
-// BPE-dropout: thr(p) = 2^32 for p = 1, else floor(p * 2^32) (exact in binary64); p outside [0, 1] or NaN is BPE_ERR_ARG.
-// p = 0 drops nothing: the deterministic pipeline runs.
-static int dropout_args(bpe_tok *tok, double p, uint64_t seed, EncDrop *d) {
-    if (!(p >= 0.0 && p <= 1.0)) return tok ? bpe_set_error(tok->ctx, BPE_ERR_ARG, "dropout probability must be in [0, 1]") : BPE_ERR_ARG;
-    memset(d, 0, sizeof(*d));
-    d->thr = p == 1.0 ? (1ull << 32) : (u64)(p * 4294967296.0);
-    u64 z = seed + 0x9E3779B97F4A7C15ull;        // mix(seed), as splitmix64 on the device
+    // BPE-dropout: thr(p) = 2^32 for p = 1, else floor(p * 2^32) (exact in binary64); p outside [0, 1] or NaN is BPE_ERR_ARG.
+    // thr = 0 (p = 0, or p below 2^-32) drops nothing: the deterministic pipeline runs.
+    if (!(o.dropout >= 0.0 && o.dropout <= 1.0)) return bpe_set_error(ctx, BPE_ERR_ARG, "dropout probability must be in [0, 1]");
+    EncDrop d{};
+    d.thr = o.dropout == 1.0 ? (1ull << 32) : (u64)(o.dropout * 4294967296.0);
+    u64 z = o.seed + 0x9E3779B97F4A7C15ull;      // mix(seed), as splitmix64 on the device
     z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
     z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-    d->seed_mix = z ^ (z >> 31);
-    return BPE_OK;
-}
-
-BPE_API int bpe_encode_dropout(bpe_tok *tok, const uint8_t *text_host, uint64_t n, double p, uint64_t seed, int out_dtype, void *out,
-                               uint64_t cap, uint64_t *n_out, bpe_encode_stats *stats) {
-    if (!tok) return BPE_ERR_ARG;
-    EncDrop d;
-    BPE_TRY(dropout_args(tok, p, seed, &d));
-    return encode_pipeline(tok, text_host, n, nullptr, 0, out_dtype, out, cap, n_out, nullptr, stats, d.thr ? &d : nullptr);
-}
-
-BPE_API int bpe_encode_batch_dropout(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
-                                     double p, uint64_t seed, int out_dtype, void *out, uint64_t cap, uint64_t *n_out,
-                                     uint64_t *id_offs_out, bpe_encode_stats *stats) {
-    if (!tok) return BPE_ERR_ARG;
-    EncDrop d;
-    BPE_TRY(dropout_args(tok, p, seed, &d));
-    return encode_batch_impl(tok, text_host, n, doc_offs_host, n_docs, out_dtype, out, cap, n_out, id_offs_out, stats, d.thr ? &d : nullptr);
-}
-
-// ---- token offsets: the ids of the four calls above and a span of the input for every token -------------------------------------
-static int offsets_args(bpe_tok *tok, int unit, const void *out, const int64_t *offs_out) {
-    if (!tok) return BPE_ERR_ARG;
-    if (unit != BPE_OFF_BYTES && unit != BPE_OFF_CHARS) return bpe_set_error(tok->ctx, BPE_ERR_ARG, "unknown offset unit %d", unit);
-    if (out && !offs_out) return bpe_set_error(tok->ctx, BPE_ERR_ARG, "offs_out is null");
-    return BPE_OK;
-}
-
-BPE_API int bpe_encode_offsets(bpe_tok *tok, const uint8_t *text_host, uint64_t n, int out_dtype, void *out, uint64_t cap, uint64_t *n_out,
-                               int unit, int64_t *offs_out, bpe_encode_stats *stats) {
-    BPE_TRY(offsets_args(tok, unit, out, offs_out));
-    return encode_pipeline(tok, text_host, n, nullptr, 0, out_dtype, out, cap, n_out, nullptr, stats, nullptr, unit, offs_out);
-}
-
-BPE_API int bpe_encode_batch_offsets(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
-                                     int out_dtype, void *out, uint64_t cap, uint64_t *n_out, uint64_t *id_offs_out, int unit,
-                                     int64_t *offs_out, bpe_encode_stats *stats) {
-    BPE_TRY(offsets_args(tok, unit, out, offs_out));
-    return encode_batch_impl(tok, text_host, n, doc_offs_host, n_docs, out_dtype, out, cap, n_out, id_offs_out, stats, nullptr, unit, offs_out);
-}
-
-BPE_API int bpe_encode_dropout_offsets(bpe_tok *tok, const uint8_t *text_host, uint64_t n, double p, uint64_t seed, int out_dtype, void *out,
-                                       uint64_t cap, uint64_t *n_out, int unit, int64_t *offs_out, bpe_encode_stats *stats) {
-    BPE_TRY(offsets_args(tok, unit, out, offs_out));
-    EncDrop d;
-    BPE_TRY(dropout_args(tok, p, seed, &d));
-    return encode_pipeline(tok, text_host, n, nullptr, 0, out_dtype, out, cap, n_out, nullptr, stats, d.thr ? &d : nullptr, unit, offs_out);
-}
-
-BPE_API int bpe_encode_batch_dropout_offsets(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs_host, uint64_t n_docs,
-                                             double p, uint64_t seed, int out_dtype, void *out, uint64_t cap, uint64_t *n_out,
-                                             uint64_t *id_offs_out, int unit, int64_t *offs_out, bpe_encode_stats *stats) {
-    BPE_TRY(offsets_args(tok, unit, out, offs_out));
-    EncDrop d;
-    BPE_TRY(dropout_args(tok, p, seed, &d));
-    return encode_batch_impl(tok, text_host, n, doc_offs_host, n_docs, out_dtype, out, cap, n_out, id_offs_out, stats, d.thr ? &d : nullptr,
-                             unit, offs_out);
+    d.seed_mix = z ^ (z >> 31);
+    if (o.doc_offs || o.n_docs) {
+        const uint64_t *doc_offs = o.doc_offs, n_docs = o.n_docs;
+        if (!n_out || !o.id_offs_out || !doc_offs) return BPE_ERR_ARG;
+        for (uint64_t j = 0; j < n_docs; j++)
+            if (doc_offs[j] > doc_offs[j + 1]) return bpe_set_error(ctx, BPE_ERR_ARG, "bpe_encode_ex: document offsets must not decrease");
+        if (n_docs ? (doc_offs[0] != 0 || doc_offs[n_docs] != n) : n != 0)
+            return bpe_set_error(ctx, BPE_ERR_ARG, "bpe_encode_ex: document offsets must run from 0 to n");
+        if (n_docs && tok->doc_sep < 0)
+            return bpe_set_error(ctx, BPE_ERR_UNSUPPORTED, "bpe_encode_ex: every ASCII byte but '\\r' occurs in a special token (no boundary byte)");
+        if (n_docs == 0) {
+            BPE_TRY(encode_check_args(tok, text_host, 0, out_dtype, n_out));
+            if (stats) memset(stats, 0, sizeof(*stats));
+            o.id_offs_out[0] = 0;
+            return BPE_OK;
+        }
+    }
+    return encode_pipeline(tok, text_host, n, o.doc_offs, o.n_docs, out_dtype, out, cap, n_out, o.id_offs_out, stats, d.thr ? &d : nullptr,
+                           o.offset_unit, o.with_offsets ? o.offs_out : nullptr);
 }
 
 BPE_API int bpe_encode_dev(bpe_tok *tok, const uint8_t *text_dev, uint64_t n, int out_dtype, void *out_dev, uint64_t cap, uint64_t *n_out,

@@ -200,57 +200,58 @@ class Tokenizer:
         ctx.check(rc)
 
     # ---- encode (tokenizer.py:111-138) -------------------------------------------------------------
-    def encode_to_numpy(self, data, dtype=np.int32, *, dropout: float = 0.0, seed: int = 0) -> np.ndarray:
-        """Token ids of UTF-8 `data` (bytes / uint8 array) as a numpy array of `dtype` (uint16 or int32).  dropout > 0: BPE-dropout
-        (every pretoken occurrence merged with each candidate pair of each round dropped with that probability; a pure function of
-        the text, dropout and seed -- see bpe_encode_dropout in include/bpe_sm100.h)."""
-        dropout, seed = _check_dropout(dropout, seed)
+    def _encode_ex(self, data, dtype, out=None, *, docs=None, texts=None, drop=(0.0, 0), unit=None):
+        """bpe_encode_ex of UTF-8 `data` into `out` (or a new array) of `dtype` (uint16 or int32): (ids, spans or None, id offsets or
+        None).  docs: uint64 document offsets into `data` (a batch; `texts` are the items they came from, when known); drop: (p, seed)
+        of BPE-dropout; unit: _lib.OFF_* for the int64 spans [n, 2] of the tokens."""
         tok = self._device_tok()
         ctx = self._tok_ctx
         L = _lib.lib()
         arr = _lib.as_u8(data)
         code = {np.dtype(np.uint16): _lib.DTYPE_U16, np.dtype(np.int32): _lib.DTYPE_I32}[np.dtype(dtype)]
-        out = np.empty(max(arr.size, 1), dtype=dtype)             # a token covers at least one byte
+        if out is None:
+            out = np.empty(max(arr.size, 1), dtype=dtype)         # a token covers at least one byte
+        opts = _lib.EncodeOpts(dropout=drop[0], seed=drop[1])
+        spans = id_offs = None
+        if docs is not None:
+            id_offs = np.zeros(docs.size, dtype=np.uint64)
+            opts.doc_offs, opts.n_docs, opts.id_offs_out = docs.ctypes.data, docs.size - 1, id_offs.ctypes.data
+        if unit is not None:
+            spans = np.empty((out.size, 2), dtype=np.int64)
+            opts.with_offsets, opts.offset_unit, opts.offs_out = 1, unit, spans.ctypes.data
         n_out = C.c_uint64(0)
         stats = _lib.EncodeStats()
         with ctx.lock:
-            if dropout:
-                rc = L.bpe_encode_dropout(tok, _lib.ptr(arr) if arr.size else None, arr.size, dropout, seed, code, _lib.ptr(out), out.size,
-                                          C.byref(n_out), C.byref(stats))
-            else:
-                rc = L.bpe_encode(tok, _lib.ptr(arr) if arr.size else None, arr.size, code, _lib.ptr(out), out.size, C.byref(n_out), C.byref(stats))
+            rc = L.bpe_encode_ex(tok, _lib.ptr(arr) if arr.size else None, arr.size, C.byref(opts), code, _lib.ptr(out), out.size,
+                                 C.byref(n_out), C.byref(stats))
+            if rc == _lib.ERR_UTF8 and texts is not None:
+                # the device reports invalid UTF-8 in a chunk before a KeyError in it: the documents before the invalid one
+                # go first, then that document fails as its decode does
+                k = int(np.searchsorted(docs, L.bpe_last_error_detail(ctx.handle), side="right")) - 1
+                self._encode_ex(arr[: int(docs[k])], dtype, docs=docs[: k + 1], drop=drop)
+                item = texts[k]
+                if isinstance(item, (bytes, bytearray, memoryview)):
+                    bytes(item).decode("utf-8")
             if rc != _lib.BPE_OK:
-                self._raise(ctx, rc, arr)
+                self._raise(ctx, rc, arr if docs is None else None)
         self.last_stats = stats.as_dict()
-        return out[: n_out.value]
+        n = n_out.value
+        return out[:n], None if spans is None else spans[:n], None if id_offs is None else id_offs.astype(np.int64)
+
+    def encode_to_numpy(self, data, dtype=np.int32, *, dropout: float = 0.0, seed: int = 0) -> np.ndarray:
+        """Token ids of UTF-8 `data` (bytes / uint8 array) as a numpy array of `dtype` (uint16 or int32).  dropout > 0: BPE-dropout
+        (every pretoken occurrence merged with each candidate pair of each round dropped with that probability; a pure function of
+        the text, dropout and seed -- see bpe_encode_opts in include/bpe_sm100.h)."""
+        return self._encode_ex(data, dtype, drop=_check_dropout(dropout, seed))[0]
 
     def encode_offsets_to_numpy(self, data, dtype=np.int32, *, unit: str = "byte", dropout: float = 0.0,
                                 seed: int = 0) -> Tuple[np.ndarray, np.ndarray]:
         """encode_to_numpy's ids and int64 spans [n, 2] of `data` in `unit` ("byte" or "char"), computed on the device in the same pass:
         token i came from data[start:end] ("byte"), or text[start:end] holds its bytes ("char"; a character that several tokens split
-        belongs to each of them).  See bpe_encode_offsets in include/bpe_sm100.h."""
+        belongs to each of them).  See bpe_encode_opts in include/bpe_sm100.h."""
         code_unit = _check_unit(unit)
-        dropout, seed = _check_dropout(dropout, seed)
-        tok = self._device_tok()
-        ctx = self._tok_ctx
-        L = _lib.lib()
-        arr = _lib.as_u8(data)
-        code = {np.dtype(np.uint16): _lib.DTYPE_U16, np.dtype(np.int32): _lib.DTYPE_I32}[np.dtype(dtype)]
-        out = np.empty(max(arr.size, 1), dtype=dtype)             # a token covers at least one byte
-        spans = np.empty((out.size, 2), dtype=np.int64)
-        n_out = C.c_uint64(0)
-        stats = _lib.EncodeStats()
-        src = (tok, _lib.ptr(arr) if arr.size else None, arr.size)
-        with ctx.lock:
-            if dropout:
-                rc = L.bpe_encode_dropout_offsets(*src, dropout, seed, code, _lib.ptr(out), out.size, C.byref(n_out), code_unit, _lib.ptr(spans),
-                                                  C.byref(stats))
-            else:
-                rc = L.bpe_encode_offsets(*src, code, _lib.ptr(out), out.size, C.byref(n_out), code_unit, _lib.ptr(spans), C.byref(stats))
-            if rc != _lib.BPE_OK:
-                self._raise(ctx, rc, arr)
-        self.last_stats = stats.as_dict()
-        return out[: n_out.value], spans[: n_out.value]
+        ids, spans, _ = self._encode_ex(data, dtype, drop=_check_dropout(dropout, seed), unit=code_unit)
+        return ids, spans
 
     def encode_with_offsets(self, text: str, *, dropout: float = 0.0, seed: int = 0) -> Tuple[List[int], List[Tuple[int, int]]]:
         """encode(text)'s ids and the character span (start, end) of every token in `text` (encode_offsets_to_numpy, unit="char")."""
@@ -259,20 +260,9 @@ class Tokenizer:
 
     def encode_into(self, data, out: np.ndarray) -> int:
         """encode_to_numpy into a caller-owned array (uint16 or int32; page-locked for PCIe-speed downloads).  Returns the count."""
-        tok = self._device_tok()
-        ctx = self._tok_ctx
-        L = _lib.lib()
-        arr = _lib.as_u8(data)
-        code = {np.dtype(np.uint16): _lib.DTYPE_U16, np.dtype(np.int32): _lib.DTYPE_I32}[out.dtype]
-        n_out = C.c_uint64(0)
-        stats = _lib.EncodeStats()
-        with ctx.lock:
-            rc = L.bpe_encode(tok, _lib.ptr(arr) if arr.size else None, arr.size, code, _lib.ptr(out), out.size, C.byref(n_out), C.byref(stats))
-            if rc != _lib.BPE_OK:
-                self._raise(ctx, rc, arr)
-        self.last_stats = stats.as_dict()
-        self.last_saw_cr = bool(L.bpe_tok_saw_cr(tok))
-        return int(n_out.value)
+        n = self._encode_ex(data, out.dtype, out)[0].size
+        self.last_saw_cr = bool(_lib.lib().bpe_tok_saw_cr(self._tok))
+        return n
 
     def encode(self, text: str, *, dropout: float = 0.0, seed: int = 0) -> List[int]:
         """Token ids of `text`; dropout > 0 samples a BPE-dropout segmentation (see encode_to_numpy)."""
@@ -281,8 +271,8 @@ class Tokenizer:
 
     def encode_batch(self, texts: Sequence[str], *, dropout: float = 0.0, seed: int = 0) -> List[List[int]]:
         """[self.encode(t) for t in texts] -- the same ids, split the same way, the same first exception -- with one device pass
-        over all documents (bpe_encode_batch) instead of one pipeline per document.  With dropout > 0, document j is sampled as
-        document j of the batch: encode(d, dropout=p, seed=s) == encode_batch([d], dropout=p, seed=s)[0]."""
+        over all documents (bpe_encode_ex with document offsets) instead of one pipeline per document.  With dropout > 0, document j
+        is sampled as document j of the batch: encode(d, dropout=p, seed=s) == encode_batch([d], dropout=p, seed=s)[0]."""
         ids, offs = self.encode_batch_to_numpy(texts, np.int32, dropout=dropout, seed=seed)
         flat, o = ids.tolist(), offs.tolist()
         return [flat[o[j]: o[j + 1]] for j in range(len(o) - 1)]
@@ -292,15 +282,9 @@ class Tokenizer:
         """Ids of every document back to back (uint16 or int32) and int64 offsets (len(texts) + 1): document j's ids are
         ids[offsets[j]:offsets[j + 1]].  A `bytes` item must be UTF-8; it fails as item.decode("utf-8") would.  Where several
         documents would fail, the error is that of the first one in list order, as in a loop over encode_to_numpy.  dropout > 0:
-        BPE-dropout with the document's index in `texts` as its `doc` (bpe_encode_batch_dropout)."""
-        drop = _check_dropout(dropout, seed)
-        kw = {"drop": drop} if drop[0] else {}
-        texts = list(texts)
-        blob, offs, bad = _pack_documents(texts)
-        if bad is not None:                      # a str that cannot be encoded: the documents before it fail first, if any does
-            self._encode_batch_packed(blob, offs, dtype, **kw)
-            raise bad
-        return self._encode_batch_packed(blob, offs, dtype, texts, **kw)
+        BPE-dropout with the document's index in `texts` as its `doc`."""
+        ids, _, offs = self._encode_batch(texts, dtype, _check_dropout(dropout, seed))
+        return ids, offs
 
     def encode_batch_offsets_to_numpy(self, texts: Sequence[str | bytes], dtype=np.int32, *, unit: str = "byte", dropout: float = 0.0,
                                       seed: int = 0) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
@@ -308,14 +292,7 @@ class Tokenizer:
         relative to its document's start: (ids, spans, offsets), and document j's tokens are [offsets[j], offsets[j + 1]).  Document j's
         spans are those of encode_offsets_to_numpy(texts[j]); the errors are those of encode_batch_to_numpy."""
         code_unit = _check_unit(unit)
-        drop = _check_dropout(dropout, seed)
-        kw = {"drop": drop} if drop[0] else {}
-        texts = list(texts)
-        blob, offs, bad = _pack_documents(texts)
-        if bad is not None:                      # as in encode_batch_to_numpy
-            self._encode_batch_packed(blob, offs, dtype, **kw)
-            raise bad
-        return self._encode_batch_packed(blob, offs, dtype, texts, unit=code_unit, **kw)
+        return self._encode_batch(texts, dtype, _check_dropout(dropout, seed), code_unit)
 
     def encode_batch_with_offsets(self, texts: Sequence[str], *, dropout: float = 0.0,
                                   seed: int = 0) -> List[Tuple[List[int], List[Tuple[int, int]]]]:
@@ -324,47 +301,14 @@ class Tokenizer:
         flat, sp, o = ids.tolist(), list(map(tuple, spans.tolist())), o.tolist()
         return [(flat[o[j]: o[j + 1]], sp[o[j]: o[j + 1]]) for j in range(len(o) - 1)]
 
-    def _encode_batch_packed(self, blob: np.ndarray, offs: np.ndarray, dtype, texts=None, drop=(0.0, 0), unit=None):
-        """(ids, id offsets), or with an offset unit (_lib.OFF_*) (ids, spans, id offsets)."""
-        tok = self._device_tok()
-        ctx = self._tok_ctx
-        L = _lib.lib()
-        code = {np.dtype(np.uint16): _lib.DTYPE_U16, np.dtype(np.int32): _lib.DTYPE_I32}[np.dtype(dtype)]
-        n_docs = offs.size - 1
-        out = np.empty(max(blob.size, 1), dtype=dtype)            # a token covers at least one byte
-        id_offs = np.zeros(n_docs + 1, dtype=np.uint64)
-        n_out = C.c_uint64(0)
-        stats = _lib.EncodeStats()
-        with ctx.lock:
-            if unit is not None:
-                spans = np.empty((out.size, 2), dtype=np.int64)
-                args = (tok, _lib.ptr(blob) if blob.size else None, blob.size, _lib.ptr(offs), n_docs)
-                tail = (code, _lib.ptr(out), out.size, C.byref(n_out), _lib.ptr(id_offs), unit, _lib.ptr(spans), C.byref(stats))
-                if drop[0]:
-                    rc = L.bpe_encode_batch_dropout_offsets(*args, drop[0], drop[1], *tail)
-                else:
-                    rc = L.bpe_encode_batch_offsets(*args, *tail)
-            elif drop[0]:
-                rc = L.bpe_encode_batch_dropout(tok, _lib.ptr(blob) if blob.size else None, blob.size, _lib.ptr(offs), n_docs, drop[0], drop[1],
-                                                code, _lib.ptr(out), out.size, C.byref(n_out), _lib.ptr(id_offs), C.byref(stats))
-            else:
-                rc = L.bpe_encode_batch(tok, _lib.ptr(blob) if blob.size else None, blob.size, _lib.ptr(offs), n_docs, code,
-                                        _lib.ptr(out), out.size, C.byref(n_out), _lib.ptr(id_offs), C.byref(stats))
-            detail = L.bpe_last_error_detail(ctx.handle)
-            if rc == _lib.ERR_UTF8 and texts is not None:
-                # the device reports invalid UTF-8 in a chunk before a KeyError in it: the documents before the invalid one
-                # go first, then that document fails as its decode does
-                k = int(np.searchsorted(offs, detail, side="right")) - 1
-                self._encode_batch_packed(blob[: int(offs[k])], offs[: k + 1], dtype, **({"drop": drop} if drop[0] else {}))
-                item = texts[k]
-                if isinstance(item, (bytes, bytearray, memoryview)):
-                    bytes(item).decode("utf-8")
-            if rc != _lib.BPE_OK:
-                self._raise(ctx, rc)
-        self.last_stats = stats.as_dict()
-        if unit is not None:
-            return out[: n_out.value], spans[: n_out.value], id_offs.astype(np.int64)
-        return out[: n_out.value], id_offs.astype(np.int64)
+    def _encode_batch(self, texts, dtype, drop, unit=None):
+        """(ids, spans or None, id offsets) of the documents `texts`, with the errors of encode_batch_to_numpy."""
+        texts = list(texts)
+        blob, offs, bad = _pack_documents(texts)
+        if bad is not None:                      # a str that cannot be encoded: the documents before it fail first, if any does
+            self._encode_ex(blob, dtype, docs=offs, drop=drop)
+            raise bad
+        return self._encode_ex(blob, dtype, docs=offs, texts=texts, drop=drop, unit=unit)
 
     def encode_sharded(self, data, dtype=np.uint16, group=None):
         """Multi-GPU encode (one process per GPU, torch.distributed initialised): every rank passes the same UTF-8 `data`
