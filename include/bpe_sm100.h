@@ -293,6 +293,13 @@ typedef struct bpe_encode_opts {
     int with_offsets;
     int offset_unit;
     int64_t *offs_out;
+    /* Device outputs (out_device != 0): `out` and `offs_out` are device pointers on the tokenizer's device. The ids (and spans) are
+     * written by the encoder's kernels straight into them, on the context's stream (bpe_ctx_set_stream). No host copy and no staging
+     * buffer is involved. id_offs_out stays a HOST array. Everything else is exactly as without the flag: the ids, spans, id offsets,
+     * two-call idiom, dtypes, errors (same order, same details) and bpe_tok_saw_cr. BPE_ERR_ARG, before anything is launched: `out`
+     * or `offs_out` not device memory of the tokenizer's device (cudaPointerGetAttributes), or offs_out not 16-byte aligned (the
+     * spans are written as 16-byte stores); these come after the checks of the other options. */
+    int out_device;
 } bpe_encode_opts;
 #define BPE_OFF_BYTES 0
 #define BPE_OFF_CHARS 1
@@ -331,6 +338,26 @@ int bpe_decode_batch(bpe_tok *tok, const int64_t *ids_host, uint64_t n, const ui
  * the array. */
 int bpe_batch_windows_dev(bpe_ctx *ctx, const void *tokens_dev, int dtype, uint64_t n_tokens, const int64_t *starts_host,
                           uint32_t batch, uint32_t context, int64_t *x_dev, int64_t *y_dev);
+
+/* Collates ragged documents (the ids of bpe_encode_ex with documents and out_device) into fixed rows, for a model's input:
+ * ids_dev holds n_ids int32 ids, row r's document is ids[id_offs[r] .. id_offs[r+1]) (id_offs_host: n_rows + 1 entries, on the
+ * host).  For row r, m = id_offs[r+1] - id_offs[r] and k = min(m, row_len):
+ *   kept tokens  ids[id_offs[r] .. +k)  (BPE_TRUNC_LEFT: the last k instead)
+ *   their place  columns [0, k)         (BPE_PAD_LEFT: [row_len - k, row_len))
+ *   ids_out[r][c] = the kept id, mask_out[r][c] = 1 and spans_out[r][c] = its span unchanged (still relative to the document, also
+ *   under left truncation); every other column gets pad_id, a mask of 0 and the span (0, 0) -- a real token's span is never empty,
+ *   so (0, 0) is unambiguous.
+ * ids_out_dev: [n_rows][row_len] int64; mask_out_dev: [n_rows][row_len] uint8, or NULL; spans_dev: [n_ids][2] int64 spans, or NULL;
+ * spans_out_dev: [n_rows][row_len][2] int64, NULL iff spans_dev is NULL.  All output pointers are device memory of ctx's device.
+ * BPE_ERR_ARG before anything is launched: a null context or a null required pointer, unknown flag bits, only one of the two span
+ * pointers, a pointer that is not device memory of ctx's device, a span pointer not 16-byte aligned, or id offsets that decrease or
+ * end past n_ids (detail = the row).  n_rows == 0 or row_len == 0 does nothing.  Stream-ordered on a caller's stream
+ * (bpe_ctx_set_stream); complete on return on the context's own stream. */
+#define BPE_PAD_LEFT   1   /* kept tokens at the END of the row, padding before them (default: kept tokens first) */
+#define BPE_TRUNC_LEFT 2   /* a document longer than the row keeps its LAST row_len tokens (default: its first) */
+int bpe_pad_rows_dev(bpe_ctx *ctx, const int32_t *ids_dev, uint64_t n_ids, const uint64_t *id_offs_host, uint64_t n_rows,
+                     const int64_t *spans_dev, uint32_t row_len, int64_t pad_id, int flags,
+                     int64_t *ids_out_dev, uint8_t *mask_out_dev, int64_t *spans_out_dev);
 
 /* ---- synthetic corpora (bench/test infrastructure; SURVEY 8d) -------------------------------- */
 #define BPE_SYNTH_TINYSTORIES 0

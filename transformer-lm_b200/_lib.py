@@ -19,6 +19,7 @@ BPE_OK = 0
 DTYPE_U16, DTYPE_I32 = 0, 1
 TRAIN_SPLIT_SPECIALS = 1
 OFF_BYTES, OFF_CHARS = 0, 1
+PAD_LEFT, TRUNC_LEFT = 1, 2
 SYNTH_TINYSTORIES, SYNTH_OWT = 0, 1
 
 
@@ -47,9 +48,10 @@ class EncodeStats(C.Structure):
 
 
 class EncodeOpts(C.Structure):
-    """bpe_encode_opts: documents, BPE-dropout and token offsets of bpe_encode_ex (all zero: bpe_encode)."""
+    """bpe_encode_opts: documents, BPE-dropout, token offsets and device outputs of bpe_encode_ex (all zero: bpe_encode)."""
     _fields_ = [("doc_offs", C.c_void_p), ("n_docs", C.c_uint64), ("id_offs_out", C.c_void_p), ("dropout", C.c_double),
-                ("seed", C.c_uint64), ("with_offsets", C.c_int), ("offset_unit", C.c_int), ("offs_out", C.c_void_p)]
+                ("seed", C.c_uint64), ("with_offsets", C.c_int), ("offset_unit", C.c_int), ("offs_out", C.c_void_p),
+                ("out_device", C.c_int)]
 
 
 _lib = None
@@ -64,7 +66,7 @@ EXPORTS = [
     "bpe_count_export_dev", "bpe_count_import", "bpe_count_import_dev", "bpe_count_pair_table",
     "bpe_train_from_counts", "bpe_last_pair_table", "bpe_train_set_live", "bpe_tok_create", "bpe_tok_destroy", "bpe_encode", "bpe_encode_ex",
     "bpe_encode_dev", "bpe_tok_key_error", "bpe_tok_saw_cr",
-    "bpe_tok_cache_reset", "bpe_decode", "bpe_decode_batch", "bpe_batch_windows_dev", "bpe_synth_dev", "bpe_synth_host", "bpe_synth_dev_at", "bpe_synth_host_at", "bpe_ctx_set_stream", "bpe_host_alloc", "bpe_host_free", "bpe_launch_count",
+    "bpe_tok_cache_reset", "bpe_decode", "bpe_decode_batch", "bpe_batch_windows_dev", "bpe_pad_rows_dev", "bpe_synth_dev", "bpe_synth_host", "bpe_synth_dev_at", "bpe_synth_host_at", "bpe_ctx_set_stream", "bpe_host_alloc", "bpe_host_free", "bpe_launch_count",
 ]
 
 
@@ -118,6 +120,7 @@ def lib():
             L.bpe_train_set_live.argtypes = [vp, vp, C.c_int]
             L.bpe_decode_batch.argtypes = [vp, vp, C.c_uint64, vp, C.c_uint64, vp, C.c_uint64, u64p, vp]
             L.bpe_batch_windows_dev.argtypes = [vp, vp, C.c_int, C.c_uint64, vp, C.c_uint32, C.c_uint32, vp, vp]
+            L.bpe_pad_rows_dev.argtypes = [vp, vp, C.c_uint64, vp, C.c_uint64, vp, C.c_uint32, C.c_int64, C.c_int, vp, vp, vp]
             L.bpe_synth_dev.argtypes = [vp, C.c_int, C.c_uint64, vp, C.c_uint64]
             L.bpe_synth_host.argtypes = [C.c_int, C.c_uint64, vp, C.c_uint64]
             L.bpe_synth_dev_at.argtypes = [vp, C.c_int, C.c_uint64, C.c_uint64, vp, C.c_uint64]

@@ -73,7 +73,7 @@ int bpe_buf_alloc(bpe_ctx *ctx, DevBuf &b, size_t bytes) {
     return pool_take(ctx, b, want);
 }
 
-BPE_API int bpe_version(void) { return 101; }
+BPE_API int bpe_version(void) { return 102; }   // 102: bpe_encode_opts.out_device, bpe_pad_rows_dev
 BPE_API const char *bpe_unicode_table_source(void) { return BPE_UNICODE_TABLE_SOURCE; }
 
 BPE_API int bpe_ctx_create(int device, bpe_ctx **out) {
@@ -147,6 +147,15 @@ BPE_API void *bpe_host_alloc(size_t bytes) {
     return p;
 }
 BPE_API void bpe_host_free(void *p) { if (p) cudaFreeHost(p); }
+
+int ctx_check_dev_ptr(bpe_ctx *ctx, const void *p, const char *what) {
+    cudaPointerAttributes a{};
+    if (!p || cudaPointerGetAttributes(&a, p) != cudaSuccess || a.type != cudaMemoryTypeDevice || a.device != ctx->device) {
+        cudaGetLastError();                      // (an unknown pointer is an argument error, not a sticky CUDA one)
+        return bpe_set_error(ctx, BPE_ERR_ARG, "%s is not device memory of device %d", what, ctx->device);
+    }
+    return BPE_OK;
+}
 
 // ---------------------------------------------------------------------------------------------
 // text arena

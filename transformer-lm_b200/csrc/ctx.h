@@ -10,6 +10,8 @@ int ctx_upload_specials(bpe_ctx *ctx, const uint8_t *blob, const u32 *offs, int 
 int ctx_run_flags(bpe_ctx *ctx, u64 *n_io, bool translate_newlines, const uint8_t *sp_blob_dev, const u32 *sp_offs_dev,
                   int n_sp, u32 sp_max_len, u64 err_lo = 0, u64 err_hi = ~0ull, const u32 *bmask = nullptr);
 void count_state_free(bpe_ctx *ctx);
+// BPE_ERR_ARG (message "<what> is not device memory of device N") unless p is device memory of ctx's device.
+int ctx_check_dev_ptr(bpe_ctx *ctx, const void *p, const char *what);
 // A position in [nominal, min(n, nominal + window)) where cutting the text changes nothing on either side: the start of a
 // special-token occurrence that no occurrence covers from the left (Tokenizer.segment splits there, tokenizer.py:63-66), or a
 // single U+0020 between two ASCII non-space bytes that no occurrence covers (SURVEY B.2).  0 = none.  Specials longest first.

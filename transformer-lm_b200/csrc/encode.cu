@@ -1669,9 +1669,10 @@ static std::vector<EncChunk> doc_chunks(const bpe_tok *tok, const uint8_t *t, u6
 //   batch encode: a chunk is uploaded as it is into one of two staging buffers; on the compute stream k_enc_expand_docs moves it
 //                 into the arena with a boundary byte after every document and sets the boundary bitmask
 // drop: BPE-dropout (thr and seed_mix set), or null.  offs_out (with out): the tokens' spans in `unit` (BPE_OFF_*), downloaded with the ids.
+// out_device: out and offs_out are device memory, and the kernels write each chunk's ids and spans at its running offset in them.
 static int encode_pipeline(bpe_tok *tok, const uint8_t *text_host, uint64_t n, const uint64_t *doc_offs, uint64_t n_docs, int out_dtype,
                            void *out, uint64_t cap, uint64_t *n_out, uint64_t *id_offs_out, bpe_encode_stats *stats,
-                           const EncDrop *drop = nullptr, int unit = BPE_OFF_BYTES, int64_t *offs_out = nullptr) {
+                           const EncDrop *drop = nullptr, int unit = BPE_OFF_BYTES, int64_t *offs_out = nullptr, bool out_device = false) {
     BPE_TRY(encode_check_args(tok, text_host, n, out_dtype, n_out));
     bpe_ctx *ctx = tok->ctx;
     cudaStream_t st = ctx->stream;
@@ -1727,7 +1728,12 @@ static int encode_pipeline(bpe_tok *tok, const uint8_t *text_host, uint64_t n, c
         if (swap) std::swap(ctx->text, ctx->text_alt);            // the arena the kernels read is always ctx->text
         CUDA_TRY(ctx, cudaStreamWaitEvent(st, ctx->ev_in[cur], 0));
         void *odev = nullptr;
-        if (out) {
+        u64 dev_cap = len;
+        const u64 w0 = std::min<u64>(total, cap);       // device outputs: where this chunk's ids start (nothing is written past cap)
+        if (out && out_device) {
+            odev = (uint8_t *)out + w0 * esz;
+            dev_cap = cap - w0;
+        } else if (out) {
             rc = bpe_buf_reserve(ctx, *obuf[cur], std::max<size_t>((m > 1 ? max_chunk : len) * esz, 16));
             if (rc != BPE_OK) { if (swap) std::swap(ctx->text, ctx->text_alt); break; }
             if (want_offs) rc = bpe_buf_reserve(ctx, tok->offs_out[cur], std::max<size_t>((m > 1 ? max_chunk : len) * 16, 16));
@@ -1739,7 +1745,7 @@ static int encode_pipeline(bpe_tok *tok, const uint8_t *text_host, uint64_t n, c
         EncOffs och{};
         const uint64_t *dofs = doc_offs ? doc_offs : one_doc;
         if (want_offs) {
-            och.chars = unit == BPE_OFF_CHARS; och.out = (long long *)tok->offs_out[cur].p; och.lo = ch.lo; och.da = ch.da; och.carry = char_carry;
+            och.chars = unit == BPE_OFF_CHARS; och.out = out_device ? (long long *)offs_out + 2 * w0 : (long long *)tok->offs_out[cur].p; och.lo = ch.lo; och.da = ch.da; och.carry = char_carry;
             och.doffs = doc_offs ? (const u64 *)ctx->doc_offs.p : nullptr;
         }
         EncOffs *op = want_offs ? &och : nullptr;
@@ -1760,7 +1766,7 @@ static int encode_pipeline(bpe_tok *tok, const uint8_t *text_host, uint64_t n, c
                     (uint8_t *)ctx->text.p + BPE_PAD, (u32 *)ctx->doc_bmask.p, (uint8_t)tok->doc_sep);
             CUDA_TRY(ctx, cudaGetLastError());
             const DocBounds db{(const u32 *)ctx->doc_bmask.p, id_dev + ch.da + 1, total};
-            rc = encode_core(tok, an, out_dtype, odev, len, &nt, stats, &db, dp, op, next_ds, next_keep);
+            rc = encode_core(tok, an, out_dtype, odev, dev_cap, &nt, stats, &db, dp, op, next_ds, next_keep);
             if (rc == BPE_ERR_UTF8 || rc == BPE_ERR_KEY) {      // arena offset -> offset in the caller's text: minus the boundaries before it
                 const u64 p = (u64)ctx->err_detail;
                 u64 a = 0, b = nb;                              // boundaries j < a lie before p (boundary j sits at ends[j] - lo + j)
@@ -1772,11 +1778,11 @@ static int encode_pipeline(bpe_tok *tok, const uint8_t *text_host, uint64_t n, c
             }
             if (rc != BPE_OK) break;
         } else {
-            rc = encode_core(tok, len, out_dtype, odev, len, &nt, stats, nullptr, dp, op, next_ds, next_keep);
+            rc = encode_core(tok, len, out_dtype, odev, dev_cap, &nt, stats, nullptr, dp, op, next_ds, next_keep);
             if (swap) std::swap(ctx->text, ctx->text_alt);
             if (rc != BPE_OK) { ctx->err_detail += (int64_t)ch.lo; break; }
         }
-        if (out && total < cap) {
+        if (out && !out_device && total < cap) {
             const u64 w = std::min<u64>(nt, cap - total);
             CUDA_TRY(ctx, cudaEventRecord(ctx->ev_done, st));
             CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->s_out, ctx->ev_done, 0));
@@ -1839,15 +1845,22 @@ BPE_API int bpe_encode_ex(bpe_tok *tok, const uint8_t *text_host, uint64_t n, co
             return bpe_set_error(ctx, BPE_ERR_ARG, "bpe_encode_ex: document offsets must run from 0 to n");
         if (n_docs && tok->doc_sep < 0)
             return bpe_set_error(ctx, BPE_ERR_UNSUPPORTED, "bpe_encode_ex: every ASCII byte but '\\r' occurs in a special token (no boundary byte)");
-        if (n_docs == 0) {
-            BPE_TRY(encode_check_args(tok, text_host, 0, out_dtype, n_out));
-            if (stats) memset(stats, 0, sizeof(*stats));
-            o.id_offs_out[0] = 0;
-            return BPE_OK;
+    }
+    if (o.out_device && out) {
+        BPE_TRY(ctx_check_dev_ptr(ctx, out, "bpe_encode_ex: out"));
+        if (o.with_offsets) {
+            BPE_TRY(ctx_check_dev_ptr(ctx, o.offs_out, "bpe_encode_ex: offs_out"));
+            if ((uintptr_t)o.offs_out % 16) return bpe_set_error(ctx, BPE_ERR_ARG, "bpe_encode_ex: offs_out must be 16-byte aligned");
         }
     }
+    if (o.doc_offs && o.n_docs == 0) {           // the empty batch
+        BPE_TRY(encode_check_args(tok, text_host, 0, out_dtype, n_out));
+        if (stats) memset(stats, 0, sizeof(*stats));
+        o.id_offs_out[0] = 0;
+        return BPE_OK;
+    }
     return encode_pipeline(tok, text_host, n, o.doc_offs, o.n_docs, out_dtype, out, cap, n_out, o.id_offs_out, stats, d.thr ? &d : nullptr,
-                           o.offset_unit, o.with_offsets ? o.offs_out : nullptr);
+                           o.offset_unit, o.with_offsets ? o.offs_out : nullptr, o.out_device != 0);
 }
 
 BPE_API int bpe_encode_dev(bpe_tok *tok, const uint8_t *text_dev, uint64_t n, int out_dtype, void *out_dev, uint64_t cap, uint64_t *n_out,

@@ -4,6 +4,7 @@
                                             .encode_batch(Sequence[str]) -> list[list[int]]
                                             .encode_iterable(Iterable[str]) -> Iterator[int]
                                             .encode_with_offsets(str) -> (list[int], list[(start, end)])
+                                            .encode_batch_padded(Sequence[str], pad_id=...) -> {"input_ids", "attention_mask"}
                                             .decode(list[int]) -> str
 
 encode / decode run on the GPU through the C ABI (bpe_tok_create / bpe_encode / bpe_decode in
@@ -12,6 +13,7 @@ tokenizer; nothing here re-implements the algorithm on the CPU (there is no fall
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
 import os
 import pickle
@@ -69,6 +71,28 @@ def _check_unit(unit) -> int:
     if not isinstance(unit, str) or unit not in _UNITS:
         raise ValueError("unit must be 'byte' or 'char', got %r" % (unit,))
     return _UNITS[unit]
+
+
+_SIDES = ("left", "right")
+
+
+@contextlib.contextmanager
+def _torch_stream(ctx):
+    """Under ctx.lock, run the library's work of the block on torch's current stream of the context's device, so that it orders with
+    torch's queued work (the outputs come from torch's caching allocator, which may hand out memory that queued work still uses);
+    yields that torch.device and restores the context's own stream afterwards.  On torch's legacy default stream (handle 0,
+    which bpe_ctx_set_stream reads as "the context's own stream", a non-blocking one) the stream is synchronised first; the
+    library's calls on its own stream are complete when they return."""
+    import torch
+    with ctx.lock:
+        stream = torch.cuda.current_stream(ctx.device)
+        if not stream.cuda_stream:
+            stream.synchronize()
+        ctx.use_stream(stream.cuda_stream)
+        try:
+            yield torch.device("cuda", ctx.device)
+        finally:
+            ctx.use_stream(None)
 
 
 class Tokenizer:
@@ -200,29 +224,42 @@ class Tokenizer:
         ctx.check(rc)
 
     # ---- encode (tokenizer.py:111-138) -------------------------------------------------------------
-    def _encode_ex(self, data, dtype, out=None, *, docs=None, texts=None, drop=(0.0, 0), unit=None):
+    def _encode_ex(self, data, dtype, out=None, *, docs=None, texts=None, drop=(0.0, 0), unit=None, device=None):
         """bpe_encode_ex of UTF-8 `data` into `out` (or a new array) of `dtype` (uint16 or int32): (ids, spans or None, id offsets or
         None).  docs: uint64 document offsets into `data` (a batch; `texts` are the items they came from, when known); drop: (p, seed)
-        of BPE-dropout; unit: _lib.OFF_* for the int64 spans [n, 2] of the tokens."""
+        of BPE-dropout; unit: _lib.OFF_* for the int64 spans [n, 2] of the tokens.  device: a torch.device (the context's, inside
+        _torch_stream) -- then the ids (int32) and spans are views of new tensors there of one id (and span) per byte, written by the
+        kernels (bpe_encode_opts.out_device)."""
         tok = self._device_tok()
         ctx = self._tok_ctx
         L = _lib.lib()
         arr = _lib.as_u8(data)
         code = {np.dtype(np.uint16): _lib.DTYPE_U16, np.dtype(np.int32): _lib.DTYPE_I32}[np.dtype(dtype)]
-        if out is None:
-            out = np.empty(max(arr.size, 1), dtype=dtype)         # a token covers at least one byte
         opts = _lib.EncodeOpts(dropout=drop[0], seed=drop[1])
+        if device is not None:
+            import torch
+            out = torch.empty(max(arr.size, 1), dtype=torch.int32, device=device)
+            out_ptr, cap, opts.out_device = C.c_void_p(out.data_ptr()), out.numel(), 1
+        else:
+            if out is None:
+                out = np.empty(max(arr.size, 1), dtype=dtype)     # a token covers at least one byte
+            out_ptr, cap = _lib.ptr(out), out.size
         spans = id_offs = None
         if docs is not None:
             id_offs = np.zeros(docs.size, dtype=np.uint64)
             opts.doc_offs, opts.n_docs, opts.id_offs_out = docs.ctypes.data, docs.size - 1, id_offs.ctypes.data
         if unit is not None:
-            spans = np.empty((out.size, 2), dtype=np.int64)
-            opts.with_offsets, opts.offset_unit, opts.offs_out = 1, unit, spans.ctypes.data
+            if device is not None:
+                spans = torch.empty((cap, 2), dtype=torch.int64, device=device)
+                opts.offs_out = spans.data_ptr()
+            else:
+                spans = np.empty((cap, 2), dtype=np.int64)
+                opts.offs_out = spans.ctypes.data
+            opts.with_offsets, opts.offset_unit = 1, unit
         n_out = C.c_uint64(0)
         stats = _lib.EncodeStats()
         with ctx.lock:
-            rc = L.bpe_encode_ex(tok, _lib.ptr(arr) if arr.size else None, arr.size, C.byref(opts), code, _lib.ptr(out), out.size,
+            rc = L.bpe_encode_ex(tok, _lib.ptr(arr) if arr.size else None, arr.size, C.byref(opts), code, out_ptr, cap,
                                  C.byref(n_out), C.byref(stats))
             if rc == _lib.ERR_UTF8 and texts is not None:
                 # the device reports invalid UTF-8 in a chunk before a KeyError in it: the documents before the invalid one
@@ -301,14 +338,103 @@ class Tokenizer:
         flat, sp, o = ids.tolist(), list(map(tuple, spans.tolist())), o.tolist()
         return [(flat[o[j]: o[j + 1]], sp[o[j]: o[j + 1]]) for j in range(len(o) - 1)]
 
-    def _encode_batch(self, texts, dtype, drop, unit=None):
-        """(ids, spans or None, id offsets) of the documents `texts`, with the errors of encode_batch_to_numpy."""
+    def _encode_batch(self, texts, dtype, drop, unit=None, device=None):
+        """(ids, spans or None, id offsets) of the documents `texts`, with the errors of encode_batch_to_numpy (device: _encode_ex)."""
         texts = list(texts)
         blob, offs, bad = _pack_documents(texts)
         if bad is not None:                      # a str that cannot be encoded: the documents before it fail first, if any does
             self._encode_ex(blob, dtype, docs=offs, drop=drop)
             raise bad
-        return self._encode_ex(blob, dtype, docs=offs, texts=texts, drop=drop, unit=unit)
+        dev = {} if device is None else {"device": device}     # (host outputs: the call of encode_batch_to_numpy, unchanged)
+        return self._encode_ex(blob, dtype, docs=offs, texts=texts, drop=drop, unit=unit, **dev)
+
+    # ---- encode into CUDA tensors: outputs written on the device, for a model on the same GPU ----------------------------------
+    # Each call runs on torch's current stream of the tokenizer's device (its outputs are ready for torch work queued after the
+    # call).  Scratch: one int32 id per input byte (+ one 16-byte span per byte with offsets) from torch's allocator, released
+    # before the call returns; the results are compact copies.
+
+    def encode_to_tensor(self, data, *, dropout: float = 0.0, seed: int = 0, offsets: str | None = None):
+        """encode_to_numpy(data, np.int32) as a 1-D int32 CUDA tensor on the tokenizer's device; with offsets="byte" or "char" also the
+        int64 spans [n, 2] of encode_offsets_to_numpy: (ids, spans).  The ids (and spans) never leave the device.  Peak scratch
+        memory: 4 bytes (+ 16 with offsets) per byte of `data`, freed before return."""
+        drop = _check_dropout(dropout, seed)
+        unit = None if offsets is None else _check_unit(offsets)
+        self._device_tok()
+        with _torch_stream(self._tok_ctx) as dev:
+            ids, spans, _ = self._encode_ex(data, np.int32, drop=drop, unit=unit, device=dev)
+            ids = ids.clone()
+            return ids if unit is None else (ids, spans.clone())
+
+    def encode_batch_to_tensor(self, texts: Sequence[str | bytes], *, dropout: float = 0.0, seed: int = 0, offsets: str | None = None):
+        """encode_batch_to_numpy(texts, np.int32) on the device: (ids int32 [n], id_offsets int64 [len(texts) + 1]) as CUDA tensors on
+        the tokenizer's device -- the ragged form that torch.nested.nested_tensor_from_jagged and variable-length attention take --
+        and with offsets="byte" or "char" (ids, id_offsets, spans int64 [n, 2]) as encode_batch_offsets_to_numpy gives them.  The
+        same errors as encode_batch_to_numpy (the first failing document in list order raises).  Peak scratch memory: 4 bytes
+        (+ 16 with offsets) per byte of UTF-8 text, freed before return."""
+        drop = _check_dropout(dropout, seed)
+        unit = None if offsets is None else _check_unit(offsets)
+        self._device_tok()
+        with _torch_stream(self._tok_ctx) as dev:
+            import torch
+            ids, spans, offs = self._encode_batch(texts, np.int32, drop, unit, device=dev)
+            out = (ids.clone(), torch.from_numpy(offs).to(dev))
+            return out if unit is None else out + (spans.clone(),)
+
+    def encode_batch_padded(self, texts: Sequence[str | bytes], *, pad_id: int, max_length: int | None = None, pad_to: str = "longest",
+                            padding_side: str = "right", truncation_side: str = "right", offsets: str | None = None,
+                            dropout: float = 0.0, seed: int = 0) -> dict:
+        """The documents `texts` as fixed-length rows on the tokenizer's device: {"input_ids": int64 [B, L], "attention_mask": bool
+        [B, L]}, and "offsets": int64 [B, L, 2] (encode_batch_offsets_to_numpy's spans in `offsets` = "byte" / "char") when asked.
+        L = max_length with pad_to="max_length" (fixed shapes, e.g. for CUDA graphs); with pad_to="longest" the longest document's
+        token count, at most max_length.  A document longer than L keeps its first L tokens (truncation_side="left": its last L); its
+        kept tokens fill the start of the row (padding_side="left": the end), and the other positions hold pad_id (any int64: no
+        default), a mask of False and the span (0, 0).  Spans stay relative to the document, also under left truncation.  Dropout and
+        errors are those of encode_batch_to_numpy; argument errors raise ValueError / TypeError before any device work.  Encode and
+        collation (bpe_pad_rows_dev) run on the device.  Peak scratch memory: 4 bytes (+ 16 with offsets) per byte of UTF-8 text,
+        freed before return; only the [B, L] outputs are kept."""
+        if isinstance(pad_id, bool) or not isinstance(pad_id, (int, np.integer)):
+            raise TypeError("pad_id must be an integer, got %r" % (pad_id,))
+        if not -2**63 <= int(pad_id) < 2**63:
+            raise ValueError("pad_id must fit int64, got %r" % (pad_id,))
+        if max_length is not None:
+            if isinstance(max_length, bool) or not isinstance(max_length, (int, np.integer)):
+                raise TypeError("max_length must be an integer or None, got %r" % (max_length,))
+            if not 1 <= int(max_length) < 2**32:
+                raise ValueError("max_length must be in [1, 2**32), got %r" % (max_length,))
+        if pad_to not in ("longest", "max_length"):
+            raise ValueError("pad_to must be 'longest' or 'max_length', got %r" % (pad_to,))
+        if pad_to == "max_length" and max_length is None:
+            raise ValueError("pad_to='max_length' needs max_length")
+        if padding_side not in _SIDES or truncation_side not in _SIDES:
+            raise ValueError("padding_side and truncation_side must be 'left' or 'right', got %r, %r" % (padding_side, truncation_side))
+        drop = _check_dropout(dropout, seed)
+        unit = None if offsets is None else _check_unit(offsets)
+        flags = (_lib.PAD_LEFT if padding_side == "left" else 0) | (_lib.TRUNC_LEFT if truncation_side == "left" else 0)
+        self._device_tok()
+        ctx = self._tok_ctx
+        with _torch_stream(ctx) as dev:
+            import torch
+            ids, spans, offs = self._encode_batch(texts, np.int32, drop, unit, device=dev)
+            n_rows = offs.size - 1
+            if pad_to == "max_length":
+                row_len = int(max_length)
+            else:
+                row_len = int(np.diff(offs).max(initial=0))
+                if max_length is not None:
+                    row_len = min(row_len, int(max_length))
+            res = {"input_ids": torch.empty((n_rows, row_len), dtype=torch.int64, device=dev),
+                   "attention_mask": torch.empty((n_rows, row_len), dtype=torch.bool, device=dev)}
+            if unit is not None:
+                res["offsets"] = torch.empty((n_rows, row_len, 2), dtype=torch.int64, device=dev)
+            if n_rows and row_len:
+                id_offs = np.ascontiguousarray(offs, dtype=np.uint64)
+                # (ids and spans are prefixes of the scratch tensors; their storage pointers stay non-null when the prefix is empty)
+                ctx.check(_lib.lib().bpe_pad_rows_dev(
+                    ctx.handle, C.c_void_p(ids.untyped_storage().data_ptr()), ids.numel(), _lib.ptr(id_offs), n_rows,
+                    None if spans is None else C.c_void_p(spans.untyped_storage().data_ptr()), row_len, int(pad_id), flags,
+                    C.c_void_p(res["input_ids"].data_ptr()), C.c_void_p(res["attention_mask"].data_ptr()),
+                    None if spans is None else C.c_void_p(res["offsets"].data_ptr())))
+            return res
 
     def encode_sharded(self, data, dtype=np.uint16, group=None):
         """Multi-GPU encode (one process per GPU, torch.distributed initialised): every rank passes the same UTF-8 `data`
